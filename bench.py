@@ -26,6 +26,9 @@ the strong-scaling efficiency, the per-layer exchange times and an in-run parity
 
 `--impl reference` times the CPU restatement of the reference (oracle/, torch CPU ops in the
 reference's op order, all host threads) on the same workload and prints the same line shape.
+
+`--dump-outputs DIR` writes what the last timed (resident) step computed as .npy files, so that two builds run with the
+same arguments, hence on the same seeded inputs, can be compared output for output.
 """
 from __future__ import annotations
 
@@ -353,11 +356,16 @@ class StepBench:
                              edge_index=graph if prebuilt else t["edge_index"], data_batch=t["batch"],
                              loc_mean=t["loc_mean"], edge_attr=None if prebuilt else t["edge_attr"])
                 # utils/train.py:104-163: MSE + weight * MMD -- one launch per direction (mse_mmd_loss), not ten torch kernels
-                loss, _mse = mse_mmd_loss(x, t["loc_t"], Z, idx, hp["sigma"], hp["weight"])
+                loss, mse = mse_mmd_loss(x, t["loc_t"], Z, idx, hp["sigma"], hp["weight"])
                 loss.backward()
                 if world > 1:
                     allreduce_grads()
             opt.step()
+            # what the step hands its caller (--dump-outputs): detached views, so no autograd state outlives the step;
+            # a captured graph's replays rewrite these same tensors
+            self.outputs = dict(node_loc=x.detach(), virtual_node_loc=Z.detach(), loss=loss.detach())
+            if not part:
+                self.outputs["mse"] = mse.detach()
             return loss
         self.train_step = train_step
         # ---- the whole step (graph prep, 4-layer fwd, losses, bwd, collectives, Adam) as ONE CUDA graph:
@@ -431,6 +439,30 @@ def timed(fn, steps, flush):
     return sum(s.elapsed_time(e) for s, e in evs) / steps     # ms
 
 
+DUMP_ARRAY_BYTES = 16_000_000        # per array; at most four arrays can reach it, so a dump stays under 64 MB
+
+
+def dump_outputs(sb, out_dir):
+    """Write what the last step of `sb` handed its caller to out_dir/<name>.npy (float32): node_loc [N,3],
+    virtual_node_loc [B,3,C], loss (and mse) [1], the parameters after the optimizer step and the gradients it applied
+    (params / grads: flat, in model.parameters() order, zeros where a parameter got no gradient).  An array above
+    DUMP_ARRAY_BYTES keeps a fixed sample of its rows: sorted row ids drawn with numpy seed 0 from the row count alone, the
+    same in every run of the same arguments."""
+    params = list(sb.model.parameters())
+    arrays = dict(sb.outputs)
+    arrays["params"] = torch.cat([p.detach().reshape(-1) for p in params])
+    arrays["grads"] = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).detach().reshape(-1)
+                                 for p in params])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.float().cpu().numpy().reshape(t.shape if t.dim() else (1,))
+        row_bytes = a[:1].nbytes
+        if a.nbytes > DUMP_ARRAY_BYTES:
+            k = DUMP_ARRAY_BYTES // row_bytes
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], k, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
+
+
 def quick_config(name, dev, flush, steps=5, warmup=3):
     """One line of the per-config table (BASELINE.json configs 1-5 on ONE GPU): ms per training step, resident."""
     if name == "large":
@@ -479,7 +511,14 @@ def main():
                     help="N > 1, default workload: skip the partitioned config-5 block (1 M nodes in N slabs)")
     ap.add_argument("--part-nodes", type=int, default=1_000_000, help="nodes of the partitioned block's graph")
     ap.add_argument("--rollout", action="store_true", help="also time the forward-only rollout mode (utils/train.py:191)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs; "
+                         "with several ranks, rank 0's share)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm's step")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -517,9 +556,7 @@ def main():
             return
         torch.set_num_threads(cores)
         step = oracle_step_fn(data, hp, model=args.model)
-        # a CPU step of the headline workload takes ~0.45 s: --steps / --warmup are honoured as given (bounded only so
-        # that a huge request still ends within minutes)
-        w, k = max(1, min(args.warmup, 50)), max(1, min(args.steps, 200))
+        w, k = args.warmup, args.steps
         t = time_cpu(step, w, k)
         val = E * LAYERS / t
         line = dict(impl="reference", metric=metric, value=val, unit="edges/s", n_gpus=args.gpus,
@@ -582,6 +619,8 @@ def main():
     ms = timed(sb.resident, args.steps, flush)
     barrier()
     launches = sb.launches(args.steps, _lib.lib.fegnn_launch_count() - launches0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(sb, args.dump_outputs)
     ms_e2e_serial = timed(sb.e2e, args.steps, flush)
     barrier()
     pipelined = not part and not args.no_graph
