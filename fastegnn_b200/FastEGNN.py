@@ -134,6 +134,7 @@ class _StackFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gx, gZ):
         mod, graph, dims = ctx.mod, ctx.graph, ctx.dims
+        L.deterministic(type(mod).__name__ + " backward", L.NO_DET_LAYERS)
         node_feat, v = ctx.saved_tensors
         dev = v.device
         N, B, Cc, Lyr = graph.N, graph.B, mod.virtual_channels, mod.n_layers
@@ -266,6 +267,7 @@ class FastEGNN(nn.Module):
 
     # -- forward --------------------------------------------------------------------------
     def forward(self, node_feat, node_loc, node_vel, edge_index, data_batch, loc_mean, edge_attr=None, node_attr=None):
+        L.deterministic(type(self).__name__, L.NO_DET_LAYERS)
         _require_cuda(node_loc, "node_loc")
         if isinstance(edge_index, CsrGraph):
             # a graph already in kernel layout (CsrGraph.from_radius, or a CsrGraph reused across steps of a static

@@ -127,6 +127,7 @@ class VNEGNN(nn.Module):
         self.to(self.device)
 
     def forward(self, node_feat, node_loc, edge_index, data_batch, virtual_node_loc, edge_attr=None, node_attr=None):
+        L.deterministic("VNEGNN", L.NO_DET_LAYERS)
         _require_cuda(node_loc, "node_loc")
         dev = node_loc.device
         C, Fe = self.virtual_channels, self._edge_attr_nf

@@ -8,6 +8,9 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import warnings
+
+import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("FEGNN_LIB") or os.path.join(HERE, "_C", "libfegnn.so")     # FEGNN_LIB: an instrumented build (tools/)
@@ -146,9 +149,10 @@ SIGNATURES = {
     "fegnn_segment_reduce": (C.c_int, [C.c_int64, i32, i32, vp, vp, i32, vp, vp, vp]),
     "fegnn_segment_reduce_backward": (C.c_int, [C.c_int64, i32, i32, vp, vp, vp, vp, vp]),
     "fegnn_adam_step": (C.c_int, [C.c_int64, vp, vp, vp, vp, vp, vp, C.c_float, C.c_double, C.c_double, C.c_float, C.c_float, vp]),
-    "fegnn_mmd_forward": (C.c_int, [i32, i32, i32, C.c_float, C.c_float, C.c_float, vp, vp, vp, vp, vp]),
+    "fegnn_loss_workspace_floats": (C.c_size_t, [i32, i32]),
+    "fegnn_mmd_forward": (C.c_int, [i32, i32, i32, C.c_float, C.c_float, C.c_float, vp, vp, vp, vp, vp, C.c_size_t, vp]),
     "fegnn_mmd_backward": (C.c_int, [i32, i32, i32, i32, C.c_float, C.c_float, C.c_float, vp, vp, vp, vp, vp, vp, vp]),
-    "fegnn_mse_mmd_forward": (C.c_int, [i32, i32, i32, i32] + [C.c_float] * 5 + [vp] * 7),
+    "fegnn_mse_mmd_forward": (C.c_int, [i32, i32, i32, i32] + [C.c_float] * 5 + [vp] * 7 + [C.c_size_t, vp]),
     "fegnn_mse_mmd_backward": (C.c_int, [i32, i32, i32, i32] + [C.c_float] * 5 + [vp] * 9),
 }
 
@@ -180,6 +184,29 @@ def set_precision(name: str) -> None:
 
 def get_mode(phase: str) -> int:
     return int(lib.fegnn_get_mode(phase.encode()))
+
+
+# Why the layer stack has no deterministic form (DESIGN.md section 9): FastEGNN, FastRF, VNEGNN, E_GCL_vel, the partitioned
+# runner and the segment helpers all reach kernels that add floats across CTAs in arrival order.
+NO_DET_LAYERS = "its edge, virtual and node kernels add sums across CTAs with float atomics"
+
+
+def deterministic(what: str, missing: str = None) -> bool:
+    """Sets the library's "deterministic" mode from torch.are_deterministic_algorithms_enabled() for one call of `what`
+    and returns the mode the call runs in.  `missing` says why `what` has no deterministic form (None: it has one).  Such
+    a call raises under the flag, as torch's own ops do, or warns and runs as without the flag under warn_only=True."""
+    on = torch.are_deterministic_algorithms_enabled()
+    if on and missing is not None:
+        msg = (f"{what} does not have a deterministic implementation ({missing}), but you set "
+               "'torch.use_deterministic_algorithms(True)'.  Use torch.use_deterministic_algorithms(True, warn_only=True) "
+               "to run it anyway.")
+        if not torch.is_deterministic_algorithms_warn_only_enabled():
+            raise RuntimeError(msg)
+        warnings.warn(msg, stacklevel=3)
+        on = False
+    if get_mode("deterministic") != int(on):
+        set_mode("deterministic", int(on))
+    return on
 
 
 def check(rc: int, what: str = "") -> None:

@@ -49,6 +49,11 @@ int fail(int code, const char* fmt, ...) {
   do {                                                                        \
     if (!(cond)) return fail(FEGNN_EINVAL, "%s: requirement failed: %s", __func__, #cond); \
   } while (0)
+#define NO_DET(why)                                                                                                \
+  do {                                                                                                             \
+    if (g_det) return fail(FEGNN_EINVAL, "%s has no deterministic form (%s); set mode \"deterministic\" to 0 to run it", \
+                           __func__, why);                                                                         \
+  } while (0)
 #define TRY(expr)            \
   do {                       \
     int rc__ = (expr);       \
@@ -81,6 +86,9 @@ const bool g_node_pre_tc3 = getenv("FEGNN_NODE_PRE_TC3") == nullptr || atoi(gete
 // walks the weight blocks, at every size (measured at 8 000 nodes: step 1.380 ms against 1.416 ms with the fp32 kernels; at
 // 160 000 nodes 11.95 ms against 12.89 ms with the (tile, block) kernel, which stays selectable by environment).
 int g_node_bwd_mode = 2;
+// "deterministic" (fegnn_set_mode): 1 = bit-reproducible forms of the entries that have one; every entry that sums floats
+// across CTAs in arrival order and has no such form refuses to run (NO_DET) instead of running nondeterministically
+int g_det = 0;
 constexpr int kNodeTcMinN = 0;
 inline bool node_bwd_tc(int N) { return g_node_bwd_mode == 1 || (g_node_bwd_mode == 2 && N >= kNodeTcMinN); }
 
@@ -92,6 +100,14 @@ int sm_count() {
     if (cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms[dev] <= 0) sms[dev] = 148;
   }
   return sms[dev];
+}
+
+// the deterministic loss forward keeps per-CTA partials in the caller's workspace (fegnn_loss_workspace_floats)
+int check_loss_ws(int N, int B, const float* ws, size_t floats) {
+  if (!g_det) return 0;
+  const size_t need = loss_det_ws_floats(N, B);
+  if (ws == nullptr || floats < need) return fail(FEGNN_ENOMEM, "loss workspace %zu < %zu floats", ws ? floats : 0, need);
+  return 0;
 }
 
 int check_dims(const fegnn_dims* d) {
@@ -243,7 +259,7 @@ SideStream* side_stream() {
 extern "C" {
 
 const char* fegnn_last_error(void) { return g_err; }
-int fegnn_version(void) { return 101; }      // 101: fegnn_layer_saved.wimg, fegnn_node_h_weight_images, FEGNN_F_WIMG_READY
+int fegnn_version(void) { return 102; }      // 102: "deterministic" mode, workspace of fegnn_mmd_forward / fegnn_mse_mmd_forward
 unsigned long long fegnn_launch_count(void) { return g_launches; }
 int fegnn_set_mode(const char* phase, int mode) {
   if (phase == nullptr) return fail(FEGNN_EINVAL, "phase is null");
@@ -270,6 +286,11 @@ int fegnn_set_mode(const char* phase, int mode) {
     (phase[8] == 'f' ? g_virt_fwd_mode : g_virt_bwd_mode) = mode;
     return 0;
   }
+  if (strcmp(phase, "deterministic") == 0) {
+    if (mode != 0 && mode != 1) return fail(FEGNN_EINVAL, "deterministic mode must be 0 or 1");
+    g_det = mode;
+    return 0;
+  }
   return fail(FEGNN_EINVAL, "unknown phase '%s'", phase);
 }
 int fegnn_get_mode(const char* phase) {
@@ -279,6 +300,7 @@ int fegnn_get_mode(const char* phase) {
   if (phase != nullptr && strcmp(phase, "node_backward") == 0) return g_node_bwd_mode;
   if (phase != nullptr && strcmp(phase, "virtual_forward") == 0) return g_virt_fwd_mode;
   if (phase != nullptr && strcmp(phase, "virtual_backward") == 0) return g_virt_bwd_mode;
+  if (phase != nullptr && strcmp(phase, "deterministic") == 0) return g_det;
   return -1;
 }
 
@@ -347,11 +369,13 @@ int fegnn_embed_forward(int32_t N, int32_t Fin, const float* node_feat, const fl
 }
 int fegnn_embed_backward(int32_t N, int32_t Fin, const float* node_feat, const float* w, const float* gh, float* gw,
                          float* gb, float* gnode_feat, void* stream) {
+  NO_DET("weight gradient flushed by many CTAs with float atomics");
   RQ(N >= 0 && Fin >= 1 && Fin <= 16 && (N == 0 || (node_feat && w && gh && gw && gb)));
   CK(launch_embed_bwd(N, Fin, node_feat, w, gh, gw, gb, gnode_feat, S(stream)));
   return 0;
 }
 int fegnn_graph_xsum(int32_t N, int32_t B, const float* x, const int32_t* batch, float* xsum, void* stream) {
+  NO_DET("per-graph sums across CTAs with float atomics");
   RQ(N >= 0 && B >= 0 && (B == 0 || xsum) && (N == 0 || (x && batch)));
   CK(cudaMemsetAsync(xsum, 0, sizeof(float) * 3 * (size_t)B, S(stream)));
   CK(launch_graph_xsum(N, x, batch, xsum, S(stream)));
@@ -361,6 +385,7 @@ int fegnn_graph_xsum(int32_t N, int32_t B, const float* x, const int32_t* batch,
 // ------------------------------------------------------------------ forward phases
 int fegnn_graph_pre_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* Z,
                             const float* Sf, const float* xsum, fegnn_layer_saved* sv, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(g && p && Z && Sf && xsum && sv);
   GraphArgs a = graph_args(d, g, p);
@@ -371,6 +396,7 @@ int fegnn_graph_pre_forward(const fegnn_dims* d, const fegnn_graph* g, const feg
 
 int fegnn_node_pre_forward(const fegnn_dims* d, const fegnn_layer_params* p, const float* h, fegnn_layer_saved* sv,
                            void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   RQ(h && sv);
@@ -384,6 +410,7 @@ int fegnn_node_pre_forward(const fegnn_dims* d, const fegnn_layer_params* p, con
 
 int fegnn_edge_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
                        fegnn_layer_saved* sv, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   RQ(g && x && sv);
@@ -400,6 +427,7 @@ int fegnn_edge_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_la
 int fegnn_virtual_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
                           const float* v, const float* Z, fegnn_layer_saved* sv, float* x_new, float* xsum_new,
                           void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   RQ(g && x && v && Z && sv && x_new && xsum_new);
@@ -416,6 +444,7 @@ int fegnn_virtual_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn
 
 int fegnn_node_h_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* h,
                          fegnn_layer_saved* sv, float* h_new, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(g && p && h && sv && h_new);
   NodeHArgs a;
@@ -453,6 +482,7 @@ int fegnn_node_h_weight_images(const fegnn_dims* d, int32_t nl, const fegnn_laye
 
 int fegnn_graph_post_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* Z,
                              const float* Sf, const fegnn_layer_saved* sv, float* Z_new, float* S_new, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(g && p && Z && Sf && sv && Z_new && ((d->flags & FEGNN_F_LAST) || S_new));
   GraphArgs a = graph_args(d, g, p);
@@ -466,6 +496,7 @@ int fegnn_graph_post_backward(const fegnn_dims* d, const fegnn_graph* g, const f
                               fegnn_layer_grads* gr, const float* Sf, const fegnn_layer_saved* sv,
                               const float* gZ_new, const float* gS_new, float* gZ, float* gS, float* gDsum,
                               float* gUsum, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   const bool last = d->flags & FEGNN_F_LAST;
   RQ(g && p && gr && sv && gZ_new && gZ && gS && gDsum && gUsum && (last || (Sf && gS_new)));
@@ -480,6 +511,7 @@ int fegnn_graph_post_backward(const fegnn_dims* d, const fegnn_graph* g, const f
 int fegnn_node_h_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
                           fegnn_layer_grads* gr, const fegnn_layer_saved* sv, const float* gh_new, float* gzh1,
                           float* gm, float* gu, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(g && p && gr && sv && gh_new && gzh1 && gm && gu);
   NodeHArgs a;
@@ -528,6 +560,7 @@ int fegnn_virtual_backward(const fegnn_dims* d, const fegnn_graph* g, const fegn
                            const fegnn_layer_saved* sv, const float* gx_new, const float* gxsum_next,
                            const float* gDsum, const float* gUsum, const float* gu, float* gAv, float* gG1, float* gx,
                            float* gZ, float* gsv, float* gsg, float* gt, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   RQ(g && gr && x && v && Z && sv && gx_new && gDsum && gAv && gG1 && gx && gZ && gsv && gt);
@@ -556,6 +589,7 @@ int fegnn_virtual_backward(const fegnn_dims* d, const fegnn_graph* g, const fegn
 int fegnn_edge_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, fegnn_layer_grads* gr,
                         const float* x, const fegnn_layer_saved* sv, const float* gm, const float* gt, float* gP,
                         float* gQ, float* gx, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   RQ(g && gr && x && sv && gt && gP && gQ && gx);
@@ -584,6 +618,7 @@ int fegnn_edge_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_l
 int fegnn_graph_pre_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
                              fegnn_layer_grads* gr, const float* Sf, const fegnn_layer_saved* sv, const float* gG1,
                              float* gS, float* gZ, float* gxsum, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(g && p && gr && Sf && sv && gG1 && gS && gZ && gxsum);
   GraphArgs a = graph_args(d, g, p);
@@ -596,6 +631,7 @@ int fegnn_graph_pre_backward(const fegnn_dims* d, const fegnn_graph* g, const fe
 int fegnn_node_pre_backward(const fegnn_dims* d, const fegnn_layer_params* p, fegnn_layer_grads* gr, const float* h,
                             const float* gP, const float* gQ, const float* gAv, const float* gUh, const float* gsv,
                             const float* gsg, float* gh, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   RQ(gr && h && gP && gQ && gAv && gsv && gh);
@@ -647,6 +683,7 @@ int fegnn_halo_push(int32_t n, const int32_t* src_row, const uint64_t* dst_q, co
 }
 int fegnn_halo_reduce_push(int32_t n, int32_t first_halo_row, const uint64_t* dst_q, const uint64_t* dst_x, const float* gQ,
                            const float* gx, void* stream) {
+  NO_DET("remote float atomics");
   RQ(n >= 0 && first_halo_row >= 0 && (n == 0 || (dst_q && dst_x && gQ && gx)));
   CK(launch_halo_reduce_push(n, first_halo_row, reinterpret_cast<const unsigned long long*>(dst_q),
                              reinterpret_cast<const unsigned long long*>(dst_x), gQ, gx, S(stream)));
@@ -688,6 +725,7 @@ int fegnn_halo_reduce_apply(int32_t n_rows, const int32_t* rows, const int32_t* 
 }
 int fegnn_p2p_allreduce(const fegnn_p2p* p, int32_t channel, int32_t nseg, float* const* seg_host, const int32_t* count_host,
                         void* stream) {
+  NO_DET("multi-GPU reductions are not covered");
   P2PArgs a;
   TRY(p2p_args(p, &a));
   RQ(channel >= 0 && channel < kP2PChannels && nseg >= 1 && nseg <= 4 && seg_host && count_host);
@@ -714,6 +752,7 @@ int fegnn_rf_vel_forward(int32_t N, const float* v, const fegnn_layer_params* p,
 }
 int fegnn_rf_vel_backward(int32_t N, const float* v, const fegnn_layer_params* p, fegnn_layer_grads* gr, const float* gsv,
                           void* stream) {
+  NO_DET("weight gradient flushed by many CTAs with float atomics");
   RQ(N >= 0 && p && gr && (N == 0 || (v && gsv)) && p->vel_w0 && p->vel_b0 && p->vel_w2);
   CK(launch_rf_vel_bwd(N, v, p->vel_w0, p->vel_b0, p->vel_w2, gsv, gr->vel_w0, gr->vel_b0, gr->vel_w2, gr->vel_b2,
                        sm_count(), S(stream)));
@@ -819,6 +858,7 @@ int fegnn_model_forward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn
                         const float* vnf, const float* node_feat, const float* x0, const float* v,
                         const float* loc_mean, float* x_out, float* Z_out, float* workspace, size_t workspace_floats,
                         void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(L >= 1 && L <= 32 && g && layers && embed_w && embed_b && vnf && workspace && x_out && Z_out);
   RQ(d->Nl == d->N);   // the partitioned path drives the phases itself (halo rows come from peers)
@@ -917,6 +957,7 @@ int fegnn_model_forward_inference(const fegnn_dims* d, int32_t L, int32_t Fin, c
                                   const float* vnf, const float* node_feat, const float* x0, const float* v,
                                   const float* loc_mean, float* x_out, float* Z_out, float* workspace,
                                   size_t workspace_floats, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(L >= 1 && L <= 32 && g && layers && embed_w && embed_b && vnf && workspace && x_out && Z_out);
   RQ(d->Nl == d->N);
@@ -1034,6 +1075,7 @@ int fegnn_model_backward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegn
                          const float* gx_out, const float* gZ_out, float* g_x0, float* g_loc_mean,
                          float* g_node_feat, const float* workspace, float* scratch, size_t scratch_floats,
                          void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(L >= 1 && L <= 32 && g && layers && grads && embed_w && g_embed_w && g_embed_b && g_vnf && workspace && scratch);
   RQ(gx_out && gZ_out && g_x0 && g_loc_mean && d->Nl == d->N);
@@ -1124,6 +1166,7 @@ int fegnn_peak_probe(int32_t kind, int32_t iters, float* sink, double* ops_host,
 // ------------------------------------------------------------------ unsorted_segment_sum / _mean (models/FastEGNN.py:279-294)
 int fegnn_segment_reduce(int64_t E, int32_t K, int32_t S_, const float* data, const int64_t* segment_ids, int32_t mean,
                          float* out, float* count, void* stream) {
+  NO_DET("scatter by segment id with float atomics");
   RQ(E >= 0 && K >= 1 && S_ >= 0 && (S_ == 0 || out) && (E == 0 || (data && segment_ids)) && (!mean || S_ == 0 || count));
   CK(launch_segment_reduce(E, K, S_, data, reinterpret_cast<const long long*>(segment_ids), mean != 0, out, count,
                            sm_count(), S(stream)));
@@ -1149,11 +1192,16 @@ int fegnn_adam_step(int64_t n, float* p, const float* g, float* m, float* v, con
 }
 
 // ------------------------------------------------------------------ MMD
+size_t fegnn_loss_workspace_floats(int32_t N, int32_t B) {
+  return g_det && N >= 0 && B >= 0 ? loss_det_ws_floats(N, B) : 0;
+}
 int fegnn_mmd_forward(int32_t B, int32_t C, int32_t ns, float sigma, float scale_vv, float scale_rv, const float* x,
-                      const float* Z, const int32_t* sample_idx, float* loss, void* stream) {
+                      const float* Z, const int32_t* sample_idx, float* loss, float* workspace, size_t workspace_floats,
+                      void* stream) {
   RQ(B >= 0 && C >= 1 && C <= FEGNN_MAX_C && ns >= 0 && sigma > 0.f && loss && (B == 0 || Z));
   RQ(B == 0 || ns == 0 || (x && sample_idx));
-  CK(launch_mmd_fwd(B, C, ns, sigma, scale_vv, scale_rv, x, Z, sample_idx, loss, S(stream)));
+  TRY(check_loss_ws(0, B, workspace, workspace_floats));
+  CK(launch_mmd_fwd(B, C, ns, sigma, scale_vv, scale_rv, x, Z, sample_idx, loss, g_det ? workspace : nullptr, S(stream)));
   return 0;
 }
 int fegnn_mmd_backward(int32_t N, int32_t B, int32_t C, int32_t ns, float sigma, float scale_vv, float scale_rv,
@@ -1161,17 +1209,19 @@ int fegnn_mmd_backward(int32_t N, int32_t B, int32_t C, int32_t ns, float sigma,
                        float* gZ, void* stream) {
   RQ(N >= 0 && B >= 0 && C >= 1 && C <= FEGNN_MAX_C && ns >= 0 && sigma > 0.f && gloss && gx && gZ);
   RQ(B == 0 || (Z && (ns == 0 || (x && sample_idx))));
-  CK(launch_mmd_bwd(N, B, C, ns, sigma, scale_vv, scale_rv, x, Z, sample_idx, gloss, gx, gZ, S(stream)));
+  CK(launch_mmd_bwd(N, B, C, ns, sigma, scale_vv, scale_rv, x, Z, sample_idx, gloss, gx, gZ, g_det != 0, S(stream)));
   return 0;
 }
 
 int fegnn_mse_mmd_forward(int32_t N, int32_t B, int32_t C, int32_t ns, float sigma, float weight, float scale_vv,
                           float scale_rv, float inv_count, const float* x, const float* target, const float* Z,
-                          const int32_t* sample_idx, float* out_total, float* out_mse, void* stream) {
+                          const int32_t* sample_idx, float* out_total, float* out_mse, float* workspace,
+                          size_t workspace_floats, void* stream) {
   RQ(N >= 0 && B >= 0 && C >= 1 && C <= FEGNN_MAX_C && ns >= 0 && sigma > 0.f && out_total && out_mse && (B == 0 || Z));
   RQ((N == 0 || (x && target)) && (B == 0 || ns == 0 || (x && sample_idx)));
+  TRY(check_loss_ws(N, B, workspace, workspace_floats));
   CK(launch_mse_mmd_fwd(N, B, C, ns, sigma, weight, scale_vv, scale_rv, inv_count, x, target, Z, sample_idx, out_total,
-                        out_mse, S(stream)));
+                        out_mse, g_det ? workspace : nullptr, S(stream)));
   return 0;
 }
 int fegnn_mse_mmd_backward(int32_t N, int32_t B, int32_t C, int32_t ns, float sigma, float weight, float scale_vv,
@@ -1181,7 +1231,7 @@ int fegnn_mse_mmd_backward(int32_t N, int32_t B, int32_t C, int32_t ns, float si
   RQ(N >= 0 && B >= 0 && C >= 1 && C <= FEGNN_MAX_C && ns >= 0 && sigma > 0.f && gx && (B == 0 || (Z && gZ)));
   RQ((N == 0 || (x && target)) && (B == 0 || ns == 0 || (x && sample_idx)));
   CK(launch_mse_mmd_bwd(N, B, C, ns, sigma, weight, scale_vv, scale_rv, inv_count, x, target, Z, sample_idx, g_total, g_mse,
-                        gx, gZ, S(stream)));
+                        gx, gZ, g_det != 0, S(stream)));
   return 0;
 }
 

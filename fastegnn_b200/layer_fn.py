@@ -125,6 +125,7 @@ class _LayerFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, spec, graph, h, x, v, Z, S, *params):
         names, flags, grav, Cc = spec
+        L.deterministic("the FastEGNN layer", L.NO_DET_LAYERS)
         dev = x.device
         named = dict(zip(names, params))
         ptrs = layer_ptrs(named, "")
@@ -143,6 +144,7 @@ class _LayerFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gh_new, gx_new, gS_new, gZ_new):
         ph = ctx.ph
+        L.deterministic("the FastEGNN layer backward", L.NO_DET_LAYERS)
         h, x, v, Z, S = ctx.saved_tensors[:5]
         params = ctx.saved_tensors[5:]
         z = lambda t, ref: torch.zeros_like(ref) if t is None else t.contiguous().float()
@@ -166,6 +168,7 @@ def layer_call(named, flags: int, gravity, virtual_channels: int, graph: CsrGrap
 def layer_forward(layer, node_feat, edge_index, coord, node_vel, virtual_coord, virtual_node_feat, data_batch,
                   edge_attr):
     """E_GCL_vel.forward: returns (node_feat, coord, virtual_node_feat, virtual_coord) (:223)."""
+    L.deterministic("E_GCL_vel", L.NO_DET_LAYERS)
     _require_cuda(coord, "coord")
     B = int(virtual_coord.size(0))
     graph = CsrGraph(edge_index, data_batch, edge_attr, B)

@@ -221,6 +221,12 @@ class SavedBlock:
 
 
 # ----------------------------------------------------------------------------- MMD
+def _loss_workspace(N: int, B: int, dev):
+    """Per-CTA partials of the deterministic loss forward (None and 0 with the mode off)."""
+    n = int(lib.fegnn_loss_workspace_floats(N, B))
+    return (torch.empty(n, device=dev, dtype=torch.float32) if n else None), n
+
+
 class _MmdFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, Z, sample_idx, sigma, scale_vv, scale_rv):
@@ -230,9 +236,12 @@ class _MmdFn(torch.autograd.Function):
         B, _, C_ = Z.shape
         ns = sample_idx.size(1)
         loss = torch.empty(1, device=x.device, dtype=torch.float32)
+        ctx.det = L.deterministic("mmd_loss")
+        ws, nws = _loss_workspace(0, B, x.device)
         with _on(x.device):
             L.check(lib.fegnn_mmd_forward(B, C_, ns, float(sigma), float(scale_vv), float(scale_rv), L.ptr(x), L.ptr(Z),
-                                          L.ptr(sample_idx), L.ptr(loss), _stream(x.device)), "fegnn_mmd_forward")
+                                          L.ptr(sample_idx), L.ptr(loss), L.ptr(ws), nws, _stream(x.device)),
+                    "fegnn_mmd_forward")
         ctx.save_for_backward(x, Z, sample_idx)
         ctx.cfg = (float(sigma), float(scale_vv), float(scale_rv))
         return loss[0]
@@ -245,6 +254,7 @@ class _MmdFn(torch.autograd.Function):
         gx = torch.empty_like(x)
         gZ = torch.empty_like(Z)
         gl = g.reshape(1).contiguous().float()
+        L.set_mode("deterministic", int(ctx.det))          # the backward takes the summation order of its forward
         with _on(x.device):
             L.check(lib.fegnn_mmd_backward(x.size(0), B, C_, idx.size(1), sigma, svv, srv, L.ptr(x), L.ptr(Z), L.ptr(idx),
                                            L.ptr(gl), L.ptr(gx), L.ptr(gZ), _stream(x.device)), "fegnn_mmd_backward")
@@ -257,8 +267,10 @@ def mmd_loss(node_loc: torch.Tensor, virtual_node_loc: torch.Tensor, sample_idx:
 
     node_loc [N,3]; virtual_node_loc [B,3,C] exactly as FastEGNN.forward returns it (the
     reference permutes it to [B,C,3] at :113); sample_idx int32 [B, ns] of GLOBAL node
-    indices (graph offset + the reference's torch.randperm(n_b)[:ns]).  scale_vv / scale_rv weight the
-    two terms (1, 1 = the reference; the partitioned path splits the sum over ranks, see fegnn.h)."""
+    indices (graph offset + the reference's torch.randperm(n_b)[:ns]).  scale_vv / scale_rv weight the two terms (1, 1 =
+    the reference; the partitioned path splits the sum over ranks, see fegnn.h).  Under
+    torch.use_deterministic_algorithms(True) the result and its gradients are bitwise reproducible as long as no node
+    index appears in the samples of two different graphs (true when each graph samples its own nodes)."""
     if sample_idx.dtype != torch.int32:
         sample_idx = sample_idx.to(torch.int32)
     return _MmdFn.apply(node_loc, virtual_node_loc, sample_idx.contiguous(), sigma, scale_vv, scale_rv)
@@ -272,10 +284,13 @@ class _MseMmdFn(torch.autograd.Function):
         B, _, C_ = Z.shape
         total = torch.empty((), device=x.device, dtype=torch.float32)
         mse = torch.empty((), device=x.device, dtype=torch.float32)
+        ctx.det = L.deterministic("mse_mmd_loss")
+        ws, nws = _loss_workspace(x.size(0), B, x.device)
         with _on(x.device):
             L.check(lib.fegnn_mse_mmd_forward(x.size(0), B, C_, sample_idx.size(1), float(sigma), float(weight),
                                               float(scale_vv), float(scale_rv), float(inv_count), L.ptr(x), L.ptr(target),
-                                              L.ptr(Z), L.ptr(sample_idx), L.ptr(total), L.ptr(mse), _stream(x.device)),
+                                              L.ptr(Z), L.ptr(sample_idx), L.ptr(total), L.ptr(mse), L.ptr(ws), nws,
+                                              _stream(x.device)),
                     "fegnn_mse_mmd_forward")
         ctx.save_for_backward(x, target, Z, sample_idx)
         ctx.cfg = (float(sigma), float(weight), float(scale_vv), float(scale_rv), float(inv_count))
@@ -291,6 +306,7 @@ class _MseMmdFn(torch.autograd.Function):
         gZ = torch.empty_like(Z)
         gt = None if g_total is None else g_total.reshape(1).contiguous().float()
         gm = None if g_mse is None else g_mse.reshape(1).contiguous().float()
+        L.set_mode("deterministic", int(ctx.det))
         with _on(x.device):
             L.check(lib.fegnn_mse_mmd_backward(x.size(0), B, C_, idx.size(1), sigma, weight, svv, srv, inv_count, L.ptr(x),
                                                L.ptr(target), L.ptr(Z), L.ptr(idx), L.ptr(gt), L.ptr(gm), L.ptr(gx), L.ptr(gZ),
@@ -303,7 +319,8 @@ def mse_mmd_loss(node_loc: torch.Tensor, target: torch.Tensor, virtual_node_loc:
     """The training step's loss of utils/train.py:104-163 in one launch per direction:
     `total = mse_loss(node_loc, target) + weight * mmd_loss(node_loc, virtual_node_loc, sample_idx, sigma)`.
     Returns (total, mse): `total` is what the loop back-propagates (:166), `mse` what it logs (:107).  No gradient flows to
-    `target`.  inv_count defaults to 1 / node_loc.numel() (torch's mean reduction)."""
+    `target`.  inv_count defaults to 1 / node_loc.numel() (torch's mean reduction).  Deterministic under
+    torch.use_deterministic_algorithms(True) on the same condition as mmd_loss."""
     if sample_idx.dtype != torch.int32:
         sample_idx = sample_idx.to(torch.int32)
     if inv_count is None:
@@ -348,4 +365,5 @@ class _SegmentFn(torch.autograd.Function):
 
 def segment_reduce(data: torch.Tensor, segment_ids: torch.Tensor, num_segments: int, mean: bool) -> torch.Tensor:
     """unsorted_segment_sum / unsorted_segment_mean of models/FastEGNN.py:279-294 (2-D data, int64 ids)."""
+    L.deterministic("unsorted_segment_mean" if mean else "unsorted_segment_sum", "a scatter by segment id with float atomics")
     return _SegmentFn.apply(data, segment_ids, int(num_segments), bool(mean))

@@ -490,6 +490,7 @@ class _PartitionedStackFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, gx_out, gZ_out):
+        L.deterministic("PartitionedFastEGNN backward", "multi-GPU runs are not covered, and " + L.NO_DET_LAYERS)
         with _on(ctx.saved_tensors[1].device):
             return _PartitionedStackFn._backward(ctx, gx_out, gZ_out)
 
@@ -599,6 +600,7 @@ class PartitionedFastEGNN:
         """node_* hold this rank's owned rows followed by its halo rows ([Nl, .]); edge_index is local
         (row < N owned, col < Nl) -- or this rank's prebuilt CsrGraph (DeviceSlabPlan.graph; edge_attr must then be None);
         loc_mean [1,3,C] is replicated.  Returns (x' of the OWNED rows, Z')."""
+        L.deterministic("PartitionedFastEGNN", "multi-GPU runs are not covered, and " + L.NO_DET_LAYERS)
         _require_cuda(node_loc, "node_loc")
         N = self.comm.N
         B = int(loc_mean.size(0))

@@ -141,7 +141,8 @@ typedef struct fegnn_layer_saved {   /* the accumulators msum, tsum, zh1, Dsum, 
 } fegnn_layer_saved;
 
 const char* fegnn_last_error(void);
-int fegnn_version(void);   /* 101 (100: before fegnn_layer_saved.wimg / fegnn_node_h_weight_images / FEGNN_F_WIMG_READY) */
+int fegnn_version(void);   /* 102 (101: before the "deterministic" mode and the loss forwards' workspace; 100: before
+                              fegnn_layer_saved.wimg / fegnn_node_h_weight_images / FEGNN_F_WIMG_READY) */
 /* kernels launched by this library so far in this process (host-side counter; bench.py reports it) */
 unsigned long long fegnn_launch_count(void);
 /* Arithmetic mode of a phase.  "edge_forward": 0 = fp32 FMA kernel, 1 = tcgen05 single-pass TF32 tiles (default),
@@ -156,7 +157,14 @@ unsigned long long fegnn_launch_count(void);
  * on tcgen05 error-compensated 3xTF32 tiles (fp32-grade) with fegnn_node_pre_forward on the fp32 FMA kernel, 1 = that plus
  * single-pass tcgen05 TF32 for fegnn_node_pre_forward (opt-in: rounding the unbounded h to TF32 costs equivariant_test.py's
  * atol 1e-4 on its U(0,10) inputs).  "node_backward": 0 = fp32 FMA kernels, 1 = tcgen05 TF32, 2 = auto (default; = 1 today)
- * for fegnn_node_pre_backward and fegnn_node_h_backward (gradients do not enter the forward equivariance).  Process-wide. */
+ * for fegnn_node_pre_backward and fegnn_node_h_backward (gradients do not enter the forward equivariance).  Process-wide.
+ * "deterministic": 0 (default) or 1.  Under 1, fegnn_mmd_forward / _backward and fegnn_mse_mmd_forward / _backward run
+ * forms whose every sum has a fixed order: repeated calls with the same inputs on the same device model and SM count give
+ * bitwise identical results, whatever the timing (eager or graph replay, other work on other streams, a fresh process);
+ * the forwards take a workspace of fegnn_loss_workspace_floats.  fegnn_adam_step, fegnn_graph_prep and the radius graph are deterministic in either mode.
+ * Every entry that adds floats across CTAs in arrival order and has no such form -- the layer phases, fegnn_model_*,
+ * fegnn_embed_backward, fegnn_graph_xsum, fegnn_rf_vel_backward, fegnn_segment_reduce, fegnn_halo_reduce_push and
+ * fegnn_p2p_allreduce -- returns FEGNN_EINVAL under 1, naming the reason, instead of running. */
 int fegnn_set_mode(const char* phase, int mode);
 int fegnn_get_mode(const char* phase);
 
@@ -368,10 +376,15 @@ int fegnn_model_backward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegn
  * loss = scale_vv * (1/(B C^2)) sum k(Z_bc,Z_bc') - scale_rv * (2/(B ns C)) sum k(x_s, Z_bc),
  * k(p,q) = exp(-|p-q| / (2 sigma^2)).  scale_vv = scale_rv = 1 is the reference; the partitioned
  * path evaluates the Z-only term on one rank (scale_vv = 0 elsewhere) and weights each rank's share of
- * the samples (scale_rv = ns_local / ns_total; ns == 0 is allowed).                                   */
+ * the samples (scale_rv = ns_local / ns_total; ns == 0 is allowed).
+ * Under the "deterministic" mode the forward keeps one partial per CTA in `workspace` (at least
+ * fegnn_loss_workspace_floats(N, B) floats; pass N = 0 for fegnn_mmd_forward) and the backward is bitwise reproducible
+ * provided no node index is sampled by two different graphs (sampling within each graph, as the reference does).  With
+ * the mode off the query returns 0 and workspace may be NULL.                                                      */
+size_t fegnn_loss_workspace_floats(int32_t N, int32_t B);
 int fegnn_mmd_forward(int32_t B, int32_t C, int32_t ns, float sigma, float scale_vv, float scale_rv,
                       const float* x /*[N,3]*/, const float* Z /*[B,3,C]*/, const int32_t* sample_idx,
-                      float* loss /*[1] zeroed here*/, void* stream);
+                      float* loss /*[1] zeroed here*/, float* workspace, size_t workspace_floats, void* stream);
 int fegnn_mmd_backward(int32_t N, int32_t B, int32_t C, int32_t ns, float sigma, float scale_vv, float scale_rv,
                        const float* x, const float* Z, const int32_t* sample_idx, const float* gloss /*[1]*/,
                        float* gx /*[N,3] zeroed here*/, float* gZ /*[B,3,C] =*/, void* stream);
@@ -383,7 +396,8 @@ int fegnn_mmd_backward(int32_t N, int32_t B, int32_t C, int32_t ns, float sigma,
  *   gx [N,3] (zeroed here) = (g_total + g_mse) * 2 inv_count (x - target) + g_total * weight * dMMD/dx ; gZ [B,3,C] =. */
 int fegnn_mse_mmd_forward(int32_t N, int32_t B, int32_t C, int32_t ns, float sigma, float weight, float scale_vv,
                           float scale_rv, float inv_count, const float* x, const float* target, const float* Z,
-                          const int32_t* sample_idx, float* out_total, float* out_mse, void* stream);
+                          const int32_t* sample_idx, float* out_total, float* out_mse, float* workspace,
+                          size_t workspace_floats, void* stream);
 int fegnn_mse_mmd_backward(int32_t N, int32_t B, int32_t C, int32_t ns, float sigma, float weight, float scale_vv,
                            float scale_rv, float inv_count, const float* x, const float* target, const float* Z,
                            const int32_t* sample_idx, const float* g_total, const float* g_mse, float* gx, float* gZ,
