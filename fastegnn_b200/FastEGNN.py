@@ -8,8 +8,11 @@ equivariant_test.py.  All arithmetic runs in libfegnn.so (hand-written sm_100a k
 explicit backward); there is no eager / CPU fallback -- non-CUDA tensors raise.
 
 Differences a caller can observe
-  * hidden_nf must be 64, act_fn must be SiLU, residual must be True, node_attr_nf must
-    be 0 (what all three mains use); anything else raises NotImplementedError.
+  * hidden_nf must be 64, act_fn must be SiLU, residual must be True (what all three mains use) and node_attr_nf
+    at most 16; anything else raises NotImplementedError.
+  * node_attr (node_attr_nf > 0) enters node_mlp.0 as its LAST node_attr_nf input columns, [h ; mean m ; vec(u) ; a]
+    (:89-93,:159).  That order is restated from the constructor's width expression and is unpinned: no golden vector
+    of the unmodified reference covers node_attr_nf > 0.  No gradient flows to node_attr (data, like node_vel).
   * the number of graphs is taken from loc_mean.size(0) instead of data_batch[-1].item()
     (:267), which removes a device synchronisation; the two agree for valid batches.
   * no gradient flows to node_vel (it is data in every caller).
@@ -23,7 +26,8 @@ import torch
 from torch import nn
 
 from . import _lib as L
-from .ops import CsrGraph, SavedBlock, _on, _require_cuda, _stream, layer_ptrs, make_dims, segment_reduce
+from .ops import (CsrGraph, SavedBlock, _on, _require_cuda, _stream, layer_ptrs, make_dims, node_attr_arg,
+                  segment_reduce)
 
 lib = L.lib
 
@@ -65,8 +69,8 @@ class E_GCL_vel(nn.Module):
             raise NotImplementedError("only act_fn=nn.SiLU() is implemented (the reference default, used by all mains)")
         if not residual:
             raise NotImplementedError("residual=False is not implemented (all reference mains use residual=True)")
-        if node_attr_nf != 0:
-            raise NotImplementedError("node_attr_nf must be 0 (the reference mains pass node_attr=None)")
+        if not 0 <= node_attr_nf <= L.MAX_FA:
+            raise NotImplementedError(f"node_attr_nf must be in [0, {L.MAX_FA}]")
         if not 1 <= virtual_channels <= L.MAX_C:
             raise NotImplementedError(f"virtual_channels must be in [1, {L.MAX_C}]")
         if not 0 <= edge_attr_nf <= L.MAX_FE:
@@ -78,6 +82,7 @@ class E_GCL_vel(nn.Module):
         self.epsilon = 1e-8
         self.virtual_channels = virtual_channels
         self.edge_attr_nf = edge_attr_nf
+        self.node_attr_nf = node_attr_nf
         H, Cc = hidden_nf, virtual_channels
         self.edge_mlp = nn.Sequential(nn.Linear(2 * H + 1 + edge_attr_nf, H), act_fn, nn.Linear(H, H), act_fn)
         self.edge_mlp_virtual = nn.Sequential(nn.Linear(2 * H + 1 + Cc, H), act_fn, nn.Linear(H, H), act_fn)
@@ -99,19 +104,21 @@ class E_GCL_vel(nn.Module):
         """(h, x, S, Z) of one layer, S in the reference's [B,H,C] layout (:192-223)."""
         if self.coords_agg not in ('sum', 'mean'):
             raise Exception('Wrong coords_agg parameter')      # raised at call time with the reference's text (:131)
+        node_attr = node_attr_arg(node_attr, self.node_attr_nf, coord.size(0))
         from .layer_fn import layer_forward     # phase-by-phase driver (also used by the partitioned path)
         return layer_forward(self, node_feat, edge_index, coord, node_vel, virtual_coord, virtual_node_feat,
-                             data_batch, edge_attr)
+                             data_batch, edge_attr, node_attr)
 
 
 class _StackFn(torch.autograd.Function):
     """FastEGNN.forward / backward as two C calls (fegnn_model_forward / _backward)."""
 
     @staticmethod
-    def forward(ctx, mod: "FastEGNN", graph: CsrGraph, node_feat, x0, v, loc_mean, *params):
+    def forward(ctx, mod: "FastEGNN", graph: CsrGraph, node_attr, node_feat, x0, v, loc_mean, *params):
         dev = x0.device
         N, B, Cc, Lyr = graph.N, graph.B, mod.virtual_channels, mod.n_layers
-        dims = make_dims(N, N, graph.E, B, Cc, graph.Fe, mod._flag_word, mod._gravity)
+        dims = make_dims(N, N, graph.E, B, Cc, graph.Fe, mod._flag_word, mod._gravity, Fa=mod._node_attr_nf,
+                         node_attr=node_attr)
         pd = C.byref(dims)
         table, names = mod._param_table()
         ws_floats = int(lib.fegnn_model_workspace_floats(pd, Lyr))
@@ -125,7 +132,7 @@ class _StackFn(torch.autograd.Function):
                                             L.ptr(x0), L.ptr(v), L.ptr(loc_mean), L.ptr(x_out), L.ptr(Z_out), L.ptr(ws),
                                             ws_floats, _stream(dev)), "fegnn_model_forward")
         ctx.mod, ctx.graph, ctx.dims, ctx.ws, ctx.Fin = mod, graph, dims, ws, Fin
-        ctx.save_for_backward(node_feat, v)
+        ctx.save_for_backward(node_feat, v, node_attr)          # node_attr: dims points at it until the backward
         ctx.names = names
         ctx.need_nf = node_feat.requires_grad
         ctx.mark_non_differentiable()
@@ -135,7 +142,7 @@ class _StackFn(torch.autograd.Function):
     def backward(ctx, gx, gZ):
         mod, graph, dims = ctx.mod, ctx.graph, ctx.dims
         L.deterministic(type(mod).__name__ + " backward", L.NO_DET_LAYERS)
-        node_feat, v = ctx.saved_tensors
+        node_feat, v, _ = ctx.saved_tensors
         dev = v.device
         N, B, Cc, Lyr = graph.N, graph.B, mod.virtual_channels, mod.n_layers
         pd = C.byref(dims)
@@ -157,15 +164,16 @@ class _StackFn(torch.autograd.Function):
                     "fegnn_model_backward")
         dead = mod._dead_names
         grads = tuple(None if n in dead else views[n] for n in names)
-        return (None, None, g_nf, g_x0, None, g_lm) + grads
+        return (None, None, None, g_nf, g_x0, None, g_lm) + grads
 
 
-def _stack_inference(mod: "FastEGNN", graph: CsrGraph, node_feat, x0, v, loc_mean):
+def _stack_inference(mod: "FastEGNN", graph: CsrGraph, node_attr, node_feat, x0, v, loc_mean):
     """FastEGNN.forward without autograd: fegnn_model_forward_inference (two ping-pong states + one shared block of
     per-layer intermediates -- a ring of four blocks up to 65 536 nodes; nothing is kept for a backward)."""
     dev = x0.device
     N, B, Cc, Lyr = graph.N, graph.B, mod.virtual_channels, mod.n_layers
-    dims = make_dims(N, N, graph.E, B, Cc, graph.Fe, mod._flag_word, mod._gravity)
+    dims = make_dims(N, N, graph.E, B, Cc, graph.Fe, mod._flag_word, mod._gravity, Fa=mod._node_attr_nf,
+                     node_attr=node_attr)
     pd = C.byref(dims)
     table, _ = mod._param_table()
     ws_floats = int(lib.fegnn_model_inference_workspace_floats(pd))
@@ -189,6 +197,7 @@ class FastEGNN(nn.Module):
     -- or under torch.no_grad() -- takes the forward-only stack (fegnn_model_forward_inference): same outputs, no saved
     activations, outputs without grad_fn.  Set eval_keeps_graph = True to get the training forward in eval mode."""
     eval_keeps_graph = False
+    _node_attr_nf = 0          # subclasses without node attributes (FastRF) inherit forward and the stack functions
 
     def __init__(self, node_feat_nf, node_attr_nf, edge_attr_nf, hidden_nf, virtual_channels, device='cpu',
                  act_fn=nn.SiLU(), n_layers=4, residual=True, attention=False, normalize=False, tanh=False,
@@ -216,6 +225,7 @@ class FastEGNN(nn.Module):
                                                     tanh=tanh, gravity=gravity))
         self._flag_word = _flags(attention, normalize, tanh, gravity)
         self._edge_attr_nf = edge_attr_nf
+        self._node_attr_nf = node_attr_nf
         self._cache = None
         last = "gcl_%d" % (n_layers - 1)
         # the final h and S are discarded (:276): these tensors receive no gradient in the reference
@@ -268,6 +278,7 @@ class FastEGNN(nn.Module):
     # -- forward --------------------------------------------------------------------------
     def forward(self, node_feat, node_loc, node_vel, edge_index, data_batch, loc_mean, edge_attr=None, node_attr=None):
         L.deterministic(type(self).__name__, L.NO_DET_LAYERS)
+        node_attr = node_attr_arg(node_attr, self._node_attr_nf, node_loc.size(0))
         _require_cuda(node_loc, "node_loc")
         if isinstance(edge_index, CsrGraph):
             # a graph already in kernel layout (CsrGraph.from_radius, or a CsrGraph reused across steps of a static
@@ -278,7 +289,7 @@ class FastEGNN(nn.Module):
             if graph.Fe != self._edge_attr_nf or graph.N != node_loc.size(0) or graph.B != loc_mean.size(0):
                 raise RuntimeError(f"prebuilt graph (N={graph.N}, B={graph.B}, Fe={graph.Fe}) does not match the inputs "
                                    f"(N={node_loc.size(0)}, B={loc_mean.size(0)}, edge_attr_nf={self._edge_attr_nf})")
-            return self._run_stack(graph, node_feat, node_loc, node_vel, loc_mean)
+            return self._run_stack(graph, node_attr, node_feat, node_loc, node_vel, loc_mean)
         if edge_attr is None:
             if self._edge_attr_nf != 0:
                 raise TypeError("edge_attr is required when edge_attr_nf > 0 (the reference's torch.cat fails on None, "
@@ -288,16 +299,16 @@ class FastEGNN(nn.Module):
                                f"{self._edge_attr_nf}")
         B = int(loc_mean.size(0))
         graph = CsrGraph(edge_index, data_batch, edge_attr, B, overlap=True)      # the sort runs under the first node phase
-        return self._run_stack(graph, node_feat, node_loc, node_vel, loc_mean)
+        return self._run_stack(graph, node_attr, node_feat, node_loc, node_vel, loc_mean)
 
-    def _run_stack(self, graph, node_feat, node_loc, node_vel, loc_mean):
+    def _run_stack(self, graph, node_attr, node_feat, node_loc, node_vel, loc_mean):
         args = (node_feat.contiguous().float(), node_loc.contiguous().float(), node_vel.contiguous().float(),
                 loc_mean.contiguous().float())
         try:
             if not torch.is_grad_enabled() or (not self.training and not self.eval_keeps_graph):
-                return _stack_inference(self, graph, *[a.detach() for a in args])
+                return _stack_inference(self, graph, node_attr, *[a.detach() for a in args])
             params = [p for _, p in self.named_parameters()]
-            return _StackFn.apply(self, graph, *args, *params)
+            return _StackFn.apply(self, graph, node_attr, *args, *params)
         finally:
             # the C call has joined the side stream of CsrGraph(overlap=True): later users of the graph (backward) need no wait
             if getattr(graph, "_ready", None) is not None:

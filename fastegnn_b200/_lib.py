@@ -18,6 +18,7 @@ LIB_PATH = os.environ.get("FEGNN_LIB") or os.path.join(HERE, "_C", "libfegnn.so"
 H = 64
 MAX_C = 16
 MAX_FE = 8
+MAX_FA = 16
 
 F_ATTENTION, F_NORMALIZE, F_TANH, F_GRAVITY, F_LAST, F_RF, F_COORDS_SUM, F_NODE_SUM, F_PREZEROED = 1, 2, 4, 8, 16, 32, 64, 128, 256
 
@@ -28,7 +29,8 @@ lp = C.POINTER(C.c_int64)
 
 class Dims(C.Structure):
     _fields_ = [("N", C.c_int32), ("Nl", C.c_int32), ("E", C.c_int32), ("B", C.c_int32), ("C", C.c_int32),
-                ("Fe", C.c_int32), ("flags", C.c_uint32), ("gravity", C.c_float * 3), ("eps", C.c_float)]
+                ("Fe", C.c_int32), ("flags", C.c_uint32), ("gravity", C.c_float * 3), ("eps", C.c_float),
+                ("Fa", C.c_int32), ("node_attr", C.c_void_p)]
 
 
 class Graph(C.Structure):

@@ -115,6 +115,10 @@ int check_dims(const fegnn_dims* d) {
   if (d->N < 0 || d->Nl < d->N || d->E < 0 || d->B < 0) return fail(FEGNN_EINVAL, "bad sizes N=%d Nl=%d E=%d B=%d", d->N, d->Nl, d->E, d->B);
   if (d->C < 1 || d->C > FEGNN_MAX_C) return fail(FEGNN_EINVAL, "virtual_channels C=%d outside [1,%d]", d->C, FEGNN_MAX_C);
   if (d->Fe < 0 || d->Fe > FEGNN_MAX_FE) return fail(FEGNN_EINVAL, "edge_attr width Fe=%d outside [0,%d]", d->Fe, FEGNN_MAX_FE);
+  if (d->Fa < 0 || d->Fa > FEGNN_MAX_FA) return fail(FEGNN_EINVAL, "node_attr width Fa=%d outside [0,%d]", d->Fa, FEGNN_MAX_FA);
+  if ((d->Fa == 0) != (d->node_attr == nullptr))
+    return fail(FEGNN_EINVAL, "node_attr must be %s with Fa=%d", d->Fa == 0 ? "NULL" : "non-NULL", d->Fa);
+  if (d->Fa > 0 && (d->flags & FEGNN_F_RF)) return fail(FEGNN_EINVAL, "FEGNN_F_RF layers have no phi_h: Fa must be 0");
   return 0;
 }
 
@@ -136,7 +140,16 @@ cudaError_t zero_pair(float* a, size_t na, float* b, size_t nb, cudaStream_t st)
 inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 inline int ld1(const fegnn_dims* d) { return 2 * kH + 1 + d->Fe; }
 inline int ldv(const fegnn_dims* d) { return 2 * kH + 1 + d->C; }
-inline int ldn(const fegnn_dims* d) { return 2 * kH + kH * d->C; }
+inline int ldn(const fegnn_dims* d) { return 2 * kH + kH * d->C + d->Fa; }
+// the attribute term of Uh: columns [ldn - Fa, ldn) of node_mlp.0.weight (and of its gradient)
+NodeAttrArgs node_attr_args(const fegnn_dims* d, const float* w0, float* gw0) {
+  NodeAttrArgs at;
+  memset(&at, 0, sizeof(at));
+  const int off = ldn(d) - d->Fa;
+  at.Fa = d->Fa; at.ldn = ldn(d); at.a = d->node_attr;
+  at.w = w0 + off; at.gw = gw0 != nullptr ? gw0 + off : nullptr;
+  return at;
+}
 
 EdgeArgs edge_args(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
                    const fegnn_layer_saved* sv) {
@@ -259,7 +272,7 @@ SideStream* side_stream() {
 extern "C" {
 
 const char* fegnn_last_error(void) { return g_err; }
-int fegnn_version(void) { return 102; }      // 102: "deterministic" mode, workspace of fegnn_mmd_forward / fegnn_mse_mmd_forward
+int fegnn_version(void) { return 103; }      // 103: fegnn_dims.Fa / .node_attr; 102: "deterministic" mode, loss workspaces
 unsigned long long fegnn_launch_count(void) { return g_launches; }
 int fegnn_set_mode(const char* phase, int mode) {
   if (phase == nullptr) return fail(FEGNN_EINVAL, "phase is null");
@@ -402,9 +415,12 @@ int fegnn_node_pre_forward(const fegnn_dims* d, const fegnn_layer_params* p, con
   RQ(h && sv);
   NodePreArgs a = node_pre_args(d, p, h);
   a.P = sv->P; a.Q = sv->Q; a.Av = sv->Av; a.Uh = sv->Uh; a.sv = sv->sv; a.sg = sv->sg;
-  if (g_node_fwd_mode == 1 && !(d->flags & FEGNN_F_RF)) CK(launch_node_pre_fwd_tc(a, sm_count(), S(stream)));
-  else if (g_node_fwd_mode == 3 && g_node_pre_tc3) CK(launch_node_pre_fwd_tc3(a, sm_count(), S(stream)));
-  else CK(launch_node_pre_fwd(a, sm_count(), S(stream)));
+  // node attributes enter Uh only; the last layer has none (its phi_h is discarded)
+  const NodeAttrArgs at_ = node_attr_args(d, p->node_w0, nullptr);
+  const NodeAttrArgs* at = d->Fa > 0 && !(d->flags & FEGNN_F_LAST) ? &at_ : nullptr;
+  if (g_node_fwd_mode == 1 && !(d->flags & FEGNN_F_RF)) CK(launch_node_pre_fwd_tc(a, sm_count(), S(stream), at));
+  else if (g_node_fwd_mode == 3 && g_node_pre_tc3) CK(launch_node_pre_fwd_tc3(a, sm_count(), S(stream), at));
+  else CK(launch_node_pre_fwd(a, sm_count(), S(stream), at));
   return 0;
 }
 
@@ -642,6 +658,9 @@ int fegnn_node_pre_backward(const fegnn_dims* d, const fegnn_layer_params* p, fe
   a.g_node_w0 = gr->node_w0; a.g_node_b0 = gr->node_b0;
   a.g_vel_w0 = gr->vel_w0; a.g_vel_b0 = gr->vel_b0; a.g_vel_w2 = gr->vel_w2; a.g_vel_b2 = gr->vel_b2;
   a.g_grav_w0 = gr->grav_w0; a.g_grav_b0 = gr->grav_b0; a.g_grav_w2 = gr->grav_w2; a.g_grav_b2 = gr->grav_b2;
+  // dU1att = sum_i gUh_i a_i^T rides on the Uh block (none in the last layer: gUh == NULL)
+  const NodeAttrArgs at_ = node_attr_args(d, p->node_w0, gr->node_w0);
+  const bool attr = d->Fa > 0 && gUh != nullptr;
   if (node_bwd_tc(d->N)) {
     // tcgen05: gh += G_blk W_blk (red.add), dW_blk += G_blk^T h, db_blk += sum G_blk for P, Q, Av [, Uh] and the phi_v
     // [/ phi_g] heads (whose G is recomputed on the tensor core from h)
@@ -662,14 +681,17 @@ int fegnn_node_pre_backward(const fegnn_dims* d, const fegnn_layer_params* p, fe
     plain(gP, p->edge_w0, a.ld1, gr->edge_w0, gr->edge_b0);
     plain(gQ, p->edge_w0 + kH, a.ld1, gr->edge_w0 ? gr->edge_w0 + kH : nullptr, nullptr);
     plain(gAv, p->edgev_w0, a.ldv, gr->edgev_w0, gr->edgev_b0);
+    dtc::AttrBlk ab;
+    ab.at = at_;
+    ab.blk = t.nblk;
     if (gUh != nullptr) plain(gUh, p->node_w0, a.ldn, gr->node_w0, gr->node_b0);
     if (!(d->flags & FEGNN_F_RF)) head(gsv, p->vel_w0, p->vel_b0, p->vel_w2, gr->vel_w0, gr->vel_b0, gr->vel_w2, gr->vel_b2);
     if (d->flags & FEGNN_F_GRAVITY)
       head(gsg, p->grav_w0, p->grav_b0, p->grav_w2, gr->grav_w0, gr->grav_b0, gr->grav_w2, gr->grav_b2);
-    CK(launch_dense_bwd_tc(t, sm_count(), S(stream)));
+    CK(launch_dense_bwd_tc(t, sm_count(), S(stream), attr ? &ab : nullptr));
     return 0;
   }
-  CK(launch_node_pre_bwd(a, sm_count(), S(stream)));
+  CK(launch_node_pre_bwd(a, sm_count(), S(stream), attr ? &at_ : nullptr));
   return 0;
 }
 

@@ -81,8 +81,16 @@ struct Smem {
 };
 constexpr uint32_t kACC = 0, kOPA = 64, kRW = 128;      // tensor-memory columns (256 allocated: two CTAs per SM)
 
-template <int CG>
-__global__ void __launch_bounds__(128 * CG, 2) dense_bwd_tc_kernel(const __grid_constant__ Args a) {
+// Node attributes (node_pre_backward with Fa > 0): block at.blk (Uh) also adds dU1att += X^T a (NodeAttrArgs) -- a column
+// walk over the X tile weighted by the attribute rows, fp32, like the bias sums.  Only the kAttr instantiations use it.
+struct AttrBlk {
+  NodeAttrArgs at;
+  int blk;
+};
+__host__ __device__ constexpr int attr_off(size_t base) { return (int)((base + 15) / 16 * 16); }
+
+template <int CG, bool kAttr>
+__global__ void __launch_bounds__(128 * CG, 2) dense_bwd_tc_kernel(const __grid_constant__ Args a, const AttrBlk ab) {
   constexpr int NT = 128 * CG, CPT = kH / CG;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (umma::smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -93,6 +101,15 @@ __global__ void __launch_bounds__(128 * CG, 2) dense_bwd_tc_kernel(const __grid_
   const int bid = blockIdx.x % a.nblk, cta = blockIdx.x / a.nblk, nctas = gridDim.x / a.nblk;
   const Blk& b = a.blk[bid];
   uint8_t *Wm = smem + Smem::off_Wm, *Wk = smem + Smem::off_Wk, *TY = smem + Smem::off_TY, *TX = smem + Smem::off_TX;
+  [[maybe_unused]] const bool attr = kAttr && bid == ab.blk;         // uniform over the CTA
+  [[maybe_unused]] float* sA = reinterpret_cast<float*>(smem + attr_off(Smem::off_vec + sizeof(Vec)));
+  [[maybe_unused]] float* sRed = sA + kTM * kMaxFa;
+  [[maybe_unused]] float sa[kMaxFa];
+  if constexpr (kAttr) {
+#pragma unroll
+    for (int f = 0; f < kMaxFa; ++f) sa[f] = 0.f;
+    for (int i = t; i < kMaxFa * kH; i += NT) sRed[i] = 0.f;
+  }
 
   // ---- prologue: weight block in both layouts (MN-major for X W; K-major only for the head recompute), vectors
   {
@@ -227,10 +244,19 @@ __global__ void __launch_bounds__(128 * CG, 2) dense_bwd_tc_kernel(const __grid_
     }
     tmem_st<CPT>(tlane + kOPA, x);
     mn_store_row<CPT>(TX, row, cg, x);
+    if constexpr (kAttr) {
+      if (attr) attr_load_tile(sA, ab.at, i0, min(kTM, a.N - i0), NT);
+    }
     tmem_st_wait();
     umma::fence_smem_to_async();
     umma::fence_before();
     __syncthreads();
+    if constexpr (kAttr) {
+      if (attr) {                                  // TX is rewritten by the next tile only after the barrier below
+        attr_wgrad_walk(sa, sA, ab.at.Fa, [&](int rr, int c) { return *reinterpret_cast<const float*>(TX + mn_off(rr, c, kTM)); });
+        __syncthreads();
+      }
+    }
     if (warp == 0) {
       umma::fence_after();
       if (umma::elect_one()) {
@@ -304,6 +330,9 @@ __global__ void __launch_bounds__(128 * CG, 2) dense_bwd_tc_kernel(const __grid_
     if (b.head && b.g_hw2 != nullptr) atomicAdd(b.g_hw2 + t, v->cw2[t]);
     if (b.head && t == 0 && b.g_hb2 != nullptr) atomicAdd(b.g_hb2, v->cb2);
   }
+  if constexpr (kAttr) {
+    if (attr && !first) attr_wgrad_flush(sa, sRed, ab.at);
+  }
   umma::fence_before();
   __syncthreads();
   if (warp == 0) umma::tmem_dealloc<256>(tmem);
@@ -362,7 +391,8 @@ __device__ __forceinline__ void gemm_ts_mn_acc(uint32_t tmem_d, uint32_t tmem_a,
 //   * the weight gradient leaves tensor memory through a [64][65] staging tile and goes out with the lanes along k
 //     (128 contiguous bytes per warp-wide reduction for wks = 1);
 //   * silu'(Y) of a block whose output gate reads the same rows (dz == Y: node_h stage 1) stays in registers.
-__global__ void __launch_bounds__(256, 1) dense_bwd_tc_rows_kernel(const __grid_constant__ Args a) {
+template <bool kAttr>
+__global__ void __launch_bounds__(256, 1) dense_bwd_tc_rows_kernel(const __grid_constant__ Args a, const AttrBlk ab) {
   constexpr int NT = 256, CG = 2, CPT = kH / CG, NWR = kH * kH / NT;     // 16 weight words per thread and block
 #ifdef FEGNN_TRACE
   long long tr_[48];
@@ -384,6 +414,15 @@ __global__ void __launch_bounds__(256, 1) dense_bwd_tc_rows_kernel(const __grid_
 
   // block range of this CTA (blockIdx.y): at a few dozen tiles the SMs left over take a share of the blocks instead of idling
   const int b0 = a.nsplit > 1 ? a.split[blockIdx.y] : 0, b1 = a.nsplit > 1 ? a.split[blockIdx.y + 1] : a.nblk;
+  [[maybe_unused]] const bool attr = kAttr && ab.blk >= b0 && ab.blk < b1;     // uniform over the CTA
+  [[maybe_unused]] float* sA = reinterpret_cast<float*>(smem + attr_off(SmemR::off_vec + sizeof(VecR)));
+  [[maybe_unused]] float* sRed = sA + kTM * kMaxFa;
+  [[maybe_unused]] float sa[kMaxFa];
+  if constexpr (kAttr) {
+#pragma unroll
+    for (int f = 0; f < kMaxFa; ++f) sa[f] = 0.f;
+    for (int i = t; i < kMaxFa * kH; i += NT) sRed[i] = 0.f;
+  }
   float wreg[NWR];
   auto load_w = [&](const Blk& b) {             // every load in flight before anything is stored
 #pragma unroll
@@ -578,6 +617,9 @@ __global__ void __launch_bounds__(256, 1) dense_bwd_tc_rows_kernel(const __grid_
       }
       // ---- X row -> A operand (tensor memory); the data gradient of block b - 1 has left the A operand
       tmem_st<CPT>(tlane + kR_OPA, xr);
+      if constexpr (kAttr) {
+        if (b == ab.blk) attr_load_tile(sA, ab.at, r0, min(kTM, a.N - r0), NT);
+      }
       tmem_st_wait();
       TR(tb_ + 2);
       if (more) load_w(a.blk[b + 1]);             // lands under the MMAs / epilogue of this block
@@ -618,6 +660,10 @@ __global__ void __launch_bounds__(256, 1) dense_bwd_tc_rows_kernel(const __grid_
 #pragma unroll 8
         for (int rr = part * 32; rr < part * 32 + 32; ++rr) sum += *reinterpret_cast<const float*>(TX(s_) + mn_off(rr, col, kTM));
         atomicAdd(&v->cb[s_][col], sum);
+      }
+      if constexpr (kAttr) {
+        if (b == ab.blk)
+          attr_wgrad_walk(sa, sA, ab.at.Fa, [&](int rr, int c) { return *reinterpret_cast<const float*>(TX(s_) + mn_off(rr, c, kTM)); });
       }
       TR(tb_ + 5);
       if (b > b0) {
@@ -693,6 +739,9 @@ __global__ void __launch_bounds__(256, 1) dense_bwd_tc_rows_kernel(const __grid_
     for (int o = 16; o > 0; o >>= 1) dmx = fmaxf(dmx, __shfl_xor_sync(0xffffffffu, dmx, o));
     if (lane == 0) atomicMax(dmx_ptr, __float_as_uint(dmx));
   }
+  if constexpr (kAttr) {
+    if (attr) attr_wgrad_flush(sa, sRed, ab.at);
+  }
   umma::fence_before();
   __syncthreads();
   if (warp == 0) umma::tmem_dealloc<256>(tmem);
@@ -720,7 +769,8 @@ inline bool dense_bwd_uses_rows(int N, int sms) {
   return (long long)ntiles <= (long long)dense_rows_max_tiles_per_sm() * sms;
 }
 
-cudaError_t launch_dense_bwd_tc(const dtc::Args& a_in, int sms, cudaStream_t st) {
+// ab != nullptr: the attribute instantiation (block ab->blk adds dU1att)
+cudaError_t launch_dense_bwd_tc(const dtc::Args& a_in, int sms, cudaStream_t st, const dtc::AttrBlk* ab = nullptr) {
   dtc::Args a = a_in;
   a.nsplit = 1;
   a.same_y_mask = a.chain_mask = 0;
@@ -732,7 +782,7 @@ cudaError_t launch_dense_bwd_tc(const dtc::Args& a_in, int sms, cudaStream_t st)
   }
   static DevOnce attr;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(dtc::dense_bwd_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(dtc::dense_bwd_tc_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)dtc::Smem::bytes);
     if (e != cudaSuccess) return e;
     attr.set();
@@ -742,7 +792,7 @@ cudaError_t launch_dense_bwd_tc(const dtc::Args& a_in, int sms, cudaStream_t st)
   if (dense_bwd_uses_rows(a.N, sms)) {   // small graphs: one CTA per node tile walks the blocks
     static DevOnce attr2;
     if (!attr2.get()) {
-      cudaError_t e = cudaFuncSetAttribute(dtc::dense_bwd_tc_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+      cudaError_t e = cudaFuncSetAttribute(dtc::dense_bwd_tc_rows_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            (int)dtc::SmemR::bytes);
       if (e != cudaSuccess) return e;
       attr2.set();
@@ -766,12 +816,35 @@ cudaError_t launch_dense_bwd_tc(const dtc::Args& a_in, int sms, cudaStream_t st)
       while (s_ < nsplit) a.split[++s_] = a.nblk;
       a.nsplit = nsplit;
     }
-    if (cudaError_t e_ = launch_pdl(dtc::dense_bwd_tc_rows_kernel, dim3(ntiles < sms ? ntiles : sms, a.nsplit), dim3(256), dtc::SmemR::bytes, st, a)) return e_;
+    const dim3 grid(ntiles < sms ? ntiles : sms, a.nsplit);
+    if (ab != nullptr) {
+      const size_t bytes = dtc::attr_off(dtc::SmemR::bytes) + kAttrGBytes;
+      static DevOnce attr3;
+      if (!attr3.get()) {
+        cudaError_t e = cudaFuncSetAttribute(dtc::dense_bwd_tc_rows_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+        if (e != cudaSuccess) return e;
+        attr3.set();
+      }
+      if (cudaError_t e_ = launch_pdl(dtc::dense_bwd_tc_rows_kernel<true>, grid, dim3(256), bytes, st, a, *ab)) return e_;
+      return cudaGetLastError();
+    }
+    if (cudaError_t e_ = launch_pdl(dtc::dense_bwd_tc_rows_kernel<false>, grid, dim3(256), dtc::SmemR::bytes, st, a, dtc::AttrBlk{})) return e_;
     return cudaGetLastError();
   }
   int per = (2 * sms) / a.nblk;                   // CTAs per block at 2 CTAs / SM
   per = per < 1 ? 1 : (per > ntiles ? ntiles : per);
-  if (cudaError_t e_ = launch_pdl(dtc::dense_bwd_tc_kernel<2>, per * a.nblk, 256, dtc::Smem::bytes, st, a)) return e_;
+  if (ab != nullptr) {
+    const size_t bytes = dtc::attr_off(dtc::Smem::bytes) + kAttrGBytes;
+    static DevOnce attr4;
+    if (!attr4.get()) {
+      cudaError_t e = cudaFuncSetAttribute(dtc::dense_bwd_tc_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+      if (e != cudaSuccess) return e;
+      attr4.set();
+    }
+    if (cudaError_t e_ = launch_pdl(dtc::dense_bwd_tc_kernel<2, true>, per * a.nblk, 256, bytes, st, a, *ab)) return e_;
+    return cudaGetLastError();
+  }
+  if (cudaError_t e_ = launch_pdl(dtc::dense_bwd_tc_kernel<2, false>, per * a.nblk, 256, dtc::Smem::bytes, st, a, dtc::AttrBlk{})) return e_;
   return cudaGetLastError();
 }
 

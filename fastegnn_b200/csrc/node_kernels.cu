@@ -95,6 +95,58 @@ struct NodePreArgs {
   float *g_vel_w0, *g_vel_b0, *g_vel_w2, *g_vel_b2, *g_grav_w0, *g_grav_b0, *g_grav_w2, *g_grav_b2;
 };
 
+// Node attributes (Fa = node_attr_nf > 0): Uh gains the rank-Fa term U1att a_i (columns [off, off + Fa) of node_w0, row
+// stride ldn) and the backward adds dU1att = sum_i gUh_i a_i^T.  Only the attribute instantiations of the node_pre kernels
+// do anything with these arguments: the <false> kernels are the Fa = 0 code, unchanged.
+struct NodeAttrArgs {
+  int Fa, ldn;
+  const float* a;    // [N, Fa]
+  const float* w;    // node_w0 + off
+  float* gw;         // g node_w0 + off, or nullptr
+};
+constexpr int kMaxFa = FEGNN_MAX_FA;
+constexpr size_t kAttrWBytes = kMaxFa * kH * sizeof(float);                   // U1att transposed: [f][n]
+constexpr size_t kAttrGBytes = (kTM * kMaxFa + kMaxFa * kH) * sizeof(float);  // a tile [128][Fa] + dU1att partials [f][n]
+
+// sW[f * 64 + n] = U1att[n][f]
+__device__ __forceinline__ void attr_stage_w(float* __restrict__ sW, const NodeAttrArgs& at, int nt) {
+  for (int i = threadIdx.x; i < at.Fa * kH; i += nt) sW[i] = at.w[(size_t)(i & 63) * at.ldn + (i >> 6)];
+}
+// sum_f a[row][f] * U1att[n][f], fp32 FMA
+__device__ __forceinline__ float attr_dot(const NodeAttrArgs& at, const float* __restrict__ sW, int row, int n) {
+  float s = 0.f;
+  const float* ar = at.a + (size_t)row * at.Fa;
+  for (int f = 0; f < at.Fa; ++f) s = fmaf(ar[f], sW[f * kH + n], s);
+  return s;
+}
+// a rows i0 .. i0 + 127 -> sA[r * Fa + f], zero past the end (the gradient rows there are zero, the product must be too)
+__device__ __forceinline__ void attr_load_tile(float* __restrict__ sA, const NodeAttrArgs& at, int i0, int nvalid, int nt) {
+  for (int i = threadIdx.x; i < kTM * at.Fa; i += nt) sA[i] = i < nvalid * at.Fa ? at.a[(size_t)i0 * at.Fa + i] : 0.f;
+}
+// dU1att partials over one tile: thread (col = tid & 63, part = tid >> 6) walks rows 32 part .. 32 part + 31 of column col
+// of the gradient tile (g(rr, col)); 256 threads
+template <typename G>
+__device__ __forceinline__ void attr_wgrad_walk(float (&sa)[kMaxFa], const float* __restrict__ sA, int Fa, G g) {
+  const int col = threadIdx.x & 63, part = threadIdx.x >> 6;
+  for (int rr = part * 32; rr < part * 32 + 32; ++rr) {
+    const float x = g(rr, col);
+#pragma unroll
+    for (int f = 0; f < kMaxFa; ++f)
+      if (f < Fa) sa[f] = fmaf(x, sA[rr * Fa + f], sa[f]);
+  }
+}
+// the four row parts add in shared memory (red: [f][64], zeroed by the caller before a barrier), then one atomic per weight
+// and CTA.  All threads call.
+__device__ __forceinline__ void attr_wgrad_flush(const float (&sa)[kMaxFa], float* __restrict__ red, const NodeAttrArgs& at) {
+  const int col = threadIdx.x & 63;
+#pragma unroll
+  for (int f = 0; f < kMaxFa; ++f)
+    if (f < at.Fa) atomicAdd(&red[f * kH + col], sa[f]);
+  __syncthreads();
+  if (at.gw != nullptr)
+    for (int i = threadIdx.x; i < at.Fa * kH; i += blockDim.x) atomicAdd(at.gw + (size_t)(i & 63) * at.ldn + (i >> 6), red[i]);
+}
+
 constexpr int kNodePreBlocks = 6;   // P, Q, Av, Uh, vel, grav
 constexpr size_t kNodePreFwdSmem = (kWFloats + kTileFloats + 2 * kH) * sizeof(float);
 
@@ -109,11 +161,13 @@ __device__ __forceinline__ int node_pre_block_id(int k, bool last, bool grav, bo
   return k;
 }
 
-__global__ void __launch_bounds__(kThreads, 3) node_pre_fwd_kernel(NodePreArgs a, int nactive) {
+template <bool kAttr>
+__global__ void __launch_bounds__(kThreads, 3) node_pre_fwd_kernel(NodePreArgs a, int nactive, NodeAttrArgs at) {
   extern __shared__ __align__(16) float smem[];
   float* Ws = smem;
   float* T0 = Ws + kWFloats;
   float* vec = T0 + kTileFloats;     // head blocks: [0] first-layer bias, [1] output weight
+  float* sWa = vec + 2 * kH;         // attribute instantiation: U1att, [f][n]
   const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
   const bool grav = a.flags & FEGNN_F_GRAVITY, last = a.flags & FEGNN_F_LAST;
   const int blk = node_pre_block_id(blockIdx.x % nactive, last, grav, a.flags & FEGNN_F_RF);
@@ -126,6 +180,9 @@ __global__ void __launch_bounds__(kThreads, 3) node_pre_fwd_kernel(NodePreArgs a
     stage_vec(vec, blk == 4 ? a.vel_b0 : a.grav_b0, kH);
     stage_vec(vec + kH, blk == 4 ? a.vel_w2 : a.grav_w2, kH);
   }
+  if constexpr (kAttr) {
+    if (blk == 3) attr_stage_w(sWa, at, kThreads);
+  }
   pdl_wait();
   const int ntiles = (a.N + kTM - 1) / kTM;
   for (int tile = cta; tile < ntiles; tile += nctas) {
@@ -136,6 +193,18 @@ __global__ void __launch_bounds__(kThreads, 3) node_pre_fwd_kernel(NodePreArgs a
     float acc[kRT][4];
     zero_acc(acc);
     gemm_nt(acc, T0, Ws, ty, tx);
+    if constexpr (kAttr) {
+      if (blk == 3) {
+#pragma unroll
+        for (int i = 0; i < kRT; ++i) {
+          const int r = ty * kRT + i;
+          if (r < nvalid) {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) acc[i][j] += attr_dot(at, sWa, i0 + r, tx * 4 + j);
+          }
+        }
+      }
+    }
     if (blk < 4) {
       const float* bias = blk == 0 ? a.edge_b0 : blk == 2 ? a.edgev_b0 : blk == 3 ? a.node_b0 : nullptr;
       float* out = blk == 0 ? a.P : blk == 1 ? a.Q : blk == 2 ? a.Av : a.Uh;
@@ -196,12 +265,15 @@ constexpr size_t kNodePreBwdSmem = (kWFloats + 2 * kTileFloats + 2 * kH) * sizeo
 
 // gh (in: dL/dh' of the residual, out: dL/dh) += G_blk W_blk ; dW_blk += G_blk^T h.
 // Work item = (node tile, block) as in the forward; gh is accumulated with red.global.add.v4.f32.
-__global__ void __launch_bounds__(kThreads, 2) node_pre_bwd_kernel(NodePreArgs a, int nactive) {
+template <bool kAttr>
+__global__ void __launch_bounds__(kThreads, 2) node_pre_bwd_kernel(NodePreArgs a, int nactive, NodeAttrArgs at) {
   extern __shared__ __align__(16) float smem[];
   float* Ws = smem;
   float* Th = Ws + kWFloats;
   float* TG = Th + kTileFloats;
   float* vec = TG + kTileFloats;   // [0] = first-layer bias of a head, [1] = its output weight
+  float* sA = vec + 2 * kH;        // attribute instantiation: a tile [128][Fa], then the dU1att partials [f][64]
+  float* sRed = sA + kTM * kMaxFa;
   const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
   const bool grav = a.flags & FEGNN_F_GRAVITY, last = a.gUh == nullptr;
   const int blk = node_pre_block_id(blockIdx.x % nactive, last, grav, a.flags & FEGNN_F_RF);
@@ -226,12 +298,24 @@ __global__ void __launch_bounds__(kThreads, 2) node_pre_bwd_kernel(NodePreArgs a
   float wg[4][4], bs[4] = {0, 0, 0, 0}, cw2[4] = {0, 0, 0, 0};
   float cb2 = 0.f;
   zero_wg(wg);
+  [[maybe_unused]] float sa[kMaxFa];
+  if constexpr (kAttr) {
+#pragma unroll
+    for (int f = 0; f < kMaxFa; ++f) sa[f] = 0.f;
+    for (int i = tid; i < kMaxFa * kH; i += kThreads) sRed[i] = 0.f;
+  }
   for (int tile = cta; tile < ntiles; tile += nctas) {
     const int i0 = tile * kTM, nvalid = min(kTM, a.N - i0);
     __syncthreads();
     load_tile(Th, a.h + (size_t)i0 * kH, kH, nvalid);
     if (!head) load_tile(TG, G + (size_t)i0 * kH, kH, nvalid);
+    if constexpr (kAttr) {
+      if (blk == 3) attr_load_tile(sA, at, i0, nvalid, kThreads);
+    }
     __syncthreads();
+    if constexpr (kAttr) {
+      if (blk == 3) attr_wgrad_walk(sa, sA, at.Fa, [&](int rr, int c) { return TG[rr * kH + c]; });
+    }
     float acc[kRT][4];
     if (head) {
       // recompute z = W h + b ; G = gs_i * w2 * silu'(z)
@@ -271,6 +355,9 @@ __global__ void __launch_bounds__(kThreads, 2) node_pre_bwd_kernel(NodePreArgs a
     colsum_flush(cw2, blk == 4 ? a.g_vel_w2 : a.g_grav_w2, 1, tx);
     float* gb2 = blk == 4 ? a.g_vel_b2 : a.g_grav_b2;
     if (tx == 0 && gb2 != nullptr) atomicAdd(gb2, cb2);
+  }
+  if constexpr (kAttr) {
+    if (blk == 3) attr_wgrad_flush(sa, sRed, at);      // uniform over the CTA
   }
 }
 
@@ -516,22 +603,37 @@ static inline int node_pre_grid(int ntiles, int nactive, int sms, int ctas_per_s
   if (per > ntiles) per = ntiles;
   return per * nactive;
 }
-cudaError_t launch_node_pre_fwd(const NodePreArgs& a, int sms, cudaStream_t st) {
-  FEGNN_SET_SMEM(node_pre_fwd_kernel, kNodePreFwdSmem);
+// at != nullptr: the attribute instantiation (Fa > 0 and a Uh block: not the last layer)
+cudaError_t launch_node_pre_fwd(const NodePreArgs& a, int sms, cudaStream_t st, const NodeAttrArgs* at = nullptr) {
+  FEGNN_SET_SMEM(node_pre_fwd_kernel<false>, kNodePreFwdSmem);
   int ntiles = (a.N + kTM - 1) / kTM;
   if (ntiles == 0) return cudaSuccess;
   const bool grav = a.flags & FEGNN_F_GRAVITY, last = a.flags & FEGNN_F_LAST;
   const int nactive = 4 + (grav ? 2 : 1) - (last ? 1 : 0) - ((a.flags & FEGNN_F_RF) ? 1 : 0);
-  if (cudaError_t e_ = launch_pdl(node_pre_fwd_kernel, node_pre_grid(ntiles, nactive, sms, 3), kThreads, kNodePreFwdSmem, st, a, nactive)) return e_;
+  if (at != nullptr) {
+    FEGNN_SET_SMEM(node_pre_fwd_kernel<true>, kNodePreFwdSmem + kAttrWBytes);
+    if (cudaError_t e_ = launch_pdl(node_pre_fwd_kernel<true>, node_pre_grid(ntiles, nactive, sms, 3), kThreads,
+                                    kNodePreFwdSmem + kAttrWBytes, st, a, nactive, *at)) return e_;
+    return cudaGetLastError();
+  }
+  if (cudaError_t e_ = launch_pdl(node_pre_fwd_kernel<false>, node_pre_grid(ntiles, nactive, sms, 3), kThreads, kNodePreFwdSmem, st, a, nactive,
+                                  NodeAttrArgs{})) return e_;
   return cudaGetLastError();
 }
-cudaError_t launch_node_pre_bwd(const NodePreArgs& a, int sms, cudaStream_t st) {
-  FEGNN_SET_SMEM(node_pre_bwd_kernel, kNodePreBwdSmem);
+cudaError_t launch_node_pre_bwd(const NodePreArgs& a, int sms, cudaStream_t st, const NodeAttrArgs* at = nullptr) {
+  FEGNN_SET_SMEM(node_pre_bwd_kernel<false>, kNodePreBwdSmem);
   int ntiles = (a.N + kTM - 1) / kTM;
   if (ntiles == 0) return cudaSuccess;
   const bool grav = a.flags & FEGNN_F_GRAVITY, last = a.gUh == nullptr;
   const int nactive = 4 + (grav ? 2 : 1) - (last ? 1 : 0) - ((a.flags & FEGNN_F_RF) ? 1 : 0);
-  if (cudaError_t e_ = launch_pdl(node_pre_bwd_kernel, node_pre_grid(ntiles, nactive, sms), kThreads, kNodePreBwdSmem, st, a, nactive)) return e_;
+  if (at != nullptr) {
+    FEGNN_SET_SMEM(node_pre_bwd_kernel<true>, kNodePreBwdSmem + kAttrGBytes);
+    if (cudaError_t e_ = launch_pdl(node_pre_bwd_kernel<true>, node_pre_grid(ntiles, nactive, sms), kThreads,
+                                    kNodePreBwdSmem + kAttrGBytes, st, a, nactive, *at)) return e_;
+    return cudaGetLastError();
+  }
+  if (cudaError_t e_ = launch_pdl(node_pre_bwd_kernel<false>, node_pre_grid(ntiles, nactive, sms), kThreads, kNodePreBwdSmem, st, a, nactive,
+                                  NodeAttrArgs{})) return e_;
   return cudaGetLastError();
 }
 cudaError_t launch_node_h_fwd(const NodeHArgs& a, int sms, cudaStream_t st, bool zero = true) {

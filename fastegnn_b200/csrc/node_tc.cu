@@ -56,14 +56,18 @@ struct PreSmem {
   static constexpr int off_A = 3 * 16384;            // h tile [128][64] K-major
   static constexpr int off_vec = off_A + 32768;
   static constexpr size_t bytes = off_vec + sizeof(PreVec) + 1024;
+  static constexpr int off_attr = (off_vec + sizeof(PreVec) + 15) / 16 * 16;
+  static constexpr size_t attr_bytes = bytes + 16 + kAttrWBytes;
 };
 
-__global__ void __launch_bounds__(256, 2) node_pre_fwd_tc_kernel(NodePreArgs a) {
+template <bool kAttr>
+__global__ void __launch_bounds__(256, 2) node_pre_fwd_tc_kernel(NodePreArgs a, NodeAttrArgs at) {
   constexpr int NT = 256, CPT = 32;
   using SM = PreSmem;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (umma::smem_u32(smem_raw) & 1023u)) & 1023u);
   PreVec* v = reinterpret_cast<PreVec*>(smem + SM::off_vec);
+  [[maybe_unused]] float* sWa = reinterpret_cast<float*>(smem + SM::off_attr);     // attribute instantiation: U1att [f][n]
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
   const int quarter = warp & 3, cg = warp >> 2, row = quarter * 32 + lane, c0 = cg * CPT;
   const bool grav = a.flags & FEGNN_F_GRAVITY, last = a.flags & FEGNN_F_LAST;
@@ -89,6 +93,9 @@ __global__ void __launch_bounds__(256, 2) node_pre_fwd_tc_kernel(NodePreArgs a) 
     for (int i = t; i < kH; i += NT) {
       v->bias[j * kH + i] = bias != nullptr ? bias[i] : 0.f;
       v->w2[j * kH + i] = w2 != nullptr ? w2[i] : 0.f;
+    }
+    if constexpr (kAttr) {
+      if (b == 3) attr_stage_w(sWa, at, NT);
     }
   }
   if (t == 0) {
@@ -148,6 +155,16 @@ __global__ void __launch_bounds__(256, 2) node_pre_fwd_tc_kernel(NodePreArgs a) 
       tmem_ld<CPT>(tlane + j * kH, z);
       if (b < 4) {
         float* out = b == 0 ? a.P : b == 1 ? a.Q : b == 2 ? a.Av : a.Uh;
+        if constexpr (kAttr) {
+          if (b == 3 && row < nvalid) {                  // + U1att a_i in fp32
+            const float* ar = at.a + (size_t)(i0 + row) * at.Fa;
+            for (int f = 0; f < at.Fa; ++f) {
+              const float af = ar[f];
+#pragma unroll
+              for (int jj = 0; jj < CPT; ++jj) z[jj] = fmaf(af, sWa[f * kH + c0 + jj], z[jj]);
+            }
+          }
+        }
         if (row < nvalid) {
           float4* dst = reinterpret_cast<float4*>(out + (size_t)(i0 + row) * kH + c0);
 #pragma unroll
@@ -479,15 +496,20 @@ struct P3Smem {
   static constexpr int off_vec = off_ST + kT;
   static constexpr size_t bytes = off_vec + sizeof(P3Vec) + 1024;
   static_assert(bytes <= 232448, "node_pre forward (3xTF32): shared memory");
+  static constexpr int off_attr = (off_vec + sizeof(P3Vec) + 15) / 16 * 16;
+  static constexpr size_t attr_bytes = bytes + 16 + kAttrWBytes;
+  static_assert(attr_bytes <= 232448, "node_pre forward (3xTF32, node attributes): shared memory");
 };
 
-__global__ void __launch_bounds__(256, 1) node_pre_fwd_tc3_kernel(NodePreArgs a, int nactive) {
+template <bool kAttr>
+__global__ void __launch_bounds__(256, 1) node_pre_fwd_tc3_kernel(NodePreArgs a, int nactive, NodeAttrArgs at) {
   constexpr int NT = 256, CPT = 32, NA = kTM * 16 / NT, NWR = kH * kH / NT;
   using SM = P3Smem;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (umma::smem_u32(smem_raw) & 1023u)) & 1023u);
   pdl_trigger();
   P3Vec* v = reinterpret_cast<P3Vec*>(smem + SM::off_vec);
+  [[maybe_unused]] float* sWa = reinterpret_cast<float*>(smem + SM::off_attr);     // attribute instantiation: U1att [f][n]
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
   const int quarter = warp & 3, cg = warp >> 2, row = quarter * 32 + lane, c0 = cg * CPT;
   const int rr0 = t >> 4, c16 = t & 15;
@@ -553,6 +575,9 @@ __global__ void __launch_bounds__(256, 1) node_pre_fwd_tc3_kernel(NodePreArgs a,
 
   // ---- prologue (weights only)
   load_w(kb);
+  if constexpr (kAttr) {
+    if (!last) attr_stage_w(sWa, at, NT);
+  }
   if (t == 0) {
     umma::mbar_init(&v->bar[0], 1);
     umma::mbar_init(&v->bar[1], 1);
@@ -606,9 +631,20 @@ __global__ void __launch_bounds__(256, 1) node_pre_fwd_tc3_kernel(NodePreArgs a,
 #pragma unroll
       for (int j = 0; j < NA; ++j) {
         const int rr = rr0 + 16 * j;
-        if (i0 + rr < a.N)
-          *reinterpret_cast<float4*>(out + (size_t)(i0 + rr) * kH + 4 * c16) =
-              *reinterpret_cast<const float4*>(ST + umma::tile_chunk_off(rr, c16, kTM));
+        if (i0 + rr < a.N) {
+          float4 o = *reinterpret_cast<const float4*>(ST + umma::tile_chunk_off(rr, c16, kTM));
+          if constexpr (kAttr) {
+            if (b == 3) {                          // + U1att a_i in fp32
+              const float* ar = at.a + (size_t)(i0 + rr) * at.Fa;
+              for (int f = 0; f < at.Fa; ++f) {
+                const float af = ar[f];
+                const float4 w = *reinterpret_cast<const float4*>(sWa + f * kH + 4 * c16);
+                o.x = fmaf(af, w.x, o.x); o.y = fmaf(af, w.y, o.y); o.z = fmaf(af, w.z, o.z); o.w = fmaf(af, w.w, o.w);
+              }
+            }
+          }
+          *reinterpret_cast<float4*>(out + (size_t)(i0 + rr) * kH + 4 * c16) = o;
+        }
       }
     } else {
       float s = 0.f;
@@ -662,26 +698,35 @@ __global__ void __launch_bounds__(256, 1) node_pre_fwd_tc3_kernel(NodePreArgs a,
 
 }  // namespace ntc
 
-cudaError_t launch_node_pre_fwd_tc(const NodePreArgs& a, int sms, cudaStream_t st) {
+// at != nullptr: the attribute instantiation (Fa > 0 and a Uh block: not the last layer)
+cudaError_t launch_node_pre_fwd_tc(const NodePreArgs& a, int sms, cudaStream_t st, const NodeAttrArgs* at = nullptr) {
   static DevOnce attr;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(ntc::node_pre_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(ntc::node_pre_fwd_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)ntc::PreSmem::bytes);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(ntc::node_pre_fwd_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)ntc::PreSmem::attr_bytes);
     if (e != cudaSuccess) return e;
     attr.set();
   }
   const int ntiles = (a.N + kTM - 1) / kTM;
   if (ntiles == 0) return cudaSuccess;
   int per = ntiles < sms ? ntiles : sms;          // CTAs per group; 2 groups -> up to 2 CTAs / SM
-  ntc::node_pre_fwd_tc_kernel<<<2 * per, 256, ntc::PreSmem::bytes, st>>>(a); ++g_launches;
+  if (at != nullptr) ntc::node_pre_fwd_tc_kernel<true><<<2 * per, 256, ntc::PreSmem::attr_bytes, st>>>(a, *at);
+  else ntc::node_pre_fwd_tc_kernel<false><<<2 * per, 256, ntc::PreSmem::bytes, st>>>(a, NodeAttrArgs{});
+  ++g_launches;
   return cudaGetLastError();
 }
 
-cudaError_t launch_node_pre_fwd_tc3(const NodePreArgs& a, int sms, cudaStream_t st) {
+cudaError_t launch_node_pre_fwd_tc3(const NodePreArgs& a, int sms, cudaStream_t st, const NodeAttrArgs* at = nullptr) {
   static DevOnce attr;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(ntc::node_pre_fwd_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(ntc::node_pre_fwd_tc3_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)ntc::P3Smem::bytes);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(ntc::node_pre_fwd_tc3_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)ntc::P3Smem::attr_bytes);
     if (e != cudaSuccess) return e;
     attr.set();
   }
@@ -690,8 +735,13 @@ cudaError_t launch_node_pre_fwd_tc3(const NodePreArgs& a, int sms, cudaStream_t 
   const bool grav = a.flags & FEGNN_F_GRAVITY, last = a.flags & FEGNN_F_LAST;
   const int nactive = 4 + (grav ? 2 : 1) - (last ? 1 : 0) - ((a.flags & FEGNN_F_RF) ? 1 : 0);
   const int nsplit = 2 * ntiles <= sms ? 2 : 1;   // few tiles: two CTAs per tile, half of the blocks each
-  if (cudaError_t e_ = launch_pdl(ntc::node_pre_fwd_tc3_kernel, dim3(ntiles < sms ? ntiles : sms, nsplit), 256, ntc::P3Smem::bytes,
-                                  st, a, nactive))
+  const dim3 grid(ntiles < sms ? ntiles : sms, nsplit);
+  if (at != nullptr) {
+    if (cudaError_t e_ = launch_pdl(ntc::node_pre_fwd_tc3_kernel<true>, grid, 256, ntc::P3Smem::attr_bytes, st, a, nactive, *at))
+      return e_;
+    return cudaGetLastError();
+  }
+  if (cudaError_t e_ = launch_pdl(ntc::node_pre_fwd_tc3_kernel<false>, grid, 256, ntc::P3Smem::bytes, st, a, nactive, NodeAttrArgs{}))
     return e_;
   return cudaGetLastError();
 }

@@ -123,13 +123,14 @@ class _LayerFn(torch.autograd.Function):
     its own parameters (fastegnn_b200/VNEGNN.py).  spec = (names, flag word, gravity list or None, virtual channels)."""
 
     @staticmethod
-    def forward(ctx, spec, graph, h, x, v, Z, S, *params):
+    def forward(ctx, spec, graph, node_attr, h, x, v, Z, S, *params):
         names, flags, grav, Cc = spec
         L.deterministic("the FastEGNN layer", L.NO_DET_LAYERS)
         dev = x.device
         named = dict(zip(names, params))
         ptrs = layer_ptrs(named, "")
-        dims = make_dims(graph.N, graph.N, graph.E, graph.B, Cc, graph.Fe, flags, grav)
+        Fa = 0 if node_attr is None else node_attr.size(1)
+        dims = make_dims(graph.N, graph.N, graph.E, graph.B, Cc, graph.Fe, flags, grav, Fa=Fa, node_attr=node_attr)
         ph = LayerPhases(dims, graph, ptrs, dev)
         xsum = torch.empty(graph.B, 3, device=dev, dtype=torch.float32)
         with _on(dev):
@@ -137,6 +138,7 @@ class _LayerFn(torch.autograd.Function):
                     "graph_xsum")
         h_new, x_new, Z_new, S_new, _ = ph.forward(h, x, v, Z, S, xsum)
         ctx.ph = ph
+        ctx.node_attr = node_attr          # ph.d points at it until the backward
         ctx.save_for_backward(h, x, v, Z, S, *params)
         ctx.names = names
         return h_new, x_new, S_new, Z_new
@@ -154,19 +156,20 @@ class _LayerFn(torch.autograd.Function):
         gptrs = layer_ptrs(views, "")
         gh, gx, gZ, gS, gxsum = ph.backward(gptrs, h, x, v, Z, S, gh_new, gx_new, gZ_new, gS_new, None)
         gx = gx + gxsum[ph.g.batch.long()]       # xbar of this layer comes from its own input coordinates
-        return (None, None, gh, gx, None, gZ, gS) + tuple(views[n] for n in ctx.names)
+        return (None, None, None, gh, gx, None, gZ, gS) + tuple(views[n] for n in ctx.names)
 
 
-def layer_call(named, flags: int, gravity, virtual_channels: int, graph: CsrGraph, h, x, v, Z, S):
+def layer_call(named, flags: int, gravity, virtual_channels: int, graph: CsrGraph, h, x, v, Z, S, *, node_attr=None):
     """(h', x', S', Z') of one layer from a dict of weight tensors keyed by the reference's state_dict suffixes
-    (edge_mlp.0.weight, ...); S / S' in kernel layout [B,C,H].  Tensors must be contiguous fp32 CUDA."""
+    (edge_mlp.0.weight, ...); S / S' in kernel layout [B,C,H].  Tensors must be contiguous fp32 CUDA.  node_attr: [N, Fa]
+    contiguous fp32 CUDA data (no gradient) or None; node_mlp.0.weight then has Fa more columns."""
     names = tuple(named.keys())
     spec = (names, int(flags), gravity, int(virtual_channels))
-    return _LayerFn.apply(spec, graph, _f32(h), _f32(x), _f32(v), _f32(Z), _f32(S), *[named[n] for n in names])
+    return _LayerFn.apply(spec, graph, node_attr, _f32(h), _f32(x), _f32(v), _f32(Z), _f32(S), *[named[n] for n in names])
 
 
 def layer_forward(layer, node_feat, edge_index, coord, node_vel, virtual_coord, virtual_node_feat, data_batch,
-                  edge_attr):
+                  edge_attr, node_attr=None):
     """E_GCL_vel.forward: returns (node_feat, coord, virtual_node_feat, virtual_coord) (:223)."""
     L.deterministic("E_GCL_vel", L.NO_DET_LAYERS)
     _require_cuda(coord, "coord")
@@ -179,5 +182,5 @@ def layer_forward(layer, node_feat, edge_index, coord, node_vel, virtual_coord, 
     grav = None if layer.gravity is None else [float(t) for t in layer.gravity.detach().cpu().tolist()]
     named = dict(_layer_named(layer))
     h_new, x_new, S_new, Z_new = layer_call(named, flags, grav, layer.virtual_channels, graph, node_feat, coord, node_vel,
-                                            virtual_coord, S.float())
+                                            virtual_coord, S.float(), node_attr=node_attr)
     return h_new, x_new, S_new.permute(0, 2, 1), Z_new

@@ -181,13 +181,34 @@ class CsrGraph:
 
 
 def make_dims(N: int, Nl: int, E: int, B: int, C_: int, Fe: int, flags: int,
-              gravity: Optional[Sequence[float]] = None, eps: float = 1e-8) -> L.Dims:
+              gravity: Optional[Sequence[float]] = None, eps: float = 1e-8, Fa: int = 0,
+              node_attr: Optional[torch.Tensor] = None) -> L.Dims:
+    """fegnn_dims.  node_attr: [N, Fa] fp32 tensor (kept alive by the caller while the dims are in use) or None."""
     d = L.Dims()
     d.N, d.Nl, d.E, d.B, d.C, d.Fe, d.flags = N, Nl, E, B, C_, Fe, flags
     g = (0.0, 0.0, 0.0) if gravity is None else tuple(float(x) for x in gravity)
     d.gravity[0], d.gravity[1], d.gravity[2] = g
     d.eps = eps
+    d.Fa, d.node_attr = Fa, L.ptr(node_attr)
     return d
+
+
+def node_attr_arg(node_attr, node_attr_nf: int, n_nodes: int) -> Optional[torch.Tensor]:
+    """Checks the node_attr argument of a forward against the module's node_attr_nf (before any device work, as
+    edge_attr is checked) and returns it as a contiguous fp32 CUDA tensor, or None when the module takes none."""
+    if node_attr is None:
+        if node_attr_nf != 0:
+            raise TypeError(f"node_attr is required when node_attr_nf > 0 (got None, node_attr_nf={node_attr_nf}; the "
+                            "reference's torch.cat fails on None, models/FastEGNN.py:159)")
+        return None
+    if node_attr_nf == 0:
+        raise RuntimeError("node_attr was given to a model built with node_attr_nf=0")
+    if node_attr.dim() != 2 or node_attr.size(1) != node_attr_nf:
+        raise RuntimeError(f"node_attr has shape {tuple(node_attr.shape)}, model was built with node_attr_nf={node_attr_nf}")
+    if node_attr.size(0) != n_nodes:
+        raise RuntimeError(f"node_attr has {node_attr.size(0)} rows for {n_nodes} nodes")
+    _require_cuda(node_attr, "node_attr")
+    return node_attr.detach().contiguous().float()
 
 
 def layer_ptrs(tensors: Dict[str, torch.Tensor], prefix: str) -> L.LayerPtrs:

@@ -583,6 +583,8 @@ class PartitionedFastEGNN:
     def __init__(self, model, plan: SlabPlan, rank: int, device, group=None, halo: str = "nccl"):
         """halo = "nccl": pack + all-to-all + unpack; "p2p": direct peer stores / remote atomics over NVLink
         (P2PHaloComm; needs torch symmetric memory, i.e. all ranks on one NVLink / NVSwitch domain)."""
+        if getattr(model, "_node_attr_nf", 0) != 0:
+            raise NotImplementedError("the partitioned path has no node attributes: build the model with node_attr_nf=0")
         self.model, self.plan, self.rank = model, plan, rank
         if halo == "fused":
             self.comm = FusedHaloComm(plan, rank, device, model.n_layers, group)

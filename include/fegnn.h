@@ -16,7 +16,7 @@
  *     thread-local message.
  *   - fp32 everywhere, indices int32 after graph prep (the reference's int64
  *     edge_index / data_batch are converted once by fegnn_graph_prep).
- *   - H (hidden_nf) must be 64; 1 <= C <= FEGNN_MAX_C; 0 <= Fe <= FEGNN_MAX_FE.
+ *   - H (hidden_nf) must be 64; 1 <= C <= FEGNN_MAX_C; 0 <= Fe <= FEGNN_MAX_FE; 0 <= Fa <= FEGNN_MAX_FA.
  *   - "reference layout" = torch.nn.Linear weight [out, in] row-major, the tensors
  *     of the reference state_dict, untouched.  Kernels re-tile them in shared memory.
  */
@@ -33,6 +33,7 @@ extern "C" {
 #define FEGNN_H 64
 #define FEGNN_MAX_C 16
 #define FEGNN_MAX_FE 8
+#define FEGNN_MAX_FA 16
 
 #define FEGNN_OK 0
 #define FEGNN_EINVAL (-1)   /* bad argument (shape / flag / null pointer)  */
@@ -77,6 +78,9 @@ typedef struct fegnn_dims {
   uint32_t flags;   /* FEGNN_F_*                                                    */
   float gravity[3]; /* models/FastEGNN.py:258-259                                   */
   float eps;        /* normalize epsilon, :21                                       */
+  int32_t Fa;       /* node_attr width (node_attr_nf, :89-93); 0 = no node attributes (FastRF: must be 0) */
+  const float* node_attr; /* [N,Fa] fp32, NULL iff Fa == 0: the last Fa columns of node_mlp.0's input (:159), read
+                             by fegnn_node_pre_forward / _backward (Uh += U1att a) and the fegnn_model_* entries */
 } fegnn_dims;
 
 /* CSR-by-row graph, produced by fegnn_graph_prep (all int32 / fp32, device). */
@@ -103,7 +107,7 @@ typedef struct fegnn_layer_params {
   const float *cvv_w0, *cvv_b0, *cvv_w2;                      /* coord_mlp_v_virtual                                 */
   const float *vel_w0, *vel_b0, *vel_w2, *vel_b2;             /* coord_mlp_vel.{0,2}      [H,H],[H],[1,H],[1]       */
   const float *grav_w0, *grav_b0, *grav_w2, *grav_b2;         /* gravity_mlp.{0,2}                                   */
-  const float *node_w0, *node_b0, *node_w2, *node_b2;         /* node_mlp.{0,2}           [H,2H+H*C],[H],[H,H],[H]  */
+  const float *node_w0, *node_b0, *node_w2, *node_b2;         /* node_mlp.{0,2}           [H,2H+H*C+Fa],[H],[H,H],[H] */
   const float *nodev_w0, *nodev_b0, *nodev_w2, *nodev_b2;     /* node_mlp_virtual.{0,2}   [H,2H],[H],[H,H],[H]      */
   const float *att_w, *att_b, *attv_w, *attv_b;               /* att_mlp.0, att_mlp_virtual.0  [1,H],[1]            */
 } fegnn_layer_params;
@@ -141,7 +145,7 @@ typedef struct fegnn_layer_saved {   /* the accumulators msum, tsum, zh1, Dsum, 
 } fegnn_layer_saved;
 
 const char* fegnn_last_error(void);
-int fegnn_version(void);   /* 102 (101: before the "deterministic" mode and the loss forwards' workspace; 100: before
+int fegnn_version(void);   /* 103 (102: before fegnn_dims.Fa / .node_attr; 101: before the "deterministic" mode and the loss forwards' workspace; 100: before
                               fegnn_layer_saved.wimg / fegnn_node_h_weight_images / FEGNN_F_WIMG_READY) */
 /* kernels launched by this library so far in this process (host-side counter; bench.py reports it) */
 unsigned long long fegnn_launch_count(void);
@@ -225,7 +229,8 @@ int fegnn_graph_xsum(int32_t N, int32_t B, const float* x, const int32_t* batch,
 /* xbar, centred Gram M and G1 = V1s S_c + V1m M[:,c]        (:212-214, per-graph part of :112-115) */
 int fegnn_graph_pre_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
                             const float* Z, const float* S, const float* xsum, fegnn_layer_saved* sv, void* stream);
-/* P,Q,Av,Uh and phi_v / phi_g heads: the h-dependent half of every first Linear (:104,115,139,142,162) */
+/* P,Q,Av,Uh and phi_v / phi_g heads: the h-dependent half of every first Linear (:104,115,139,142,162); with Fa > 0
+ * Uh also carries the node-attribute term U1att a_i (columns [2H + H*C, 2H + H*C + Fa) of node_mlp.0.weight) */
 int fegnn_node_pre_forward(const fegnn_dims* d, const fegnn_layer_params* p, const float* h, fegnn_layer_saved* sv,
                            void* stream);
 /* fused real-edge phase: gather, phi_e, phi_x, segment sums by row (:102-108,:125-129,:156) */
