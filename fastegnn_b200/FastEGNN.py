@@ -12,10 +12,12 @@ Differences a caller can observe
     at most 16; anything else raises NotImplementedError.
   * node_attr (node_attr_nf > 0) enters node_mlp.0 as its LAST node_attr_nf input columns, [h ; mean m ; vec(u) ; a]
     (:89-93,:159).  That order is restated from the constructor's width expression and is unpinned: no golden vector
-    of the unmodified reference covers node_attr_nf > 0.  No gradient flows to node_attr (data, like node_vel).
+    of the unmodified reference covers node_attr_nf > 0.
+  * node_vel, node_attr and edge_attr receive gradients as in the reference, computed only when they require grad
+    (fegnn_model_backward_inputs).  Exceptions: FastRF's node_vel (none), and the edge_attr a prebuilt CsrGraph carries
+    (data of the graph: pass graph.edge_index() and a tensor to differentiate it).
   * the number of graphs is taken from loc_mean.size(0) instead of data_batch[-1].item()
     (:267), which removes a device synchronisation; the two agree for valid batches.
-  * no gradient flows to node_vel (it is data in every caller).
 """
 from __future__ import annotations
 
@@ -104,17 +106,22 @@ class E_GCL_vel(nn.Module):
         """(h, x, S, Z) of one layer, S in the reference's [B,H,C] layout (:192-223)."""
         if self.coords_agg not in ('sum', 'mean'):
             raise Exception('Wrong coords_agg parameter')      # raised at call time with the reference's text (:131)
+        attr_in = node_attr
         node_attr = node_attr_arg(node_attr, self.node_attr_nf, coord.size(0))
         from .layer_fn import layer_forward     # phase-by-phase driver (also used by the partitioned path)
         return layer_forward(self, node_feat, edge_index, coord, node_vel, virtual_coord, virtual_node_feat,
-                             data_batch, edge_attr, node_attr)
+                             data_batch, edge_attr, node_attr, attr_in)
 
 
 class _StackFn(torch.autograd.Function):
-    """FastEGNN.forward / backward as two C calls (fegnn_model_forward / _backward)."""
+    """FastEGNN.forward / backward as two C calls (fegnn_model_forward / fegnn_model_backward_inputs).
+
+    node_attr is the contiguous fp32 copy the kernels read; attr_in / edge_attr_in are the caller's tensors (or None), which
+    are inputs here only so that autograd can hand them their gradients.  The kernels read edge_attr from the graph."""
 
     @staticmethod
-    def forward(ctx, mod: "FastEGNN", graph: CsrGraph, node_attr, node_feat, x0, v, loc_mean, *params):
+    def forward(ctx, mod: "FastEGNN", graph: CsrGraph, node_attr, attr_in, edge_attr_in, node_feat, x0, v, loc_mean,
+                *params):
         dev = x0.device
         N, B, Cc, Lyr = graph.N, graph.B, mod.virtual_channels, mod.n_layers
         dims = make_dims(N, N, graph.E, B, Cc, graph.Fe, mod._flag_word, mod._gravity, Fa=mod._node_attr_nf,
@@ -135,6 +142,8 @@ class _StackFn(torch.autograd.Function):
         ctx.save_for_backward(node_feat, v, node_attr)          # node_attr: dims points at it until the backward
         ctx.names = names
         ctx.need_nf = node_feat.requires_grad
+        ctx.in_dtypes = (None if attr_in is None else attr_in.dtype, None if edge_attr_in is None else edge_attr_in.dtype,
+                         v.dtype)
         ctx.mark_non_differentiable()
         return x_out, Z_out
 
@@ -155,16 +164,25 @@ class _StackFn(torch.autograd.Function):
         g_x0 = torch.empty(N, 3, device=dev, dtype=torch.float32)
         g_lm = torch.empty(B, 3, Cc, device=dev, dtype=torch.float32)
         g_nf = torch.empty_like(node_feat) if ctx.need_nf else None
+        # the input gradients exactly as requested; FastRF's velocity enters through |v| and has none (not implemented)
+        need = ctx.needs_input_grad
+        f32 = dict(device=dev, dtype=torch.float32)
+        g_na = torch.empty(N, dims.Fa, **f32) if need[3] else None
+        g_ea = (torch.empty if graph.Fe else torch.zeros)(graph.E, graph.Fe, **f32) if need[4] else None
+        g_v = torch.empty(N, 3, **f32) if need[7] and not (mod._flag_word & L.F_RF) else None
+        ig = L.InputGrads(L.ptr(g_v), L.ptr(g_na), L.ptr(g_ea) if graph.Fe else None, L.ptr(graph.perm))
         with _on(dev):
-            L.check(lib.fegnn_model_backward(pd, Lyr, ctx.Fin, C.byref(graph.c), table, gtable,
-                                             L.ptr(mod.embedding_in.weight), L.ptr(views["embedding_in.weight"]),
-                                             L.ptr(views["embedding_in.bias"]), L.ptr(views["virtual_node_feat"]),
-                                             L.ptr(node_feat), L.ptr(v), L.ptr(gx), L.ptr(gZ), L.ptr(g_x0), L.ptr(g_lm),
-                                             L.ptr(g_nf), L.ptr(ctx.ws), L.ptr(scratch), scr_floats, _stream(dev)),
-                    "fegnn_model_backward")
+            L.check(lib.fegnn_model_backward_inputs(pd, Lyr, ctx.Fin, C.byref(graph.c), table, gtable,
+                                                    L.ptr(mod.embedding_in.weight), L.ptr(views["embedding_in.weight"]),
+                                                    L.ptr(views["embedding_in.bias"]), L.ptr(views["virtual_node_feat"]),
+                                                    L.ptr(node_feat), L.ptr(v), L.ptr(gx), L.ptr(gZ), L.ptr(g_x0),
+                                                    L.ptr(g_lm), L.ptr(g_nf), L.ptr(ctx.ws), L.ptr(scratch), scr_floats,
+                                                    C.byref(ig), _stream(dev)), "fegnn_model_backward_inputs")
         dead = mod._dead_names
         grads = tuple(None if n in dead else views[n] for n in names)
-        return (None, None, None, g_nf, g_x0, None, g_lm) + grads
+        dt_na, dt_ea, dt_v = ctx.in_dtypes
+        cast = lambda g, dt: None if g is None else g.to(dt)
+        return (None, None, None, cast(g_na, dt_na), cast(g_ea, dt_ea), g_nf, g_x0, cast(g_v, dt_v), g_lm) + grads
 
 
 def _stack_inference(mod: "FastEGNN", graph: CsrGraph, node_attr, node_feat, x0, v, loc_mean):
@@ -278,6 +296,7 @@ class FastEGNN(nn.Module):
     # -- forward --------------------------------------------------------------------------
     def forward(self, node_feat, node_loc, node_vel, edge_index, data_batch, loc_mean, edge_attr=None, node_attr=None):
         L.deterministic(type(self).__name__, L.NO_DET_LAYERS)
+        attr_in = node_attr
         node_attr = node_attr_arg(node_attr, self._node_attr_nf, node_loc.size(0))
         _require_cuda(node_loc, "node_loc")
         if isinstance(edge_index, CsrGraph):
@@ -289,7 +308,8 @@ class FastEGNN(nn.Module):
             if graph.Fe != self._edge_attr_nf or graph.N != node_loc.size(0) or graph.B != loc_mean.size(0):
                 raise RuntimeError(f"prebuilt graph (N={graph.N}, B={graph.B}, Fe={graph.Fe}) does not match the inputs "
                                    f"(N={node_loc.size(0)}, B={loc_mean.size(0)}, edge_attr_nf={self._edge_attr_nf})")
-            return self._run_stack(graph, node_attr, node_feat, node_loc, node_vel, loc_mean)
+            # node_attr still gets its gradient; the graph's edge_attr is data of the graph (no autograd input here)
+            return self._run_stack(graph, node_attr, attr_in, None, node_feat, node_loc, node_vel, loc_mean)
         if edge_attr is None:
             if self._edge_attr_nf != 0:
                 raise TypeError("edge_attr is required when edge_attr_nf > 0 (the reference's torch.cat fails on None, "
@@ -299,16 +319,16 @@ class FastEGNN(nn.Module):
                                f"{self._edge_attr_nf}")
         B = int(loc_mean.size(0))
         graph = CsrGraph(edge_index, data_batch, edge_attr, B, overlap=True)      # the sort runs under the first node phase
-        return self._run_stack(graph, node_attr, node_feat, node_loc, node_vel, loc_mean)
+        return self._run_stack(graph, node_attr, attr_in, edge_attr, node_feat, node_loc, node_vel, loc_mean)
 
-    def _run_stack(self, graph, node_attr, node_feat, node_loc, node_vel, loc_mean):
+    def _run_stack(self, graph, node_attr, attr_in, edge_attr_in, node_feat, node_loc, node_vel, loc_mean):
         args = (node_feat.contiguous().float(), node_loc.contiguous().float(), node_vel.contiguous().float(),
                 loc_mean.contiguous().float())
         try:
             if not torch.is_grad_enabled() or (not self.training and not self.eval_keeps_graph):
                 return _stack_inference(self, graph, node_attr, *[a.detach() for a in args])
             params = [p for _, p in self.named_parameters()]
-            return _StackFn.apply(self, graph, node_attr, *args, *params)
+            return _StackFn.apply(self, graph, node_attr, attr_in, edge_attr_in, *args, *params)
         finally:
             # the C call has joined the side stream of CsrGraph(overlap=True): later users of the graph (backward) need no wait
             if getattr(graph, "_ready", None) is not None:

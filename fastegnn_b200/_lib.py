@@ -68,6 +68,12 @@ class LayerPtrs(C.Structure):
     _fields_ = [(n, C.c_void_p) for n, _ in LAYER_FIELDS]
 
 
+class InputGrads(C.Structure):
+    """fegnn_input_grads: requested gradients to node_vel [N,3], node_attr [N,Fa], edge_attr [E,Fe] (NULL = not requested)
+    and the CSR -> caller edge order map (NULL = CSR order)."""
+    _fields_ = [("node_vel", C.c_void_p), ("node_attr", C.c_void_p), ("edge_attr", C.c_void_p), ("perm", C.c_void_p)]
+
+
 SAVED_FIELDS = ["P", "Q", "Av", "Uh", "sv", "sg", "M", "Zc", "G1", "msum", "tsum", "u", "zh1", "Dsum", "Usum", "scratch", "wimg"]
 
 
@@ -102,6 +108,7 @@ lib = _load()
 vp = C.c_void_p
 i32 = C.c_int32
 _PD, _PG, _PP, _PS = C.POINTER(Dims), C.POINTER(Graph), C.POINTER(LayerPtrs), C.POINTER(Saved)
+_PI = C.POINTER(InputGrads)
 
 SIGNATURES = {
     "fegnn_last_error": (C.c_char_p, []),
@@ -131,6 +138,9 @@ SIGNATURES = {
     "fegnn_edge_backward": (C.c_int, [_PD, _PG, _PP, _PP, vp, _PS, vp, vp, vp, vp, vp, vp]),
     "fegnn_graph_pre_backward": (C.c_int, [_PD, _PG, _PP, _PP, vp, _PS, vp, vp, vp, vp, vp]),
     "fegnn_node_pre_backward": (C.c_int, [_PD, _PP, _PP, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "fegnn_virtual_backward_inputs": (C.c_int, [_PD, _PG, _PP, _PP, vp, vp, vp, _PS] + [vp] * 12 + [_PI, vp]),
+    "fegnn_edge_backward_inputs": (C.c_int, [_PD, _PG, _PP, _PP, vp, _PS, vp, vp, vp, vp, vp, _PI, vp]),
+    "fegnn_node_pre_backward_inputs": (C.c_int, [_PD, _PP, _PP, vp, vp, vp, vp, vp, vp, vp, vp, _PI, vp]),
     "fegnn_halo_push": (C.c_int, [i32, vp, vp, vp, vp, vp, vp]),
     "fegnn_halo_reduce_push": (C.c_int, [i32, i32, vp, vp, vp, vp, vp]),
     "fegnn_halo_push_signal": (C.c_int, [C.POINTER(P2P), i32, i32, vp, i32, vp, vp, vp, vp, vp]),
@@ -147,6 +157,7 @@ SIGNATURES = {
     "fegnn_model_inference_workspace_floats": (C.c_size_t, [_PD]),
     "fegnn_model_forward_inference": (C.c_int, [_PD, i32, i32, _PG, _PP] + [vp] * 9 + [vp, C.c_size_t, vp]),
     "fegnn_model_backward": (C.c_int, [_PD, i32, i32, _PG, _PP, _PP] + [vp] * 11 + [vp, vp, C.c_size_t, vp]),
+    "fegnn_model_backward_inputs": (C.c_int, [_PD, i32, i32, _PG, _PP, _PP] + [vp] * 11 + [vp, vp, C.c_size_t, _PI, vp]),
     "fegnn_peak_probe": (C.c_int, [i32, i32, vp, C.POINTER(C.c_double), vp]),
     "fegnn_segment_reduce": (C.c_int, [C.c_int64, i32, i32, vp, vp, i32, vp, vp, vp]),
     "fegnn_segment_reduce_backward": (C.c_int, [C.c_int64, i32, i32, vp, vp, vp, vp, vp]),

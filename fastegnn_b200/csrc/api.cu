@@ -26,6 +26,7 @@
 #include "dense_tc.cu"
 #include "segment.cu"
 #include "peak_probe.cu"
+#include "input_grads.cu"
 
 using namespace fegnn;
 
@@ -122,6 +123,23 @@ int check_dims(const fegnn_dims* d) {
   return 0;
 }
 
+// Requested input gradients (fegnn_input_grads): refused before any launch where the layer has no such input or the
+// selected kernel cannot form the gradient.  The edge_attr gradient needs gz1, which only the fp32 kernel (mode 0) and the
+// packed-fp16 kernel with 256 threads per tile (mode 7, and 6 = auto) form it from; auto then picks 7 where it applies,
+// else 0.  The environment-only tensor-core forms (1, 2, 4, 5, 8) refuse a request.
+int check_input_grads(const fegnn_dims* d, const fegnn_input_grads* ig) {
+  if (ig == nullptr) return 0;
+  if (ig->node_attr != nullptr && d->Fa == 0) return fail(FEGNN_EINVAL, "node_attr gradient requested with Fa = 0");
+  if (ig->edge_attr != nullptr && d->Fe == 0) return fail(FEGNN_EINVAL, "edge_attr gradient requested with Fe = 0");
+  if (ig->node_vel != nullptr && (d->flags & FEGNN_F_RF))
+    return fail(FEGNN_EINVAL, "node_vel gradient requested on FEGNN_F_RF layers (v enters through |v|; not implemented)");
+  const bool tc_ok = d->Fe <= kTcMaxFe && !(d->flags & FEGNN_F_ATTENTION);
+  const int m = g_edge_bwd_mode;
+  if (ig->edge_attr != nullptr && tc_ok && m != 0 && m != 6 && m != 7)
+    return fail(FEGNN_EINVAL, "edge_backward mode %d has no edge_attr gradient (modes 0, 6 = auto and 7 have)", m);
+  return 0;
+}
+
 inline size_t al4(size_t n) { return (n + 3) & ~(size_t)3; }
 // Zero two float buffers with ONE memset node when they are neighbours in the caller's block (the model driver's
 // workspaces place them so; padding between 16-byte aligned slots is owned by the block), else with two.
@@ -154,7 +172,7 @@ NodeAttrArgs node_attr_args(const fegnn_dims* d, const float* w0, float* gw0) {
 EdgeArgs edge_args(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
                    const fegnn_layer_saved* sv) {
   EdgeArgs a;
-  memset(&a, 0, sizeof(a));
+  memset(&a, 0, sizeof(a));   // msum / tsum share their slots with the backward's g_ea / perm (EdgeArgs): set per direction
   a.N = d->N; a.Nl = d->Nl; a.E = d->E; a.Fe = d->Fe; a.ld1 = ld1(d); a.flags = d->flags; a.eps = d->eps;
   a.row = g->row; a.col = g->col; a.ea = g->edge_attr; a.x = x; a.P = sv->P; a.Q = sv->Q;
   a.w1 = p->edge_w0; a.W2 = p->edge_w2; a.b2 = p->edge_b2; a.W3 = p->cr_w0; a.b3 = p->cr_b0; a.w4 = p->cr_w2;
@@ -576,9 +594,18 @@ int fegnn_virtual_backward(const fegnn_dims* d, const fegnn_graph* g, const fegn
                            const fegnn_layer_saved* sv, const float* gx_new, const float* gxsum_next,
                            const float* gDsum, const float* gUsum, const float* gu, float* gAv, float* gG1, float* gx,
                            float* gZ, float* gsv, float* gsg, float* gt, void* stream) {
+  return fegnn_virtual_backward_inputs(d, g, p, gr, x, v, Z, sv, gx_new, gxsum_next, gDsum, gUsum, gu, gAv, gG1, gx, gZ, gsv,
+                                       gsg, gt, nullptr, stream);
+}
+int fegnn_virtual_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
+                                  fegnn_layer_grads* gr, const float* x, const float* v, const float* Z,
+                                  const fegnn_layer_saved* sv, const float* gx_new, const float* gxsum_next,
+                                  const float* gDsum, const float* gUsum, const float* gu, float* gAv, float* gG1, float* gx,
+                                  float* gZ, float* gsv, float* gsg, float* gt, const fegnn_input_grads* ig, void* stream) {
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
+  TRY(check_input_grads(d, ig));
   RQ(g && gr && x && v && Z && sv && gx_new && gDsum && gAv && gG1 && gx && gZ && gsv && gt);
   RQ(!(d->flags & FEGNN_F_GRAVITY) || gsg);
   VirtArgs a = virt_args(d, g, p, x, v, Z, sv);
@@ -599,15 +626,23 @@ int fegnn_virtual_backward(const fegnn_dims* d, const fegnn_graph* g, const fegn
   } else {
     CK(launch_virtual_bwd(a, sm_count(), S(stream)));
   }
+  if (ig != nullptr && ig->node_vel != nullptr)
+    CK(launch_input_grad_vel(d->N, sv->sv, gx_new, gxsum_next, g->batch, ig->node_vel, S(stream)));
   return 0;
 }
 
 int fegnn_edge_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, fegnn_layer_grads* gr,
                         const float* x, const fegnn_layer_saved* sv, const float* gm, const float* gt, float* gP,
                         float* gQ, float* gx, void* stream) {
+  return fegnn_edge_backward_inputs(d, g, p, gr, x, sv, gm, gt, gP, gQ, gx, nullptr, stream);
+}
+int fegnn_edge_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, fegnn_layer_grads* gr,
+                               const float* x, const fegnn_layer_saved* sv, const float* gm, const float* gt, float* gP,
+                               float* gQ, float* gx, const fegnn_input_grads* ig, void* stream) {
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
+  TRY(check_input_grads(d, ig));
   RQ(g && gr && x && sv && gt && gP && gQ && gx);
   EdgeArgs a = edge_args(d, g, p, x, sv);
   a.gm = gm; a.gt = gt; a.gP = gP; a.gQ = gQ; a.gx = gx;
@@ -620,6 +655,18 @@ int fegnn_edge_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_l
   if (mode == 6) mode = (tc_ok && sv->scratch != nullptr) ? 7 : 4;      // auto: the packed-fp16 kernel wherever it applies
   if ((mode == 7 || mode == 8) && (!tc_ok || sv->scratch == nullptr)) mode = 4;
   const bool pre = !(d->flags & FEGNN_F_STATS_READY);      // the bound pre-pass (its statistics came with the layer's other phases)
+  if (ig != nullptr && ig->edge_attr != nullptr) {
+    // dL/d edge_attr: the kEa instantiations (modes checked above); the output rides in the slots the forward uses for
+    // msum / tsum, so the argument block is the default one's
+    a.g_ea = ig->edge_attr;
+    a.perm = ig->perm;
+    if (tc_ok && sv->scratch != nullptr && mode == 7) {
+      CK((launch_edge_bwd_tc4<2, true>(a, reinterpret_cast<unsigned*>(sv->scratch), sm_count(), S(stream), zero && pre, pre)));
+    } else {
+      CK(launch_edge_bwd<true>(a, sm_count(), S(stream)));
+    }
+    return 0;
+  }
   if (mode == 7) CK(launch_edge_bwd_tc4<2>(a, reinterpret_cast<unsigned*>(sv->scratch), sm_count(), S(stream), zero && pre, pre));
   else if (mode == 8) CK(launch_edge_bwd_tc4<4>(a, reinterpret_cast<unsigned*>(sv->scratch), sm_count(), S(stream), zero && pre, pre));
   else if (mode == 5 && tc_ok && sv->scratch != nullptr)
@@ -647,9 +694,17 @@ int fegnn_graph_pre_backward(const fegnn_dims* d, const fegnn_graph* g, const fe
 int fegnn_node_pre_backward(const fegnn_dims* d, const fegnn_layer_params* p, fegnn_layer_grads* gr, const float* h,
                             const float* gP, const float* gQ, const float* gAv, const float* gUh, const float* gsv,
                             const float* gsg, float* gh, void* stream) {
+  return fegnn_node_pre_backward_inputs(d, p, gr, h, gP, gQ, gAv, gUh, gsv, gsg, gh, nullptr, stream);
+}
+int fegnn_node_pre_backward_inputs(const fegnn_dims* d, const fegnn_layer_params* p, fegnn_layer_grads* gr, const float* h,
+                                   const float* gP, const float* gQ, const float* gAv, const float* gUh, const float* gsv,
+                                   const float* gsg, float* gh, const fegnn_input_grads* ig, void* stream) {
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
+  TRY(check_input_grads(d, ig));
+  // dL/da += gUh U1att: the last layer has no Uh (gUh == NULL) and adds nothing
+  const bool want_ga = ig != nullptr && ig->node_attr != nullptr && gUh != nullptr;
   RQ(gr && h && gP && gQ && gAv && gsv && gh);
   RQ(!(d->flags & FEGNN_F_GRAVITY) || gsg);
   NodePreArgs a = node_pre_args(d, p, h);
@@ -689,9 +744,10 @@ int fegnn_node_pre_backward(const fegnn_dims* d, const fegnn_layer_params* p, fe
     if (d->flags & FEGNN_F_GRAVITY)
       head(gsg, p->grav_w0, p->grav_b0, p->grav_w2, gr->grav_w0, gr->grav_b0, gr->grav_w2, gr->grav_b2);
     CK(launch_dense_bwd_tc(t, sm_count(), S(stream), attr ? &ab : nullptr));
-    return 0;
+  } else {
+    CK(launch_node_pre_bwd(a, sm_count(), S(stream), attr ? &at_ : nullptr));
   }
-  CK(launch_node_pre_bwd(a, sm_count(), S(stream), attr ? &at_ : nullptr));
+  if (want_ga) CK(launch_input_grad_attr(d->N, d->Fa, at_.ldn, at_.w, gUh, ig->node_attr, S(stream)));
   return 0;
 }
 
@@ -1097,8 +1153,18 @@ int fegnn_model_backward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegn
                          const float* gx_out, const float* gZ_out, float* g_x0, float* g_loc_mean,
                          float* g_node_feat, const float* workspace, float* scratch, size_t scratch_floats,
                          void* stream) {
+  return fegnn_model_backward_inputs(d, L, Fin, g, layers, grads, embed_w, g_embed_w, g_embed_b, g_vnf, node_feat, v, gx_out,
+                                     gZ_out, g_x0, g_loc_mean, g_node_feat, workspace, scratch, scratch_floats, nullptr, stream);
+}
+int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn_graph* g,
+                                const fegnn_layer_params* layers, fegnn_layer_grads* grads, const float* embed_w,
+                                float* g_embed_w, float* g_embed_b, float* g_vnf, const float* node_feat, const float* v,
+                                const float* gx_out, const float* gZ_out, float* g_x0, float* g_loc_mean,
+                                float* g_node_feat, const float* workspace, float* scratch, size_t scratch_floats,
+                                const fegnn_input_grads* ig, void* stream) {
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
+  TRY(check_input_grads(d, ig));
   RQ(L >= 1 && L <= 32 && g && layers && grads && embed_w && g_embed_w && g_embed_b && g_vnf && workspace && scratch);
   RQ(gx_out && gZ_out && g_x0 && g_loc_mean && d->Nl == d->N);
   if (scratch_floats < bwd_scratch_floats(d))
@@ -1110,6 +1176,12 @@ int fegnn_model_backward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegn
   bwd_scratch_bind(d, scratch, &s);
   const size_t N = d->N, B = d->B, C = d->C;
   CK(cudaMemsetAsync(s.gh, 0, sizeof(float) * kH * N, st));
+  // the requested input gradients are sums over layers: filled here, then every layer adds its term
+  if (ig != nullptr) {
+    if (ig->node_vel != nullptr) CK(cudaMemsetAsync(ig->node_vel, 0, sizeof(float) * 3 * N, st));
+    if (ig->node_attr != nullptr) CK(cudaMemsetAsync(ig->node_attr, 0, sizeof(float) * d->Fa * N, st));
+    if (ig->edge_attr != nullptr) CK(cudaMemsetAsync(ig->edge_attr, 0, sizeof(float) * d->Fe * (size_t)d->E, st));
+  }
   // [gG1 | gx] and [gP | gQ] exist twice: layer l accumulates into set `cur` while the side stream zero-fills the other set
   // (whose last readers, virtual_backward(l) and node_pre_backward(l + 1), lie before the fork) for layer l - 1 -- no fill
   // stands between two kernels of the main chain
@@ -1145,19 +1217,20 @@ int fegnn_model_backward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegn
                                   side));                                                   // side, under node_h_bwd
     if (!last) TRY(fegnn_node_h_backward(&dl, g, p, gr, sv, s.gh, s.gzh1, s.gm, s.gu, stream));
     JOIN(sd, st);
-    TRY(fegnn_virtual_backward(&dl, g, p, gr, w.x[l], v, w.Z[l], sv, gx_new, gxsum_next, s.gDsum,
-                               last ? nullptr : s.gUsum, s.gu, s.gAv, s.gG1[cur], s.gx[cur], s.gZ[cur],
-                               s.gsv, s.gsg, s.gt, stream));
+    TRY(fegnn_virtual_backward_inputs(&dl, g, p, gr, w.x[l], v, w.Z[l], sv, gx_new, gxsum_next, s.gDsum,
+                                      last ? nullptr : s.gUsum, s.gu, s.gAv, s.gG1[cur], s.gx[cur], s.gZ[cur],
+                                      s.gsv, s.gsg, s.gt, ig, stream));
     FORK(sd, st);                                 // side: graph_pre_bwd(l) -> graph_post_bwd(l-1), under edge_bwd, node_pre_bwd
     TRY(fegnn_graph_pre_backward(&dl, g, p, gr, w.Sx[ls], sv, s.gG1[cur], s.gS[cur], s.gZ[cur], s.gxsum[cur], side));
     if (l > 0) {                                  // side: the other set, for layer l - 1
       CK(cudaMemsetAsync(s.gG1[cur ^ 1], 0, sizeof(float) * s.set_a_floats, S(side)));
       CK(cudaMemsetAsync(s.gP[cur ^ 1], 0, sizeof(float) * s.set_b_floats, S(side)));
     }
-    TRY(fegnn_edge_backward(&dl, g, p, gr, w.x[l], sv, last ? nullptr : s.gm, s.gt, s.gP[cur], s.gQ[cur], s.gx[cur], stream));
+    TRY(fegnn_edge_backward_inputs(&dl, g, p, gr, w.x[l], sv, last ? nullptr : s.gm, s.gt, s.gP[cur], s.gQ[cur], s.gx[cur],
+                                   ig, stream));
     if (rf) TRY(fegnn_rf_vel_backward(d->N, v, p, gr, s.gsv, stream));
-    TRY(fegnn_node_pre_backward(&dl, p, gr, w.h[ls], s.gP[cur], s.gQ[cur], s.gAv, last ? nullptr : s.gzh1, s.gsv, s.gsg, s.gh,
-                                stream));
+    TRY(fegnn_node_pre_backward_inputs(&dl, p, gr, w.h[ls], s.gP[cur], s.gQ[cur], s.gAv, last ? nullptr : s.gzh1, s.gsv, s.gsg,
+                                       s.gh, ig, stream));
     gx_new = s.gx[cur]; gZ_new = s.gZ[cur]; gS_new = s.gS[cur]; gxsum_next = s.gxsum[cur];
     cur ^= 1;
   }

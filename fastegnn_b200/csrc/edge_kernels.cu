@@ -18,8 +18,11 @@ struct EdgeArgs {
   const int *row, *col;
   const float *ea, *x, *P, *Q;
   const float *w1, *W2, *b2, *W3, *b3, *w4, *wa, *ba;   // w1 = edge_mlp.0.weight (for wq / Wa columns)
-  // forward outputs
-  float *msum, *tsum;
+  // forward outputs.  The backward writes neither: its edge_attr-gradient instantiations (kEa) take their output and the
+  // CSR -> caller edge order map in the same two slots, so the default backward launches keep their argument block.
+  // A backward kernel must never read msum / tsum (it would get g_ea / perm), nor a forward kernel g_ea / perm.
+  union { float* msum; float* g_ea; };       // g_ea: [E,Fe] dL/d edge_attr in the caller's order, += (one owner per edge)
+  union { float* tsum; const int* perm; };   // perm: [E] caller index of CSR edge e, or nullptr (CSR order is the caller's)
   // backward inputs / outputs
   const float *gm, *gt;
   float *gP, *gQ, *gx;
@@ -194,6 +197,8 @@ __global__ void __launch_bounds__(kThreads, 2) edge_fwd_kernel(EdgeArgs a) {
   }
 }
 
+// kEa: also g_ea[perm[e]][f] += sum_k gz1[e][k] Wa[f][k] (edge_attr enters phi_e's first Linear only)
+template <bool kEa>
 __global__ void __launch_bounds__(kThreads, 1) edge_bwd_kernel(EdgeArgs a) {
   extern __shared__ __align__(16) float smem[];
   float* W2s = smem;
@@ -375,6 +380,21 @@ __global__ void __launch_bounds__(kThreads, 1) edge_bwd_kernel(EdgeArgs a) {
         if (tail && r >= 0) atomicAdd(a.gx + (size_t)r * 3 + k, tot);
       }
     }
+    if constexpr (kEa) {
+      const int e = tile * kTM + tid;
+      if (tid < kTM && e < a.E) {
+        const float* gz = TD1 + tid * kH;
+        float* dst = a.g_ea + (size_t)(a.perm != nullptr ? a.perm[e] : e) * a.Fe;
+        for (int f = 0; f < a.Fe; ++f) {
+          float s = 0.f;
+          for (int j = 0; j < kH; ++j) {
+            const int k = (j + tid) & (kH - 1);        // rotated start: the 128 row walks hit different banks
+            s = fmaf(gz[k], v->Wa[f * kH + k], s);
+          }
+          dst[f] += s;
+        }
+      }
+    }
   }
   // ---- per-CTA weight-gradient partials -> reference-layout gradients
   wgrad_flush(wgW3, a.g_W3, kH, 0, 1);
@@ -408,17 +428,18 @@ cudaError_t launch_edge_fwd(const EdgeArgs& a, int sms, cudaStream_t st) {
   edge_fwd_kernel<<<grid, kThreads, kEdgeFwdSmem, st>>>(a); ++g_launches;
   return cudaGetLastError();
 }
+template <bool kEa = false>
 cudaError_t launch_edge_bwd(const EdgeArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(edge_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEdgeBwdSmem);
+    cudaError_t e = cudaFuncSetAttribute(edge_bwd_kernel<kEa>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEdgeBwdSmem);
     if (e != cudaSuccess) return e;
     attr.set();
   }
   int ntiles = (a.E + kTM - 1) / kTM;
   if (ntiles == 0) return cudaSuccess;
   int grid = ntiles < sms ? ntiles : sms;
-  edge_bwd_kernel<<<grid, kThreads, kEdgeBwdSmem, st>>>(a); ++g_launches;
+  edge_bwd_kernel<kEa><<<grid, kThreads, kEdgeBwdSmem, st>>>(a); ++g_launches;
   return cudaGetLastError();
 }
 

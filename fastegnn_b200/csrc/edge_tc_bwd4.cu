@@ -159,7 +159,11 @@ __device__ __forceinline__ float pow2_to(float bound, int e_target) {   // large
   return ldexpf(1.f, e);
 }
 
-template <int CG>
+// kEa: also g_ea[perm[e]][f] += gz1[e] . Wa_f (edge_attr enters phi_e's first Linear only), from the fp16 gz1 values of
+// epilogue 4 and the packed 0.5 Wa of the assembly, widened to fp32 and accumulated in fp32.  The per-column-group partials
+// go to T3, which holds nothing between the dw4 GEMM (waited in epilogue 3) and the next tile's assembly; the edge's owning
+// thread sums them in the tail.
+template <int CG, bool kEa>
 __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, const unsigned* stats) {
   VTR_DECL();
   constexpr int NTG = 128 * CG, NT = 2 * NTG, CPT = kH / CG, NP = CPT / 2, NWG = NTG / 32, RPW = kTM / NWG;
@@ -607,6 +611,23 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
       }
       store_row<NP>(TM, row, cg, pd);
       v->sgqp[cg * kTM + row] = gq;
+      if constexpr (kEa) {
+        float* sge = reinterpret_cast<float*>(T3);
+        for (int f = 0; f < a.Fe; ++f) {
+          float ge = 0.f;
+#pragma unroll
+          for (int j = 0; j < NP; j += 4) {
+            const uint4 w = *reinterpret_cast<const uint4*>(sv->hWah + f * (kH / 2) + (c0 >> 1) + j);
+            const uint32_t wa4[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+              const float2 g2 = __half22float2(u2h(pd[j + k])), w2 = __half22float2(u2h(wa4[k]));
+              ge = fmaf(g2.x, w2.x, fmaf(g2.y, w2.y, ge));
+            }
+          }
+          sge[(f * CG + cg) * kTM + row] = ge;
+        }
+      }
     }
     umma::fence_smem_to_async();
     umma::fence_before();
@@ -677,6 +698,18 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
         for (int k = 0; k < 3; ++k) atomicAdd(a.gx + (size_t)r * 3 + k, gd[k]);
       }
     }
+    if constexpr (kEa) {
+      if (tg < kTM && geo->srow[tg] >= 0) {
+        const int e = tile * kTM + tg;
+        float* dst = a.g_ea + (size_t)(a.perm != nullptr ? a.perm[e] : e) * a.Fe;
+        for (int f = 0; f < a.Fe; ++f) {
+          float ge = 0.f;
+#pragma unroll
+          for (int g = 0; g < CG; ++g) ge += reinterpret_cast<const float*>(T3)[(f * CG + g) * kTM + tg];
+          dst[f] += ge * (2.f * r1);               // gz1 is stored times s1, hWah holds Wa / 2
+        }
+      }
+    }
     VTR();
   }
   // ---- flush: each group waits for its last aux GEMM; then the whole CTA meets and group 0's warps read BOTH groups'
@@ -741,13 +774,13 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
 }  // namespace bwd4
 
 // stats: 4 unsigned of caller scratch (device)
-template <int CG>
+template <int CG, bool kEa = false>
 inline cudaError_t launch_edge_bwd_tc4(const EdgeArgs& a, unsigned* stats, int sms, cudaStream_t st, bool zero_stats = true,
                                        bool run_stats = true) {
   static DevOnce attr;
   const size_t bytes = bwd4::Smem4<CG>::bytes;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(bwd4::edge_bwd_tc4_kernel<CG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    cudaError_t e = cudaFuncSetAttribute(bwd4::edge_bwd_tc4_kernel<CG, kEa>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
     attr.set();
   }
@@ -766,7 +799,7 @@ inline cudaError_t launch_edge_bwd_tc4(const EdgeArgs& a, unsigned* stats, int s
     e = launch_pdl(bwd3::edge_bwd_stats_kernel, sblocks, 256, 0, st, a.N, a.Nl, a.x, a.gt, a.gm, stats);
     if (e != cudaSuccess) return e;
   }
-  e = launch_pdl(bwd4::edge_bwd_tc4_kernel<CG>, grid, 256 * CG, bytes, st, a, (const unsigned*)stats);
+  e = launch_pdl(bwd4::edge_bwd_tc4_kernel<CG, kEa>, grid, 256 * CG, bytes, st, a, (const unsigned*)stats);
   if (e != cudaSuccess) return e;
   return cudaGetLastError();
 }

@@ -40,9 +40,11 @@ class LayerPhases:
         with _on(self.dev):                      # the C ABI launches on the runtime's current device
             return self._forward(h, x, v, Z, S, xsum, hooks)
 
-    def backward(self, grads, h, x, v, Z, S, gh_new, gx_new, gZ_new, gS_new, gxsum_next, hooks=None, graph_grads=None):
+    def backward(self, grads, h, x, v, Z, S, gh_new, gx_new, gZ_new, gS_new, gxsum_next, hooks=None, graph_grads=None,
+                 input_grads: Optional[L.InputGrads] = None):
         with _on(self.dev):
-            return self._backward(grads, h, x, v, Z, S, gh_new, gx_new, gZ_new, gS_new, gxsum_next, hooks, graph_grads)
+            return self._backward(grads, h, x, v, Z, S, gh_new, gx_new, gZ_new, gS_new, gxsum_next, hooks, graph_grads,
+                                  input_grads)
 
     def _forward(self, h, x, v, Z, S, xsum, hooks=None):
         d, g, p, sv, st = self.d, self.g, self.p, self.saved, _stream(self.dev)
@@ -71,13 +73,15 @@ class LayerPhases:
 
     # ---- backward
     def _backward(self, grads: L.LayerPtrs, h, x, v, Z, S, gh_new, gx_new, gZ_new, gS_new, gxsum_next, hooks=None,
-                  graph_grads: Optional[L.LayerPtrs] = None):
+                  graph_grads: Optional[L.LayerPtrs] = None, input_grads: Optional[L.InputGrads] = None):
         """gh_new is consumed in place (becomes dL/dh).  Returns (gh, gx, gZ, gS, gxsum).
         graph_grads: weight-gradient table for the per-graph phases (replicated when partitioned, so
-        only one rank passes real pointers); defaults to `grads`."""
+        only one rank passes real pointers); defaults to `grads`.  input_grads: buffers the phases ADD this layer's
+        node_vel / node_attr / edge_attr gradients into (fegnn_input_grads), or None."""
         d, g, p, sv, st = self.d, self.g, self.p, self.saved, _stream(self.dev)
         N, Nl, B, Cc = d.N, d.Nl, d.B, d.C
         pd, pg, pp, ps, pgr = self.pd, C.byref(g.c), C.byref(p), C.byref(sv.c), C.byref(grads)
+        pig = None if input_grads is None else C.byref(input_grads)
         pgg = pgr if graph_grads is None else C.byref(graph_grads)
         gZ, gS = self._e(B, 3, Cc), self._e(B, Cc, L.H)
         gDsum, gUsum = self._e(B, 3, Cc), self._e(B, Cc, L.H)
@@ -95,21 +99,21 @@ class LayerPhases:
         gsv, gsg, gt = self._e(N), self._e(N), self._e(N, 3)
         # partitioned: the virtual phase adds only this rank's share of dZ -> keep it apart until it is all-reduced
         gZ_part = gZ if hooks is None else torch.zeros(B, 3, Cc, device=self.dev, dtype=torch.float32)
-        L.check(lib.fegnn_virtual_backward(pd, pg, pp, pgr, L.ptr(x), L.ptr(v), L.ptr(Z), ps, L.ptr(gx_new),
-                                           L.ptr(gxsum_next), L.ptr(gDsum), None if self.last else L.ptr(gUsum),
-                                           L.ptr(gu), L.ptr(gAv), L.ptr(gG1), L.ptr(gx), L.ptr(gZ_part), L.ptr(gsv),
-                                           L.ptr(gsg), L.ptr(gt), st), "virtual_backward")
+        L.check(lib.fegnn_virtual_backward_inputs(pd, pg, pp, pgr, L.ptr(x), L.ptr(v), L.ptr(Z), ps, L.ptr(gx_new),
+                                                  L.ptr(gxsum_next), L.ptr(gDsum), None if self.last else L.ptr(gUsum),
+                                                  L.ptr(gu), L.ptr(gAv), L.ptr(gG1), L.ptr(gx), L.ptr(gZ_part), L.ptr(gsv),
+                                                  L.ptr(gsg), L.ptr(gt), pig, st), "virtual_backward")
         gP = self._e(N, L.H)
-        L.check(lib.fegnn_edge_backward(pd, pg, pp, pgr, L.ptr(x), ps, L.ptr(gm), L.ptr(gt), L.ptr(gP), L.ptr(gQ),
-                                        L.ptr(gx), st), "edge_backward")
+        L.check(lib.fegnn_edge_backward_inputs(pd, pg, pp, pgr, L.ptr(x), ps, L.ptr(gm), L.ptr(gt), L.ptr(gP), L.ptr(gQ),
+                                               L.ptr(gx), pig, st), "edge_backward")
         if hooks is not None:
             hooks.after_edge_backward(self, gQ, gx, gG1, gZ_part)   # reverse halo (sum) + all-reduce of dG1 / dZ shares
             gZ.add_(gZ_part)
         gxsum = self._e(B, 3)
         L.check(lib.fegnn_graph_pre_backward(pd, pg, pp, pgg, L.ptr(S), ps, L.ptr(gG1), L.ptr(gS), L.ptr(gZ),
                                              L.ptr(gxsum), st), "graph_pre_backward")
-        L.check(lib.fegnn_node_pre_backward(pd, pp, pgr, L.ptr(h), L.ptr(gP), L.ptr(gQ), L.ptr(gAv), L.ptr(gzh1),
-                                            L.ptr(gsv), L.ptr(gsg), L.ptr(gh_new), st), "node_pre_backward")
+        L.check(lib.fegnn_node_pre_backward_inputs(pd, pp, pgr, L.ptr(h), L.ptr(gP), L.ptr(gQ), L.ptr(gAv), L.ptr(gzh1),
+                                                   L.ptr(gsv), L.ptr(gsg), L.ptr(gh_new), pig, st), "node_pre_backward")
         return gh_new, gx, gZ, gS, gxsum
 
 
@@ -120,10 +124,12 @@ def _layer_named(layer):
 class _LayerFn(torch.autograd.Function):
     """One layer through the phase calls, as a function of NAMED WEIGHT TENSORS (reference state_dict suffixes, any
     autograd history): E_GCL_vel.forward passes a layer's parameters; the VNEGNN sibling passes tensors it assembles from
-    its own parameters (fastegnn_b200/VNEGNN.py).  spec = (names, flag word, gravity list or None, virtual channels)."""
+    its own parameters (fastegnn_b200/VNEGNN.py).  spec = (names, flag word, gravity list or None, virtual channels).
+    node_attr is the fp32 copy the kernels read; attr_in / edge_attr_in are the caller's node_attr / edge_attr tensors (or
+    None), inputs only so that autograd hands them their gradients (the kernels read edge_attr from the graph)."""
 
     @staticmethod
-    def forward(ctx, spec, graph, node_attr, h, x, v, Z, S, *params):
+    def forward(ctx, spec, graph, node_attr, attr_in, edge_attr_in, h, x, v, Z, S, *params):
         names, flags, grav, Cc = spec
         L.deterministic("the FastEGNN layer", L.NO_DET_LAYERS)
         dev = x.device
@@ -141,6 +147,7 @@ class _LayerFn(torch.autograd.Function):
         ctx.node_attr = node_attr          # ph.d points at it until the backward
         ctx.save_for_backward(h, x, v, Z, S, *params)
         ctx.names = names
+        ctx.in_dtypes = (None if attr_in is None else attr_in.dtype, None if edge_attr_in is None else edge_attr_in.dtype)
         return h_new, x_new, S_new, Z_new
 
     @staticmethod
@@ -154,22 +161,36 @@ class _LayerFn(torch.autograd.Function):
         gx_new, gS_new, gZ_new = z(gx_new, x), z(gS_new, S), z(gZ_new, Z)
         views = {n: torch.zeros_like(p) for n, p in zip(ctx.names, params)}
         gptrs = layer_ptrs(views, "")
-        gh, gx, gZ, gS, gxsum = ph.backward(gptrs, h, x, v, Z, S, gh_new, gx_new, gZ_new, gS_new, None)
+        need = ctx.needs_input_grad
+        zf = lambda *shape: torch.zeros(*shape, device=x.device, dtype=torch.float32)      # the phases add into these
+        g_na = zf(ph.d.N, ph.d.Fa) if need[3] else None
+        g_ea = zf(ph.g.E, ph.g.Fe) if need[4] else None
+        g_v = zf(ph.d.N, 3) if need[7] else None
+        ig = None
+        if g_na is not None or g_ea is not None or g_v is not None:
+            ig = L.InputGrads(L.ptr(g_v), L.ptr(g_na), L.ptr(g_ea) if ph.g.Fe else None, L.ptr(ph.g.perm))
+        gh, gx, gZ, gS, gxsum = ph.backward(gptrs, h, x, v, Z, S, gh_new, gx_new, gZ_new, gS_new, None, input_grads=ig)
         gx = gx + gxsum[ph.g.batch.long()]       # xbar of this layer comes from its own input coordinates
-        return (None, None, None, gh, gx, None, gZ, gS) + tuple(views[n] for n in ctx.names)
+        dt_na, dt_ea = ctx.in_dtypes
+        cast = lambda g, dt: None if g is None else g.to(dt)
+        return (None, None, None, cast(g_na, dt_na), cast(g_ea, dt_ea), gh, gx, g_v, gZ, gS) + \
+            tuple(views[n] for n in ctx.names)
 
 
-def layer_call(named, flags: int, gravity, virtual_channels: int, graph: CsrGraph, h, x, v, Z, S, *, node_attr=None):
+def layer_call(named, flags: int, gravity, virtual_channels: int, graph: CsrGraph, h, x, v, Z, S, *, node_attr=None,
+               attr_in=None, edge_attr_in=None):
     """(h', x', S', Z') of one layer from a dict of weight tensors keyed by the reference's state_dict suffixes
     (edge_mlp.0.weight, ...); S / S' in kernel layout [B,C,H].  Tensors must be contiguous fp32 CUDA.  node_attr: [N, Fa]
-    contiguous fp32 CUDA data (no gradient) or None; node_mlp.0.weight then has Fa more columns."""
+    contiguous fp32 CUDA tensor the kernels read, or None; node_mlp.0.weight then has Fa more columns.  attr_in /
+    edge_attr_in: the tensors node_attr and graph.edge_attr were made from, to receive gradients (None: no gradient)."""
     names = tuple(named.keys())
     spec = (names, int(flags), gravity, int(virtual_channels))
-    return _LayerFn.apply(spec, graph, node_attr, _f32(h), _f32(x), _f32(v), _f32(Z), _f32(S), *[named[n] for n in names])
+    return _LayerFn.apply(spec, graph, node_attr, attr_in, edge_attr_in, _f32(h), _f32(x), _f32(v), _f32(Z), _f32(S),
+                          *[named[n] for n in names])
 
 
 def layer_forward(layer, node_feat, edge_index, coord, node_vel, virtual_coord, virtual_node_feat, data_batch,
-                  edge_attr, node_attr=None):
+                  edge_attr, node_attr=None, attr_in=None):
     """E_GCL_vel.forward: returns (node_feat, coord, virtual_node_feat, virtual_coord) (:223)."""
     L.deterministic("E_GCL_vel", L.NO_DET_LAYERS)
     _require_cuda(coord, "coord")
@@ -182,5 +203,6 @@ def layer_forward(layer, node_feat, edge_index, coord, node_vel, virtual_coord, 
     grav = None if layer.gravity is None else [float(t) for t in layer.gravity.detach().cpu().tolist()]
     named = dict(_layer_named(layer))
     h_new, x_new, S_new, Z_new = layer_call(named, flags, grav, layer.virtual_channels, graph, node_feat, coord, node_vel,
-                                            virtual_coord, S.float(), node_attr=node_attr)
+                                            virtual_coord, S.float(), node_attr=node_attr, attr_in=attr_in,
+                                            edge_attr_in=edge_attr)
     return h_new, x_new, S_new.permute(0, 2, 1), Z_new

@@ -286,6 +286,41 @@ int fegnn_node_pre_backward(const fegnn_dims* d, const fegnn_layer_params* p, fe
                             const float* gsv, const float* gsg, float* gh /*[N,H] in: dL/dh' (residual), out: dL/dh*/,
                             void* stream);
 
+/* ------------------------------------------------------------------ gradients to the data inputs
+ * The reference's autograd reaches node_vel, node_attr and edge_attr (models/FastEGNN.py:104,142,159); these entries add
+ * those gradients.  A NULL member is not requested; when nothing is requested the _inputs forms run exactly the kernels
+ * of the plain forms, which are these entries called with NULL.
+ *   node_vel  [N,3]  : sum over layers of phi_v(h_i) dL/dx'_i (the layer adds phi_v(h) v to x, :142)
+ *   node_attr [N,Fa] : sum over the layers with a Uh block (all but the last) of dL/dUh_i U1att
+ *   edge_attr [E,Fe] : sum over layers of dL/dz1_e W1[:, 2H+1 ..] (edge_attr enters phi_e's first Linear only, :104), in
+ *                      the CALLER's edge order: row perm[e] receives CSR edge e (perm of fegnn_graph_prep), or CSR order
+ *                      when perm is NULL (fegnn_radius_graph_fill has no other order)
+ * The per-phase forms ADD (+=) their layer's term, one owner per element (no atomics); fegnn_model_backward_inputs fills
+ * the requested buffers.  Refused with FEGNN_EINVAL before any launch: node_attr with Fa == 0, edge_attr with Fe == 0,
+ * node_vel on FEGNN_F_RF layers (v enters FastRF through |v|), and edge_attr under an "edge_backward" mode whose kernel
+ * has no such term (1, 2, 4, 5, 8; modes 0, 6 = auto and 7 have it).  With edge_attr requested, auto and mode 7 take the
+ * fp32 kernel (mode 0) wherever the packed-fp16 kernel does not apply (attention, Fe > 4, no saved scratch).          */
+typedef struct fegnn_input_grads {
+  float* node_vel;       /* [N,3]  or NULL */
+  float* node_attr;      /* [N,Fa] or NULL */
+  float* edge_attr;      /* [E,Fe] or NULL */
+  const int32_t* perm;   /* [E] CSR edge -> caller edge, or NULL (CSR order) */
+} fegnn_input_grads;
+int fegnn_virtual_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
+                                  fegnn_layer_grads* gr, const float* x, const float* v, const float* Z,
+                                  const fegnn_layer_saved* sv, const float* gx_new, const float* gxsum_next,
+                                  const float* gDsum, const float* gUsum, const float* gu, float* gAv, float* gG1,
+                                  float* gx, float* gZ, float* gsv, float* gsg, float* gt,
+                                  const fegnn_input_grads* ig /*node_vel +=*/, void* stream);
+int fegnn_edge_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
+                               fegnn_layer_grads* gr, const float* x, const fegnn_layer_saved* sv, const float* gm,
+                               const float* gt, float* gP, float* gQ, float* gx,
+                               const fegnn_input_grads* ig /*edge_attr +=, perm*/, void* stream);
+int fegnn_node_pre_backward_inputs(const fegnn_dims* d, const fegnn_layer_params* p, fegnn_layer_grads* gr,
+                                   const float* h, const float* gP, const float* gQ, const float* gAv,
+                                   const float* gUh, const float* gsv, const float* gsg, float* gh,
+                                   const fegnn_input_grads* ig /*node_attr +=*/, void* stream);
+
 /* ------------------------------------------------------------------ halo exchange over peer memory
  * Multi-GPU form of the layer (one big graph in spatial slabs, fastegnn_b200/partitioned.py): a node is owned by one
  * rank; rows [N, Nl) of Q / x are copies of remote neighbours ("halo").  These two calls move the rows over NVLink
@@ -374,6 +409,13 @@ int fegnn_model_backward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegn
                          const float* gx_out /*[N,3]*/, const float* gZ_out /*[B,3,C]*/,
                          float* g_x0 /*[N,3]*/, float* g_loc_mean /*[B,3,C]*/, float* g_node_feat /*[N,Fin] or NULL*/,
                          const float* workspace, float* scratch, size_t scratch_floats, void* stream);
+/* fegnn_model_backward plus the requested input gradients (fegnn_input_grads above; the buffers are filled here) */
+int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn_graph* g,
+                                const fegnn_layer_params* layers_host, fegnn_layer_grads* grads_host /*[L]*/,
+                                const float* embed_w, float* g_embed_w, float* g_embed_b, float* g_virtual_node_feat,
+                                const float* node_feat, const float* v, const float* gx_out, const float* gZ_out,
+                                float* g_x0, float* g_loc_mean, float* g_node_feat, const float* workspace, float* scratch,
+                                size_t scratch_floats, const fegnn_input_grads* ig, void* stream);
 
 /* ------------------------------------------------------------------ MMD regulariser
  * utils/train.py:17-20,111-165 with the random sample made explicit:
