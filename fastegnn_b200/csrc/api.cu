@@ -90,6 +90,12 @@ int g_node_bwd_mode = 2;
 // "deterministic" (fegnn_set_mode): 1 = bit-reproducible forms of the entries that have one; every entry that sums floats
 // across CTAs in arrival order and has no such form refuses to run (NO_DET) instead of running nondeterministically
 int g_det = 0;
+// "layer_overlap" (fegnn_set_mode; environment FEGNN_LAYER_OVERLAP): in fegnn_model_backward_inputs each layer's virtual
+// backward runs on a second stream next to its edge backward (DESIGN 3.7) -- 2 = at every size, 1 = auto (default: where
+// it measured faster), 0 = never (the two one after the other)
+int g_layer_overlap = getenv("FEGNN_LAYER_OVERLAP") ? atoi(getenv("FEGNN_LAYER_OVERLAP")) : 1;
+// SMs of the virtual backward in that arrangement (the edge backward gets the rest): 0 = its share of the layer's SM time
+const int g_overlap_vsms = getenv("FEGNN_OVERLAP_VSMS") ? atoi(getenv("FEGNN_OVERLAP_VSMS")) : 0;   // experiment switch
 constexpr int kNodeTcMinN = 0;
 inline bool node_bwd_tc(int N) { return g_node_bwd_mode == 1 || (g_node_bwd_mode == 2 && N >= kNodeTcMinN); }
 
@@ -257,9 +263,11 @@ namespace {
 
 // The per-graph phases run one CTA per graph.  fegnn_model_forward / backward put them on a second stream (fork / join
 // with events, all capturable) so they overlap the node- and edge-parallel kernels instead of idling 147 SMs.
+//
+// The backward's virtual branch (layer_overlap) runs on a third stream, `vst`, forked and joined with vfork / vjoin.
 struct SideStream {
-  cudaStream_t st = nullptr;
-  cudaEvent_t fork = nullptr, join = nullptr, aux = nullptr;
+  cudaStream_t st = nullptr, vst = nullptr;
+  cudaEvent_t fork = nullptr, join = nullptr, aux = nullptr, vfork = nullptr, vjoin = nullptr;
 };
 SideStream* side_stream() {
   static SideStream per_dev[64];
@@ -271,6 +279,9 @@ SideStream* side_stream() {
     if (cudaEventCreateWithFlags(&s->fork, cudaEventDisableTiming) != cudaSuccess) return nullptr;
     if (cudaEventCreateWithFlags(&s->join, cudaEventDisableTiming) != cudaSuccess) return nullptr;
     if (cudaEventCreateWithFlags(&s->aux, cudaEventDisableTiming) != cudaSuccess) return nullptr;
+    if (cudaStreamCreateWithFlags(&s->vst, cudaStreamNonBlocking) != cudaSuccess) return nullptr;
+    if (cudaEventCreateWithFlags(&s->vfork, cudaEventDisableTiming) != cudaSuccess) return nullptr;
+    if (cudaEventCreateWithFlags(&s->vjoin, cudaEventDisableTiming) != cudaSuccess) return nullptr;
   }
   return s;
 }
@@ -322,6 +333,11 @@ int fegnn_set_mode(const char* phase, int mode) {
     g_det = mode;
     return 0;
   }
+  if (strcmp(phase, "layer_overlap") == 0) {
+    if (mode < 0 || mode > 2) return fail(FEGNN_EINVAL, "layer_overlap mode must be 0, 1 (auto) or 2");
+    g_layer_overlap = mode;
+    return 0;
+  }
   return fail(FEGNN_EINVAL, "unknown phase '%s'", phase);
 }
 int fegnn_get_mode(const char* phase) {
@@ -332,6 +348,7 @@ int fegnn_get_mode(const char* phase) {
   if (phase != nullptr && strcmp(phase, "virtual_forward") == 0) return g_virt_fwd_mode;
   if (phase != nullptr && strcmp(phase, "virtual_backward") == 0) return g_virt_bwd_mode;
   if (phase != nullptr && strcmp(phase, "deterministic") == 0) return g_det;
+  if (phase != nullptr && strcmp(phase, "layer_overlap") == 0) return g_layer_overlap;
   return -1;
 }
 
@@ -597,16 +614,24 @@ int fegnn_virtual_backward(const fegnn_dims* d, const fegnn_graph* g, const fegn
   return fegnn_virtual_backward_inputs(d, g, p, gr, x, v, Z, sv, gx_new, gxsum_next, gDsum, gUsum, gu, gAv, gG1, gx, gZ, gsv,
                                        gsg, gt, nullptr, stream);
 }
-int fegnn_virtual_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
-                                  fegnn_layer_grads* gr, const float* x, const float* v, const float* Z,
-                                  const fegnn_layer_saved* sv, const float* gx_new, const float* gxsum_next,
-                                  const float* gDsum, const float* gUsum, const float* gu, float* gAv, float* gG1, float* gx,
-                                  float* gZ, float* gsv, float* gsg, float* gt, const fegnn_input_grads* ig, void* stream) {
+// the virtual backward runs on its two tensor-core kernels (else on the fp32 kernel)
+static bool virt_bwd_tc(const fegnn_dims* d, const float* gu) {
+  return g_virt_bwd_mode == 1 && !(d->flags & FEGNN_F_ATTENTION) && gu != nullptr;
+}
+// gt_ahead: gt and its bound statistics were formed by launch_virtual_bwd_gt (fegnn_model_backward_inputs, layer_overlap;
+// tensor-core kernels only), which the heads kernel then skips.  cap: grid cap of the tensor-core kernels.
+static int virtual_backward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
+                                fegnn_layer_grads* gr, const float* x, const float* v, const float* Z,
+                                const fegnn_layer_saved* sv, const float* gx_new, const float* gxsum_next,
+                                const float* gDsum, const float* gUsum, const float* gu, float* gAv, float* gG1, float* gx,
+                                float* gZ, float* gsv, float* gsg, float* gt, const fegnn_input_grads* ig, bool gt_ahead,
+                                int cap, void* stream) {
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   TRY(check_input_grads(d, ig));
   RQ(g && gr && x && v && Z && sv && gx_new && gDsum && gAv && gG1 && gx && gZ && gsv && gt);
+  RQ(!gt_ahead || virt_bwd_tc(d, gu));
   RQ(!(d->flags & FEGNN_F_GRAVITY) || gsg);
   VirtArgs a = virt_args(d, g, p, x, v, Z, sv);
   a.gx_new = gx_new; a.gxsum_next = gxsum_next; a.gDsum = gDsum; a.gUsum = gUsum; a.gu = gu;
@@ -618,11 +643,12 @@ int fegnn_virtual_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, con
   if (!(d->flags & FEGNN_F_PREZEROED)) CK(zero_pair(gG1, kH * d->C * (size_t)d->B, gx, 3 * (size_t)d->Nl, S(stream)));
   // tensor-core form: two kernels; `gu` doubles as the [N,C,H] scratch that carries the total dL/du between them
   if (d->flags & FEGNN_F_LAST) a.gu = nullptr;        // last layer: phi_h is discarded, a gu buffer holds no input
-  if (g_virt_bwd_mode == 1 && !(d->flags & FEGNN_F_ATTENTION) && gu != nullptr) {
+  if (virt_bwd_tc(d, gu)) {
     a.gu_work = const_cast<float*>(gu);
     a.u = sv->u;                                       // the heads are recomputed from the saved u
     a.stats = reinterpret_cast<unsigned*>(sv->scratch);   // max|gt|, max|x - x_0| for the edge backward (FEGNN_F_STATS_READY)
-    CK(launch_virtual_bwd_tc<4>(a, sm_count(), S(stream)));
+    if (gt_ahead) { a.gt = nullptr; a.stats = nullptr; }
+    CK(launch_virtual_bwd_tc<4>(a, cap, S(stream)));
   } else {
     CK(launch_virtual_bwd(a, sm_count(), S(stream)));
   }
@@ -630,15 +656,24 @@ int fegnn_virtual_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, con
     CK(launch_input_grad_vel(d->N, sv->sv, gx_new, gxsum_next, g->batch, ig->node_vel, S(stream)));
   return 0;
 }
+int fegnn_virtual_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
+                                  fegnn_layer_grads* gr, const float* x, const float* v, const float* Z,
+                                  const fegnn_layer_saved* sv, const float* gx_new, const float* gxsum_next,
+                                  const float* gDsum, const float* gUsum, const float* gu, float* gAv, float* gG1, float* gx,
+                                  float* gZ, float* gsv, float* gsg, float* gt, const fegnn_input_grads* ig, void* stream) {
+  return virtual_backward_run(d, g, p, gr, x, v, Z, sv, gx_new, gxsum_next, gDsum, gUsum, gu, gAv, gG1, gx, gZ, gsv, gsg, gt,
+                              ig, false, sm_count(), stream);
+}
 
 int fegnn_edge_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, fegnn_layer_grads* gr,
                         const float* x, const fegnn_layer_saved* sv, const float* gm, const float* gt, float* gP,
                         float* gQ, float* gx, void* stream) {
   return fegnn_edge_backward_inputs(d, g, p, gr, x, sv, gm, gt, gP, gQ, gx, nullptr, stream);
 }
-int fegnn_edge_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, fegnn_layer_grads* gr,
-                               const float* x, const fegnn_layer_saved* sv, const float* gm, const float* gt, float* gP,
-                               float* gQ, float* gx, const fegnn_input_grads* ig, void* stream) {
+// claim: NULL (static tile split) or a zeroed word from which the packed-fp16 kernels claim their tiles; cap: their grid cap
+static int edge_backward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, fegnn_layer_grads* gr,
+                             const float* x, const fegnn_layer_saved* sv, const float* gm, const float* gt, float* gP,
+                             float* gQ, float* gx, const fegnn_input_grads* ig, unsigned* claim, int cap, void* stream) {
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
@@ -661,14 +696,14 @@ int fegnn_edge_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const 
     a.g_ea = ig->edge_attr;
     a.perm = ig->perm;
     if (tc_ok && sv->scratch != nullptr && mode == 7) {
-      CK((launch_edge_bwd_tc4<2, true>(a, reinterpret_cast<unsigned*>(sv->scratch), sm_count(), S(stream), zero && pre, pre)));
+      CK((launch_edge_bwd_tc4<2, true>(a, reinterpret_cast<unsigned*>(sv->scratch), cap, S(stream), zero && pre, pre, claim)));
     } else {
       CK(launch_edge_bwd<true>(a, sm_count(), S(stream)));
     }
     return 0;
   }
-  if (mode == 7) CK(launch_edge_bwd_tc4<2>(a, reinterpret_cast<unsigned*>(sv->scratch), sm_count(), S(stream), zero && pre, pre));
-  else if (mode == 8) CK(launch_edge_bwd_tc4<4>(a, reinterpret_cast<unsigned*>(sv->scratch), sm_count(), S(stream), zero && pre, pre));
+  if (mode == 7) CK(launch_edge_bwd_tc4<2>(a, reinterpret_cast<unsigned*>(sv->scratch), cap, S(stream), zero && pre, pre, claim));
+  else if (mode == 8) CK(launch_edge_bwd_tc4<4>(a, reinterpret_cast<unsigned*>(sv->scratch), cap, S(stream), zero && pre, pre, claim));
   else if (mode == 5 && tc_ok && sv->scratch != nullptr)
     CK(launch_edge_bwd_tc3(a, reinterpret_cast<unsigned*>(sv->scratch), sm_count(), S(stream), zero));
   else if (mode == 2 && tc_ok) CK(launch_edge_bwd_tc2<2>(a, sm_count(), S(stream)));
@@ -676,6 +711,11 @@ int fegnn_edge_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const 
   else if (mode == 1 && tc_ok) CK(launch_edge_bwd_tc(a, sm_count(), S(stream)));
   else CK(launch_edge_bwd(a, sm_count(), S(stream)));
   return 0;
+}
+int fegnn_edge_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, fegnn_layer_grads* gr,
+                               const float* x, const fegnn_layer_saved* sv, const float* gm, const float* gt, float* gP,
+                               float* gQ, float* gx, const fegnn_input_grads* ig, void* stream) {
+  return edge_backward_run(d, g, p, gr, x, sv, gm, gt, gP, gQ, gx, ig, nullptr, sm_count(), stream);
 }
 
 int fegnn_graph_pre_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
@@ -898,13 +938,14 @@ void model_ws_bind(const fegnn_dims* d, int L, float* base, ModelWs* w) {
 
 struct BwdScratch {
   float *gh, *gx[2], *gZ[2], *gS[2], *gxsum[2], *gDsum, *gUsum, *gzh1, *gm, *gu, *gAv, *gG1[2], *gsv, *gsg, *gt, *gP[2], *gQ[2];
-  size_t set_a_floats, set_b_floats;      // [gG1 | gx] and [gP | gQ] of one set, each contiguous (one zero-fill)
+  unsigned* claim[2];                     // the edge backward's tile counter (layer_overlap)
+  size_t set_a_floats, set_b_floats;      // [gG1 | gx] and [gP | gQ | claim] of one set, each contiguous (one zero-fill)
 };
 size_t bwd_scratch_floats(const fegnn_dims* d) {
   const size_t N = d->N, Nl = d->Nl, B = d->B, C = d->C;
   return al4(N * kH) + 2 * al4(Nl * 3) + 2 * al4(B * 3 * C) + 2 * al4(B * C * kH) + 2 * al4(B * 3) + al4(B * 3 * C) +
          al4(B * C * kH) + 2 * al4(N * kH) + al4(N * C * kH) + al4(N * kH) + 2 * al4(B * C * kH) + 2 * al4(N) +
-         al4(N * 3) + 2 * (al4(N * kH) + al4(Nl * kH));
+         al4(N * 3) + 2 * (al4(N * kH) + al4(Nl * kH) + 4);
 }
 void bwd_scratch_bind(const fegnn_dims* d, float* base, BwdScratch* s) {
   const size_t N = d->N, Nl = d->Nl, B = d->B, C = d->C;
@@ -920,8 +961,10 @@ void bwd_scratch_bind(const fegnn_dims* d, float* base, BwdScratch* s) {
   s->gzh1 = take(N * kH); s->gm = take(N * kH); s->gu = take(N * C * kH);
   s->gAv = take(N * kH);
   s->gsv = take(N); s->gsg = take(N); s->gt = take(N * 3);
-  for (int k = 0; k < 2; ++k) { s->gP[k] = take(N * kH); s->gQ[k] = take(Nl * kH); }        // set k: [gP | gQ] contiguous
-  s->set_b_floats = al4(N * kH) + Nl * kH;
+  for (int k = 0; k < 2; ++k) {                                                             // set k: [gP | gQ | claim]
+    s->gP[k] = take(N * kH); s->gQ[k] = take(Nl * kH); s->claim[k] = reinterpret_cast<unsigned*>(take(4));
+  }
+  s->set_b_floats = al4(N * kH) + al4(Nl * kH) + 4;
 }
 
 }  // namespace
@@ -1217,17 +1260,50 @@ int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, con
                                   side));                                                   // side, under node_h_bwd
     if (!last) TRY(fegnn_node_h_backward(&dl, g, p, gr, sv, s.gh, s.gzh1, s.gm, s.gu, stream));
     JOIN(sd, st);
-    TRY(fegnn_virtual_backward_inputs(&dl, g, p, gr, w.x[l], v, w.Z[l], sv, gx_new, gxsum_next, s.gDsum,
-                                      last ? nullptr : s.gUsum, s.gu, s.gAv, s.gG1[cur], s.gx[cur], s.gZ[cur],
-                                      s.gsv, s.gsg, s.gt, ig, stream));
-    FORK(sd, st);                                 // side: graph_pre_bwd(l) -> graph_post_bwd(l-1), under edge_bwd, node_pre_bwd
+    // layer_overlap: gt on this stream, then the virtual backward on `vst` next to the edge backward here (they share
+    // only gx, to which both add); vst is joined in front of node_pre_bwd, which reads gAv / gsv / gsg
+    // Auto: only where the virtual backward's tiles leave most of a second wave idle (more than one and at most 1.5 waves
+    // of one CTA per SM).  In one wave there is no idle wave to fill and the extra launch and events cost (N-body-5: +2 %
+    // per step); with more (N-body-100: 1.6 waves, protein batch: 6.9) both kernels fill the machine anyway and the split
+    // measured slower than one after the other (B200: +1.0 % / +1.9 %; config 5 at 1 M nodes -1.2 %; DESIGN 3.7).
+    const int vtiles = (d->N + kTM / d->C - 1) / (kTM / d->C);
+    const bool overlap = virt_bwd_tc(&dl, s.gu) &&
+                         (g_layer_overlap == 2 || (g_layer_overlap == 1 && vtiles > sm_count() && 2 * vtiles <= 3 * sm_count()));
+    void* vstream = overlap ? static_cast<void*>(sd->vst) : stream;
+    // Each kernel takes one CTA per SM and a whole SM's shared memory, so the two share the machine by SMs: the first
+    // launched would hold every SM it can fill.  The virtual backward gets `vsms` persistent CTAs, the edge backward the
+    // remaining SMs -- in proportion to their SM time (B200, Water-3D: one (node, channel) tile through the heads and trunk
+    // kernels costs about as much as 2.9 edge tiles; DESIGN 3.7).
+    int vsms = g_overlap_vsms;
+    if (overlap && vsms <= 0) {
+      const double wv = 2.9 * vtiles, we = (double)((d->E + kTM - 1) / kTM);
+      vsms = (int)(sm_count() * wv / (wv + we) + 0.5);
+    }
+    vsms = min(max(vsms, 1), sm_count() - 1);
+    if (overlap) {
+      VirtArgs ga = virt_args(&dl, g, p, w.x[l], v, w.Z[l], sv);
+      ga.gx_new = gx_new; ga.gxsum_next = gxsum_next; ga.gt = s.gt;
+      CK(launch_virtual_bwd_gt(ga, reinterpret_cast<unsigned*>(sv->scratch), st));
+      CK(cudaEventRecord(sd->vfork, st));                  // after gt: the set fills forked from vst below overwrite gx_new
+      CK(cudaStreamWaitEvent(sd->vst, sd->vfork, 0));
+    }
+    TRY(virtual_backward_run(&dl, g, p, gr, w.x[l], v, w.Z[l], sv, gx_new, gxsum_next, s.gDsum, last ? nullptr : s.gUsum, s.gu,
+                             s.gAv, s.gG1[cur], s.gx[cur], s.gZ[cur], s.gsv, s.gsg, s.gt, ig, overlap,
+                             overlap ? vsms : sm_count(), vstream));
+    // side: graph_pre_bwd(l) -> graph_post_bwd(l-1), under edge_bwd, node_pre_bwd
+    CK(cudaEventRecord(sd->fork, S(vstream)));
+    CK(cudaStreamWaitEvent(sd->st, sd->fork, 0));
     TRY(fegnn_graph_pre_backward(&dl, g, p, gr, w.Sx[ls], sv, s.gG1[cur], s.gS[cur], s.gZ[cur], s.gxsum[cur], side));
     if (l > 0) {                                  // side: the other set, for layer l - 1
       CK(cudaMemsetAsync(s.gG1[cur ^ 1], 0, sizeof(float) * s.set_a_floats, S(side)));
       CK(cudaMemsetAsync(s.gP[cur ^ 1], 0, sizeof(float) * s.set_b_floats, S(side)));
     }
-    TRY(fegnn_edge_backward_inputs(&dl, g, p, gr, w.x[l], sv, last ? nullptr : s.gm, s.gt, s.gP[cur], s.gQ[cur], s.gx[cur],
-                                   ig, stream));
+    TRY(edge_backward_run(&dl, g, p, gr, w.x[l], sv, last ? nullptr : s.gm, s.gt, s.gP[cur], s.gQ[cur], s.gx[cur], ig,
+                          overlap ? s.claim[cur] : nullptr, overlap ? sm_count() - vsms : sm_count(), stream));
+    if (overlap) {
+      CK(cudaEventRecord(sd->vjoin, sd->vst));
+      CK(cudaStreamWaitEvent(st, sd->vjoin, 0));
+    }
     if (rf) TRY(fegnn_rf_vel_backward(d->N, v, p, gr, s.gsv, stream));
     TRY(fegnn_node_pre_backward_inputs(&dl, p, gr, w.h[ls], s.gP[cur], s.gQ[cur], s.gAv, last ? nullptr : s.gzh1, s.gsv, s.gsg,
                                        s.gh, ig, stream));

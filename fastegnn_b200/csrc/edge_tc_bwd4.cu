@@ -128,6 +128,8 @@ struct GroupVec {
   float iea[kTM * kTcMaxFe];       // written and read by thread tg only
   float spart[CG * kTM], sgqp[CG * kTM], ss[kTM];
   uint64_t bar[6];
+  int qt[4];                       // this group's tiles: slot n & 3 holds its n-th (current, next, the one after)
+  int had;                         // the group processed a tile (its weight-gradient lanes are defined)
 };
 __device__ __forceinline__ void cp_async4(void* dst, const void* src) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" :: "r"(umma::smem_u32(dst)), "l"(src) : "memory");
@@ -163,8 +165,12 @@ __device__ __forceinline__ float pow2_to(float bound, int e_target) {   // large
 // epilogue 4 and the packed 0.5 Wa of the assembly, widened to fp32 and accumulated in fp32.  The per-column-group partials
 // go to T3, which holds nothing between the dw4 GEMM (waited in epilogue 3) and the next tile's assembly; the edge's owning
 // thread sums them in the tail.
+//
+// claim: NULL = static split (group G of CTA b takes tiles 2 b + G + n 2 gridDim.x); else a zeroed counter from which
+// each group takes its tiles one at a time, two ahead of the one it works on, so that a CTA that starts late (its SM held
+// by a kernel of another stream) takes what is left instead of a fixed share.
 template <int CG, bool kEa>
-__global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, const unsigned* stats) {
+__global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, const unsigned* stats, unsigned* claim) {
   VTR_DECL();
   constexpr int NTG = 128 * CG, NT = 2 * NTG, CPT = kH / CG, NP = CPT / 2, NWG = NTG / 32, RPW = kTM / NWG;
   using SM = Smem4<CG>;
@@ -285,11 +291,12 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
   const uint64_t dTMa = make_desc_h(umma::smem_u32(TM), kTileBytes);              // A = gz1 (after m is dead)
   const uint64_t dT3a = make_desc_h(umma::smem_u32(T3), kTileBytes);              // A = a3
   const uint64_t dAUX = make_desc_h(umma::smem_u32(AUX), kTileBytes);             // B = AUX, N = 8
-  uint32_t phase = 0;
   bool first_tile = true;
   const int l16 = lane & 15, hsel = lane >> 4;
 
-  const int ntiles = (a.E + kTM - 1) / kTM, tstride = gridDim.x * 2;
+  const int ntiles = (a.E + kTM - 1) / kTM;
+  // the tile after `prev` of this group (one thread per group asks; the answer goes through v->qt)
+  auto claim_tile = [&](int prev) { return claim != nullptr ? (int)atomicAdd(claim, 1u) : prev + (int)gridDim.x * 2; };
   // indices / edge attributes of tile `tl` -> this thread's landing slots (asynchronous; rows past E get row = -1)
   auto load_idx_async = [&](int tl) {
     const int e = tl * kTM + tg;
@@ -336,14 +343,23 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
     gg->sgte[tg * 3 + 0] = g0; gg->sgte[tg * 3 + 1] = g1; gg->sgte[tg * 3 + 2] = g2;
     gg->sgs[tg] = d0 * g0 + d1 * g1 + d2 * g2;
   };
-  int cur = 0;
-  if (tg < kTM && blockIdx.x * 2 + G < ntiles) {          // first tile: nothing to hide the gathers under
-    load_idx_async(blockIdx.x * 2 + G);
-    geometry(&v->geo[0]);
-    if (blockIdx.x * 2 + G + tstride < ntiles) load_idx_async(blockIdx.x * 2 + G + tstride);
+  if (tg == 0) {
+    v->qt[0] = claim != nullptr ? (int)atomicAdd(claim, 1u) : (int)blockIdx.x * 2 + G;
+    v->qt[1] = claim_tile(v->qt[0]);
   }
-  for (int tile = blockIdx.x * 2 + G; tile < ntiles; tile += tstride, cur ^= 1) {
-    const Geo* geo = &v->geo[cur];
+  group_sync();
+  if (tg < kTM && v->qt[0] < ntiles) {                   // first tile: nothing to hide the gathers under
+    load_idx_async(v->qt[0]);
+    geometry(&v->geo[0]);
+    if (v->qt[1] < ntiles) load_idx_async(v->qt[1]);
+  }
+  // k: this group's tile count; its tile is v->qt[k & 3] (the ids stay in shared memory: the kernel is at its register cap)
+  // the mbarrier phase of tile k is k & 1
+  int k = 0;
+  for (; v->qt[k & 3] < ntiles; ++k) {
+    const uint32_t phase = k & 1;
+    const Geo* geo = &v->geo[k & 1];
+    if (tg == 0) v->qt[(k + 2) & 3] = claim_tile(v->qt[(k + 1) & 3]);   // read after the group barriers below; its slot was last read in tile k - 1
     if (!first_tile) {                           // the previous tile's last GEMMs still read AUX, TM, TA, TG
       umma::mbar_wait(&v->bar[4], phase ^ 1);
     VTR();
@@ -432,9 +448,9 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
       __syncwarp();
     }
     // ---- under G1: geometry of the NEXT tile (its indices landed long ago), then the indices of the one after
-    if (tg < kTM && tile + tstride < ntiles) {
-      geometry(&v->geo[cur ^ 1]);
-      if (tile + 2 * tstride < ntiles) load_idx_async(tile + 2 * tstride);
+    if (tg < kTM && v->qt[(k + 1) & 3] < ntiles) {
+      geometry(&v->geo[(k & 1) ^ 1]);
+      if (v->qt[(k + 2) & 3] < ntiles) load_idx_async(v->qt[(k + 2) & 3]);
     }
     umma::mbar_wait(&v->bar[0], phase);
     VTR();
@@ -641,7 +657,6 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
       }
       __syncwarp();
     }
-    phase ^= 1;
     first_tile = false;
     // ---- gQ (by col) and gP (by row) from the fp16 gz1 tile: a half-warp owns RPW / 2 consecutive rows, 4 columns per
     //      lane; one vector red per row for gQ, one per row run for gP
@@ -700,7 +715,7 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
     }
     if constexpr (kEa) {
       if (tg < kTM && geo->srow[tg] >= 0) {
-        const int e = tile * kTM + tg;
+        const int e = v->qt[k & 3] * kTM + tg;
         float* dst = a.g_ea + (size_t)(a.perm != nullptr ? a.perm[e] : e) * a.Fe;
         for (int f = 0; f < a.Fe; ++f) {
           float ge = 0.f;
@@ -714,16 +729,17 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
   }
   // ---- flush: each group waits for its last aux GEMM; then the whole CTA meets and group 0's warps read BOTH groups'
   //      weight-gradient tiles (M = 64 layout: row n of group g in lane (n / 16) * 32 + n % 16 + 16 g)
-  if (!first_tile) umma::mbar_wait(&v->bar[4], phase ^ 1);
+  if (!first_tile) umma::mbar_wait(&v->bar[4], (k & 1) ^ 1);
     VTR();
+  if (tg == 0) v->had = first_tile ? 0 : 1;
   umma::fence_after();
   umma::fence_before();
   __syncthreads();
     VTR();
   umma::fence_after();
-  // a group that saw no tile left its accumulator lanes undefined: only groups with first_tile == false contribute.
-  // (blockIdx.x * 2 + G < ntiles decides that for every thread of the CTA without communication.)
-  const bool has0 = blockIdx.x * 2 + 0 < ntiles, has1 = blockIdx.x * 2 + 1 < ntiles;
+  // a group that saw no tile left its accumulator lanes undefined: only groups with a tile contribute
+  const bool has0 = reinterpret_cast<const GV*>(smem + SM::off_groups + SM::g_vec)->had != 0;
+  const bool has1 = reinterpret_cast<const GV*>(smem + SM::off_groups + SM::g_bytes + SM::g_vec)->had != 0;
   if (G == 0) {
     const int n = quarter * 16 + (lane & 15);
     const bool mine = (lane < 16) ? has0 : has1;
@@ -773,10 +789,11 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
 
 }  // namespace bwd4
 
-// stats: 4 unsigned of caller scratch (device)
+// stats: 4 unsigned of caller scratch (device); claim: NULL (static tile split) or a zeroed word (tiles claimed dynamically);
+// sms: the grid's cap
 template <int CG, bool kEa = false>
 inline cudaError_t launch_edge_bwd_tc4(const EdgeArgs& a, unsigned* stats, int sms, cudaStream_t st, bool zero_stats = true,
-                                       bool run_stats = true) {
+                                       bool run_stats = true, unsigned* claim = nullptr) {
   static DevOnce attr;
   const size_t bytes = bwd4::Smem4<CG>::bytes;
   if (!attr.get()) {
@@ -799,7 +816,7 @@ inline cudaError_t launch_edge_bwd_tc4(const EdgeArgs& a, unsigned* stats, int s
     e = launch_pdl(bwd3::edge_bwd_stats_kernel, sblocks, 256, 0, st, a.N, a.Nl, a.x, a.gt, a.gm, stats);
     if (e != cudaSuccess) return e;
   }
-  e = launch_pdl(bwd4::edge_bwd_tc4_kernel<CG, kEa>, grid, 256 * CG, bytes, st, a, (const unsigned*)stats);
+  e = launch_pdl(bwd4::edge_bwd_tc4_kernel<CG, kEa>, grid, 256 * CG, bytes, st, a, (const unsigned*)stats, claim);
   if (e != cudaSuccess) return e;
   return cudaGetLastError();
 }

@@ -773,8 +773,14 @@ __global__ void __launch_bounds__(128 * CG, 1) virtual_bwd_heads_tc_kernel(VirtA
           const float g = v->g.sgxn[t * 3 + k];
           float sum = 0.f;
           for (int c = 0; c < C; ++c) sum += v->g.sgD[(t * C + c) * 3 + k];
-          a.gx[(size_t)i * 3 + k] = g - sum;          // the trunk kernel subtracts the rho term
-          a.gt[(size_t)i * 3 + k] = g * di;
+          // gt == NULL: virtual_bwd_gt_kernel wrote gt, and the edge backward may be adding its row and col terms to the
+          // zeroed gx right now (fegnn_model_backward_inputs, "layer_overlap"), so this kernel and the trunk add too
+          if (a.gt != nullptr) {
+            a.gx[(size_t)i * 3 + k] = g - sum;        // the trunk kernel subtracts the rho term
+            a.gt[(size_t)i * 3 + k] = g * di;
+          } else {
+            atomicAdd(a.gx + (size_t)i * 3 + k, g - sum);
+          }
           if (a.stats != nullptr) {
             st_gt = fmaxf(st_gt, fabsf(g * di));
             st_x = fmaxf(st_x, fabsf(a.x[(size_t)i * 3 + k] - a.x[k]));
@@ -1189,7 +1195,8 @@ __global__ void __launch_bounds__(128 * CG, 1) virtual_bwd_trunk_tc_kernel(VirtA
         for (int k = 0; k < 3; ++k) {
           float sum = 0.f;
           for (int c = 0; c < C; ++c) sum += v->g.sgD[(t * C + c) * 3 + k];
-          a.gx[(size_t)i * 3 + k] -= sum;             // the heads kernel wrote g - (head terms)
+          if (a.gt != nullptr) a.gx[(size_t)i * 3 + k] -= sum;     // the heads kernel wrote g - (head terms)
+          else atomicAdd(a.gx + (size_t)i * 3 + k, -sum);            // layer_overlap (see the heads kernel)
         }
       }
     }
@@ -1254,8 +1261,10 @@ cudaError_t launch_virtual_fwd_tc(const VirtArgs& a, int sms, cudaStream_t st) {
 }  // namespace fegnn
 
 namespace fegnn {
+// grid = min(tiles, cap): cap = sms keeps one persistent CTA per SM; a larger cap leaves the extra tiles to the block
+// scheduler, which places them wherever an SM frees up (next to the edge backward on another stream)
 template <int CG>
-cudaError_t launch_virtual_bwd_tc(const VirtArgs& a, int sms, cudaStream_t st) {
+cudaError_t launch_virtual_bwd_tc(const VirtArgs& a, int cap, cudaStream_t st) {
   static DevOnce attr;
   if (!attr.get()) {
     cudaError_t e = cudaFuncSetAttribute(vtc::virtual_bwd_heads_tc_kernel<CG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -1269,11 +1278,55 @@ cudaError_t launch_virtual_bwd_tc(const VirtArgs& a, int sms, cudaStream_t st) {
   const int TN = kTM / a.C;
   const int ntiles = (a.N + TN - 1) / TN;
   if (ntiles == 0) return cudaSuccess;
-  const int grid = ntiles < sms ? ntiles : sms;
+  const int grid = ntiles < cap ? ntiles : cap;
   if (cudaError_t e_ = launch_pdl(vtc::virtual_bwd_heads_tc_kernel<CG>, grid, 128 * CG, vtc::HeadsSmem::bytes, st, a)) return e_;
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   if (cudaError_t e_ = launch_pdl(vtc::virtual_bwd_trunk_tc_kernel<CG>, grid, 128 * CG, vtc::TrunkSmem::bytes, st, a)) return e_;
+  return cudaGetLastError();
+}
+
+// gt = (dL/dx'_i + gxsum_next[batch_i]) dinv_i, the coordinate gradient the edge backward gathers by row: the heads kernel's
+// expression, formed ahead of the virtual backward so that the edge backward need not wait for it.  With `stats` it also
+// folds max|gt| and max|x - x_0| into stats[0] / stats[2] (the FEGNN_F_STATS_READY bounds): one atomicMax pair per CTA.
+// One thread per (node, component).  gx_new / gxsum_next come from the kernels ahead: plain loads after the wait.
+constexpr int kGtThreads = 256;
+__global__ void __launch_bounds__(kGtThreads) virtual_bwd_gt_kernel(int N, const float* __restrict__ x, const float* gx_new,
+                                                                   const float* gxsum_next, const int* __restrict__ batch,
+                                                                   const float* __restrict__ dinv, float* gt, unsigned* stats) {
+  __shared__ float red[2][kGtThreads / 32];
+  pdl_trigger();
+  pdl_wait();
+  const int idx = blockIdx.x * kGtThreads + threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  float mg = 0.f, mx = 0.f;
+  if (idx < N * 3) {
+    const int i = idx / 3, k = idx - i * 3;
+    float g = gx_new[idx];
+    if (gxsum_next != nullptr) g += gxsum_next[batch[i] * 3 + k];
+    g *= dinv != nullptr ? dinv[i] : 1.f;
+    gt[idx] = g;
+    mg = fabsf(g);
+    mx = fabsf(x[idx] - x[k]);
+  }
+  if (stats == nullptr) return;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    mg = fmaxf(mg, __shfl_xor_sync(0xffffffffu, mg, o));
+    mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  }
+  if (lane == 0) { red[0][warp] = mg; red[1][warp] = mx; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int w = 1; w < kGtThreads / 32; ++w) { mg = fmaxf(mg, red[0][w]); mx = fmaxf(mx, red[1][w]); }
+    atomicMax(stats + 0, __float_as_uint(mg));     // non-negative floats order like their bit patterns
+    atomicMax(stats + 2, __float_as_uint(mx));
+  }
+}
+inline cudaError_t launch_virtual_bwd_gt(const VirtArgs& a, unsigned* stats, cudaStream_t st) {
+  if (a.N == 0) return cudaSuccess;
+  if (cudaError_t e = launch_pdl(virtual_bwd_gt_kernel, (a.N * 3 + kGtThreads - 1) / kGtThreads, kGtThreads, 0, st, a.N, a.x,
+                                 a.gx_new, a.gxsum_next, a.batch, a.dinv, a.gt, stats))
+    return e;
   return cudaGetLastError();
 }
 }  // namespace fegnn

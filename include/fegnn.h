@@ -168,7 +168,12 @@ unsigned long long fegnn_launch_count(void);
  * the forwards take a workspace of fegnn_loss_workspace_floats.  fegnn_adam_step, fegnn_graph_prep and the radius graph are deterministic in either mode.
  * Every entry that adds floats across CTAs in arrival order and has no such form -- the layer phases, fegnn_model_*,
  * fegnn_embed_backward, fegnn_graph_xsum, fegnn_rf_vel_backward, fegnn_segment_reduce, fegnn_halo_reduce_push and
- * fegnn_p2p_allreduce -- returns FEGNN_EINVAL under 1, naming the reason, instead of running. */
+ * fegnn_p2p_allreduce -- returns FEGNN_EINVAL under 1, naming the reason, instead of running.
+ * "layer_overlap": 1 (default, auto), 2 or 0; the environment variable FEGNN_LAYER_OVERLAP sets the starting value.
+ * Under 2, fegnn_model_backward(_inputs) runs each layer's virtual backward on a second internal stream next to its edge
+ * backward (the edge backward's tiles are then claimed dynamically); under 0 the two run one after the other on `stream`;
+ * under 1 the first where the virtual backward has more than one and at most 1.5 waves of tiles (one CTA per SM), else
+ * the second.  Both arrangements run the same arithmetic; float sums are added in arrival order either way. */
 int fegnn_set_mode(const char* phase, int mode);
 int fegnn_get_mode(const char* phase);
 
