@@ -194,7 +194,8 @@ def _stack_inference(mod: "FastEGNN", graph: CsrGraph, node_attr, node_feat, x0,
                      node_attr=node_attr)
     pd = C.byref(dims)
     table, _ = mod._param_table()
-    ws_floats = int(lib.fegnn_model_inference_workspace_floats(pd))
+    # + the scratch of the deterministic kernels, behind it (0 with the mode off)
+    ws_floats = int(lib.fegnn_model_inference_workspace_floats(pd)) + int(lib.fegnn_model_inference_det_workspace_floats(pd))
     ws = torch.empty(ws_floats, device=dev, dtype=torch.float32)
     x_out = torch.empty(N, 3, device=dev, dtype=torch.float32)
     Z_out = torch.empty(B, 3, Cc, device=dev, dtype=torch.float32)
@@ -294,8 +295,13 @@ class FastEGNN(nn.Module):
         return flat, views, gtable
 
     # -- forward --------------------------------------------------------------------------
+    def _inference_route(self):
+        """True when forward takes the forward-only stack (no autograd graph)."""
+        return not torch.is_grad_enabled() or (not self.training and not self.eval_keeps_graph)
+
     def forward(self, node_feat, node_loc, node_vel, edge_index, data_batch, loc_mean, edge_attr=None, node_attr=None):
-        L.deterministic(type(self).__name__, L.NO_DET_LAYERS)
+        # the forward-only stack has deterministic forms of its kernels; the training forward and its backward have none
+        L.deterministic(type(self).__name__, None if self._inference_route() else L.NO_DET_LAYERS)
         attr_in = node_attr
         node_attr = node_attr_arg(node_attr, self._node_attr_nf, node_loc.size(0))
         _require_cuda(node_loc, "node_loc")
@@ -325,7 +331,7 @@ class FastEGNN(nn.Module):
         args = (node_feat.contiguous().float(), node_loc.contiguous().float(), node_vel.contiguous().float(),
                 loc_mean.contiguous().float())
         try:
-            if not torch.is_grad_enabled() or (not self.training and not self.eval_keeps_graph):
+            if self._inference_route():
                 return _stack_inference(self, graph, node_attr, *[a.detach() for a in args])
             params = [p for _, p in self.named_parameters()]
             return _StackFn.apply(self, graph, node_attr, attr_in, edge_attr_in, *args, *params)

@@ -155,6 +155,7 @@ SIGNATURES = {
     "fegnn_model_backward_scratch_floats": (C.c_size_t, [_PD]),
     "fegnn_model_forward": (C.c_int, [_PD, i32, i32, _PG, _PP] + [vp] * 9 + [vp, C.c_size_t, vp]),
     "fegnn_model_inference_workspace_floats": (C.c_size_t, [_PD]),
+    "fegnn_model_inference_det_workspace_floats": (C.c_size_t, [_PD]),
     "fegnn_model_forward_inference": (C.c_int, [_PD, i32, i32, _PG, _PP] + [vp] * 9 + [vp, C.c_size_t, vp]),
     "fegnn_model_backward": (C.c_int, [_PD, i32, i32, _PG, _PP, _PP] + [vp] * 11 + [vp, vp, C.c_size_t, vp]),
     "fegnn_model_backward_inputs": (C.c_int, [_PD, i32, i32, _PG, _PP, _PP] + [vp] * 11 + [vp, vp, C.c_size_t, _PI, vp]),

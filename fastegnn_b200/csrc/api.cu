@@ -224,6 +224,23 @@ NodePreArgs node_pre_args(const fegnn_dims* d, const fegnn_layer_params* p, cons
   return a;
 }
 
+// Scratch of the deterministic forward-only stack (fegnn_model_inference_det_workspace_floats), behind the stack's workspace.
+// The phases below take it as `det`: nullptr = the default kernels, else their kDet forms.
+struct DetWs {
+  float* eslab;   // edge forward: tile-boundary row sums (edge_det_slab_floats)
+  float* dval;    // virtual forward: the rows D sX, [N, C, 3]
+  float* gslab;   // per-graph sums: chunk-boundary slots (det_graph_slab_floats)
+};
+inline int det_graph_width(const fegnn_dims* d) { return d->C * kH + 3 * d->C + 3; }   // Usum, Dsum, xsum_new
+size_t det_ws_floats(const fegnn_dims* d) {
+  return al4(edge_det_slab_floats(d->E)) + al4((size_t)d->N * d->C * 3) + al4(det_graph_slab_floats(d->N, det_graph_width(d)));
+}
+void det_ws_bind(const fegnn_dims* d, float* p, DetWs* w) {
+  w->eslab = p; p += al4(edge_det_slab_floats(d->E));
+  w->dval = p; p += al4((size_t)d->N * d->C * 3);
+  w->gslab = p;
+}
+
 int check_flags_params(const fegnn_dims* d, const fegnn_layer_params* p) {
   if (p == nullptr) return fail(FEGNN_EINVAL, "layer params is null");
   if ((d->flags & FEGNN_F_ATTENTION) && (!p->att_w || !p->att_b || !p->attv_w || !p->attv_b))
@@ -422,18 +439,34 @@ int fegnn_embed_backward(int32_t N, int32_t Fin, const float* node_feat, const f
   CK(launch_embed_bwd(N, Fin, node_feat, w, gh, gw, gb, gnode_feat, S(stream)));
   return 0;
 }
-int fegnn_graph_xsum(int32_t N, int32_t B, const float* x, const int32_t* batch, float* xsum, void* stream) {
-  NO_DET("per-graph sums across CTAs with float atomics");
+}  // extern "C"
+namespace {
+int graph_xsum_run(int32_t N, int32_t B, const float* x, const int32_t* batch, float* xsum, const DetWs* det, void* stream) {
   RQ(N >= 0 && B >= 0 && (B == 0 || xsum) && (N == 0 || (x && batch)));
   CK(cudaMemsetAsync(xsum, 0, sizeof(float) * 3 * (size_t)B, S(stream)));
-  CK(launch_graph_xsum(N, x, batch, xsum, S(stream)));
+  if (det != nullptr) {
+    DetSegArgs sa;
+    memset(&sa, 0, sizeof(sa));
+    sa.N = N; sa.n = 1; sa.batch = batch; sa.slab = det->gslab;
+    sa.X[0] = x; sa.W[0] = 3; sa.out[0] = xsum;
+    CK(launch_det_graph_sums(sa, S(stream)));
+  } else {
+    CK(launch_graph_xsum(N, x, batch, xsum, S(stream)));
+  }
   return 0;
+}
+}  // namespace
+extern "C" {
+int fegnn_graph_xsum(int32_t N, int32_t B, const float* x, const int32_t* batch, float* xsum, void* stream) {
+  NO_DET("per-graph sums across CTAs with float atomics");
+  return graph_xsum_run(N, B, x, batch, xsum, nullptr, stream);
 }
 
 // ------------------------------------------------------------------ forward phases
-int fegnn_graph_pre_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* Z,
-                            const float* Sf, const float* xsum, fegnn_layer_saved* sv, void* stream) {
-  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+}  // extern "C"
+namespace {
+int graph_pre_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* Z,
+                          const float* Sf, const float* xsum, fegnn_layer_saved* sv, void* stream) {
   TRY(check_dims(d));
   RQ(g && p && Z && Sf && xsum && sv);
   GraphArgs a = graph_args(d, g, p);
@@ -442,9 +475,8 @@ int fegnn_graph_pre_forward(const fegnn_dims* d, const fegnn_graph* g, const feg
   return 0;
 }
 
-int fegnn_node_pre_forward(const fegnn_dims* d, const fegnn_layer_params* p, const float* h, fegnn_layer_saved* sv,
-                           void* stream) {
-  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+int node_pre_forward_run(const fegnn_dims* d, const fegnn_layer_params* p, const float* h, fegnn_layer_saved* sv,
+                         void* stream) {
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   RQ(h && sv);
@@ -459,9 +491,8 @@ int fegnn_node_pre_forward(const fegnn_dims* d, const fegnn_layer_params* p, con
   return 0;
 }
 
-int fegnn_edge_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
-                       fegnn_layer_saved* sv, void* stream) {
-  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+int edge_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
+                     fegnn_layer_saved* sv, const DetWs* det, void* stream) {
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   RQ(g && x && sv);
@@ -469,16 +500,22 @@ int fegnn_edge_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_la
   a.msum = sv->msum; a.tsum = sv->tsum;
   if (!(d->flags & FEGNN_F_PREZEROED)) CK(zero_pair(sv->msum, kH * (size_t)d->N, sv->tsum, 3 * (size_t)d->N, S(stream)));
   const int mode = d->Fe <= kTcMaxFe ? g_edge_fwd_mode : 0;
+  if (det != nullptr) {
+    a.slab = det->eslab;
+    if (mode == 3) CK((launch_edge_fwd_tc<3, true>(a, sm_count(), S(stream))));
+    else if (mode == 1) CK((launch_edge_fwd_tc<1, true>(a, sm_count(), S(stream))));
+    else CK(launch_edge_fwd<true>(a, sm_count(), S(stream)));
+    return 0;
+  }
   if (mode == 3) CK(launch_edge_fwd_tc<3>(a, sm_count(), S(stream)));
   else if (mode == 1) CK(launch_edge_fwd_tc<1>(a, sm_count(), S(stream)));
   else CK(launch_edge_fwd(a, sm_count(), S(stream)));
   return 0;
 }
 
-int fegnn_virtual_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
-                          const float* v, const float* Z, fegnn_layer_saved* sv, float* x_new, float* xsum_new,
-                          void* stream) {
-  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+int virtual_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
+                        const float* v, const float* Z, fegnn_layer_saved* sv, float* x_new, float* xsum_new,
+                        const DetWs* det, void* stream) {
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   RQ(g && x && v && Z && sv && x_new && xsum_new);
@@ -488,14 +525,28 @@ int fegnn_virtual_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn
     CK(zero_pair(sv->Dsum, 3 * d->C * (size_t)d->B, sv->Usum, kH * d->C * (size_t)d->B, S(stream)));
     CK(cudaMemsetAsync(xsum_new, 0, sizeof(float) * 3 * (size_t)d->B, S(stream)));
   }
-  if (g_virt_fwd_mode == 1 && !(d->flags & FEGNN_F_ATTENTION)) CK(launch_virtual_fwd_tc<2>(a, sm_count(), S(stream)));
+  const bool tc = g_virt_fwd_mode == 1 && !(d->flags & FEGNN_F_ATTENTION);
+  if (det != nullptr) {
+    // the kernel writes u, x_new and the rows D sX (into the Dsum slot); their per-graph sums follow in graph order
+    a.Dsum = det->dval;
+    if (tc) CK((launch_virtual_fwd_tc<2, true>(a, sm_count(), S(stream))));
+    else CK(launch_virtual_fwd<true>(a, sm_count(), S(stream)));
+    DetSegArgs sa;
+    memset(&sa, 0, sizeof(sa));
+    sa.N = d->N; sa.n = 3; sa.batch = g->batch; sa.slab = det->gslab;
+    sa.X[0] = sv->u; sa.W[0] = d->C * kH; sa.out[0] = sv->Usum;
+    sa.X[1] = det->dval; sa.W[1] = 3 * d->C; sa.out[1] = sv->Dsum; sa.remapC[1] = d->C;
+    sa.X[2] = x_new; sa.W[2] = 3; sa.out[2] = xsum_new;
+    CK(launch_det_graph_sums(sa, S(stream)));
+    return 0;
+  }
+  if (tc) CK(launch_virtual_fwd_tc<2>(a, sm_count(), S(stream)));
   else CK(launch_virtual_fwd(a, sm_count(), S(stream)));
   return 0;
 }
 
-int fegnn_node_h_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* h,
-                         fegnn_layer_saved* sv, float* h_new, void* stream) {
-  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+int node_h_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* h,
+                       fegnn_layer_saved* sv, float* h_new, const DetWs* det, void* stream) {
   TRY(check_dims(d));
   RQ(g && p && h && sv && h_new);
   NodeHArgs a;
@@ -514,10 +565,13 @@ int fegnn_node_h_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_
     }
     CK(launch_node_h_fwd_tc(a, sm_count(), S(stream)));
   }
+  else if (det != nullptr) CK(launch_node_h_fwd<true>(a, sm_count(), S(stream)));
   else CK(launch_node_h_fwd(a, sm_count(), S(stream), !(d->flags & FEGNN_F_PREZEROED)));
   return 0;
 }
 
+}  // namespace
+extern "C" {
 int fegnn_node_h_weight_images(const fegnn_dims* d, int32_t nl, const fegnn_layer_params* layers, float* const* wimg,
                                void* stream) {
   TRY(check_dims(d));
@@ -530,16 +584,56 @@ int fegnn_node_h_weight_images(const fegnn_dims* d, int32_t nl, const fegnn_laye
   CK(launch_node_h_wprep(d->C, ldn(d), nl, w0, w2, wimg, S(stream)));
   return 0;
 }
+}  // extern "C"
+namespace {
 
-int fegnn_graph_post_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* Z,
-                             const float* Sf, const fegnn_layer_saved* sv, float* Z_new, float* S_new, void* stream) {
-  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+int graph_post_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* Z,
+                           const float* Sf, const fegnn_layer_saved* sv, float* Z_new, float* S_new, void* stream) {
   TRY(check_dims(d));
   RQ(g && p && Z && Sf && sv && Z_new && ((d->flags & FEGNN_F_LAST) || S_new));
   GraphArgs a = graph_args(d, g, p);
   a.Z = Z; a.S = Sf; a.Dsum = sv->Dsum; a.Usum = sv->Usum; a.Z_new = Z_new; a.S_new = S_new;
   CK(launch_graph_post_fwd(a, S(stream)));
   return 0;
+}
+
+}  // namespace
+extern "C" {
+int fegnn_graph_pre_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* Z,
+                            const float* Sf, const float* xsum, fegnn_layer_saved* sv, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+  return graph_pre_forward_run(d, g, p, Z, Sf, xsum, sv, stream);
+}
+
+int fegnn_node_pre_forward(const fegnn_dims* d, const fegnn_layer_params* p, const float* h, fegnn_layer_saved* sv,
+                           void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+  return node_pre_forward_run(d, p, h, sv, stream);
+}
+
+int fegnn_edge_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
+                       fegnn_layer_saved* sv, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+  return edge_forward_run(d, g, p, x, sv, nullptr, stream);
+}
+
+int fegnn_virtual_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
+                          const float* v, const float* Z, fegnn_layer_saved* sv, float* x_new, float* xsum_new,
+                          void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+  return virtual_forward_run(d, g, p, x, v, Z, sv, x_new, xsum_new, nullptr, stream);
+}
+
+int fegnn_node_h_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* h,
+                         fegnn_layer_saved* sv, float* h_new, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+  return node_h_forward_run(d, g, p, h, sv, h_new, nullptr, stream);
+}
+
+int fegnn_graph_post_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* Z,
+                             const float* Sf, const fegnn_layer_saved* sv, float* Z_new, float* S_new, void* stream) {
+  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
+  return graph_post_forward_run(d, g, p, Z, Sf, sv, Z_new, S_new, stream);
 }
 
 // ------------------------------------------------------------------ backward phases
@@ -1072,18 +1166,29 @@ size_t fegnn_model_inference_workspace_floats(const fegnn_dims* d) {
   // two ping-pong states + the (h, S) of the embedding (FastRF) + the shared block(s) of per-layer intermediates
   return 3 * per_state + infer_blocks(d) * fegnn_layer_saved_floats(d);
 }
+// the deterministic forms' scratch (DetWs), which follows that workspace
+size_t fegnn_model_inference_det_workspace_floats(const fegnn_dims* d) {
+  return g_det && d != nullptr && check_dims(d) == 0 ? det_ws_floats(d) : 0;
+}
 
 int fegnn_model_forward_inference(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn_graph* g,
                                   const fegnn_layer_params* layers, const float* embed_w, const float* embed_b,
                                   const float* vnf, const float* node_feat, const float* x0, const float* v,
                                   const float* loc_mean, float* x_out, float* Z_out, float* workspace,
                                   size_t workspace_floats, void* stream) {
-  NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(L >= 1 && L <= 32 && g && layers && embed_w && embed_b && vnf && workspace && x_out && Z_out);
   RQ(d->Nl == d->N);
-  if (workspace_floats < fegnn_model_inference_workspace_floats(d))
-    return fail(FEGNN_ENOMEM, "inference workspace %zu < %zu floats", workspace_floats, fegnn_model_inference_workspace_floats(d));
+  // deterministic mode: the kDet forms of the phases, with their scratch behind the workspace
+  const size_t base_floats = fegnn_model_inference_workspace_floats(d);
+  const size_t need = base_floats + fegnn_model_inference_det_workspace_floats(d);
+  if (workspace_floats < need) return fail(FEGNN_ENOMEM, "inference workspace %zu < %zu floats", workspace_floats, need);
+  DetWs det_;
+  const DetWs* det = nullptr;
+  if (g_det) {
+    det_ws_bind(d, workspace + base_floats, &det_);
+    det = &det_;
+  }
   cudaStream_t st = S(stream);
   const size_t N = d->N, Nl = d->Nl, B = d->B, C = d->C;
   float* p = workspace;
@@ -1129,10 +1234,10 @@ int fegnn_model_forward_inference(const fegnn_dims* d, int32_t L, int32_t Fin, c
     fegnn_dims d0 = *d;
     d0.flags |= FEGNN_F_PREZEROED;
     if (rf || L == 1) d0.flags |= FEGNN_F_LAST;
-    TRY(fegnn_node_pre_forward(&d0, &layers[0], h[2], &sv_[0], stream));
+    TRY(node_pre_forward_run(&d0, &layers[0], h[2], &sv_[0], stream));
     CK(cudaStreamWaitEvent(st, static_cast<cudaEvent_t>(g->ready_event), 0));
   }
-  TRY(fegnn_graph_xsum(d->N, d->B, x[2], g->batch, xsum[2], stream));
+  TRY(graph_xsum_run(d->N, d->B, x[2], g->batch, xsum[2], det, stream));
   SideStream* sd = side_stream();
   RQ(sd != nullptr);
   void* side = sd->st;
@@ -1158,12 +1263,12 @@ int fegnn_model_forward_inference(const fegnn_dims* d, int32_t L, int32_t Fin, c
     // ... and the per-graph coordinate sums of the state this layer produces on the side stream (last read by the per-graph
     // kernels of the layer that consumed that state, earlier on the same stream; joined in front of virtual_forward)
     CK(cudaMemsetAsync(xsum[nxt], 0, sizeof(float) * 3 * B, S(side)));
-    TRY(fegnn_graph_pre_forward(&dl, g, pl, Z[cur], Sx[hs], xsum[cur], sv, side));
-    if (!(graph_pending && l == 0)) TRY(fegnn_node_pre_forward(&dl, pl, h[hs], sv, stream));
+    TRY(graph_pre_forward_run(&dl, g, pl, Z[cur], Sx[hs], xsum[cur], sv, side));
+    if (!(graph_pending && l == 0)) TRY(node_pre_forward_run(&dl, pl, h[hs], sv, stream));
     if (rf) TRY(fegnn_rf_vel_forward(d->N, v, pl, sv->sv, stream));
-    TRY(fegnn_edge_forward(&dl, g, pl, x[cur], sv, stream));
+    TRY(edge_forward_run(&dl, g, pl, x[cur], sv, det, stream));
     JOIN(sd, st);
-    TRY(fegnn_virtual_forward(&dl, g, pl, x[cur], v, Z[cur], sv, x[nxt], xsum[nxt], stream));
+    TRY(virtual_forward_run(&dl, g, pl, x[cur], v, Z[cur], sv, x[nxt], xsum[nxt], det, stream));
     FORK(sd, st);
     if (two && l + 1 >= nb && l + 1 < L) {
       // the accumulators of the ring block that layer l + 1 reuses: last read by layer l + 1 - nb (node phase on this stream
@@ -1171,8 +1276,8 @@ int fegnn_model_forward_inference(const fegnn_dims* d, int32_t L, int32_t Fin, c
       CK(cudaMemsetAsync(sv_[(l + 1) % nb].msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), S(side)));
       CK(cudaEventRecord(sd->aux, S(side)));
     }
-    if (!last) TRY(fegnn_node_h_forward(&dl, g, pl, h[cur], sv, h[nxt], stream));
-    TRY(fegnn_graph_post_forward(&dl, g, pl, Z[cur], Sx[hs], sv, Z[nxt], Sx[nxt], side));
+    if (!last) TRY(node_h_forward_run(&dl, g, pl, h[cur], sv, h[nxt], det, stream));
+    TRY(graph_post_forward_run(&dl, g, pl, Z[cur], Sx[hs], sv, Z[nxt], Sx[nxt], side));
     if (img_ahead && l + 2 < L && l + 1 >= nimg_top) CK(weight_images(l + 1, 1, S(side)));
     // the shared block is rewritten by the next layer: its per-graph kernels (side) must not start before this layer's
     // node_h (main) has read u / msum, and its main-stream kernels not before this layer's graph_post (side) has read

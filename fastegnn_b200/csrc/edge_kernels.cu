@@ -25,9 +25,99 @@ struct EdgeArgs {
   union { float* tsum; const int* perm; };   // perm: [E] caller index of CSR edge e, or nullptr (CSR order is the caller's)
   // backward inputs / outputs
   const float *gm, *gt;
-  float *gP, *gQ, *gx;
+  // slab: the deterministic forward's (kDet) tile-boundary row sums, [ntiles][2][kDetSlot] (edge_det_msum); a forward
+  // kernel never reads gP
+  union { float* gP; float* slab; };
+  float *gQ, *gx;
   float *g_w1, *g_W2, *g_b2, *g_W3, *g_b3, *g_w4, *g_wa, *g_ba;
 };
+
+// ---- deterministic forward (kDet): msum / tsum without arrival-order float sums
+// Each tile sums its runs of equal row ids in row order.  A run that stays inside the tile is the row's only contribution:
+// ONE add into the zero-filled msum / tsum.  A run that continues into the previous or next tile goes to the tile's
+// boundary slab instead -- slot 0 for the run that starts at the tile's first edge, slot 1 for the one that ends at its
+// last -- and edge_det_fixup_kernel adds the slots of such a row in tile order and stores the total.
+constexpr int kDetSlot = 68;      // floats per slot: 64 msum columns, 3 tsum columns, 1 pad (16-byte slots)
+inline size_t edge_det_slab_floats(int E) { return (size_t)((E + kTM - 1) / kTM) * 2 * kDetSlot; }
+
+// does the row of this tile's first (last) edge continue from the previous (into the next) tile?
+__device__ __forceinline__ bool edge_det_cont_in(const EdgeArgs& a, const int* srow, int tile) {
+  return tile > 0 && a.row[tile * kTM - 1] == srow[0];
+}
+__device__ __forceinline__ bool edge_det_cont_out(const EdgeArgs& a, const int* srow, int tile) {
+  const int e1 = (tile + 1) * kTM;
+  return e1 < a.E && a.row[e1] == srow[kTM - 1];
+}
+// msum: thread (c4 = tid & 15, grp = tid >> 4) takes the runs that START in rows 8 grp .. 8 grp + 7 and walks each to its
+// end in row order over column quad c4.  mget(rr, c4) = float4 of columns 4 c4 .. 4 c4 + 3 of edge row rr's message.
+template <typename MGet>
+__device__ __forceinline__ void edge_det_msum(const EdgeArgs& a, const int* srow, int tile, MGet mget) {
+  const int c4 = threadIdx.x & 15, grp = threadIdx.x >> 4;
+  const bool cin = edge_det_cont_in(a, srow, tile), cout = edge_det_cont_out(a, srow, tile);
+  for (int r0 = grp * 8; r0 < grp * 8 + 8; ++r0) {
+    const int k = srow[r0];
+    if (k < 0 || (r0 > 0 && srow[r0 - 1] == k)) continue;
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    int r = r0;
+    for (; r < kTM && srow[r] == k; ++r) {
+      const float4 m = mget(r, c4);
+      acc.x += m.x; acc.y += m.y; acc.z += m.z; acc.w += m.w;
+    }
+    if ((r0 == 0 && cin) || (r == kTM && cout))
+      *reinterpret_cast<float4*>(a.slab + ((size_t)tile * 2 + (r0 == 0 ? 0 : 1)) * kDetSlot + c4 * 4) = acc;
+    else
+      atomicAdd(reinterpret_cast<float4*>(a.msum + (size_t)k * kH + c4 * 4), acc);
+  }
+}
+// tsum: thread t < 128 takes the run that starts at row t, if any.  tget(rr, k) = coordinate k of edge row rr's term.
+template <typename TGet>
+__device__ __forceinline__ void edge_det_tsum(const EdgeArgs& a, const int* srow, int tile, TGet tget) {
+  const int r0 = threadIdx.x;
+  if (r0 >= kTM) return;
+  const int k = srow[r0];
+  if (k < 0 || (r0 > 0 && srow[r0 - 1] == k)) return;
+  float acc[3] = {0.f, 0.f, 0.f};
+  int r = r0;
+  for (; r < kTM && srow[r] == k; ++r) {
+#pragma unroll
+    for (int j = 0; j < 3; ++j) acc[j] += tget(r, j);
+  }
+  const bool cross = (r0 == 0 && edge_det_cont_in(a, srow, tile)) || (r == kTM && edge_det_cont_out(a, srow, tile));
+#pragma unroll
+  for (int j = 0; j < 3; ++j) {
+    if (cross) a.slab[((size_t)tile * 2 + (r0 == 0 ? 0 : 1)) * kDetSlot + kH + j] = acc[j];
+    else atomicAdd(a.tsum + (size_t)k * 3 + j, acc[j]);
+  }
+}
+// One warp per tile boundary b (between tiles b - 1 and b): if a row r crosses it and b is r's first crossing, r's sums are
+// its slot in tile b - 1 plus slot 0 of every following tile it reaches, added in tile order.  Nothing else adds into r.
+__global__ void __launch_bounds__(256) edge_det_fixup_kernel(EdgeArgs a) {
+  pdl_trigger();
+  const int lane = threadIdx.x & 31;
+  const int b = (int)((blockIdx.x * 256u + threadIdx.x) >> 5) + 1;
+  const int ntiles = (a.E + kTM - 1) / kTM;
+  pdl_wait();
+  if (b >= ntiles) return;
+  const int e = b * kTM, s = e - kTM, r = a.row[e];
+  if (a.row[e - 1] != r) return;
+  if (s > 0 && a.row[s] == r && a.row[s - 1] == r) return;      // r starts before tile b - 1: an earlier boundary's warp
+  const int slot = a.row[s] == r ? 0 : 1;                        // r's run in tile b - 1 starts at its first edge
+  for (int j = lane; j < kH + 3; j += 32) {
+    float acc = a.slab[((size_t)(b - 1) * 2 + slot) * kDetSlot + j];
+    for (int t = b;; ++t) {
+      acc += a.slab[(size_t)t * 2 * kDetSlot + j];
+      if ((t + 1) * kTM >= a.E || a.row[(t + 1) * kTM] != r) break;
+    }
+    if (j < kH) a.msum[(size_t)r * kH + j] = acc;
+    else a.tsum[(size_t)r * 3 + (j - kH)] = acc;
+  }
+}
+inline cudaError_t launch_edge_det_fixup(const EdgeArgs& a, cudaStream_t st) {
+  const int nb = (a.E + kTM - 1) / kTM - 1;      // tile boundaries
+  if (nb <= 0) return cudaSuccess;
+  if (cudaError_t e_ = launch_pdl(edge_det_fixup_kernel, (nb + 7) / 8, 256, 0, st, a)) return e_;
+  return cudaGetLastError();
+}
 
 struct EdgeSmemVec {
   float wq[kH], Wa[FEGNN_MAX_FE * kH], b2[kH], b3[kH], w4[kH], wa[kH];
@@ -131,6 +221,8 @@ __device__ __forceinline__ void edge_assemble(const EdgeArgs& a, const EdgeSmemV
 constexpr size_t kEdgeFwdSmem = (2 * kWFloats + 2 * kTileFloats) * sizeof(float) + sizeof(EdgeSmemVec);
 constexpr size_t kEdgeBwdSmem = (2 * kWFloats + 5 * kTileFloats) * sizeof(float) + sizeof(EdgeSmemVec);
 
+// kDet: msum / tsum through edge_det_msum / edge_det_tsum and the boundary slab (same terms, summed in row order)
+template <bool kDet>
 __global__ void __launch_bounds__(kThreads, 2) edge_fwd_kernel(EdgeArgs a) {
   extern __shared__ __align__(16) float smem[];
   float* W2s = smem;
@@ -168,7 +260,10 @@ __global__ void __launch_bounds__(kThreads, 2) edge_fwd_kernel(EdgeArgs a) {
       }
     }
     __syncthreads();
-    tile_segsum_rows(T2, v->srow, a.msum);
+    if constexpr (kDet) edge_det_msum(a, v->srow, tile, [&](int rr, int c4) {
+      return *reinterpret_cast<const float4*>(T2 + rr * kH + c4 * 4);
+    });
+    else tile_segsum_rows(T2, v->srow, a.msum);
     zero_acc(acc);
     gemm_nt(acc, T2, W3s, ty, tx);
     {
@@ -184,7 +279,9 @@ __global__ void __launch_bounds__(kThreads, 2) edge_fwd_kernel(EdgeArgs a) {
       }
     }
     __syncthreads();
-    if (tid < kTM) {
+    if constexpr (kDet) {
+      edge_det_tsum(a, v->srow, tile, [&](int rr, int k) { return v->sdn[rr * 3 + k] * v->ss[rr]; });
+    } else if (tid < kTM) {
       const int r = v->srow[tid];
       const float s = v->ss[tid];
 #pragma unroll
@@ -415,18 +512,20 @@ __global__ void __launch_bounds__(kThreads, 1) edge_bwd_kernel(EdgeArgs a) {
 }
 
 // ---------------------------------------------------------------------------- host side
+template <bool kDet = false>
 cudaError_t launch_edge_fwd(const EdgeArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(edge_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEdgeFwdSmem);
+    cudaError_t e = cudaFuncSetAttribute(edge_fwd_kernel<kDet>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEdgeFwdSmem);
     if (e != cudaSuccess) return e;
     attr.set();
   }
   int ntiles = (a.E + kTM - 1) / kTM;
   if (ntiles == 0) return cudaSuccess;
   int grid = ntiles < 2 * sms ? ntiles : 2 * sms;
-  edge_fwd_kernel<<<grid, kThreads, kEdgeFwdSmem, st>>>(a); ++g_launches;
-  return cudaGetLastError();
+  edge_fwd_kernel<kDet><<<grid, kThreads, kEdgeFwdSmem, st>>>(a); ++g_launches;
+  if (cudaError_t e_ = cudaGetLastError()) return e_;
+  return kDet ? launch_edge_det_fixup(a, st) : cudaSuccess;
 }
 template <bool kEa = false>
 cudaError_t launch_edge_bwd(const EdgeArgs& a, int sms, cudaStream_t st) {

@@ -131,7 +131,9 @@ __device__ __forceinline__ float tc_silu_hb(float z, float b) {
   return fmaf(t, th, t);
 }
 
-template <int SPLIT>
+// kDet: msum / tsum through edge_det_msum / edge_det_tsum and the boundary slab (edge_kernels.cu; same terms, summed in row
+// order)
+template <int SPLIT, bool kDet>
 __global__ void __launch_bounds__(kTcThreads, EdgeTcSmem<SPLIT>::ctas_per_sm) edge_fwd_tc_kernel(EdgeArgs a) {
   using SM = EdgeTcSmem<SPLIT>;
   extern __shared__ uint8_t smem_raw[];
@@ -296,7 +298,17 @@ __global__ void __launch_bounds__(kTcThreads, EdgeTcSmem<SPLIT>::ctas_per_sm) ed
     // ---- msum: walk over the m tile while the tensor core runs (read-only on both sides).  Thread (c4, grp) owns the
     //      16-byte column quad c4 of the 8 rows of swizzle atom grp: one LDS.128 per row, one red.global.add.v4.f32 per
     //      run of equal row ids (the scalar 32-row column walk this replaces was 17 % of the kernel's instructions).
-    {
+    if constexpr (kDet) {
+      edge_det_msum(a, v->srow, tile, [&](int rr, int c4) {
+        const uint32_t o = (c4 >> 3) * (kTM * 128) + (rr >> 3) * 1024 + (rr & 7) * 128 + (((c4 & 7) ^ (rr & 7)) << 4);
+        float4 mv = *reinterpret_cast<const float4*>(At + o);
+        if (SPLIT == 3) {
+          const float4 lo = *reinterpret_cast<const float4*>(At + SM::kT + o);
+          mv.x += lo.x; mv.y += lo.y; mv.z += lo.z; mv.w += lo.w;
+        }
+        return mv;
+      });
+    } else {
       const int c4 = t & 15, grp = t >> 4;
       const uint8_t* gbase = At + (c4 >> 3) * (kTM * 128) + grp * 1024;
       int cur = -1;
@@ -331,7 +343,15 @@ __global__ void __launch_bounds__(kTcThreads, EdgeTcSmem<SPLIT>::ctas_per_sm) ed
       for (int j = 0; j < 32; ++j) s = fmaf(tc_silu_hb<SPLIT>(z[j], v->b3[half * 32 + j]), v->w4[half * 32 + j], s);
       if (half == 1) v->spart[row] = s;
       __syncthreads();
-      if (half == 0) {
+      if constexpr (kDet) {
+        if (half == 0) {
+          s += v->spart[row];
+          if (use_tanh) s = tanhf(s);
+          v->sq[row] = s;                  // sq (|x_i - x_j|^2) was last read by the assembly
+        }
+        __syncthreads();
+        edge_det_tsum(a, v->srow, tile, [&](int rr, int k) { return v->sdn[rr * 3 + k] * v->sq[rr]; });
+      } else if (half == 0) {
         s += v->spart[row];
         if (use_tanh) s = tanhf(s);
         const int r = v->srow[row];
@@ -349,12 +369,12 @@ __global__ void __launch_bounds__(kTcThreads, EdgeTcSmem<SPLIT>::ctas_per_sm) ed
   if (warp == 0) umma::tmem_dealloc<128>(tmem);
 }
 
-template <int SPLIT>
+template <int SPLIT, bool kDet = false>
 cudaError_t launch_edge_fwd_tc(const EdgeArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   const size_t bytes = EdgeTcSmem<SPLIT>::bytes;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(edge_fwd_tc_kernel<SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    cudaError_t e = cudaFuncSetAttribute(edge_fwd_tc_kernel<SPLIT, kDet>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
     attr.set();
   }
@@ -362,8 +382,9 @@ cudaError_t launch_edge_fwd_tc(const EdgeArgs& a, int sms, cudaStream_t st) {
   if (ntiles == 0) return cudaSuccess;
   const int per_sm = EdgeTcSmem<SPLIT>::ctas_per_sm;
   const int grid = ntiles < per_sm * sms ? ntiles : per_sm * sms;
-  if (cudaError_t e_ = launch_pdl(edge_fwd_tc_kernel<SPLIT>, grid, kTcThreads, bytes, st, a)) return e_;
-  return cudaGetLastError();
+  if (cudaError_t e_ = launch_pdl(edge_fwd_tc_kernel<SPLIT, kDet>, grid, kTcThreads, bytes, st, a)) return e_;
+  if (cudaError_t e_ = cudaGetLastError()) return e_;
+  return kDet ? launch_edge_det_fixup(a, st) : cudaSuccess;
 }
 
 }  // namespace fegnn

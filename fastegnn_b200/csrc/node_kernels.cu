@@ -80,6 +80,102 @@ __global__ void graph_xsum_kernel(int N, const float* __restrict__ x, const int*
   }
 }
 
+// ---- per-graph sums of the deterministic forward: out_m[b][w] = sum over the nodes i of graph b of X_m[i][w], for up to
+// three row-major matrices in one pair of launches (graph_xsum; Usum, Dsum and xsum_new of the virtual forward).  The nodes
+// are cut into chunks of K rows, K a function of N alone.  Pass 1, one CTA per chunk, sums each column of the chunk in node
+// order per graph run: a graph that lies inside the chunk gets its total stored; a run that continues into the previous or
+// next chunk goes to the chunk's slot 0 (run at its first row) or 1 (run at its last).  Pass 2 adds the slots of each graph
+// that spans chunks in chunk order -- 8 fixed parts of its chunk range per column, then the 8 part sums in part order -- and
+// stores the total.  Graphs without nodes get nothing: the caller zero-fills out.
+struct DetSegArgs {
+  int N, K, n, Wtot;               // nodes, rows per chunk, matrices, their total width
+  const int* batch;                // [N] non-decreasing
+  const float* X[3];               // [N][W[m]]
+  int W[3];
+  float* out[3];                   // [B][W[m]]; remapC[m] = C > 0: column w = 3 c + k goes to [B][3][C] position k C + c
+  int remapC[3];
+  float* slab;                     // [nchunks][2][Wtot]
+};
+inline int det_chunk_rows(int N) { return N <= 262144 ? 256 : (N + 1023) / 1024; }     // at most 1 024 chunks
+inline size_t det_graph_slab_floats(int N, int Wtot) {
+  const int K = det_chunk_rows(N);
+  return (size_t)((N + K - 1) / K) * 2 * Wtot;
+}
+__device__ __forceinline__ void det_graph_store(const DetSegArgs& a, int m, int b, int w, float v) {
+  const int C = a.remapC[m];
+  a.out[m][(size_t)b * a.W[m] + (C > 0 ? (w % 3) * C + w / 3 : w)] = v;
+}
+__global__ void __launch_bounds__(256) det_graph_sums_chunk_kernel(DetSegArgs a) {
+  pdl_trigger();
+  const int j = blockIdx.x, i0 = j * a.K, i1 = min(a.N, i0 + a.K);
+  pdl_wait();
+  const bool cin = i0 > 0 && a.batch[i0 - 1] == a.batch[i0], cout = i1 < a.N && a.batch[i1] == a.batch[i1 - 1];
+  int wbase = 0;
+  for (int m = 0; m < a.n; ++m) {
+    const int W = a.W[m];
+    const float* __restrict__ X = a.X[m];
+    for (int w = threadIdx.x; w < W; w += blockDim.x) {
+      for (int r0 = i0, r1; r0 < i1; r0 = r1) {
+        const int b = a.batch[r0];
+        for (r1 = r0 + 1; r1 < i1 && a.batch[r1] == b; ++r1) {}
+        float acc = 0.f;
+        for (int i = r0; i < r1; ++i) acc += X[(size_t)i * W + w];
+        if ((r0 == i0 && cin) || (r1 == i1 && cout)) a.slab[((size_t)j * 2 + (r0 == i0 ? 0 : 1)) * a.Wtot + wbase + w] = acc;
+        else det_graph_store(a, m, b, w, acc);
+      }
+    }
+    wbase += W;
+  }
+}
+// grid (chunks - 1, ceil(Wtot / 32)): block (j - 1, y) serves the graph that crosses the boundary in front of chunk j if
+// that is its first crossing; thread (col, part) sums part `part` of the graph's slot list in column 32 y + col
+__global__ void __launch_bounds__(256) det_graph_sums_fix_kernel(DetSegArgs a) {
+  pdl_trigger();
+  __shared__ float red[8][32];
+  const int j = blockIdx.x + 1, i = j * a.K, s = i - a.K;
+  pdl_wait();
+  const int b = a.batch[i];
+  if (a.batch[i - 1] != b) return;
+  if (s > 0 && a.batch[s] == b && a.batch[s - 1] == b) return;     // the graph starts before chunk j - 1
+  const int slot = a.batch[s] == b ? 0 : 1;                        // its run in chunk j - 1 starts at that chunk's first row
+  int lo = i, hi = a.N;                                             // last node of the graph: batch is non-decreasing
+  while (hi - lo > 1) {
+    const int mid = lo + (hi - lo) / 2;
+    if (a.batch[mid] == b) lo = mid; else hi = mid;
+  }
+  const int n = lo / a.K - j + 2;                                   // slots: chunk j - 1, then chunks j .. lo / K
+  const int col = threadIdx.x & 31, part = threadIdx.x >> 5, w = blockIdx.y * 32 + col;
+  float acc = 0.f;
+  if (w < a.Wtot) {
+    for (int e = part * n / 8; e < (part + 1) * n / 8; ++e) {
+      const size_t sl = e == 0 ? (size_t)(j - 1) * 2 + slot : (size_t)(j - 1 + e) * 2;
+      acc += a.slab[sl * a.Wtot + w];
+    }
+  }
+  red[part][col] = acc;
+  __syncthreads();
+  if (part == 0 && w < a.Wtot) {
+    float tot = 0.f;
+#pragma unroll
+    for (int p = 0; p < 8; ++p) tot += red[p][col];
+    int m = 0, wl = w;
+    while (wl >= a.W[m]) wl -= a.W[m++];
+    det_graph_store(a, m, b, wl, tot);
+  }
+}
+// a.slab must hold det_graph_slab_floats(N, Wtot) floats
+inline cudaError_t launch_det_graph_sums(DetSegArgs a, cudaStream_t st) {
+  if (a.N == 0) return cudaSuccess;
+  a.K = det_chunk_rows(a.N);
+  a.Wtot = 0;
+  for (int m = 0; m < a.n; ++m) a.Wtot += a.W[m];
+  const int nch = (a.N + a.K - 1) / a.K;
+  if (cudaError_t e_ = launch_pdl(det_graph_sums_chunk_kernel, nch, 256, 0, st, a)) return e_;
+  if (nch > 1)
+    if (cudaError_t e_ = launch_pdl(det_graph_sums_fix_kernel, dim3(nch - 1, (a.Wtot + 31) / 32), 256, 0, st, a)) return e_;
+  return cudaGetLastError();
+}
+
 // ------------------------------------------------------------------------------------------- node_pre
 struct NodePreArgs {
   int N, ld1, ldv, ldn;
@@ -393,14 +489,56 @@ constexpr size_t kNodeHSmem = (kWFloats + 2 * kTileFloats) * sizeof(float);
 
 // zh1 += [Uh +] W_blk A_blk for one (node tile, K-block) work item; zh1 is zero-filled by the launcher and
 // accumulated with red.global.add.v4.f32 (block 0 = message mean + the h term Uh, block 1+c = u[:,c,:]).
+// kDet: one CTA per node tile walks the K-blocks in block order, adds each block's product to a running total in
+// registers and stores zh1 once (the same terms, in block order).
+template <bool kDet>
 __global__ void __launch_bounds__(kThreads, 2) node_h_z_kernel(NodeHArgs a) {
   extern __shared__ __align__(16) float smem[];
   float* Ws = smem;
   float* T0 = Ws + kWFloats;
   const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
   const int nblk = a.C + 1;
-  const int blk = blockIdx.x % nblk, cta = blockIdx.x / nblk, nctas = gridDim.x / nblk;
   const int ntiles = (a.N + kTM - 1) / kTM;
+  if constexpr (kDet) {
+    pdl_trigger();
+    pdl_wait();
+    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+      const int i0 = tile * kTM, nvalid = min(kTM, a.N - i0);
+      float tot[kRT][4];
+      for (int blk = 0; blk < nblk; ++blk) {
+        __syncthreads();
+        if (blk == 0) {
+          stage_weight(Ws, a.node_w0, a.ldn, kH, 1);
+          load_tile_rowscaled(T0, a.msum + (size_t)i0 * kH, kH, nvalid, a.dinv != nullptr ? a.dinv + i0 : nullptr);
+        } else {
+          stage_weight(Ws, a.node_w0, a.ldn, 2 * kH + (blk - 1), a.C);
+          load_tile(T0, a.u + ((size_t)i0 * a.C + (blk - 1)) * kH, (size_t)a.C * kH, nvalid);
+        }
+        __syncthreads();
+        float acc[kRT][4];
+#pragma unroll
+        for (int i = 0; i < kRT; ++i) {
+          const int r = ty * kRT + i;
+          float4 g0 = make_float4(0, 0, 0, 0);
+          if (blk == 0 && r < nvalid) g0 = *reinterpret_cast<const float4*>(a.Uh + (size_t)(i0 + r) * kH + tx * 4);
+          acc[i][0] = g0.x; acc[i][1] = g0.y; acc[i][2] = g0.z; acc[i][3] = g0.w;
+        }
+        gemm_nt(acc, T0, Ws, ty, tx);
+#pragma unroll
+        for (int i = 0; i < kRT; ++i)
+#pragma unroll
+          for (int j = 0; j < 4; ++j) tot[i][j] = blk == 0 ? acc[i][j] : tot[i][j] + acc[i][j];
+      }
+#pragma unroll
+      for (int i = 0; i < kRT; ++i) {
+        const int r = ty * kRT + i;
+        if (r < nvalid)
+          *reinterpret_cast<float4*>(a.zh1 + (size_t)(i0 + r) * kH + tx * 4) = make_float4(tot[i][0], tot[i][1], tot[i][2], tot[i][3]);
+      }
+    }
+    return;
+  }
+  const int blk = blockIdx.x % nblk, cta = blockIdx.x / nblk, nctas = gridDim.x / nblk;
   pdl_trigger();
   if (blk == 0) stage_weight(Ws, a.node_w0, a.ldn, kH, 1);
   else stage_weight(Ws, a.node_w0, a.ldn, 2 * kH + (blk - 1), a.C);
@@ -636,8 +774,9 @@ cudaError_t launch_node_pre_bwd(const NodePreArgs& a, int sms, cudaStream_t st, 
                                   NodeAttrArgs{})) return e_;
   return cudaGetLastError();
 }
+template <bool kDet = false>
 cudaError_t launch_node_h_fwd(const NodeHArgs& a, int sms, cudaStream_t st, bool zero = true) {
-  FEGNN_SET_SMEM(node_h_z_kernel, kNodeHSmem);
+  FEGNN_SET_SMEM(node_h_z_kernel<kDet>, kNodeHSmem);
   {
     static DevOnce done2_;
     if (!done2_.get()) {
@@ -648,9 +787,10 @@ cudaError_t launch_node_h_fwd(const NodeHArgs& a, int sms, cudaStream_t st, bool
   }
   int ntiles = (a.N + kTM - 1) / kTM;
   if (ntiles == 0) return cudaSuccess;
-  cudaError_t e = zero ? cudaMemsetAsync(a.zh1, 0, sizeof(float) * kH * (size_t)a.N, st) : cudaSuccess;
+  cudaError_t e = zero && !kDet ? cudaMemsetAsync(a.zh1, 0, sizeof(float) * kH * (size_t)a.N, st) : cudaSuccess;
   if (e != cudaSuccess) return e;
-  if (cudaError_t e_ = launch_pdl(node_h_z_kernel, node_pre_grid(ntiles, a.C + 1, sms), kThreads, kNodeHSmem, st, a)) return e_;
+  const int zgrid = kDet ? persistent_grid(ntiles, 2 * sms) : node_pre_grid(ntiles, a.C + 1, sms);
+  if (cudaError_t e_ = launch_pdl(node_h_z_kernel<kDet>, zgrid, kThreads, kNodeHSmem, st, a)) return e_;
   if (cudaError_t e_ = launch_pdl(node_h_out_kernel, persistent_grid(ntiles, 2 * sms), kThreads, kNodeHSmem, st, a)) return e_;
   return cudaGetLastError();
 }

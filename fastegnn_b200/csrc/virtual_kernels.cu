@@ -17,7 +17,8 @@ struct VirtArgs {
   const int* batch;
   const float *x, *v, *Z, *Av, *G1, *tsum, *dinv, *sv, *sg;
   const float *wv1, *V2, *c2, *Wxv, *bxv, *wxv, *WX, *bX, *wX, *wav, *bav;
-  // forward outputs
+  // forward outputs.  The deterministic forward kernels (kDet) form no per-graph sum: Dsum then carries the [N, C, 3] rows
+  // D sX that det_graph_sums adds per graph (with u into Usum and x_new into xsum_new)
   float *u, *x_new, *Dsum, *Usum, *xsum_new;
   // backward inputs
   const float *gx_new, *gxsum_next, *gDsum, *gUsum, *gu;
@@ -190,6 +191,7 @@ __device__ __forceinline__ void virt_rows_to_graph(const float* __restrict__ T, 
 constexpr size_t kVirtFwdSmem = (3 * kWFloats + 2 * kTileFloats) * sizeof(float) + sizeof(VirtSmem);
 constexpr size_t kVirtBwdSmem = (3 * kWFloats + 5 * kTileFloats) * sizeof(float) + sizeof(VirtSmem);
 
+template <bool kDet>
 __global__ void __launch_bounds__(kThreads, 1) virtual_fwd_kernel(VirtArgs a) {
   extern __shared__ __align__(16) float smem[];
   float* V2s = smem;
@@ -209,7 +211,7 @@ __global__ void __launch_bounds__(kThreads, 1) virtual_fwd_kernel(VirtArgs a) {
     virt_geometry<false>(a, s, tile, TN);
     __syncthreads();
     const bool single = s->b_first == s->b_last;
-    if (!single || s->b_first != cur_b) {
+    if (!kDet && (!single || s->b_first != cur_b)) {
       const int nb = single ? s->b_first : -1;
       virt_flush(s, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
       cur_b = nb;
@@ -238,7 +240,7 @@ __global__ void __launch_bounds__(kThreads, 1) virtual_fwd_kernel(VirtArgs a) {
       }
     }
     __syncthreads();
-    virt_rows_to_graph(T2, s, C, TN, single, a.Usum);
+    if (!kDet) virt_rows_to_graph(T2, s, C, TN, single, a.Usum);
     // phi_xv head
     zero_acc(acc);
     gemm_nt(acc, T2, Wxvs, ty, tx);
@@ -277,7 +279,8 @@ __global__ void __launch_bounds__(kThreads, 1) virtual_fwd_kernel(VirtArgs a) {
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
           float val = s->sD[tid * 3 + k] * sX;
-          if (single) atomicAdd(&s->accSmall[k * C + c], val);
+          if (kDet) a.Dsum[((size_t)tile * TN * C + tid) * 3 + k] = val;
+          else if (single) atomicAdd(&s->accSmall[k * C + c], val);
           else atomicAdd(a.Dsum + ((size_t)b * 3 + k) * C + c, val);
         }
       }
@@ -298,13 +301,14 @@ __global__ void __launch_bounds__(kThreads, 1) virtual_fwd_kernel(VirtArgs a) {
                      svi * a.v[(size_t)i * 3 + k];
           if (grav) xn += sgi * a.grav[k];
           a.x_new[(size_t)i * 3 + k] = xn;
+          if (kDet) continue;
           if (single) atomicAdd(&s->accX[k], xn);
           else atomicAdd(a.xsum_new + (size_t)b * 3 + k, xn);
         }
       }
     }
   }
-  virt_flush(s, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
+  if (!kDet) virt_flush(s, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
 }
 
 __global__ void __launch_bounds__(kThreads, 1) virtual_bwd_kernel(VirtArgs a) {
@@ -557,10 +561,11 @@ __global__ void __launch_bounds__(kThreads, 1) virtual_bwd_kernel(VirtArgs a) {
   }
 }
 
+template <bool kDet = false>
 cudaError_t launch_virtual_fwd(const VirtArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(virtual_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kVirtFwdSmem);
+    cudaError_t e = cudaFuncSetAttribute(virtual_fwd_kernel<kDet>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kVirtFwdSmem);
     if (e != cudaSuccess) return e;
     attr.set();
   }
@@ -568,7 +573,7 @@ cudaError_t launch_virtual_fwd(const VirtArgs& a, int sms, cudaStream_t st) {
   int ntiles = (a.N + TN - 1) / TN;
   if (ntiles == 0) return cudaSuccess;
   int grid = ntiles < sms ? ntiles : sms;
-  virtual_fwd_kernel<<<grid, kThreads, kVirtFwdSmem, st>>>(a); ++g_launches;
+  virtual_fwd_kernel<kDet><<<grid, kThreads, kVirtFwdSmem, st>>>(a); ++g_launches;
   return cudaGetLastError();
 }
 cudaError_t launch_virtual_bwd(const VirtArgs& a, int sms, cudaStream_t st) {

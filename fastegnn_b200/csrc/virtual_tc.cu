@@ -213,7 +213,8 @@ struct FwdSmem {
 };
 constexpr uint32_t kF_ACC0 = 0, kF_ACCH = 64, kF_OPA = 192;    // 256 columns
 
-template <int CG>
+// kDet: no per-graph sums; the rows D sX go to the [N, C, 3] buffer in the Dsum slot (VirtArgs)
+template <int CG, bool kDet>
 __global__ void __launch_bounds__(128 * CG, 2) virtual_fwd_tc_kernel(VirtArgs a) {
   VTR_DECL();
   constexpr int NT = 128 * CG, CPT = kH / CG, NW = NT / 32;
@@ -297,7 +298,7 @@ __global__ void __launch_bounds__(128 * CG, 2) virtual_fwd_tc_kernel(VirtArgs a)
     __syncthreads();
     VTR();
     const bool single = v->b_first == v->b_last;
-    if (!single || v->b_first != cur_b) {
+    if (!kDet && (!single || v->b_first != cur_b)) {
       const int nb = single ? v->b_first : -1;
       acc_flush<NT>(&v->acc, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
       cur_b = nb;
@@ -384,7 +385,7 @@ __global__ void __launch_bounds__(128 * CG, 2) virtual_fwd_tc_kernel(VirtArgs a)
           *reinterpret_cast<float4*>(ubase + (size_t)rr * kH + 4 * c16) = *reinterpret_cast<const float4*>(T + mn_chunk_off(rr, c16, kTM));
       }
     }
-    rows_to_graph<NT>(T, v->skey, &v->acc, C, TN, single, a.Usum);                 // overlaps GH
+    if (!kDet) rows_to_graph<NT>(T, v->skey, &v->acc, C, TN, single, a.Usum);       // overlaps GH
     umma::mbar_wait(&v->bar[1], phase);
     VTR();
     umma::fence_after();
@@ -417,14 +418,15 @@ __global__ void __launch_bounds__(128 * CG, 2) virtual_fwd_tc_kernel(VirtArgs a)
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
           val[k] = v->sD[t * 3 + k] * sX;
-          if (!single) atomicAdd(a.Dsum + ((size_t)b * 3 + k) * C + c, val[k]);
+          if (kDet) a.Dsum[((size_t)tile * TN * C + t) * 3 + k] = val[k];
+          else if (!single) atomicAdd(a.Dsum + ((size_t)b * 3 + k) * C + c, val[k]);
         }
       }
       v->sval[t * 3 + 0] = val[0]; v->sval[t * 3 + 1] = val[1]; v->sval[t * 3 + 2] = val[2];
     }
     __syncthreads();
     VTR();
-    if (single && warp == NW - 1) small_from_rows(v->sval, &v->acc, C, TN, lane);
+    if (!kDet && single && warp == NW - 1) small_from_rows(v->sval, &v->acc, C, TN, lane);
     if (warp * 32 < TN) {                 // x' (models/FastEGNN.py:133-142) and its per-graph sum
       const int i = tile * TN + t;
       float xs[3] = {0.f, 0.f, 0.f};
@@ -441,10 +443,10 @@ __global__ void __launch_bounds__(128 * CG, 2) virtual_fwd_tc_kernel(VirtArgs a)
           if (grav) xn += sgi * a.grav[k];
           a.x_new[(size_t)i * 3 + k] = xn;
           xs[k] = xn;
-          if (!single) atomicAdd(a.xsum_new + (size_t)b * 3 + k, xn);
+          if (!kDet && !single) atomicAdd(a.xsum_new + (size_t)b * 3 + k, xn);
         }
       }
-      if (single) {                       // one shared atomic per warp and coordinate instead of one per node
+      if (!kDet && single) {                       // one shared atomic per warp and coordinate instead of one per node
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
           float sum = xs[k];
@@ -455,7 +457,7 @@ __global__ void __launch_bounds__(128 * CG, 2) virtual_fwd_tc_kernel(VirtArgs a)
       }
     }
   }
-  acc_flush<NT>(&v->acc, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
+  if (!kDet) acc_flush<NT>(&v->acc, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
   umma::fence_before();
   __syncthreads();
     VTR();
@@ -1241,12 +1243,12 @@ __global__ void __launch_bounds__(128 * CG, 1) virtual_bwd_trunk_tc_kernel(VirtA
 
 }  // namespace vtc
 
-template <int CG>
+template <int CG, bool kDet = false>
 cudaError_t launch_virtual_fwd_tc(const VirtArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   const size_t bytes = vtc::FwdSmem::bytes;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(vtc::virtual_fwd_tc_kernel<CG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    cudaError_t e = cudaFuncSetAttribute(vtc::virtual_fwd_tc_kernel<CG, kDet>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
     attr.set();
   }
@@ -1254,7 +1256,7 @@ cudaError_t launch_virtual_fwd_tc(const VirtArgs& a, int sms, cudaStream_t st) {
   const int ntiles = (a.N + TN - 1) / TN;
   if (ntiles == 0) return cudaSuccess;
   const int grid = ntiles < 2 * sms ? ntiles : 2 * sms;
-  if (cudaError_t e_ = launch_pdl(vtc::virtual_fwd_tc_kernel<CG>, grid, 128 * CG, bytes, st, a)) return e_;
+  if (cudaError_t e_ = launch_pdl(vtc::virtual_fwd_tc_kernel<CG, kDet>, grid, 128 * CG, bytes, st, a)) return e_;
   return cudaGetLastError();
 }
 

@@ -166,7 +166,10 @@ unsigned long long fegnn_launch_count(void);
  * forms whose every sum has a fixed order: repeated calls with the same inputs on the same device model and SM count give
  * bitwise identical results, whatever the timing (eager or graph replay, other work on other streams, a fresh process);
  * the forwards take a workspace of fegnn_loss_workspace_floats.  fegnn_adam_step, fegnn_graph_prep and the radius graph are deterministic in either mode.
- * Every entry that adds floats across CTAs in arrival order and has no such form -- the layer phases, fegnn_model_*,
+ * fegnn_model_forward_inference runs the same way under 1, with the extra workspace of
+ * fegnn_model_inference_det_workspace_floats.
+ * Every entry that adds floats across CTAs in arrival order and has no such form -- the layer phases, fegnn_model_forward,
+ * fegnn_model_backward[_inputs],
  * fegnn_embed_backward, fegnn_graph_xsum, fegnn_rf_vel_backward, fegnn_segment_reduce, fegnn_halo_reduce_push and
  * fegnn_p2p_allreduce -- returns FEGNN_EINVAL under 1, naming the reason, instead of running.
  * "layer_overlap": 1 (default, auto), 2 or 0; the environment variable FEGNN_LAYER_OVERLAP sets the starting value.
@@ -400,8 +403,13 @@ int fegnn_model_forward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn
  * as fegnn_model_forward, but nothing is kept for a backward -- the layers ping-pong between two state sets and share ONE
  * block of per-layer intermediates (workspace = 3 states + 1 block instead of (L + 1) states + L blocks); up to 65 536 nodes
  * a ring of FOUR blocks (layer l uses block l % 4), which takes the per-layer join + fork, the accumulator fills and the
- * phi_h weight images out of the kernel chain. */
+ * phi_h weight images out of the kernel chain.
+ * Under the "deterministic" mode the phases run their deterministic forms, which need workspace_floats >= the sum of the two
+ * queries below (FEGNN_ENOMEM before any launch otherwise); their scratch lies behind the first query's floats. */
 size_t fegnn_model_inference_workspace_floats(const fegnn_dims* d);
+/* 0 with the "deterministic" mode off; with it on, the scratch of the deterministic forms (edge tile-boundary row sums, the
+ * virtual phase's per-row D sX and the per-graph chunk sums) */
+size_t fegnn_model_inference_det_workspace_floats(const fegnn_dims* d);
 int fegnn_model_forward_inference(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn_graph* g,
                                   const fegnn_layer_params* layers_host, const float* embed_w, const float* embed_b,
                                   const float* virtual_node_feat, const float* node_feat, const float* x0, const float* v,

@@ -7,9 +7,11 @@ Make each log from a checkout of the build it describes (nvcc prints the listing
 
     python tools/ptxas_compare.py parent.log this.log > profiles/input_grads_ptxas.txt
 
-Kernels are matched by mangled name after two renamings that do not change the code: the anonymous namespace of api.cu
-(its hash depends on the source path) and the `kEa = false` instantiations of edge_bwd_kernel / edge_bwd_tc4_kernel, which
-are the parent's untemplated (resp. single-parameter) kernels.  Every kernel of both builds is listed with its resource
+Kernels are matched by mangled name, a name the parent lacks after renamings that do not change the code: the anonymous
+namespace of api.cu (its hash depends on the source path), the `kEa = false` instantiations of edge_bwd_kernel /
+edge_bwd_tc4_kernel and the `kDet = false` instantiations of the forward kernels (edge_fwd_kernel, edge_fwd_tc_kernel,
+virtual_fwd_kernel, virtual_fwd_tc_kernel, node_h_z_kernel), which are a parent's untemplated (resp. one-parameter
+fewer) kernels.  Every kernel of both builds is listed with its resource
 lines (stack frame, spills, registers, barriers, shared memory; constant-bank sizes are left out)."""
 import re
 import sys
@@ -30,14 +32,25 @@ def parse(path):
     return out
 
 
-def to_parent(name):
-    name = name.replace("edge_bwd_kernelILb0EEEvNS_8EdgeArgsE", "edge_bwd_kernelENS_8EdgeArgsE")
-    return re.sub(r"edge_bwd_tc4_kernelILi(\d)ELb0EEEvNS_8EdgeArgsEPKj", r"edge_bwd_tc4_kernelILi\1EEEvNS_8EdgeArgsEPKj", name)
+# a trailing bool template parameter (false) that a parent does not have: "kernelI<args>Lb0EEEv" -> "kernelI<args>EEv",
+# and a kernel whose only template parameter it is: "kernelILb0EEEvNS_" -> "kernelENS_"
+BOOL_ADDED = ("edge_bwd_kernel", "edge_bwd_tc4_kernel", "edge_fwd_kernel", "edge_fwd_tc_kernel", "virtual_fwd_kernel",
+              "virtual_fwd_tc_kernel", "node_h_z_kernel")
+
+
+def to_parent(name, parent):
+    if name in parent:
+        return name
+    for k in BOOL_ADDED:
+        if f"{len(k)}{k}I" in name:
+            name = name.replace(f"{k}ILb0EEEvNS_", f"{k}ENS_")
+            return re.sub(rf"({k}I(?:Li\d+E)+)Lb0EEEv", r"\1EEv", name)
+    return name
 
 
 def main(parent_log, this_log):
     a, b = parse(parent_log), parse(this_log)
-    matched = {k: to_parent(k) for k in b if to_parent(k) in a}
+    matched = {k: to_parent(k, a) for k in b if to_parent(k, a) in a}
     same = sum(a[p] == b[k] for k, p in matched.items())
     new = [k for k in b if k not in matched]
     gone = [p for p in a if p not in set(matched.values())]
