@@ -117,15 +117,20 @@ class _StackFn(torch.autograd.Function):
     """FastEGNN.forward / backward as two C calls (fegnn_model_forward / fegnn_model_backward_inputs).
 
     node_attr is the contiguous fp32 copy the kernels read; attr_in / edge_attr_in are the caller's tensors (or None), which
-    are inputs here only so that autograd can hand them their gradients.  The kernels read edge_attr from the graph."""
+    are inputs here only so that autograd can hand them their gradients.  The kernels read edge_attr from the graph.
+    With mod.recompute the flag word carries FEGNN_F_RECOMPUTE: the workspace holds the states and two saved blocks, and
+    the backward (which reads the flag from ctx.dims, not from the module) rebuilds each layer's block.  A recompute
+    backward leaves the two blocks holding other layers than the forward did, so a further backward over the same graph
+    (retain_graph=True) passes FEGNN_F_REBUILD_ALL and rebuilds every layer."""
 
     @staticmethod
     def forward(ctx, mod: "FastEGNN", graph: CsrGraph, node_attr, attr_in, edge_attr_in, node_feat, x0, v, loc_mean,
                 *params):
         dev = x0.device
         N, B, Cc, Lyr = graph.N, graph.B, mod.virtual_channels, mod.n_layers
-        dims = make_dims(N, N, graph.E, B, Cc, graph.Fe, mod._flag_word, mod._gravity, Fa=mod._node_attr_nf,
-                         node_attr=node_attr)
+        recompute = bool(mod.recompute)
+        flags = mod._flag_word | (L.F_RECOMPUTE if recompute else 0)
+        dims = make_dims(N, N, graph.E, B, Cc, graph.Fe, flags, mod._gravity, Fa=mod._node_attr_nf, node_attr=node_attr)
         pd = C.byref(dims)
         table, names = mod._param_table()
         ws_floats = int(lib.fegnn_model_workspace_floats(pd, Lyr))
@@ -139,6 +144,8 @@ class _StackFn(torch.autograd.Function):
                                             L.ptr(x0), L.ptr(v), L.ptr(loc_mean), L.ptr(x_out), L.ptr(Z_out), L.ptr(ws),
                                             ws_floats, _stream(dev)), "fegnn_model_forward")
         ctx.mod, ctx.graph, ctx.dims, ctx.ws, ctx.Fin = mod, graph, dims, ws, Fin
+        ctx.recompute = recompute                               # the backward follows this step's forward
+        ctx.blocks_consumed = False                             # recompute: set by the first backward (see above)
         ctx.save_for_backward(node_feat, v, node_attr)          # node_attr: dims points at it until the backward
         ctx.names = names
         ctx.need_nf = node_feat.requires_grad
@@ -154,6 +161,9 @@ class _StackFn(torch.autograd.Function):
         node_feat, v, _ = ctx.saved_tensors
         dev = v.device
         N, B, Cc, Lyr = graph.N, graph.B, mod.virtual_channels, mod.n_layers
+        if ctx.recompute and ctx.blocks_consumed:
+            dims = type(dims).from_buffer_copy(dims)
+            dims.flags |= L.F_REBUILD_ALL
         pd = C.byref(dims)
         gx = torch.zeros(N, 3, device=dev) if gx is None else gx.contiguous().float()
         gZ = torch.zeros(B, 3, Cc, device=dev) if gZ is None else gZ.contiguous().float()
@@ -178,6 +188,7 @@ class _StackFn(torch.autograd.Function):
                                                     L.ptr(node_feat), L.ptr(v), L.ptr(gx), L.ptr(gZ), L.ptr(g_x0),
                                                     L.ptr(g_lm), L.ptr(g_nf), L.ptr(ctx.ws), L.ptr(scratch), scr_floats,
                                                     C.byref(ig), _stream(dev)), "fegnn_model_backward_inputs")
+        ctx.blocks_consumed = ctx.recompute
         dead = mod._dead_names
         grads = tuple(None if n in dead else views[n] for n in names)
         dt_na, dt_ea, dt_v = ctx.in_dtypes
@@ -214,8 +225,15 @@ class FastEGNN(nn.Module):
     eval_keeps_graph (attribute, default False): the reference's evaluation epochs (utils/train.py:24-27,191-192) run the
     model under model.eval() WITHOUT torch.no_grad(), building an autograd graph nobody uses.  Here a forward in eval mode
     -- or under torch.no_grad() -- takes the forward-only stack (fegnn_model_forward_inference): same outputs, no saved
-    activations, outputs without grad_fn.  Set eval_keeps_graph = True to get the training forward in eval mode."""
+    activations, outputs without grad_fn.  Set eval_keeps_graph = True to get the training forward in eval mode.
+
+    recompute (attribute, default False): activation checkpointing for the training stack.  The forward keeps only the
+    n_layers + 1 layer states and the backward rebuilds each layer's intermediates just before that layer's backward, so a
+    step holds two saved blocks instead of n_layers (about 1.5 KB + 256 B * virtual_channels per node each) for about one
+    more forward per step (DESIGN 3.8).  Same results up to float summation order.  A step's backward follows the setting
+    of its forward.  The eval() / no_grad forward-only stack is unaffected."""
     eval_keeps_graph = False
+    recompute = False
     _node_attr_nf = 0          # subclasses without node attributes (FastRF) inherit forward and the stack functions
 
     def __init__(self, node_feat_nf, node_attr_nf, edge_attr_nf, hidden_nf, virtual_channels, device='cpu',

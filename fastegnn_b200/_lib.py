@@ -21,6 +21,8 @@ MAX_FE = 8
 MAX_FA = 16
 
 F_ATTENTION, F_NORMALIZE, F_TANH, F_GRAVITY, F_LAST, F_RF, F_COORDS_SUM, F_NODE_SUM, F_PREZEROED = 1, 2, 4, 8, 16, 32, 64, 128, 256
+F_RECOMPUTE = 2048          # training stack: two saved blocks, each layer's rebuilt in the backward (DESIGN 3.8)
+F_REBUILD_ALL = 4096        # with F_RECOMPUTE: a backward after another one over the same forward rebuilds every layer
 
 fp = C.POINTER(C.c_float)
 ip = C.POINTER(C.c_int32)

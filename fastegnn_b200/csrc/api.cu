@@ -55,6 +55,14 @@ int fail(int code, const char* fmt, ...) {
     if (g_det) return fail(FEGNN_EINVAL, "%s has no deterministic form (%s); set mode \"deterministic\" to 0 to run it", \
                            __func__, why);                                                                         \
   } while (0)
+// FEGNN_F_RECOMPUTE is read by the fegnn_model_* entries (and selects the saved-only forms of the virtual and phi_h forwards);
+// every other per-layer entry refuses it
+#define NO_RECOMPUTE(d)                                                                                            \
+  do {                                                                                                             \
+    if ((d) != nullptr && ((d)->flags & (FEGNN_F_RECOMPUTE | FEGNN_F_REBUILD_ALL)))                                \
+      return fail(FEGNN_EINVAL, "%s: FEGNN_F_RECOMPUTE is a flag of the fegnn_model_* entries (and of the saved-only " \
+                  "fegnn_virtual_forward / fegnn_node_h_forward)", __func__);                                       \
+  } while (0)
 #define TRY(expr)            \
   do {                       \
     int rc__ = (expr);       \
@@ -518,14 +526,23 @@ int virtual_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_l
                         const DetWs* det, void* stream) {
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
-  RQ(g && x && v && Z && sv && x_new && xsum_new);
+  // FEGNN_F_RECOMPUTE: the saved-only form (u, Dsum, Usum; x' and xsum_new are the next layer's state already)
+  const bool saved_only = d->flags & FEGNN_F_RECOMPUTE;
+  RQ(g && x && v && Z && sv && (saved_only || (x_new && xsum_new)));
+  RQ(!saved_only || det == nullptr);
   VirtArgs a = virt_args(d, g, p, x, v, Z, sv);
   a.u = sv->u; a.x_new = x_new; a.Dsum = sv->Dsum; a.Usum = sv->Usum; a.xsum_new = xsum_new;
   if (!(d->flags & FEGNN_F_PREZEROED)) {
     CK(zero_pair(sv->Dsum, 3 * d->C * (size_t)d->B, sv->Usum, kH * d->C * (size_t)d->B, S(stream)));
-    CK(cudaMemsetAsync(xsum_new, 0, sizeof(float) * 3 * (size_t)d->B, S(stream)));
+    if (!saved_only) CK(cudaMemsetAsync(xsum_new, 0, sizeof(float) * 3 * (size_t)d->B, S(stream)));
   }
   const bool tc = g_virt_fwd_mode == 1 && !(d->flags & FEGNN_F_ATTENTION);
+  if (saved_only) {
+    a.x_new = nullptr; a.xsum_new = nullptr;
+    if (tc) CK((launch_virtual_fwd_tc<2, false, true>(a, sm_count(), S(stream))));
+    else CK((launch_virtual_fwd<false, true>(a, sm_count(), S(stream))));
+    return 0;
+  }
   if (det != nullptr) {
     // the kernel writes u, x_new and the rows D sX (into the Dsum slot); their per-graph sums follow in graph order
     a.Dsum = det->dval;
@@ -548,7 +565,10 @@ int virtual_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_l
 int node_h_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* h,
                        fegnn_layer_saved* sv, float* h_new, const DetWs* det, void* stream) {
   TRY(check_dims(d));
-  RQ(g && p && h && sv && h_new);
+  // FEGNN_F_RECOMPUTE: the saved-only form (zh1; h' is the next layer's state already)
+  const bool saved_only = d->flags & FEGNN_F_RECOMPUTE;
+  RQ(g && p && h && sv && (saved_only || h_new));
+  RQ(!saved_only || det == nullptr);
   NodeHArgs a;
   memset(&a, 0, sizeof(a));
   a.N = d->N; a.C = d->C; a.ldn = ldn(d);
@@ -563,8 +583,10 @@ int node_h_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_la
       float* img = sv->wimg;
       CK(launch_node_h_wprep(d->C, ldn(d), 1, &w0, &w2, &img, S(stream)));
     }
-    CK(launch_node_h_fwd_tc(a, sm_count(), S(stream)));
+    if (saved_only) CK(launch_node_h_fwd_tc<true>(a, sm_count(), S(stream)));
+    else CK(launch_node_h_fwd_tc(a, sm_count(), S(stream)));
   }
+  else if (saved_only) CK((launch_node_h_fwd<false, true>(a, sm_count(), S(stream), !(d->flags & FEGNN_F_PREZEROED))));
   else if (det != nullptr) CK(launch_node_h_fwd<true>(a, sm_count(), S(stream)));
   else CK(launch_node_h_fwd(a, sm_count(), S(stream), !(d->flags & FEGNN_F_PREZEROED)));
   return 0;
@@ -574,6 +596,7 @@ int node_h_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_la
 extern "C" {
 int fegnn_node_h_weight_images(const fegnn_dims* d, int32_t nl, const fegnn_layer_params* layers, float* const* wimg,
                                void* stream) {
+  NO_RECOMPUTE(d);
   TRY(check_dims(d));
   RQ(nl >= 0 && nl <= 32 && (nl == 0 || (layers && wimg)));
   const float *w0[32], *w2[32];
@@ -601,18 +624,21 @@ int graph_post_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegn
 extern "C" {
 int fegnn_graph_pre_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* Z,
                             const float* Sf, const float* xsum, fegnn_layer_saved* sv, void* stream) {
+  NO_RECOMPUTE(d);
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   return graph_pre_forward_run(d, g, p, Z, Sf, xsum, sv, stream);
 }
 
 int fegnn_node_pre_forward(const fegnn_dims* d, const fegnn_layer_params* p, const float* h, fegnn_layer_saved* sv,
                            void* stream) {
+  NO_RECOMPUTE(d);
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   return node_pre_forward_run(d, p, h, sv, stream);
 }
 
 int fegnn_edge_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* x,
                        fegnn_layer_saved* sv, void* stream) {
+  NO_RECOMPUTE(d);
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   return edge_forward_run(d, g, p, x, sv, nullptr, stream);
 }
@@ -632,6 +658,7 @@ int fegnn_node_h_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_
 
 int fegnn_graph_post_forward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, const float* Z,
                              const float* Sf, const fegnn_layer_saved* sv, float* Z_new, float* S_new, void* stream) {
+  NO_RECOMPUTE(d);
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   return graph_post_forward_run(d, g, p, Z, Sf, sv, Z_new, S_new, stream);
 }
@@ -641,6 +668,7 @@ int fegnn_graph_post_backward(const fegnn_dims* d, const fegnn_graph* g, const f
                               fegnn_layer_grads* gr, const float* Sf, const fegnn_layer_saved* sv,
                               const float* gZ_new, const float* gS_new, float* gZ, float* gS, float* gDsum,
                               float* gUsum, void* stream) {
+  NO_RECOMPUTE(d);
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   const bool last = d->flags & FEGNN_F_LAST;
@@ -656,6 +684,7 @@ int fegnn_graph_post_backward(const fegnn_dims* d, const fegnn_graph* g, const f
 int fegnn_node_h_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
                           fegnn_layer_grads* gr, const fegnn_layer_saved* sv, const float* gh_new, float* gzh1,
                           float* gm, float* gu, void* stream) {
+  NO_RECOMPUTE(d);
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(g && p && gr && sv && gh_new && gzh1 && gm && gu);
@@ -755,6 +784,7 @@ int fegnn_virtual_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, con
                                   const fegnn_layer_saved* sv, const float* gx_new, const float* gxsum_next,
                                   const float* gDsum, const float* gUsum, const float* gu, float* gAv, float* gG1, float* gx,
                                   float* gZ, float* gsv, float* gsg, float* gt, const fegnn_input_grads* ig, void* stream) {
+  NO_RECOMPUTE(d);
   return virtual_backward_run(d, g, p, gr, x, v, Z, sv, gx_new, gxsum_next, gDsum, gUsum, gu, gAv, gG1, gx, gZ, gsv, gsg, gt,
                               ig, false, sm_count(), stream);
 }
@@ -809,12 +839,14 @@ static int edge_backward_run(const fegnn_dims* d, const fegnn_graph* g, const fe
 int fegnn_edge_backward_inputs(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p, fegnn_layer_grads* gr,
                                const float* x, const fegnn_layer_saved* sv, const float* gm, const float* gt, float* gP,
                                float* gQ, float* gx, const fegnn_input_grads* ig, void* stream) {
+  NO_RECOMPUTE(d);
   return edge_backward_run(d, g, p, gr, x, sv, gm, gt, gP, gQ, gx, ig, nullptr, sm_count(), stream);
 }
 
 int fegnn_graph_pre_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_params* p,
                              fegnn_layer_grads* gr, const float* Sf, const fegnn_layer_saved* sv, const float* gG1,
                              float* gS, float* gZ, float* gxsum, void* stream) {
+  NO_RECOMPUTE(d);
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(g && p && gr && Sf && sv && gG1 && gS && gZ && gxsum);
@@ -833,6 +865,7 @@ int fegnn_node_pre_backward(const fegnn_dims* d, const fegnn_layer_params* p, fe
 int fegnn_node_pre_backward_inputs(const fegnn_dims* d, const fegnn_layer_params* p, fegnn_layer_grads* gr, const float* h,
                                    const float* gP, const float* gQ, const float* gAv, const float* gUh, const float* gsv,
                                    const float* gsg, float* gh, const fegnn_input_grads* ig, void* stream) {
+  NO_RECOMPUTE(d);
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
@@ -1008,13 +1041,15 @@ namespace {
 struct ModelWs {
   // per layer l in [0, L]: state entering layer l (index L = outputs)
   float *h[33], *x[33], *Z[33], *Sx[33], *xsum[33];
-  fegnn_layer_saved saved[32];
+  fegnn_layer_saved saved[32];      // FEGNN_F_RECOMPUTE: layer l's block is block l % 2 of a ring of two (DESIGN 3.8)
 };
 
+// saved blocks of the training stack: one per layer, or with FEGNN_F_RECOMPUTE a ring of min(L, 2)
+inline int model_blocks(const fegnn_dims* d, int L) { return (d->flags & FEGNN_F_RECOMPUTE) ? (L < 2 ? L : 2) : L; }
 size_t model_ws_floats(const fegnn_dims* d, int L) {
   const size_t N = d->N, Nl = d->Nl, B = d->B, C = d->C;
   size_t per_state = al4(N * kH) + al4(Nl * 3) + al4(B * 3 * C) + al4(B * C * kH) + al4(B * 3);
-  return (size_t)(L + 1) * per_state + (size_t)L * fegnn_layer_saved_floats(d);
+  return (size_t)(L + 1) * per_state + (size_t)model_blocks(d, L) * fegnn_layer_saved_floats(d);
 }
 void model_ws_bind(const fegnn_dims* d, int L, float* base, ModelWs* w) {
   const size_t N = d->N, Nl = d->Nl, B = d->B, C = d->C;
@@ -1024,9 +1059,14 @@ void model_ws_bind(const fegnn_dims* d, int L, float* base, ModelWs* w) {
   for (int l = 0; l <= L; ++l) {
     w->h[l] = take(N * kH); w->x[l] = take(Nl * 3); w->Z[l] = take(B * 3 * C); w->Sx[l] = take(B * C * kH);
   }
+  const int nb = model_blocks(d, L);
   for (int l = 0; l < L; ++l) {
-    fegnn_layer_saved_bind(d, p, &w->saved[l]);
-    p += fegnn_layer_saved_floats(d);
+    if (l < nb) {
+      fegnn_layer_saved_bind(d, p, &w->saved[l]);
+      p += fegnn_layer_saved_floats(d);
+    } else {
+      w->saved[l] = w->saved[l % nb];
+    }
   }
 }
 
@@ -1092,18 +1132,24 @@ int fegnn_model_forward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn
   }
   // every accumulator of the step is zero-filled here, ahead of the kernel chain (the phases then skip their own fills):
   // the per-graph coordinate sums of all states, and the accumulator head of every layer's saved block
+  // (FEGNN_F_RECOMPUTE: the blocks form a ring of nb = min(L, 2); the block of a layer l >= nb is filled on the side stream
+  // during layer l - 1, below -- a memset node between two kernels of the chain would cut their programmatic overlap)
+  const bool rc = d->flags & FEGNN_F_RECOMPUTE;
+  const int nb = model_blocks(d, L);
   CK(cudaMemsetAsync(w.xsum[0], 0, sizeof(float) * ((size_t)L * al4(B * 3) + B * 3), st));
-  for (int l = 0; l < L; ++l)
+  for (int l = 0; l < nb; ++l)
     CK(cudaMemsetAsync(w.saved[l].msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), st));
   const bool rf = d->flags & FEGNN_F_RF;          // FastRF: h and S pass through every layer (models/FastRF.py:186)
   // phi_h on the tensor cores: the operand-tile images of every layer's weight blocks in ONE launch here -- weights only, so it
-  // runs ahead of the chain and (graph_pending) under the CSR sort
+  // runs ahead of the chain and (graph_pending) under the CSR sort.  Ring: the first nb layers' here, layer l + 1 >= nb's on
+  // the side stream next to graph_post(l) (its block's images were last read by phi_h of layer l + 1 - nb, ahead of the fork)
   bool wimg_ready = false;
+  const int nimg_top = nb < L - 1 ? nb : L - 1;   // the last layer has no phi_h
   if (g_node_fwd_mode != 0 && !rf && L > 1) {
     const float *w0[32], *w2[32];
     float* img[32];
-    for (int l = 0; l + 1 < L; ++l) { w0[l] = layers[l].node_w0; w2[l] = layers[l].node_w2; img[l] = w.saved[l].wimg; }
-    CK(launch_node_h_wprep(d->C, ldn(d), L - 1, w0, w2, img, st));
+    for (int l = 0; l < nimg_top; ++l) { w0[l] = layers[l].node_w0; w2[l] = layers[l].node_w2; img[l] = w.saved[l].wimg; }
+    CK(launch_node_h_wprep(d->C, ldn(d), nimg_top, w0, w2, img, st));
     wimg_ready = true;
   }
   const bool graph_pending = g->ready_event != nullptr;
@@ -1111,6 +1157,7 @@ int fegnn_model_forward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn
     // the CSR sort is still running on another stream: everything above and the first layer's node phase read no graph
     // array and run under it; this stream joins the sort here
     fegnn_dims d0 = *d;
+    d0.flags &= ~(FEGNN_F_RECOMPUTE | FEGNN_F_REBUILD_ALL);
     d0.flags |= FEGNN_F_PREZEROED;
     if (rf || L == 1) d0.flags |= FEGNN_F_LAST;
     TRY(fegnn_node_pre_forward(&d0, &layers[0], w.h[0], &w.saved[0], stream));
@@ -1123,6 +1170,7 @@ int fegnn_model_forward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn
   FORK(sd, st);                                   // side: graph_pre(0)
   for (int l = 0; l < L; ++l) {
     fegnn_dims dl = *d;
+    dl.flags &= ~(FEGNN_F_RECOMPUTE | FEGNN_F_REBUILD_ALL);   // the phases run their full forms
     dl.flags |= FEGNN_F_PREZEROED;
     if (wimg_ready) dl.flags |= FEGNN_F_WIMG_READY;
     const bool last = rf || l == L - 1;
@@ -1130,6 +1178,7 @@ int fegnn_model_forward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn
     const fegnn_layer_params* p = &layers[l];
     fegnn_layer_saved* sv = &w.saved[l];
     const int ls = rf ? 0 : l;                    // layer whose (h, S) state this layer reads
+    if (rc && l >= nb) CK(cudaStreamWaitEvent(st, sd->aux, 0));        // ring: this block's fill (side, during layer l - 1)
     TRY(fegnn_graph_pre_forward(&dl, g, p, w.Z[l], w.Sx[ls], w.xsum[l], sv, side));      // side (1 CTA per graph)
     if (!(graph_pending && l == 0)) TRY(fegnn_node_pre_forward(&dl, p, w.h[ls], sv, stream));
     if (rf) TRY(fegnn_rf_vel_forward(d->N, v, p, sv->sv, stream));
@@ -1137,8 +1186,19 @@ int fegnn_model_forward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn
     JOIN(sd, st);                                 // virtual needs G1, M of graph_pre
     TRY(fegnn_virtual_forward(&dl, g, p, w.x[l], v, w.Z[l], sv, w.x[l + 1], w.xsum[l + 1], stream));
     FORK(sd, st);                                 // side: graph_post(l) [-> graph_pre(l+1)] under node_h, node_pre, edge
+    if (rc && l + 1 >= nb && l + 1 < L) {
+      // ring: the accumulators of the block layer l + 1 reuses, last read by layer l + 1 - nb (node phase on this stream ahead
+      // of the fork, per-graph kernels earlier on the side stream)
+      CK(cudaMemsetAsync(w.saved[l + 1].msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), S(side)));
+      CK(cudaEventRecord(sd->aux, S(side)));
+    }
     if (!last) TRY(fegnn_node_h_forward(&dl, g, p, w.h[l], sv, w.h[l + 1], stream));
     TRY(fegnn_graph_post_forward(&dl, g, p, w.Z[l], w.Sx[ls], sv, w.Z[l + 1], w.Sx[l + 1], side));
+    if (rc && wimg_ready && l + 2 < L && l + 1 >= nimg_top) {
+      const float *w0 = layers[l + 1].node_w0, *w2 = layers[l + 1].node_w2;
+      float* img = w.saved[l + 1].wimg;
+      CK(launch_node_h_wprep(d->C, ldn(d), 1, &w0, &w2, &img, S(side)));     // joined in front of virtual_forward(l + 1)
+    }
   }
   JOIN(sd, st);
   CK(cudaMemcpyAsync(x_out, w.x[L], sizeof(float) * 3 * N, cudaMemcpyDeviceToDevice, st));
@@ -1179,6 +1239,9 @@ int fegnn_model_forward_inference(const fegnn_dims* d, int32_t L, int32_t Fin, c
   TRY(check_dims(d));
   RQ(L >= 1 && L <= 32 && g && layers && embed_w && embed_b && vnf && workspace && x_out && Z_out);
   RQ(d->Nl == d->N);
+  fegnn_dims d_full = *d;                         // FEGNN_F_RECOMPUTE is a training-stack flag: nothing is kept here anyway
+  d_full.flags &= ~(FEGNN_F_RECOMPUTE | FEGNN_F_REBUILD_ALL);
+  d = &d_full;
   // deterministic mode: the kDet forms of the phases, with their scratch behind the workspace
   const size_t base_floats = fegnn_model_inference_workspace_floats(d);
   const size_t need = base_floats + fegnn_model_inference_det_workspace_floats(d);
@@ -1315,6 +1378,7 @@ int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, con
   TRY(check_input_grads(d, ig));
   RQ(L >= 1 && L <= 32 && g && layers && grads && embed_w && g_embed_w && g_embed_b && g_vnf && workspace && scratch);
   RQ(gx_out && gZ_out && g_x0 && g_loc_mean && d->Nl == d->N);
+  RQ(!(d->flags & FEGNN_F_REBUILD_ALL) || (d->flags & FEGNN_F_RECOMPUTE));
   if (scratch_floats < bwd_scratch_floats(d))
     return fail(FEGNN_ENOMEM, "backward scratch %zu < %zu floats", scratch_floats, bwd_scratch_floats(d));
   cudaStream_t st = S(stream);
@@ -1345,15 +1409,58 @@ int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, con
   void* side = sd->st;
   FORK(sd, st);                                   // side: graph_post_bwd(L-1)
   const bool rf = d->flags & FEGNN_F_RF;
-  for (int l = L - 1; l >= 0; --l) {
+  // FEGNN_F_RECOMPUTE (DESIGN 3.8): layer l's block is block l % 2.  The forward leaves the blocks of layers L - 1 and L - 2
+  // complete (unless a backward has run since: FEGNN_F_REBUILD_ALL); every layer below is rebuilt from its input state just before its backward (recompute(l)).  Its accumulator fill,
+  // phi_h weight images and graph_pre run on the side stream during backward(l + 1), behind the last readers of the block
+  // (backward(l + 2), ahead of the fork in front of graph_pre_bwd(l + 1)); the main stream waits for them (aux) at recompute(l).
+  // A backward leaves the ring blocks holding layers 0 / 1, not L - 1 / L - 2: a further backward over the same forward
+  // passes FEGNN_F_REBUILD_ALL and then rebuilds those two as well (the top layer's preparation runs ahead of the loop).
+  const bool rc = d->flags & FEGNN_F_RECOMPUTE;
+  const bool rebuild_all = d->flags & FEGNN_F_REBUILD_ALL;
+  const bool rc_img = g_node_fwd_mode != 0 && !rf;
+  auto recomputed = [&](int l) { return rc && l >= 0 && (rebuild_all || l + 2 < L); };
+  auto layer_dims = [&](int l) {
     fegnn_dims dl = *d;
+    dl.flags &= ~(FEGNN_F_RECOMPUTE | FEGNN_F_REBUILD_ALL);
     dl.flags |= FEGNN_F_PREZEROED;
+    if (rf || l == L - 1) dl.flags |= FEGNN_F_LAST;
+    return dl;
+  };
+  // side stream, ahead of recompute(l): the block's accumulator fill, layer l's phi_h weight images and graph_pre(l)
+  auto prepare = [&](int l) -> int {
+    const fegnn_dims dp = layer_dims(l);
+    fegnn_layer_saved* svp = &w.saved[l];
+    CK(cudaMemsetAsync(svp->msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), S(side)));
+    if (rc_img && !(dp.flags & FEGNN_F_LAST)) {
+      const float *w0 = layers[l].node_w0, *w2 = layers[l].node_w2;
+      CK(launch_node_h_wprep(d->C, ldn(d), 1, &w0, &w2, &svp->wimg, S(side)));
+    }
+    TRY(graph_pre_forward_run(&dp, g, &layers[l], w.Z[l], w.Sx[rf ? 0 : l], w.xsum[l], svp, side));
+    CK(cudaEventRecord(sd->aux, S(side)));
+    return 0;
+  };
+  if (recomputed(L - 1)) TRY(prepare(L - 1));     // rebuild_all: behind the fork above (the caller's stream order)
+  for (int l = L - 1; l >= 0; --l) {
+    fegnn_dims dl = layer_dims(l);
     const bool last = rf || l == L - 1;
-    if (last) dl.flags |= FEGNN_F_LAST;
     const fegnn_layer_params* p = &layers[l];
     fegnn_layer_grads* gr = &grads[l];
-    const fegnn_layer_saved* sv = &w.saved[l];
+    fegnn_layer_saved* sv = &w.saved[l];
     const int ls = rf ? 0 : l;
+    if (recomputed(l)) {
+      // recompute(l): node_pre, edge, virtual (u, Dsum, Usum) and phi_h (zh1) forwards of layer l from state l.  graph_post's
+      // forward is not rerun: it writes only Z' / S' (state l + 1), and its backward reads S, Usum and the gradients.
+      CK(cudaStreamWaitEvent(st, sd->aux, 0));                    // fill, weight images, graph_pre(l) (M, Zc, G1)
+      TRY(node_pre_forward_run(&dl, p, w.h[ls], sv, stream));
+      if (rf) TRY(fegnn_rf_vel_forward(d->N, v, p, sv->sv, stream));
+      TRY(edge_forward_run(&dl, g, p, w.x[l], sv, nullptr, stream));
+      fegnn_dims ds = dl;
+      ds.flags |= FEGNN_F_RECOMPUTE;                              // the saved-only forms
+      if (rc_img) ds.flags |= FEGNN_F_WIMG_READY;
+      TRY(virtual_forward_run(&ds, g, p, w.x[l], v, w.Z[l], sv, nullptr, nullptr, nullptr, stream));
+      FORK(sd, st);                                               // graph_post_bwd(l) reads Usum
+      if (!last) TRY(node_h_forward_run(&ds, g, p, w.h[l], sv, nullptr, nullptr, stream));
+    }
     // the edge backward's bound statistics come out of this layer's virtual backward (max|gt|, max|x - x_0|) and node_h
     // backward (max|gm|; the last layer has no gm) when those run on their tensor-core kernels: no pre-pass kernel on the chain
     static const bool stats_fused = getenv("FEGNN_STATS_FUSED") == nullptr || atoi(getenv("FEGNN_STATS_FUSED")) != 0;   // experiment switch
@@ -1403,6 +1510,7 @@ int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, con
       CK(cudaMemsetAsync(s.gG1[cur ^ 1], 0, sizeof(float) * s.set_a_floats, S(side)));
       CK(cudaMemsetAsync(s.gP[cur ^ 1], 0, sizeof(float) * s.set_b_floats, S(side)));
     }
+    if (recomputed(l - 1)) TRY(prepare(l - 1));   // side: into the block backward(l + 1) has left
     TRY(edge_backward_run(&dl, g, p, gr, w.x[l], sv, last ? nullptr : s.gm, s.gt, s.gP[cur], s.gQ[cur], s.gx[cur], ig,
                           overlap ? s.claim[cur] : nullptr, overlap ? sm_count() - vsms : sm_count(), stream));
     if (overlap) {

@@ -774,7 +774,9 @@ cudaError_t launch_node_pre_bwd(const NodePreArgs& a, int sms, cudaStream_t st, 
                                   NodeAttrArgs{})) return e_;
   return cudaGetLastError();
 }
-template <bool kDet = false>
+// kSaved: the saved-only form of a backward's recompute (FEGNN_F_RECOMPUTE): zh1 only -- h' is already in the next layer's
+// state, so the write-out kernel (U2 silu(zh1) + e2 and the residual add) does not run
+template <bool kDet = false, bool kSaved = false>
 cudaError_t launch_node_h_fwd(const NodeHArgs& a, int sms, cudaStream_t st, bool zero = true) {
   FEGNN_SET_SMEM(node_h_z_kernel<kDet>, kNodeHSmem);
   {
@@ -791,6 +793,7 @@ cudaError_t launch_node_h_fwd(const NodeHArgs& a, int sms, cudaStream_t st, bool
   if (e != cudaSuccess) return e;
   const int zgrid = kDet ? persistent_grid(ntiles, 2 * sms) : node_pre_grid(ntiles, a.C + 1, sms);
   if (cudaError_t e_ = launch_pdl(node_h_z_kernel<kDet>, zgrid, kThreads, kNodeHSmem, st, a)) return e_;
+  if constexpr (kSaved) return cudaGetLastError();
   if (cudaError_t e_ = launch_pdl(node_h_out_kernel, persistent_grid(ntiles, 2 * sms), kThreads, kNodeHSmem, st, a)) return e_;
   return cudaGetLastError();
 }

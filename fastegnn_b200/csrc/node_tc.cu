@@ -257,6 +257,9 @@ __global__ void __launch_bounds__(256) node_h_wprep_kernel(const __grid_constant
   }
 }
 
+// kSaved: the saved-only form of a backward's recompute (FEGNN_F_RECOMPUTE): zh1 only -- h' is already in the next layer's
+// state, so the output Linear, its residual add and the h' write-out do not run
+template <bool kSaved = false>
 __global__ void __launch_bounds__(256, 1) node_h_fwd_tc_kernel(NodeHArgs a) {
   VTR_DECL();
   constexpr int NT = 256, CPT = 32, NA = kTM * 16 / NT;
@@ -394,7 +397,7 @@ __global__ void __launch_bounds__(256, 1) node_h_fwd_tc_kernel(NodeHArgs a) {
       else if (more) load_a(par, (tile + gridDim.x) * kTM, areg, sc);
       if (b == nb1 - 1) {                          // the rows the write-out phases add: Uh (zh1) and h (h')
         load_rows(uh, a.Uh, kH, i0);
-        load_rows(hr, a.h, kH, i0);
+        if constexpr (!kSaved) load_rows(hr, a.h, kH, i0);
       }
       issue(tmem + kNH_ACC1, s_, wq, b > 0);
       pend_bits |= 1u << s_;
@@ -430,9 +433,15 @@ __global__ void __launch_bounds__(256, 1) node_h_fwd_tc_kernel(NodeHArgs a) {
       float4 z = *reinterpret_cast<const float4*>(ST + umma::tile_chunk_off(rr, c16, kTM));
       z.x += uh[j].x; z.y += uh[j].y; z.z += uh[j].z; z.w += uh[j].w;
       if (i0 + rr < a.N) *reinterpret_cast<float4*>(a.zh1 + (size_t)(i0 + rr) * kH + 4 * c16) = z;
-      store_split(At(s2), j, make_float4(silu_f(z.x), silu_f(z.y), silu_f(z.z), silu_f(z.w)));
+      if constexpr (!kSaved) store_split(At(s2), j, make_float4(silu_f(z.x), silu_f(z.y), silu_f(z.z), silu_f(z.w)));
     }
     cp_async_wait_group<1>();                      // the output Linear's weights have landed
+    if constexpr (kSaved) {                        // same slot and weight-ring sequence, no output Linear
+      ++g;
+      wq = wn;
+      __syncthreads();                             // ST has been read
+      continue;
+    }
     umma::fence_smem_to_async();
     umma::fence_before();
     __syncthreads();
@@ -757,17 +766,18 @@ cudaError_t launch_node_h_wprep(int C, int ldn, int nl, const float* const* w0, 
   return cudaGetLastError();
 }
 
+template <bool kSaved = false>
 cudaError_t launch_node_h_fwd_tc(const NodeHArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(ntc::node_h_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(ntc::node_h_fwd_tc_kernel<kSaved>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)ntc::HSmem::bytes);
     if (e != cudaSuccess) return e;
     attr.set();
   }
   const int ntiles = (a.N + kTM - 1) / kTM;
   if (ntiles == 0) return cudaSuccess;
-  if (cudaError_t e_ = launch_pdl(ntc::node_h_fwd_tc_kernel, ntiles < sms ? ntiles : sms, 256, ntc::HSmem::bytes, st, a)) return e_;
+  if (cudaError_t e_ = launch_pdl(ntc::node_h_fwd_tc_kernel<kSaved>, ntiles < sms ? ntiles : sms, 256, ntc::HSmem::bytes, st, a)) return e_;
   return cudaGetLastError();
 }
 

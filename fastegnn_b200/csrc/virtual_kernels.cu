@@ -191,7 +191,9 @@ __device__ __forceinline__ void virt_rows_to_graph(const float* __restrict__ T, 
 constexpr size_t kVirtFwdSmem = (3 * kWFloats + 2 * kTileFloats) * sizeof(float) + sizeof(VirtSmem);
 constexpr size_t kVirtBwdSmem = (3 * kWFloats + 5 * kTileFloats) * sizeof(float) + sizeof(VirtSmem);
 
-template <bool kDet>
+// kSaved: the saved-only form of a backward's recompute (FEGNN_F_RECOMPUTE): u, Dsum and Usum only -- x' and its per-graph
+// sum are already in the next layer's state, and adding xsum_new again would double it
+template <bool kDet, bool kSaved = false>
 __global__ void __launch_bounds__(kThreads, 1) virtual_fwd_kernel(VirtArgs a) {
   extern __shared__ __align__(16) float smem[];
   float* V2s = smem;
@@ -213,7 +215,8 @@ __global__ void __launch_bounds__(kThreads, 1) virtual_fwd_kernel(VirtArgs a) {
     const bool single = s->b_first == s->b_last;
     if (!kDet && (!single || s->b_first != cur_b)) {
       const int nb = single ? s->b_first : -1;
-      virt_flush(s, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
+      if constexpr (kSaved) virt_flush(s, cur_b, C, a.Usum, a.Dsum, nullptr);
+      else virt_flush(s, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
       cur_b = nb;
     }
     virt_assemble<0>(a, s, T1, nullptr);
@@ -286,6 +289,7 @@ __global__ void __launch_bounds__(kThreads, 1) virtual_fwd_kernel(VirtArgs a) {
       }
     }
     // per-node: x' (models/FastEGNN.py:133-142) and its per-graph sum
+    if constexpr (kSaved) continue;
     if (tid < TN) {
       const int i = tile * TN + tid;
       if (i < a.N) {
@@ -308,7 +312,8 @@ __global__ void __launch_bounds__(kThreads, 1) virtual_fwd_kernel(VirtArgs a) {
       }
     }
   }
-  if (!kDet) virt_flush(s, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
+  if constexpr (kSaved) virt_flush(s, cur_b, C, a.Usum, a.Dsum, nullptr);
+  else if (!kDet) virt_flush(s, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
 }
 
 __global__ void __launch_bounds__(kThreads, 1) virtual_bwd_kernel(VirtArgs a) {
@@ -561,11 +566,11 @@ __global__ void __launch_bounds__(kThreads, 1) virtual_bwd_kernel(VirtArgs a) {
   }
 }
 
-template <bool kDet = false>
+template <bool kDet = false, bool kSaved = false>
 cudaError_t launch_virtual_fwd(const VirtArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(virtual_fwd_kernel<kDet>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kVirtFwdSmem);
+    cudaError_t e = cudaFuncSetAttribute(virtual_fwd_kernel<kDet, kSaved>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kVirtFwdSmem);
     if (e != cudaSuccess) return e;
     attr.set();
   }
@@ -573,7 +578,7 @@ cudaError_t launch_virtual_fwd(const VirtArgs& a, int sms, cudaStream_t st) {
   int ntiles = (a.N + TN - 1) / TN;
   if (ntiles == 0) return cudaSuccess;
   int grid = ntiles < sms ? ntiles : sms;
-  virtual_fwd_kernel<kDet><<<grid, kThreads, kVirtFwdSmem, st>>>(a); ++g_launches;
+  virtual_fwd_kernel<kDet, kSaved><<<grid, kThreads, kVirtFwdSmem, st>>>(a); ++g_launches;
   return cudaGetLastError();
 }
 cudaError_t launch_virtual_bwd(const VirtArgs& a, int sms, cudaStream_t st) {

@@ -214,7 +214,9 @@ struct FwdSmem {
 constexpr uint32_t kF_ACC0 = 0, kF_ACCH = 64, kF_OPA = 192;    // 256 columns
 
 // kDet: no per-graph sums; the rows D sX go to the [N, C, 3] buffer in the Dsum slot (VirtArgs)
-template <int CG, bool kDet>
+// kSaved: the saved-only form of a backward's recompute (FEGNN_F_RECOMPUTE): u, Dsum and Usum only -- x' and its per-graph
+// sum are already in the next layer's state, and adding xsum_new again would double it
+template <int CG, bool kDet, bool kSaved = false>
 __global__ void __launch_bounds__(128 * CG, 2) virtual_fwd_tc_kernel(VirtArgs a) {
   VTR_DECL();
   constexpr int NT = 128 * CG, CPT = kH / CG, NW = NT / 32;
@@ -300,7 +302,8 @@ __global__ void __launch_bounds__(128 * CG, 2) virtual_fwd_tc_kernel(VirtArgs a)
     const bool single = v->b_first == v->b_last;
     if (!kDet && (!single || v->b_first != cur_b)) {
       const int nb = single ? v->b_first : -1;
-      acc_flush<NT>(&v->acc, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
+      if constexpr (kSaved) acc_flush<NT>(&v->acc, cur_b, C, a.Usum, a.Dsum, nullptr);
+      else acc_flush<NT>(&v->acc, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
       cur_b = nb;
     }
     // ---- assembly: a1 = silu(Av[node] + G1[key] + rho vr) -> T (K-major).  Half-warp per row, float4 per lane.
@@ -427,6 +430,7 @@ __global__ void __launch_bounds__(128 * CG, 2) virtual_fwd_tc_kernel(VirtArgs a)
     __syncthreads();
     VTR();
     if (!kDet && single && warp == NW - 1) small_from_rows(v->sval, &v->acc, C, TN, lane);
+    if constexpr (kSaved) continue;
     if (warp * 32 < TN) {                 // x' (models/FastEGNN.py:133-142) and its per-graph sum
       const int i = tile * TN + t;
       float xs[3] = {0.f, 0.f, 0.f};
@@ -457,7 +461,8 @@ __global__ void __launch_bounds__(128 * CG, 2) virtual_fwd_tc_kernel(VirtArgs a)
       }
     }
   }
-  if (!kDet) acc_flush<NT>(&v->acc, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
+  if constexpr (kSaved) acc_flush<NT>(&v->acc, cur_b, C, a.Usum, a.Dsum, nullptr);
+  else if (!kDet) acc_flush<NT>(&v->acc, cur_b, C, a.Usum, a.Dsum, a.xsum_new);
   umma::fence_before();
   __syncthreads();
     VTR();
@@ -1243,12 +1248,12 @@ __global__ void __launch_bounds__(128 * CG, 1) virtual_bwd_trunk_tc_kernel(VirtA
 
 }  // namespace vtc
 
-template <int CG, bool kDet = false>
+template <int CG, bool kDet = false, bool kSaved = false>
 cudaError_t launch_virtual_fwd_tc(const VirtArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   const size_t bytes = vtc::FwdSmem::bytes;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(vtc::virtual_fwd_tc_kernel<CG, kDet>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    cudaError_t e = cudaFuncSetAttribute(vtc::virtual_fwd_tc_kernel<CG, kDet, kSaved>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
     attr.set();
   }
@@ -1256,7 +1261,7 @@ cudaError_t launch_virtual_fwd_tc(const VirtArgs& a, int sms, cudaStream_t st) {
   const int ntiles = (a.N + TN - 1) / TN;
   if (ntiles == 0) return cudaSuccess;
   const int grid = ntiles < 2 * sms ? ntiles : 2 * sms;
-  if (cudaError_t e_ = launch_pdl(vtc::virtual_fwd_tc_kernel<CG, kDet>, grid, 128 * CG, bytes, st, a)) return e_;
+  if (cudaError_t e_ = launch_pdl(vtc::virtual_fwd_tc_kernel<CG, kDet, kSaved>, grid, 128 * CG, bytes, st, a)) return e_;
   return cudaGetLastError();
 }
 

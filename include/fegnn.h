@@ -67,6 +67,22 @@ extern "C" {
 #define FEGNN_F_STATS_READY 1024u /* fegnn_edge_backward (tensor-core modes 7 / 8): saved.scratch[0..2] already hold the bound
                                     statistics (max|gt|, max|gm|, max|x - x_0|) -- written by fegnn_virtual_backward and
                                     fegnn_node_h_backward of the same layer on their tensor-core kernels: skip the pre-pass */
+#define FEGNN_F_RECOMPUTE 2048u /* recompute ("activation checkpointing") for the training stack: fegnn_model_workspace_floats,
+                                  fegnn_model_forward and fegnn_model_backward[_inputs] keep the L + 1 layer states and min(L, 2)
+                                  saved blocks instead of L; the backward rebuilds a layer's block from its input state just
+                                  before that layer's backward (DESIGN 3.8).  On fegnn_virtual_forward / fegnn_node_h_forward it
+                                  selects the saved-only forms of a recompute: u, Dsum, Usum (resp. zh1) are written, x',
+                                  xsum_new (resp. h') are not (x_new, xsum_new, h_new may be NULL).  Every other per-layer phase
+                                  and fegnn_node_h_weight_images return FEGNN_EINVAL with it; fegnn_model_forward_inference
+                                  ignores it (it keeps no blocks). */
+#define FEGNN_F_REBUILD_ALL 4096u /* with FEGNN_F_RECOMPUTE, read by fegnn_model_backward[_inputs] only: the saved blocks are not as
+                                    fegnn_model_forward left them, so rebuild every layer.  A recompute backward rebuilds the
+                                    lower layers into the two blocks the forward left holding layers L - 1 and L - 2 (for L >= 3),
+                                    so a SECOND backward over the same forward (autograd's retain_graph) must pass this flag, or
+                                    it reads the wrong layers' intermediates.  The first backward after a forward may pass it
+                                    too (it then also rebuilds the top two layers).  Without FEGNN_F_RECOMPUTE the backward
+                                    refuses it with FEGNN_EINVAL; the forward entries ignore it; every other per-layer entry
+                                    refuses it like FEGNN_F_RECOMPUTE. */
 
 typedef struct fegnn_dims {
   int32_t N;        /* owned real nodes                                             */
@@ -390,6 +406,8 @@ size_t fegnn_layer_saved_floats(const fegnn_dims* d);
 /* words of the accumulator head of a saved block (from .msum): what FEGNN_F_PREZEROED expects zero-filled */
 size_t fegnn_layer_saved_accum_floats(const fegnn_dims* d);
 int fegnn_layer_saved_bind(const fegnn_dims* d, float* block, fegnn_layer_saved* out);
+/* (L + 1) states + L saved blocks; with FEGNN_F_RECOMPUTE in d->flags (L + 1) states + min(L, 2) saved blocks.  The forward
+ * and the backward of one step must see the same flag. */
 size_t fegnn_model_workspace_floats(const fegnn_dims* d, int32_t L);
 size_t fegnn_model_backward_scratch_floats(const fegnn_dims* d);
 
@@ -422,7 +440,8 @@ int fegnn_model_backward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegn
                          const float* gx_out /*[N,3]*/, const float* gZ_out /*[B,3,C]*/,
                          float* g_x0 /*[N,3]*/, float* g_loc_mean /*[B,3,C]*/, float* g_node_feat /*[N,Fin] or NULL*/,
                          const float* workspace, float* scratch, size_t scratch_floats, void* stream);
-/* fegnn_model_backward plus the requested input gradients (fegnn_input_grads above; the buffers are filled here) */
+/* fegnn_model_backward plus the requested input gradients (fegnn_input_grads above; the buffers are filled here).
+ * With FEGNN_F_RECOMPUTE both backward entries rewrite the saved blocks of the workspace (the states are only read). */
 int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn_graph* g,
                                 const fegnn_layer_params* layers_host, fegnn_layer_grads* grads_host /*[L]*/,
                                 const float* embed_w, float* g_embed_w, float* g_embed_b, float* g_virtual_node_feat,

@@ -10,8 +10,8 @@ Make each log from a checkout of the build it describes (nvcc prints the listing
 Kernels are matched by mangled name, a name the parent lacks after renamings that do not change the code: the anonymous
 namespace of api.cu (its hash depends on the source path), the `kEa = false` instantiations of edge_bwd_kernel /
 edge_bwd_tc4_kernel and the `kDet = false` instantiations of the forward kernels (edge_fwd_kernel, edge_fwd_tc_kernel,
-virtual_fwd_kernel, virtual_fwd_tc_kernel, node_h_z_kernel), which are a parent's untemplated (resp. one-parameter
-fewer) kernels.  Every kernel of both builds is listed with its resource
+virtual_fwd_kernel, virtual_fwd_tc_kernel, node_h_z_kernel), the `kSaved = false` instantiations of virtual_fwd_kernel,
+virtual_fwd_tc_kernel and node_h_fwd_tc_kernel, which are a parent's untemplated (resp. one-parameter fewer) kernels.  Every kernel of both builds is listed with its resource
 lines (stack frame, spills, registers, barriers, shared memory; constant-bank sizes are left out)."""
 import re
 import sys
@@ -35,12 +35,19 @@ def parse(path):
 # a trailing bool template parameter (false) that a parent does not have: "kernelI<args>Lb0EEEv" -> "kernelI<args>EEv",
 # and a kernel whose only template parameter it is: "kernelILb0EEEvNS_" -> "kernelENS_"
 BOOL_ADDED = ("edge_bwd_kernel", "edge_bwd_tc4_kernel", "edge_fwd_kernel", "edge_fwd_tc_kernel", "virtual_fwd_kernel",
-              "virtual_fwd_tc_kernel", "node_h_z_kernel")
+              "virtual_fwd_tc_kernel", "node_h_z_kernel", "node_h_fwd_tc_kernel")
+# a second trailing bool (the kSaved = false forms of the recompute, FEGNN_F_RECOMPUTE) after the kDet one
+BOOL2_ADDED = ("virtual_fwd_kernel", "virtual_fwd_tc_kernel")
 
 
 def to_parent(name, parent):
     if name in parent:
         return name
+    for k in BOOL2_ADDED:
+        if f"{len(k)}{k}I" in name:
+            trimmed = re.sub(rf"({k}I(?:L[ib]\d+E)+)Lb0EEEv", r"\1EEv", name)
+            if trimmed in parent:
+                return trimmed
     for k in BOOL_ADDED:
         if f"{len(k)}{k}I" in name:
             name = name.replace(f"{k}ILb0EEEvNS_", f"{k}ENS_")
