@@ -1038,18 +1038,38 @@ size_t fegnn_layer_saved_accum_floats(const fegnn_dims* d) {
 
 namespace {
 
+// A stack's workspace as its drivers see it.  What differs between the training stack and the forward-only stack is
+// data here, not code in forward_stack.
 struct ModelWs {
   // per layer l in [0, L]: state entering layer l (index L = outputs)
   float *h[33], *x[33], *Z[33], *Sx[33], *xsum[33];
-  fegnn_layer_saved saved[32];      // FEGNN_F_RECOMPUTE: layer l's block is block l % 2 of a ring of two (DESIGN 3.8)
+  fegnn_layer_saved saved[32];      // layer l's block is block l % nb of a ring of nb <= L blocks
+  int nb;
+  bool xsum_ahead;                  // the x sums of all states are distinct and contiguous: ONE zero-fill ahead of the chain
+  const DetWs* det;                 // the deterministic forms' scratch (forward-only stack), else nullptr: the default kernels
 };
 
-// saved blocks of the training stack: one per layer, or with FEGNN_F_RECOMPUTE a ring of min(L, 2)
+void bind_blocks(const fegnn_dims* d, int L, int nb, float* p, ModelWs* w) {
+  w->nb = nb < L ? nb : L;
+  for (int l = 0; l < L; ++l) {
+    if (l < w->nb) {
+      fegnn_layer_saved_bind(d, p, &w->saved[l]);
+      p += fegnn_layer_saved_floats(d);
+    } else {
+      w->saved[l] = w->saved[l % w->nb];
+    }
+  }
+}
+
+// saved blocks of the training stack: one per layer, or with FEGNN_F_RECOMPUTE a ring of min(L, 2) (DESIGN 3.8)
 inline int model_blocks(const fegnn_dims* d, int L) { return (d->flags & FEGNN_F_RECOMPUTE) ? (L < 2 ? L : 2) : L; }
-size_t model_ws_floats(const fegnn_dims* d, int L) {
+// one state: h, x, Z, S and the per-graph x sums
+size_t state_floats(const fegnn_dims* d) {
   const size_t N = d->N, Nl = d->Nl, B = d->B, C = d->C;
-  size_t per_state = al4(N * kH) + al4(Nl * 3) + al4(B * 3 * C) + al4(B * C * kH) + al4(B * 3);
-  return (size_t)(L + 1) * per_state + (size_t)model_blocks(d, L) * fegnn_layer_saved_floats(d);
+  return al4(N * kH) + al4(Nl * 3) + al4(B * 3 * C) + al4(B * C * kH) + al4(B * 3);
+}
+size_t model_ws_floats(const fegnn_dims* d, int L) {
+  return (size_t)(L + 1) * state_floats(d) + (size_t)model_blocks(d, L) * fegnn_layer_saved_floats(d);
 }
 void model_ws_bind(const fegnn_dims* d, int L, float* base, ModelWs* w) {
   const size_t N = d->N, Nl = d->Nl, B = d->B, C = d->C;
@@ -1059,15 +1079,39 @@ void model_ws_bind(const fegnn_dims* d, int L, float* base, ModelWs* w) {
   for (int l = 0; l <= L; ++l) {
     w->h[l] = take(N * kH); w->x[l] = take(Nl * 3); w->Z[l] = take(B * 3 * C); w->Sx[l] = take(B * C * kH);
   }
-  const int nb = model_blocks(d, L);
-  for (int l = 0; l < L; ++l) {
-    if (l < nb) {
-      fegnn_layer_saved_bind(d, p, &w->saved[l]);
-      p += fegnn_layer_saved_floats(d);
-    } else {
-      w->saved[l] = w->saved[l % nb];
-    }
+  w->xsum_ahead = true;
+  w->det = nullptr;
+  bind_blocks(d, L, model_blocks(d, L), p, w);
+}
+
+// Forward-only stack (rollout / evaluation; utils/train.py:24-27,191-192: validation and test run the model with
+// backprop=False).  Nothing is kept for a backward: the layers ping-pong between two state slots and share ONE block of
+// per-layer intermediates, so the workspace is 3 states + 1 block instead of (L + 1) states + L blocks (3.4 GB instead of
+// 13.4 GB at 1 M nodes, C = 8, L = 4).  Small graphs get a RING of kInferBlocks blocks (a stack of up to that many layers
+// has a block per layer): with ONE block the per-graph kernels of layer l + 1 (side stream) must not start before layer
+// l's node phase has read u / msum, and the next main-stream kernels not before graph_post(l) has read Dsum / Usum -- a
+// join + fork per layer that puts 12 us of one-CTA kernels on the chain -- and every layer needs its accumulator fill and
+// its phi_h weight images inside the chain.  With the ring the stack has the training forward's structure: fills and
+// weight images ahead of the first kernel, one fork / join pair per layer.  Large graphs keep one block: there all of this
+// is noise and the block is gigabytes.
+constexpr int kInferRingMaxN = 65536, kInferBlocks = 4;      // 4 = n_layers of every reference main
+inline int infer_blocks(const fegnn_dims* d) { return d->N <= kInferRingMaxN ? kInferBlocks : 1; }
+void infer_ws_bind(const fegnn_dims* d, int L, float* base, const DetWs* det, ModelWs* w) {
+  const size_t N = d->N, Nl = d->Nl, B = d->B, C = d->C;
+  float* p = base;
+  auto take = [&](size_t n) { float* r = p; p += al4(n); return r; };
+  float *h[3], *x[3], *Z[3], *Sx[3], *xsum[3];
+  for (int i = 0; i < 3; ++i) {
+    h[i] = take(N * kH); x[i] = take(Nl * 3); Z[i] = take(B * 3 * C); Sx[i] = take(B * C * kH); xsum[i] = take(B * 3);
   }
+  // slot 2 keeps the embedding state (h0, S0), which FastRF reads in every layer; the layers' outputs alternate 0, 1, 0, ...
+  for (int l = 0; l <= L; ++l) {
+    const int s = l == 0 ? 2 : (l - 1) & 1;
+    w->h[l] = h[s]; w->x[l] = x[s]; w->Z[l] = Z[s]; w->Sx[l] = Sx[s]; w->xsum[l] = xsum[s];
+  }
+  w->xsum_ahead = false;
+  w->det = det;
+  bind_blocks(d, L, infer_blocks(d), p, w);
 }
 
 struct BwdScratch {
@@ -1101,6 +1145,146 @@ void bwd_scratch_bind(const fegnn_dims* d, float* base, BwdScratch* s) {
   s->set_b_floats = al4(N * kH) + al4(Nl * kH) + 4;
 }
 
+// every layer's parameters against the flags, before a stack's first launch
+int check_layers(const fegnn_dims* d, int L, const fegnn_layer_params* layers) {
+  char why[sizeof(g_err)];
+  for (int l = 0; l < L; ++l) {
+    if (check_flags_params(d, &layers[l]) == 0) continue;
+    memcpy(why, g_err, sizeof(why));
+    return fail(FEGNN_EINVAL, "layer %d: %s", l, why);
+  }
+  return 0;
+}
+
+// the dims of layer l's phases in a stack: their full forms (FEGNN_F_RECOMPUTE is the stack's flag), accumulators
+// zero-filled by the stack, FEGNN_F_LAST on the last layer and on every FastRF layer (h passes through: models/FastRF.py:186)
+fegnn_dims layer_dims(const fegnn_dims* d, int L, int l) {
+  fegnn_dims dl = *d;
+  dl.flags &= ~(FEGNN_F_RECOMPUTE | FEGNN_F_REBUILD_ALL);
+  dl.flags |= FEGNN_F_PREZEROED;
+  if ((d->flags & FEGNN_F_RF) || l == L - 1) dl.flags |= FEGNN_F_LAST;
+  return dl;
+}
+
+// the accumulator head of a saved block (fegnn_layer_saved_accum_floats words from msum)
+cudaError_t fill_block(const fegnn_dims* d, const fegnn_layer_saved& sv, cudaStream_t s) {
+  return cudaMemsetAsync(sv.msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), s);
+}
+
+// phi_h on the tensor cores: the operand-tile images of layers l0 .. l0 + n - 1 into their blocks, in one launch
+cudaError_t weight_images(const fegnn_dims* d, const fegnn_layer_params* layers, const ModelWs& w, int l0, int n,
+                          cudaStream_t s) {
+  const float *w0[32], *w2[32];
+  float* img[32];
+  for (int l = 0; l < n; ++l) { w0[l] = layers[l0 + l].node_w0; w2[l] = layers[l0 + l].node_w2; img[l] = w.saved[l0 + l].wimg; }
+  return launch_node_h_wprep(d->C, ldn(d), n, w0, w2, img, s);
+}
+
+// The ring block that layer l reuses, filled on the side stream behind its last readers (a memset node between two kernels
+// of the chain would cut their programmatic overlap); the main stream waits for `aux` before layer l (layer_forward)
+int ring_fill(const fegnn_dims* d, const fegnn_layer_saved& sv, SideStream* sd) {
+  CK(fill_block(d, sv, sd->st));
+  CK(cudaEventRecord(sd->aux, sd->st));
+  return 0;
+}
+
+// Layer l's forward on the main stream, from state l to state l + 1: [the wait for its ring block's fill,] node_pre,
+// FastRF's velocity head, the edge forward, the join (the virtual forward reads graph_pre's M and G1), the virtual
+// forward, the fork and phi_h.  The caller puts graph_pre on the side stream ahead of it and graph_post (the backward's
+// rebuild: graph_post_backward) behind it.  With FEGNN_F_RECOMPUTE in dl the saved-only forms run: x', xsum' and h' are
+// state l + 1 already.
+int layer_forward(const fegnn_dims* dl, const fegnn_graph* g, const fegnn_layer_params* p, const float* v, ModelWs& w, int l,
+                  bool ring_wait, bool node_pre, SideStream* sd, void* stream) {
+  cudaStream_t st = S(stream);
+  const bool rf = dl->flags & FEGNN_F_RF, saved_only = dl->flags & FEGNN_F_RECOMPUTE;
+  fegnn_layer_saved* sv = &w.saved[l];
+  if (ring_wait) CK(cudaStreamWaitEvent(st, sd->aux, 0));
+  if (node_pre) TRY(node_pre_forward_run(dl, p, w.h[rf ? 0 : l], sv, stream));
+  if (rf) TRY(fegnn_rf_vel_forward(dl->N, v, p, sv->sv, stream));
+  TRY(edge_forward_run(dl, g, p, w.x[l], sv, w.det, stream));
+  JOIN(sd, st);
+  TRY(virtual_forward_run(dl, g, p, w.x[l], v, w.Z[l], sv, saved_only ? nullptr : w.x[l + 1],
+                          saved_only ? nullptr : w.xsum[l + 1], w.det, stream));
+  FORK(sd, st);
+  if (!(dl->flags & FEGNN_F_LAST)) TRY(node_h_forward_run(dl, g, p, w.h[l], sv, saved_only ? nullptr : w.h[l + 1], w.det, stream));
+  return 0;
+}
+
+// The forward of both stacks (fegnn_model_forward, fegnn_model_forward_inference): the prologue, the layer loop and the
+// output copies.  The per-graph phases run one CTA per graph on the side stream, under the main chain.
+int forward_stack(const fegnn_dims* d, int L, int Fin, const fegnn_graph* g, const fegnn_layer_params* layers,
+                  const float* embed_w, const float* embed_b, const float* vnf, const float* node_feat, const float* x0,
+                  const float* v, const float* loc_mean, float* x_out, float* Z_out, ModelWs& w, void* stream) {
+  cudaStream_t st = S(stream);
+  const size_t N = d->N, B = d->B, C = d->C;
+  const bool rf = d->flags & FEGNN_F_RF;          // FastRF: h and S of state 0 enter every layer
+  const int nb = w.nb;
+  TRY(fegnn_embed_forward(d->N, Fin, node_feat, embed_w, embed_b, w.h[0], stream));
+  CK(cudaMemcpyAsync(w.x[0], x0, sizeof(float) * 3 * N, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(w.Z[0], loc_mean, sizeof(float) * 3 * C * B, cudaMemcpyDeviceToDevice, st));
+  if (B > 0) {
+    broadcast_vnf_kernel<<<(unsigned)((B * C * kH + 255) / 256), 256, 0, st>>>(d->B, d->C, vnf, w.Sx[0]); ++g_launches;
+    CK(cudaGetLastError());
+  }
+  // the accumulators are zero-filled ahead of the kernel chain (the phases then skip their own fills): the x sums of every
+  // state where the states are distinct, and the accumulator head of every block.  A ring (nb > 1) refills the block of a
+  // layer l >= nb on the side stream during layer l - 1; a single block is refilled in the chain in front of each layer.
+  if (w.xsum_ahead) CK(cudaMemsetAsync(w.xsum[0], 0, sizeof(float) * ((size_t)L * al4(B * 3) + B * 3), st));
+  for (int l = 0; l < nb; ++l) CK(fill_block(d, w.saved[l], st));
+  // phi_h on the tensor cores with a ring: the first blocks' weight images in ONE launch here -- weights only, so it runs
+  // ahead of the chain and (graph_pending) under the CSR sort -- and layer l + 1 >= nb's on the side stream next to
+  // graph_post(l) (its block's images were last read by phi_h of layer l + 1 - nb, ahead of the fork).  A single block:
+  // phi_h writes its own images in the chain.
+  const bool img_ahead = nb > 1 && g_node_fwd_mode != 0 && !rf;
+  const int nimg_top = nb < L - 1 ? nb : L - 1;   // the last layer has no phi_h
+  if (img_ahead) CK(weight_images(d, layers, w, 0, nimg_top, st));
+  const bool graph_pending = g->ready_event != nullptr;
+  if (graph_pending) {
+    // the CSR sort is still running on another stream: everything above and the first layer's node phase read no graph
+    // array and run under it; this stream joins the sort here
+    const fegnn_dims d0 = layer_dims(d, L, 0);
+    TRY(node_pre_forward_run(&d0, &layers[0], w.h[0], &w.saved[0], stream));
+    CK(cudaStreamWaitEvent(st, static_cast<cudaEvent_t>(g->ready_event), 0));
+  }
+  if (w.xsum_ahead) CK(launch_graph_xsum(d->N, w.x[0], g->batch, w.xsum[0], st));
+  else TRY(graph_xsum_run(d->N, d->B, w.x[0], g->batch, w.xsum[0], w.det, stream));
+  SideStream* sd = side_stream();
+  RQ(sd != nullptr);
+  void* side = sd->st;
+  FORK(sd, st);                                   // side: graph_pre(0)
+  for (int l = 0; l < L; ++l) {
+    fegnn_dims dl = layer_dims(d, L, l);
+    if (img_ahead) dl.flags |= FEGNN_F_WIMG_READY;
+    const fegnn_layer_params* p = &layers[l];
+    fegnn_layer_saved* sv = &w.saved[l];
+    const int ls = rf ? 0 : l;                    // layer whose (h, S) state this layer reads
+    if (nb == 1 && l > 0) CK(fill_block(d, *sv, st));
+    // states in shared slots: the x sums of the state this layer produces, on the side stream (last read by the per-graph
+    // kernels of the layer that consumed that slot's state, earlier on the same stream; joined in front of virtual_forward)
+    if (!w.xsum_ahead) CK(cudaMemsetAsync(w.xsum[l + 1], 0, sizeof(float) * 3 * B, S(side)));
+    TRY(graph_pre_forward_run(&dl, g, p, w.Z[l], w.Sx[ls], w.xsum[l], sv, side));
+    TRY(layer_forward(&dl, g, p, v, w, l, nb > 1 && l >= nb, !(graph_pending && l == 0), sd, stream));
+    // side: [the fill of the block layer l + 1 reuses,] graph_post(l) [-> graph_pre(l + 1)] under phi_h(l), node_pre(l + 1),
+    // edge(l + 1).  The fill's block was last read by layer l + 1 - nb: its node phase on the main stream ahead of the
+    // fork, its per-graph kernels earlier on the side stream.
+    if (nb > 1 && l + 1 >= nb && l + 1 < L) TRY(ring_fill(d, w.saved[l + 1], sd));
+    TRY(graph_post_forward_run(&dl, g, p, w.Z[l], w.Sx[ls], sv, w.Z[l + 1], w.Sx[l + 1], side));
+    if (img_ahead && l + 2 < L && l + 1 >= nimg_top) CK(weight_images(d, layers, w, l + 1, 1, S(side)));
+    // a single block is rewritten by the next layer: its per-graph kernels (side) must not start before this layer's
+    // phi_h (main) has read u / msum, and its main-stream kernels not before this layer's graph_post (side) has read
+    // Dsum / Usum.  (Ring: block l % nb is next written by layer l + nb, whose kernels are ordered behind both by the
+    // joins in front of the virtual forwards in between.)
+    if (nb == 1 && l + 1 < L) {
+      JOIN(sd, st);
+      FORK(sd, st);
+    }
+  }
+  JOIN(sd, st);
+  CK(cudaMemcpyAsync(x_out, w.x[L], sizeof(float) * 3 * N, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(Z_out, w.Z[L], sizeof(float) * 3 * C * B, cudaMemcpyDeviceToDevice, st));
+  return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1119,112 +1303,16 @@ int fegnn_model_forward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn
   RQ(d->Nl == d->N);   // the partitioned path drives the phases itself (halo rows come from peers)
   if (workspace_floats < model_ws_floats(d, L))
     return fail(FEGNN_ENOMEM, "model workspace %zu < %zu floats", workspace_floats, model_ws_floats(d, L));
-  cudaStream_t st = S(stream);
+  TRY(check_layers(d, L, layers));
   ModelWs w;
   model_ws_bind(d, L, workspace, &w);
-  const size_t N = d->N, B = d->B, C = d->C;
-  TRY(fegnn_embed_forward(d->N, Fin, node_feat, embed_w, embed_b, w.h[0], stream));
-  CK(cudaMemcpyAsync(w.x[0], x0, sizeof(float) * 3 * N, cudaMemcpyDeviceToDevice, st));
-  CK(cudaMemcpyAsync(w.Z[0], loc_mean, sizeof(float) * 3 * C * B, cudaMemcpyDeviceToDevice, st));
-  if (B > 0) {
-    broadcast_vnf_kernel<<<(unsigned)((B * C * kH + 255) / 256), 256, 0, st>>>(d->B, d->C, vnf, w.Sx[0]); ++g_launches;
-    CK(cudaGetLastError());
-  }
-  // every accumulator of the step is zero-filled here, ahead of the kernel chain (the phases then skip their own fills):
-  // the per-graph coordinate sums of all states, and the accumulator head of every layer's saved block
-  // (FEGNN_F_RECOMPUTE: the blocks form a ring of nb = min(L, 2); the block of a layer l >= nb is filled on the side stream
-  // during layer l - 1, below -- a memset node between two kernels of the chain would cut their programmatic overlap)
-  const bool rc = d->flags & FEGNN_F_RECOMPUTE;
-  const int nb = model_blocks(d, L);
-  CK(cudaMemsetAsync(w.xsum[0], 0, sizeof(float) * ((size_t)L * al4(B * 3) + B * 3), st));
-  for (int l = 0; l < nb; ++l)
-    CK(cudaMemsetAsync(w.saved[l].msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), st));
-  const bool rf = d->flags & FEGNN_F_RF;          // FastRF: h and S pass through every layer (models/FastRF.py:186)
-  // phi_h on the tensor cores: the operand-tile images of every layer's weight blocks in ONE launch here -- weights only, so it
-  // runs ahead of the chain and (graph_pending) under the CSR sort.  Ring: the first nb layers' here, layer l + 1 >= nb's on
-  // the side stream next to graph_post(l) (its block's images were last read by phi_h of layer l + 1 - nb, ahead of the fork)
-  bool wimg_ready = false;
-  const int nimg_top = nb < L - 1 ? nb : L - 1;   // the last layer has no phi_h
-  if (g_node_fwd_mode != 0 && !rf && L > 1) {
-    const float *w0[32], *w2[32];
-    float* img[32];
-    for (int l = 0; l < nimg_top; ++l) { w0[l] = layers[l].node_w0; w2[l] = layers[l].node_w2; img[l] = w.saved[l].wimg; }
-    CK(launch_node_h_wprep(d->C, ldn(d), nimg_top, w0, w2, img, st));
-    wimg_ready = true;
-  }
-  const bool graph_pending = g->ready_event != nullptr;
-  if (graph_pending) {
-    // the CSR sort is still running on another stream: everything above and the first layer's node phase read no graph
-    // array and run under it; this stream joins the sort here
-    fegnn_dims d0 = *d;
-    d0.flags &= ~(FEGNN_F_RECOMPUTE | FEGNN_F_REBUILD_ALL);
-    d0.flags |= FEGNN_F_PREZEROED;
-    if (rf || L == 1) d0.flags |= FEGNN_F_LAST;
-    TRY(fegnn_node_pre_forward(&d0, &layers[0], w.h[0], &w.saved[0], stream));
-    CK(cudaStreamWaitEvent(st, static_cast<cudaEvent_t>(g->ready_event), 0));
-  }
-  CK(launch_graph_xsum(d->N, w.x[0], g->batch, w.xsum[0], st));
-  SideStream* sd = side_stream();
-  RQ(sd != nullptr);
-  void* side = sd->st;
-  FORK(sd, st);                                   // side: graph_pre(0)
-  for (int l = 0; l < L; ++l) {
-    fegnn_dims dl = *d;
-    dl.flags &= ~(FEGNN_F_RECOMPUTE | FEGNN_F_REBUILD_ALL);   // the phases run their full forms
-    dl.flags |= FEGNN_F_PREZEROED;
-    if (wimg_ready) dl.flags |= FEGNN_F_WIMG_READY;
-    const bool last = rf || l == L - 1;
-    if (last) dl.flags |= FEGNN_F_LAST;
-    const fegnn_layer_params* p = &layers[l];
-    fegnn_layer_saved* sv = &w.saved[l];
-    const int ls = rf ? 0 : l;                    // layer whose (h, S) state this layer reads
-    if (rc && l >= nb) CK(cudaStreamWaitEvent(st, sd->aux, 0));        // ring: this block's fill (side, during layer l - 1)
-    TRY(fegnn_graph_pre_forward(&dl, g, p, w.Z[l], w.Sx[ls], w.xsum[l], sv, side));      // side (1 CTA per graph)
-    if (!(graph_pending && l == 0)) TRY(fegnn_node_pre_forward(&dl, p, w.h[ls], sv, stream));
-    if (rf) TRY(fegnn_rf_vel_forward(d->N, v, p, sv->sv, stream));
-    TRY(fegnn_edge_forward(&dl, g, p, w.x[l], sv, stream));
-    JOIN(sd, st);                                 // virtual needs G1, M of graph_pre
-    TRY(fegnn_virtual_forward(&dl, g, p, w.x[l], v, w.Z[l], sv, w.x[l + 1], w.xsum[l + 1], stream));
-    FORK(sd, st);                                 // side: graph_post(l) [-> graph_pre(l+1)] under node_h, node_pre, edge
-    if (rc && l + 1 >= nb && l + 1 < L) {
-      // ring: the accumulators of the block layer l + 1 reuses, last read by layer l + 1 - nb (node phase on this stream ahead
-      // of the fork, per-graph kernels earlier on the side stream)
-      CK(cudaMemsetAsync(w.saved[l + 1].msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), S(side)));
-      CK(cudaEventRecord(sd->aux, S(side)));
-    }
-    if (!last) TRY(fegnn_node_h_forward(&dl, g, p, w.h[l], sv, w.h[l + 1], stream));
-    TRY(fegnn_graph_post_forward(&dl, g, p, w.Z[l], w.Sx[ls], sv, w.Z[l + 1], w.Sx[l + 1], side));
-    if (rc && wimg_ready && l + 2 < L && l + 1 >= nimg_top) {
-      const float *w0 = layers[l + 1].node_w0, *w2 = layers[l + 1].node_w2;
-      float* img = w.saved[l + 1].wimg;
-      CK(launch_node_h_wprep(d->C, ldn(d), 1, &w0, &w2, &img, S(side)));     // joined in front of virtual_forward(l + 1)
-    }
-  }
-  JOIN(sd, st);
-  CK(cudaMemcpyAsync(x_out, w.x[L], sizeof(float) * 3 * N, cudaMemcpyDeviceToDevice, st));
-  CK(cudaMemcpyAsync(Z_out, w.Z[L], sizeof(float) * 3 * C * B, cudaMemcpyDeviceToDevice, st));
-  return 0;
+  return forward_stack(d, L, Fin, g, layers, embed_w, embed_b, vnf, node_feat, x0, v, loc_mean, x_out, Z_out, w, stream);
 }
 
 // ------------------------------------------------------------------ forward-only stack (rollout / evaluation)
-// utils/train.py:24-27,191-192: validation and test run the model with backprop=False.  Nothing is kept for a backward:
-// the layers ping-pong between two state sets and share ONE block of per-layer intermediates, so the workspace is
-// 2 states + 1 block instead of (L + 1) states + L blocks (3.4 GB instead of 13.4 GB at 1 M nodes, C = 8, L = 4).
-// Small graphs get a RING of kInferBlocks blocks (layer l uses block l % kInferBlocks; a stack of up to that many layers has a
-// block per layer): with ONE block the per-graph kernels of layer l + 1 (side stream) must not start before layer l's node
-// phase has read u / msum, and the next main-stream kernels not before graph_post(l) has read Dsum / Usum -- a join + fork
-// per layer that puts 12 us of one-CTA kernels on the chain -- and every layer needs its accumulator fill and its phi_h
-// weight images inside the chain.  With the ring the stack has the training forward's structure: fills and weight images
-// ahead of the first kernel, one fork / join pair per layer.  Large graphs keep one block: there all of this is noise and the
-// block is gigabytes.
-constexpr int kInferRingMaxN = 65536, kInferBlocks = 4;      // 4 = n_layers of every reference main
-static inline size_t infer_blocks(const fegnn_dims* d) { return d->N <= kInferRingMaxN ? kInferBlocks : 1; }
-
 size_t fegnn_model_inference_workspace_floats(const fegnn_dims* d) {
-  const size_t N = d->N, Nl = d->Nl, B = d->B, C = d->C;
-  const size_t per_state = al4(N * kH) + al4(Nl * 3) + al4(B * 3 * C) + al4(B * C * kH) + al4(B * 3);
   // two ping-pong states + the (h, S) of the embedding (FastRF) + the shared block(s) of per-layer intermediates
-  return 3 * per_state + infer_blocks(d) * fegnn_layer_saved_floats(d);
+  return 3 * state_floats(d) + infer_blocks(d) * fegnn_layer_saved_floats(d);
 }
 // the deterministic forms' scratch (DetWs), which follows that workspace
 size_t fegnn_model_inference_det_workspace_floats(const fegnn_dims* d) {
@@ -1239,123 +1327,16 @@ int fegnn_model_forward_inference(const fegnn_dims* d, int32_t L, int32_t Fin, c
   TRY(check_dims(d));
   RQ(L >= 1 && L <= 32 && g && layers && embed_w && embed_b && vnf && workspace && x_out && Z_out);
   RQ(d->Nl == d->N);
-  fegnn_dims d_full = *d;                         // FEGNN_F_RECOMPUTE is a training-stack flag: nothing is kept here anyway
-  d_full.flags &= ~(FEGNN_F_RECOMPUTE | FEGNN_F_REBUILD_ALL);
-  d = &d_full;
   // deterministic mode: the kDet forms of the phases, with their scratch behind the workspace
   const size_t base_floats = fegnn_model_inference_workspace_floats(d);
   const size_t need = base_floats + fegnn_model_inference_det_workspace_floats(d);
   if (workspace_floats < need) return fail(FEGNN_ENOMEM, "inference workspace %zu < %zu floats", workspace_floats, need);
-  DetWs det_;
-  const DetWs* det = nullptr;
-  if (g_det) {
-    det_ws_bind(d, workspace + base_floats, &det_);
-    det = &det_;
-  }
-  cudaStream_t st = S(stream);
-  const size_t N = d->N, Nl = d->Nl, B = d->B, C = d->C;
-  float* p = workspace;
-  auto take = [&](size_t n) { float* r = p; p += al4(n); return r; };
-  float *h[3], *x[3], *Z[3], *Sx[3], *xsum[3];
-  for (int i = 0; i < 3; ++i) {
-    h[i] = take(N * kH); x[i] = take(Nl * 3); Z[i] = take(B * 3 * C); Sx[i] = take(B * C * kH); xsum[i] = take(B * 3);
-  }
-  const int nb = (int)infer_blocks(d);            // ring of blocks (1: large graphs)
-  const bool two = nb > 1;
-  fegnn_layer_saved sv_[kInferBlocks];
-  for (int i = 0; i < kInferBlocks; ++i) {
-    if (i < nb) fegnn_layer_saved_bind(d, p + (size_t)i * fegnn_layer_saved_floats(d), &sv_[i]);
-    else sv_[i] = sv_[0];
-  }
-  const int ntop = nb < L ? nb : L;               // blocks filled (and layers whose weight images are written) ahead of the chain
-  // slot 2 keeps the embedding state (h0, S0): FastRF reads it in every layer; slots 0 / 1 ping-pong
-  TRY(fegnn_embed_forward(d->N, Fin, node_feat, embed_w, embed_b, h[2], stream));
-  CK(cudaMemcpyAsync(x[2], x0, sizeof(float) * 3 * N, cudaMemcpyDeviceToDevice, st));
-  CK(cudaMemcpyAsync(Z[2], loc_mean, sizeof(float) * 3 * C * B, cudaMemcpyDeviceToDevice, st));
-  if (B > 0) {
-    broadcast_vnf_kernel<<<(unsigned)((B * C * kH + 255) / 256), 256, 0, st>>>(d->B, d->C, vnf, Sx[2]); ++g_launches;
-    CK(cudaGetLastError());
-  }
-  const bool rf = d->flags & FEGNN_F_RF;
-  for (int i = 0; i < ntop; ++i)
-    CK(cudaMemsetAsync(sv_[i].msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), st));
-  // phi_h weight images off the chain (ring): the first ntop layers' here in one launch, layer l + 1 >= ntop's on the side
-  // stream next to graph_post(l) (the image buffer of that block was last read by phi_h of layer l + 1 - nb, ahead of the fork)
-  const bool img_ahead = two && g_node_fwd_mode != 0 && !rf && L > 1;
-  auto weight_images = [&](int l0, int nl, cudaStream_t s_) -> cudaError_t {
-    const float *w0[32], *w2[32];
-    float* img[32];
-    for (int l = 0; l < nl; ++l) { w0[l] = layers[l0 + l].node_w0; w2[l] = layers[l0 + l].node_w2; img[l] = sv_[(l0 + l) % nb].wimg; }
-    return launch_node_h_wprep(d->C, ldn(d), nl, w0, w2, img, s_);
-  };
-  const int nimg_top = ntop < L - 1 ? ntop : L - 1;      // the last layer has no phi_h
-  if (img_ahead && nimg_top > 0) CK(weight_images(0, nimg_top, st));
-  const bool graph_pending = g->ready_event != nullptr;
-  if (graph_pending) {
-    // the CSR sort is still running on another stream: everything above and the first layer's node phase read no graph
-    // array and run under it; this stream joins the sort here
-    fegnn_dims d0 = *d;
-    d0.flags |= FEGNN_F_PREZEROED;
-    if (rf || L == 1) d0.flags |= FEGNN_F_LAST;
-    TRY(node_pre_forward_run(&d0, &layers[0], h[2], &sv_[0], stream));
-    CK(cudaStreamWaitEvent(st, static_cast<cudaEvent_t>(g->ready_event), 0));
-  }
-  TRY(graph_xsum_run(d->N, d->B, x[2], g->batch, xsum[2], det, stream));
-  SideStream* sd = side_stream();
-  RQ(sd != nullptr);
-  void* side = sd->st;
-  FORK(sd, st);
-  int cur = 2;                                    // state entering the layer
-  for (int l = 0; l < L; ++l) {
-    fegnn_dims dl = *d;
-    const bool last = rf || l == L - 1;
-    if (last) dl.flags |= FEGNN_F_LAST;
-    dl.flags |= FEGNN_F_PREZEROED;                // one fill of the block's accumulators here instead of one per phase ...
-    if (img_ahead) dl.flags |= FEGNN_F_WIMG_READY;
-    const fegnn_layer_params* pl = &layers[l];
-    const int nxt = cur == 2 ? 0 : (cur ^ 1);
-    const int hs = rf ? 2 : cur;                  // layer whose (h, S) this layer reads
-    fegnn_layer_saved* sv = &sv_[l % nb];
-    // ring: the first ntop blocks are filled ahead of the chain, the block of a layer l >= nb on the side stream during layer
-    // l - 1 (below) -- a memset node between two kernels of the chain would cut their programmatic overlap
-    if (two) {
-      if (l >= nb) CK(cudaStreamWaitEvent(st, sd->aux, 0));
-    } else if (l > 0) {
-      CK(cudaMemsetAsync(sv->msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), st));
-    }
-    // ... and the per-graph coordinate sums of the state this layer produces on the side stream (last read by the per-graph
-    // kernels of the layer that consumed that state, earlier on the same stream; joined in front of virtual_forward)
-    CK(cudaMemsetAsync(xsum[nxt], 0, sizeof(float) * 3 * B, S(side)));
-    TRY(graph_pre_forward_run(&dl, g, pl, Z[cur], Sx[hs], xsum[cur], sv, side));
-    if (!(graph_pending && l == 0)) TRY(node_pre_forward_run(&dl, pl, h[hs], sv, stream));
-    if (rf) TRY(fegnn_rf_vel_forward(d->N, v, pl, sv->sv, stream));
-    TRY(edge_forward_run(&dl, g, pl, x[cur], sv, det, stream));
-    JOIN(sd, st);
-    TRY(virtual_forward_run(&dl, g, pl, x[cur], v, Z[cur], sv, x[nxt], xsum[nxt], det, stream));
-    FORK(sd, st);
-    if (two && l + 1 >= nb && l + 1 < L) {
-      // the accumulators of the ring block that layer l + 1 reuses: last read by layer l + 1 - nb (node phase on this stream
-      // ahead of the fork, per-graph kernels earlier on the side stream)
-      CK(cudaMemsetAsync(sv_[(l + 1) % nb].msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), S(side)));
-      CK(cudaEventRecord(sd->aux, S(side)));
-    }
-    if (!last) TRY(node_h_forward_run(&dl, g, pl, h[cur], sv, h[nxt], det, stream));
-    TRY(graph_post_forward_run(&dl, g, pl, Z[cur], Sx[hs], sv, Z[nxt], Sx[nxt], side));
-    if (img_ahead && l + 2 < L && l + 1 >= nimg_top) CK(weight_images(l + 1, 1, S(side)));
-    // the shared block is rewritten by the next layer: its per-graph kernels (side) must not start before this layer's
-    // node_h (main) has read u / msum, and its main-stream kernels not before this layer's graph_post (side) has read
-    // Dsum / Usum.  (Ring: block l % nb is next written by layer l + nb, whose kernels are ordered behind both by the
-    // joins in front of the virtual_forward calls in between.)
-    if (!two) {
-      JOIN(sd, st);
-      FORK(sd, st);
-    }
-    cur = nxt;
-  }
-  JOIN(sd, st);
-  CK(cudaMemcpyAsync(x_out, x[cur], sizeof(float) * 3 * N, cudaMemcpyDeviceToDevice, st));
-  CK(cudaMemcpyAsync(Z_out, Z[cur], sizeof(float) * 3 * C * B, cudaMemcpyDeviceToDevice, st));
-  return 0;
+  TRY(check_layers(d, L, layers));
+  DetWs det;
+  if (g_det) det_ws_bind(d, workspace + base_floats, &det);
+  ModelWs w;                                      // FEGNN_F_RECOMPUTE is a training-stack flag: nothing is kept here anyway
+  infer_ws_bind(d, L, workspace, g_det ? &det : nullptr, &w);
+  return forward_stack(d, L, Fin, g, layers, embed_w, embed_b, vnf, node_feat, x0, v, loc_mean, x_out, Z_out, w, stream);
 }
 
 int fegnn_model_backward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn_graph* g,
@@ -1381,6 +1362,7 @@ int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, con
   RQ(!(d->flags & FEGNN_F_REBUILD_ALL) || (d->flags & FEGNN_F_RECOMPUTE));
   if (scratch_floats < bwd_scratch_floats(d))
     return fail(FEGNN_ENOMEM, "backward scratch %zu < %zu floats", scratch_floats, bwd_scratch_floats(d));
+  TRY(check_layers(d, L, layers));
   cudaStream_t st = S(stream);
   ModelWs w;
   model_ws_bind(d, L, const_cast<float*>(workspace), &w);
@@ -1410,38 +1392,27 @@ int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, con
   FORK(sd, st);                                   // side: graph_post_bwd(L-1)
   const bool rf = d->flags & FEGNN_F_RF;
   // FEGNN_F_RECOMPUTE (DESIGN 3.8): layer l's block is block l % 2.  The forward leaves the blocks of layers L - 1 and L - 2
-  // complete (unless a backward has run since: FEGNN_F_REBUILD_ALL); every layer below is rebuilt from its input state just before its backward (recompute(l)).  Its accumulator fill,
-  // phi_h weight images and graph_pre run on the side stream during backward(l + 1), behind the last readers of the block
-  // (backward(l + 2), ahead of the fork in front of graph_pre_bwd(l + 1)); the main stream waits for them (aux) at recompute(l).
+  // complete (unless a backward has run since: FEGNN_F_REBUILD_ALL); every layer below is rebuilt from its input state just
+  // before its backward (recompute(l)).  Its accumulator fill, phi_h weight images and graph_pre run on the side stream during
+  // backward(l + 1), behind the last readers of the block (backward(l + 2), ahead of the fork in front of graph_pre_bwd(l + 1)).
+  // recompute(l) waits for the fill (aux) before its first kernel and for the rest at its join in front of the virtual forward.
   // A backward leaves the ring blocks holding layers 0 / 1, not L - 1 / L - 2: a further backward over the same forward
   // passes FEGNN_F_REBUILD_ALL and then rebuilds those two as well (the top layer's preparation runs ahead of the loop).
   const bool rc = d->flags & FEGNN_F_RECOMPUTE;
   const bool rebuild_all = d->flags & FEGNN_F_REBUILD_ALL;
   const bool rc_img = g_node_fwd_mode != 0 && !rf;
   auto recomputed = [&](int l) { return rc && l >= 0 && (rebuild_all || l + 2 < L); };
-  auto layer_dims = [&](int l) {
-    fegnn_dims dl = *d;
-    dl.flags &= ~(FEGNN_F_RECOMPUTE | FEGNN_F_REBUILD_ALL);
-    dl.flags |= FEGNN_F_PREZEROED;
-    if (rf || l == L - 1) dl.flags |= FEGNN_F_LAST;
-    return dl;
-  };
   // side stream, ahead of recompute(l): the block's accumulator fill, layer l's phi_h weight images and graph_pre(l)
   auto prepare = [&](int l) -> int {
-    const fegnn_dims dp = layer_dims(l);
-    fegnn_layer_saved* svp = &w.saved[l];
-    CK(cudaMemsetAsync(svp->msum, 0, sizeof(float) * fegnn_layer_saved_accum_floats(d), S(side)));
-    if (rc_img && !(dp.flags & FEGNN_F_LAST)) {
-      const float *w0 = layers[l].node_w0, *w2 = layers[l].node_w2;
-      CK(launch_node_h_wprep(d->C, ldn(d), 1, &w0, &w2, &svp->wimg, S(side)));
-    }
-    TRY(graph_pre_forward_run(&dp, g, &layers[l], w.Z[l], w.Sx[rf ? 0 : l], w.xsum[l], svp, side));
-    CK(cudaEventRecord(sd->aux, S(side)));
+    const fegnn_dims dp = layer_dims(d, L, l);
+    TRY(ring_fill(d, w.saved[l], sd));
+    if (rc_img && !(dp.flags & FEGNN_F_LAST)) CK(weight_images(d, layers, w, l, 1, S(side)));
+    TRY(graph_pre_forward_run(&dp, g, &layers[l], w.Z[l], w.Sx[rf ? 0 : l], w.xsum[l], &w.saved[l], side));
     return 0;
   };
   if (recomputed(L - 1)) TRY(prepare(L - 1));     // rebuild_all: behind the fork above (the caller's stream order)
   for (int l = L - 1; l >= 0; --l) {
-    fegnn_dims dl = layer_dims(l);
+    fegnn_dims dl = layer_dims(d, L, l);
     const bool last = rf || l == L - 1;
     const fegnn_layer_params* p = &layers[l];
     fegnn_layer_grads* gr = &grads[l];
@@ -1450,16 +1421,10 @@ int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, con
     if (recomputed(l)) {
       // recompute(l): node_pre, edge, virtual (u, Dsum, Usum) and phi_h (zh1) forwards of layer l from state l.  graph_post's
       // forward is not rerun: it writes only Z' / S' (state l + 1), and its backward reads S, Usum and the gradients.
-      CK(cudaStreamWaitEvent(st, sd->aux, 0));                    // fill, weight images, graph_pre(l) (M, Zc, G1)
-      TRY(node_pre_forward_run(&dl, p, w.h[ls], sv, stream));
-      if (rf) TRY(fegnn_rf_vel_forward(d->N, v, p, sv->sv, stream));
-      TRY(edge_forward_run(&dl, g, p, w.x[l], sv, nullptr, stream));
       fegnn_dims ds = dl;
       ds.flags |= FEGNN_F_RECOMPUTE;                              // the saved-only forms
       if (rc_img) ds.flags |= FEGNN_F_WIMG_READY;
-      TRY(virtual_forward_run(&ds, g, p, w.x[l], v, w.Z[l], sv, nullptr, nullptr, nullptr, stream));
-      FORK(sd, st);                                               // graph_post_bwd(l) reads Usum
-      if (!last) TRY(node_h_forward_run(&ds, g, p, w.h[l], sv, nullptr, nullptr, stream));
+      TRY(layer_forward(&ds, g, p, v, w, l, true, true, sd, stream));    // its fork: graph_post_bwd(l) reads Usum
     }
     // the edge backward's bound statistics come out of this layer's virtual backward (max|gt|, max|x - x_0|) and node_h
     // backward (max|gm|; the last layer has no gm) when those run on their tensor-core kernels: no pre-pass kernel on the chain
