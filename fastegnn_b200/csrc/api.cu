@@ -107,14 +107,19 @@ const int g_overlap_vsms = getenv("FEGNN_OVERLAP_VSMS") ? atoi(getenv("FEGNN_OVE
 constexpr int kNodeTcMinN = 0;
 inline bool node_bwd_tc(int N) { return g_node_bwd_mode == 1 || (g_node_bwd_mode == 2 && N >= kNodeTcMinN); }
 
+// "grid_sms" (fegnn_set_mode; test-only): 0 = the device's SM count (default), n >= 2 = min(n, that count).  sm_count()
+// sizes launch shapes only (persistent grids, the layer_overlap SM split), never a workspace, so a small cap makes every
+// persistent kernel run many tiles per CTA at sizes where the fp64 reference is instant.
+int g_grid_sms = 0;
+
 int sm_count() {
   static int sms[64] = {};                  // per device ordinal (a process may drive several GPUs)
   int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 148;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return g_grid_sms > 0 ? min(g_grid_sms, 148) : 148;
   if (sms[dev] == 0) {
     if (cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms[dev] <= 0) sms[dev] = 148;
   }
-  return sms[dev];
+  return g_grid_sms > 0 ? min(g_grid_sms, sms[dev]) : sms[dev];
 }
 
 // the deterministic loss forward keeps per-CTA partials in the caller's workspace (fegnn_loss_workspace_floats)
@@ -363,6 +368,12 @@ int fegnn_set_mode(const char* phase, int mode) {
     g_layer_overlap = mode;
     return 0;
   }
+  if (strcmp(phase, "grid_sms") == 0) {
+    // layer_overlap splits the SMs between two kernels (at least one each): a cap needs two
+    if (mode != 0 && mode < 2) return fail(FEGNN_EINVAL, "grid_sms must be 0 (the device's SM count) or at least 2");
+    g_grid_sms = mode;
+    return 0;
+  }
   return fail(FEGNN_EINVAL, "unknown phase '%s'", phase);
 }
 int fegnn_get_mode(const char* phase) {
@@ -374,6 +385,7 @@ int fegnn_get_mode(const char* phase) {
   if (phase != nullptr && strcmp(phase, "virtual_backward") == 0) return g_virt_bwd_mode;
   if (phase != nullptr && strcmp(phase, "deterministic") == 0) return g_det;
   if (phase != nullptr && strcmp(phase, "layer_overlap") == 0) return g_layer_overlap;
+  if (phase != nullptr && strcmp(phase, "grid_sms") == 0) return g_grid_sms;
   return -1;
 }
 

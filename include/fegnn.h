@@ -192,7 +192,10 @@ unsigned long long fegnn_launch_count(void);
  * Under 2, fegnn_model_backward(_inputs) runs each layer's virtual backward on a second internal stream next to its edge
  * backward (the edge backward's tiles are then claimed dynamically); under 0 the two run one after the other on `stream`;
  * under 1 the first where the virtual backward has more than one and at most 1.5 waves of tiles (one CTA per SM), else
- * the second.  Both arrangements run the same arithmetic; float sums are added in arrival order either way. */
+ * the second.  Both arrangements run the same arithmetic; float sums are added in arrival order either way.
+ * "grid_sms" (test-only): 0 (default) = every persistent grid is sized from the device's SM count; n >= 2 = from
+ * min(n, that count), so that each CTA of a small problem runs several tiles (1 and negatives are refused: layer_overlap
+ * splits the SMs between two kernels).  It changes launch shapes only (which CTA takes which tile), no workspace size. */
 int fegnn_set_mode(const char* phase, int mode);
 int fegnn_get_mode(const char* phase);
 
