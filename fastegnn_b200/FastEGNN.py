@@ -28,8 +28,8 @@ import torch
 from torch import nn
 
 from . import _lib as L
-from .ops import (CsrGraph, SavedBlock, _on, _require_cuda, _stream, layer_ptrs, make_dims, node_attr_arg,
-                  segment_reduce)
+from .ops import (CsrGraph, SavedBlock, _on, _require_cuda, _stream, layer_ptrs, live_flag, make_dims,
+                  node_attr_arg, segment_reduce)
 
 lib = L.lib
 
@@ -129,7 +129,7 @@ class _StackFn(torch.autograd.Function):
         dev = x0.device
         N, B, Cc, Lyr = graph.N, graph.B, mod.virtual_channels, mod.n_layers
         recompute = bool(mod.recompute)
-        flags = mod._flag_word | (L.F_RECOMPUTE if recompute else 0)
+        flags = mod._flag_word | (L.F_RECOMPUTE if recompute else 0) | live_flag(graph)
         dims = make_dims(N, N, graph.E, B, Cc, graph.Fe, flags, mod._gravity, Fa=mod._node_attr_nf, node_attr=node_attr)
         pd = C.byref(dims)
         table, names = mod._param_table()
@@ -201,8 +201,8 @@ def _stack_inference(mod: "FastEGNN", graph: CsrGraph, node_attr, node_feat, x0,
     per-layer intermediates -- a ring of four blocks up to 65 536 nodes; nothing is kept for a backward)."""
     dev = x0.device
     N, B, Cc, Lyr = graph.N, graph.B, mod.virtual_channels, mod.n_layers
-    dims = make_dims(N, N, graph.E, B, Cc, graph.Fe, mod._flag_word, mod._gravity, Fa=mod._node_attr_nf,
-                     node_attr=node_attr)
+    dims = make_dims(N, N, graph.E, B, Cc, graph.Fe, mod._flag_word | live_flag(graph), mod._gravity,
+                     Fa=mod._node_attr_nf, node_attr=node_attr)
     pd = C.byref(dims)
     table, _ = mod._param_table()
     # + the scratch of the deterministic kernels, behind it (0 with the mode off)

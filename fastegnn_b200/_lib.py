@@ -23,6 +23,9 @@ MAX_FA = 16
 F_ATTENTION, F_NORMALIZE, F_TANH, F_GRAVITY, F_LAST, F_RF, F_COORDS_SUM, F_NODE_SUM, F_PREZEROED = 1, 2, 4, 8, 16, 32, 64, 128, 256
 F_RECOMPUTE = 2048          # training stack: two saved blocks, each layer's rebuilt in the backward (DESIGN 3.8)
 F_REBUILD_ALL = 4096        # with F_RECOMPUTE: a backward after another one over the same forward rebuilds every layer
+F_LIVE_EDGES = 8192         # fegnn_dims.E is a capacity; the live edge count is the device word fegnn_graph.n_edges
+# sticky status bits of fegnn_graph_prep_live / fegnn_radius_graph_fill_live
+LIVE_BAD_COUNT, LIVE_CAND_OVERFLOW, LIVE_EDGE_OVERFLOW = 1, 2, 4
 
 fp = C.POINTER(C.c_float)
 ip = C.POINTER(C.c_int32)
@@ -37,7 +40,7 @@ class Dims(C.Structure):
 
 class Graph(C.Structure):
     _fields_ = [("row", C.c_void_p), ("col", C.c_void_p), ("batch", C.c_void_p), ("edge_attr", C.c_void_p),
-                ("dinv", C.c_void_p), ("inv_nb", C.c_void_p), ("ready_event", C.c_void_p)]
+                ("dinv", C.c_void_p), ("inv_nb", C.c_void_p), ("ready_event", C.c_void_p), ("n_edges", C.c_void_p)]
 
 
 # member order of fegnn_layer_params / fegnn_layer_grads -> reference state_dict suffix
@@ -120,10 +123,13 @@ SIGNATURES = {
     "fegnn_get_mode": (C.c_int, [C.c_char_p]),
     "fegnn_graph_prep_workspace_bytes": (C.c_size_t, [i32, i32]),
     "fegnn_graph_prep": (C.c_int, [i32, i32, i32, i32] + [vp] * 12 + [vp, C.c_size_t, vp]),
+    "fegnn_graph_prep_live": (C.c_int, [i32, i32, i32, i32] + [vp] * 12 + [vp, C.c_size_t, vp, vp, vp, vp]),
     "fegnn_radius_graph_workspace_bytes": (C.c_size_t, [i32, i32]),
     "fegnn_radius_graph_count": (C.c_int, [i32, i32, vp, vp, C.c_float, vp, vp, vp, vp, vp, vp, C.c_size_t, vp]),
     "fegnn_radius_graph_fill": (C.c_int, [i32, i32, i32, C.c_float, C.c_double, vp, vp, vp, vp, i32, vp, vp, vp, i32,
                                           vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp]),
+    "fegnn_radius_graph_fill_live": (C.c_int, [i32, i32, i32, C.c_float, C.c_double, vp, vp, vp, vp, i32, vp, vp, vp, i32,
+                                               vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_size_t, vp]),
     "fegnn_embed_forward": (C.c_int, [i32, i32, vp, vp, vp, vp, vp]),
     "fegnn_embed_backward": (C.c_int, [i32, i32, vp, vp, vp, vp, vp, vp, vp]),
     "fegnn_graph_xsum": (C.c_int, [i32, i32, vp, vp, vp, vp]),

@@ -159,6 +159,18 @@ int check_input_grads(const fegnn_dims* d, const fegnn_input_grads* ig) {
   return 0;
 }
 
+// FEGNN_F_LIVE_EDGES: the graph must carry its live edge count, and the edge backward (edge_bwd) must have a kernel with a
+// live form -- modes 1, 2, 4 and 5 have none and refuse the flag.  Checked before any launch of an entry.
+int check_live(const fegnn_dims* d, const fegnn_graph* g, bool edge_bwd) {
+  if (d == nullptr || !(d->flags & FEGNN_F_LIVE_EDGES)) return 0;
+  if (g == nullptr || g->n_edges == nullptr)
+    return fail(FEGNN_EINVAL, "FEGNN_F_LIVE_EDGES is set but fegnn_graph.n_edges is NULL (the live edge count is required)");
+  const int m = g_edge_bwd_mode;
+  if (edge_bwd && (m == 1 || m == 2 || m == 4 || m == 5))
+    return fail(FEGNN_EINVAL, "edge_backward mode %d has no form for FEGNN_F_LIVE_EDGES (modes 0, 6 = auto, 7 and 8 have)", m);
+  return 0;
+}
+
 inline size_t al4(size_t n) { return (n + 3) & ~(size_t)3; }
 // Zero two float buffers with ONE memset node when they are neighbours in the caller's block (the model driver's
 // workspaces place them so; padding between 16-byte aligned slots is owned by the block), else with two.
@@ -196,6 +208,7 @@ EdgeArgs edge_args(const fegnn_dims* d, const fegnn_graph* g, const fegnn_layer_
   a.row = g->row; a.col = g->col; a.ea = g->edge_attr; a.x = x; a.P = sv->P; a.Q = sv->Q;
   a.w1 = p->edge_w0; a.W2 = p->edge_w2; a.b2 = p->edge_b2; a.W3 = p->cr_w0; a.b3 = p->cr_b0; a.w4 = p->cr_w2;
   a.wa = p->att_w; a.ba = p->att_b;
+  a.n_edges = (d->flags & FEGNN_F_LIVE_EDGES) ? g->n_edges : nullptr;
   static const unsigned exp_bits = getenv("FEGNN_EXP") ? (unsigned)atoi(getenv("FEGNN_EXP")) : 0u;
   a.exp = exp_bits;
   return a;
@@ -412,6 +425,26 @@ int fegnn_graph_prep(int32_t N, int32_t E, int32_t B, int32_t Fe, const int64_t*
   return 0;
 }
 
+int fegnn_graph_prep_live(int32_t N, int32_t E, int32_t B, int32_t Fe, const int64_t* edge_index, const int64_t* data_batch,
+                          const float* edge_attr, int32_t* perm, int32_t* rowptr, int32_t* row, int32_t* col,
+                          int32_t* batch, int32_t* gptr, float* edge_attr_sorted, float* dinv, float* inv_nb,
+                          void* workspace, size_t workspace_bytes, const int32_t* n_edges_in, int32_t* n_edges_out,
+                          uint32_t* status, void* stream) {
+  RQ(N >= 0 && E >= 0 && B >= 0 && Fe >= 0);
+  RQ(n_edges_in && n_edges_out && status);
+  RQ(rowptr && gptr && (N == 0 || (batch && data_batch && dinv)) && (B == 0 || inv_nb));
+  RQ(E == 0 || (edge_index && perm && row && col && workspace));
+  RQ(E == 0 || Fe == 0 || (edge_attr && edge_attr_sorted));
+  if (workspace_bytes < graph_prep_workspace_bytes(N, E))
+    return fail(FEGNN_ENOMEM, "graph_prep workspace %zu < %zu bytes", workspace_bytes, graph_prep_workspace_bytes(N, E));
+  SideStream* sd = E > 0 ? side_stream() : nullptr;
+  if (sd != nullptr) FORK(sd, S(stream));
+  CK(graph_prep(N, E, B, Fe, edge_index, data_batch, edge_attr, perm, rowptr, row, col, batch, gptr, edge_attr_sorted, dinv,
+                inv_nb, workspace, S(stream), sd != nullptr ? sd->st : S(stream), n_edges_in, n_edges_out, status));
+  if (sd != nullptr) JOIN(sd, S(stream));
+  return 0;
+}
+
 // ------------------------------------------------------------------ graph construction (SURVEY.md 8 f2)
 size_t fegnn_radius_graph_workspace_bytes(int32_t N, int32_t B) { return radius_graph_workspace_bytes(N, B); }
 
@@ -442,6 +475,21 @@ int fegnn_radius_graph_fill(int32_t N, int32_t B, int32_t Fe, float r, double ke
     return fail(FEGNN_ENOMEM, "radius_graph workspace %zu < %zu bytes", workspace_bytes, radius_graph_workspace_bytes(N, B));
   CK(radius_graph_fill(N, B, Fe, r, keep_frac, cand_capacity, batch, gptr, cand_rowptr, n_cand, cand_col, cand_dist,
                        cand_row, out_capacity, rowptr, row, col, edge_attr, dinv, n_edges, workspace, S(stream)));
+  return 0;
+}
+
+int fegnn_radius_graph_fill_live(int32_t N, int32_t B, int32_t Fe, float r, double keep_frac, const int32_t* batch,
+                                 const int32_t* gptr, const int32_t* cand_rowptr, const int32_t* n_cand,
+                                 int32_t cand_capacity, int32_t* cand_col, float* cand_dist, int32_t* cand_row,
+                                 int32_t out_capacity, int32_t* rowptr, int32_t* row, int32_t* col, float* edge_attr,
+                                 float* dinv, int32_t* n_edges, int32_t* n_live, uint32_t* status, void* workspace,
+                                 size_t workspace_bytes, void* stream) {
+  RQ(n_live && status);
+  TRY(fegnn_radius_graph_fill(N, B, Fe, r, keep_frac, batch, gptr, cand_rowptr, n_cand, cand_capacity, cand_col, cand_dist,
+                              cand_row, out_capacity, rowptr, row, col, edge_attr, dinv, n_edges, workspace, workspace_bytes,
+                              stream));
+  rg::live_status_kernel<<<1, 1, 0, S(stream)>>>(n_cand, cand_capacity, n_edges, out_capacity, n_live, status); ++g_launches;
+  CK(cudaGetLastError());
   return 0;
 }
 
@@ -489,6 +537,7 @@ int graph_pre_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn
                           const float* Sf, const float* xsum, fegnn_layer_saved* sv, void* stream) {
   TRY(check_dims(d));
   RQ(g && p && Z && Sf && xsum && sv);
+  TRY(check_live(d, g, false));
   GraphArgs a = graph_args(d, g, p);
   a.Z = Z; a.S = Sf; a.xsum = xsum; a.M = sv->M; a.Zc = sv->Zc; a.G1 = sv->G1;
   CK(launch_graph_pre_fwd(a, S(stream)));
@@ -516,10 +565,25 @@ int edge_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_laye
   TRY(check_dims(d));
   TRY(check_flags_params(d, p));
   RQ(g && x && sv);
+  TRY(check_live(d, g, false));
   EdgeArgs a = edge_args(d, g, p, x, sv);
   a.msum = sv->msum; a.tsum = sv->tsum;
   if (!(d->flags & FEGNN_F_PREZEROED)) CK(zero_pair(sv->msum, kH * (size_t)d->N, sv->tsum, 3 * (size_t)d->N, S(stream)));
   const int mode = d->Fe <= kTcMaxFe ? g_edge_fwd_mode : 0;
+  if (d->flags & FEGNN_F_LIVE_EDGES) {
+    // the kLive forms: grids from the capacity d->E, tiles from the live count
+    if (det != nullptr) {
+      a.slab = det->eslab;
+      if (mode == 3) CK((launch_edge_fwd_tc<3, true, true>(a, sm_count(), S(stream))));
+      else if (mode == 1) CK((launch_edge_fwd_tc<1, true, true>(a, sm_count(), S(stream))));
+      else CK((launch_edge_fwd<true, true>(a, sm_count(), S(stream))));
+      return 0;
+    }
+    if (mode == 3) CK((launch_edge_fwd_tc<3, false, true>(a, sm_count(), S(stream))));
+    else if (mode == 1) CK((launch_edge_fwd_tc<1, false, true>(a, sm_count(), S(stream))));
+    else CK((launch_edge_fwd<false, true>(a, sm_count(), S(stream))));
+    return 0;
+  }
   if (det != nullptr) {
     a.slab = det->eslab;
     if (mode == 3) CK((launch_edge_fwd_tc<3, true>(a, sm_count(), S(stream))));
@@ -542,6 +606,7 @@ int virtual_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_l
   const bool saved_only = d->flags & FEGNN_F_RECOMPUTE;
   RQ(g && x && v && Z && sv && (saved_only || (x_new && xsum_new)));
   RQ(!saved_only || det == nullptr);
+  TRY(check_live(d, g, false));
   VirtArgs a = virt_args(d, g, p, x, v, Z, sv);
   a.u = sv->u; a.x_new = x_new; a.Dsum = sv->Dsum; a.Usum = sv->Usum; a.xsum_new = xsum_new;
   if (!(d->flags & FEGNN_F_PREZEROED)) {
@@ -581,6 +646,7 @@ int node_h_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegnn_la
   const bool saved_only = d->flags & FEGNN_F_RECOMPUTE;
   RQ(g && p && h && sv && (saved_only || h_new));
   RQ(!saved_only || det == nullptr);
+  TRY(check_live(d, g, false));
   NodeHArgs a;
   memset(&a, 0, sizeof(a));
   a.N = d->N; a.C = d->C; a.ldn = ldn(d);
@@ -626,6 +692,7 @@ int graph_post_forward_run(const fegnn_dims* d, const fegnn_graph* g, const fegn
                            const float* Sf, const fegnn_layer_saved* sv, float* Z_new, float* S_new, void* stream) {
   TRY(check_dims(d));
   RQ(g && p && Z && Sf && sv && Z_new && ((d->flags & FEGNN_F_LAST) || S_new));
+  TRY(check_live(d, g, false));
   GraphArgs a = graph_args(d, g, p);
   a.Z = Z; a.S = Sf; a.Dsum = sv->Dsum; a.Usum = sv->Usum; a.Z_new = Z_new; a.S_new = S_new;
   CK(launch_graph_post_fwd(a, S(stream)));
@@ -685,6 +752,7 @@ int fegnn_graph_post_backward(const fegnn_dims* d, const fegnn_graph* g, const f
   TRY(check_dims(d));
   const bool last = d->flags & FEGNN_F_LAST;
   RQ(g && p && gr && sv && gZ_new && gZ && gS && gDsum && gUsum && (last || (Sf && gS_new)));
+  TRY(check_live(d, g, false));
   GraphArgs a = graph_args(d, g, p);
   a.S = Sf; a.Usum = sv->Usum; a.gZ_new = gZ_new; a.gS_new = gS_new;
   a.gZ = gZ; a.gS = gS; a.gDsum = gDsum; a.gUsum = gUsum;
@@ -700,6 +768,7 @@ int fegnn_node_h_backward(const fegnn_dims* d, const fegnn_graph* g, const fegnn
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(g && p && gr && sv && gh_new && gzh1 && gm && gu);
+  TRY(check_live(d, g, false));
   NodeHArgs a;
   memset(&a, 0, sizeof(a));
   a.N = d->N; a.C = d->C; a.ldn = ldn(d);
@@ -766,6 +835,7 @@ static int virtual_backward_run(const fegnn_dims* d, const fegnn_graph* g, const
   TRY(check_flags_params(d, p));
   TRY(check_input_grads(d, ig));
   RQ(g && gr && x && v && Z && sv && gx_new && gDsum && gAv && gG1 && gx && gZ && gsv && gt);
+  TRY(check_live(d, g, false));
   RQ(!gt_ahead || virt_bwd_tc(d, gu));
   RQ(!(d->flags & FEGNN_F_GRAVITY) || gsg);
   VirtArgs a = virt_args(d, g, p, x, v, Z, sv);
@@ -815,6 +885,7 @@ static int edge_backward_run(const fegnn_dims* d, const fegnn_graph* g, const fe
   TRY(check_flags_params(d, p));
   TRY(check_input_grads(d, ig));
   RQ(g && gr && x && sv && gt && gP && gQ && gx);
+  TRY(check_live(d, g, true));
   EdgeArgs a = edge_args(d, g, p, x, sv);
   a.gm = gm; a.gt = gt; a.gP = gP; a.gQ = gQ; a.gx = gx;
   a.g_w1 = gr->edge_w0; a.g_W2 = gr->edge_w2; a.g_b2 = gr->edge_b2;
@@ -823,19 +894,34 @@ static int edge_backward_run(const fegnn_dims* d, const fegnn_graph* g, const fe
   if (zero) CK(zero_pair(gP, kH * (size_t)d->N, gQ, kH * (size_t)d->Nl, S(stream)));
   const bool tc_ok = d->Fe <= kTcMaxFe && !(d->flags & FEGNN_F_ATTENTION);
   int mode = g_edge_bwd_mode;
-  if (mode == 6) mode = (tc_ok && sv->scratch != nullptr) ? 7 : 4;      // auto: the packed-fp16 kernel wherever it applies
-  if ((mode == 7 || mode == 8) && (!tc_ok || sv->scratch == nullptr)) mode = 4;
+  // FEGNN_F_LIVE_EDGES: modes 1, 2, 4 and 5 were refused above; where 7 / 8 do not apply the fp32 kernel (0) takes their place
+  const bool live = d->flags & FEGNN_F_LIVE_EDGES;
+  if (mode == 6) mode = (tc_ok && sv->scratch != nullptr) ? 7 : (live ? 0 : 4);      // auto: the packed-fp16 kernel wherever it applies
+  if ((mode == 7 || mode == 8) && (!tc_ok || sv->scratch == nullptr)) mode = live ? 0 : 4;
   const bool pre = !(d->flags & FEGNN_F_STATS_READY);      // the bound pre-pass (its statistics came with the layer's other phases)
   if (ig != nullptr && ig->edge_attr != nullptr) {
     // dL/d edge_attr: the kEa instantiations (modes checked above); the output rides in the slots the forward uses for
     // msum / tsum, so the argument block is the default one's
     a.g_ea = ig->edge_attr;
     a.perm = ig->perm;
+    if (live) {
+      if (tc_ok && sv->scratch != nullptr && mode == 7)
+        CK((launch_edge_bwd_tc4<2, true, true>(a, reinterpret_cast<unsigned*>(sv->scratch), cap, S(stream), zero && pre, pre, claim)));
+      else
+        CK((launch_edge_bwd<true, true>(a, sm_count(), S(stream))));
+      return 0;
+    }
     if (tc_ok && sv->scratch != nullptr && mode == 7) {
       CK((launch_edge_bwd_tc4<2, true>(a, reinterpret_cast<unsigned*>(sv->scratch), cap, S(stream), zero && pre, pre, claim)));
     } else {
       CK(launch_edge_bwd<true>(a, sm_count(), S(stream)));
     }
+    return 0;
+  }
+  if (live) {
+    if (mode == 7) CK((launch_edge_bwd_tc4<2, false, true>(a, reinterpret_cast<unsigned*>(sv->scratch), cap, S(stream), zero && pre, pre, claim)));
+    else if (mode == 8) CK((launch_edge_bwd_tc4<4, false, true>(a, reinterpret_cast<unsigned*>(sv->scratch), cap, S(stream), zero && pre, pre, claim)));
+    else CK((launch_edge_bwd<false, true>(a, sm_count(), S(stream))));
     return 0;
   }
   if (mode == 7) CK(launch_edge_bwd_tc4<2>(a, reinterpret_cast<unsigned*>(sv->scratch), cap, S(stream), zero && pre, pre, claim));
@@ -862,6 +948,7 @@ int fegnn_graph_pre_backward(const fegnn_dims* d, const fegnn_graph* g, const fe
   NO_DET("the layer kernels add edge, node and graph sums across CTAs with float atomics");
   TRY(check_dims(d));
   RQ(g && p && gr && Sf && sv && gG1 && gS && gZ && gxsum);
+  TRY(check_live(d, g, false));
   GraphArgs a = graph_args(d, g, p);
   a.S = Sf; a.M = sv->M; a.Zc = sv->Zc; a.gG1 = gG1; a.gS = gS; a.gZ = gZ; a.gxsum = gxsum;
   a.g_wv1 = gr->edgev_w0;
@@ -1313,6 +1400,7 @@ int fegnn_model_forward(const fegnn_dims* d, int32_t L, int32_t Fin, const fegnn
   TRY(check_dims(d));
   RQ(L >= 1 && L <= 32 && g && layers && embed_w && embed_b && vnf && workspace && x_out && Z_out);
   RQ(d->Nl == d->N);   // the partitioned path drives the phases itself (halo rows come from peers)
+  TRY(check_live(d, g, false));
   if (workspace_floats < model_ws_floats(d, L))
     return fail(FEGNN_ENOMEM, "model workspace %zu < %zu floats", workspace_floats, model_ws_floats(d, L));
   TRY(check_layers(d, L, layers));
@@ -1339,6 +1427,7 @@ int fegnn_model_forward_inference(const fegnn_dims* d, int32_t L, int32_t Fin, c
   TRY(check_dims(d));
   RQ(L >= 1 && L <= 32 && g && layers && embed_w && embed_b && vnf && workspace && x_out && Z_out);
   RQ(d->Nl == d->N);
+  TRY(check_live(d, g, false));
   // deterministic mode: the kDet forms of the phases, with their scratch behind the workspace
   const size_t base_floats = fegnn_model_inference_workspace_floats(d);
   const size_t need = base_floats + fegnn_model_inference_det_workspace_floats(d);
@@ -1372,6 +1461,7 @@ int fegnn_model_backward_inputs(const fegnn_dims* d, int32_t L, int32_t Fin, con
   RQ(L >= 1 && L <= 32 && g && layers && grads && embed_w && g_embed_w && g_embed_b && g_vnf && workspace && scratch);
   RQ(gx_out && gZ_out && g_x0 && g_loc_mean && d->Nl == d->N);
   RQ(!(d->flags & FEGNN_F_REBUILD_ALL) || (d->flags & FEGNN_F_RECOMPUTE));
+  TRY(check_live(d, g, true));
   if (scratch_floats < bwd_scratch_floats(d))
     return fail(FEGNN_ENOMEM, "backward scratch %zu < %zu floats", scratch_floats, bwd_scratch_floats(d));
   TRY(check_layers(d, L, layers));

@@ -30,7 +30,18 @@ struct EdgeArgs {
   union { float* gP; float* slab; };
   float *gQ, *gx;
   float *g_w1, *g_W2, *g_b2, *g_W3, *g_b3, *g_w4, *g_wa, *g_ba;
+  const int* n_edges;   // FEGNN_F_LIVE_EDGES: the live edge count (device word); E is then the capacity.  Read by kLive only
 };
+
+// The live edge count of a kLive kernel, clamped to [0, capacity].  An earlier kernel of the stream may have written the
+// word (graph prep, the radius graph): it is not weight-only data, so a kernel reads it once per CTA AFTER pdl_wait(), and
+// through L2 (ld.global.cg: no non-coherent load the compiler could hoist above the wait).  The kLive forms then overwrite
+// their copy of a.E with it, so every bound below (tile counts, e < a.E, the dynamic tile claim, the deterministic
+// boundaries) is the live one, and no row / col / edge_attr entry at or past the live count is read.
+__device__ __forceinline__ int live_edges(const EdgeArgs& a) {
+  const int n = __ldcg(a.n_edges);
+  return n < 0 ? 0 : (n > a.E ? a.E : n);
+}
 
 // ---- deterministic forward (kDet): msum / tsum without arrival-order float sums
 // Each tile sums its runs of equal row ids in row order.  A run that stays inside the tile is the row's only contribution:
@@ -91,12 +102,18 @@ __device__ __forceinline__ void edge_det_tsum(const EdgeArgs& a, const int* srow
 }
 // One warp per tile boundary b (between tiles b - 1 and b): if a row r crosses it and b is r's first crossing, r's sums are
 // its slot in tile b - 1 plus slot 0 of every following tile it reaches, added in tile order.  Nothing else adds into r.
+// kLive: the boundaries of the live count (FEGNN_F_LIVE_EDGES); the grid covers those of the capacity.
+template <bool kLive = false>
 __global__ void __launch_bounds__(256) edge_det_fixup_kernel(EdgeArgs a) {
   pdl_trigger();
   const int lane = threadIdx.x & 31;
   const int b = (int)((blockIdx.x * 256u + threadIdx.x) >> 5) + 1;
-  const int ntiles = (a.E + kTM - 1) / kTM;
+  int ntiles = (a.E + kTM - 1) / kTM;
   pdl_wait();
+  if constexpr (kLive) {
+    a.E = live_edges(a);
+    ntiles = (a.E + kTM - 1) / kTM;
+  }
   if (b >= ntiles) return;
   const int e = b * kTM, s = e - kTM, r = a.row[e];
   if (a.row[e - 1] != r) return;
@@ -112,10 +129,11 @@ __global__ void __launch_bounds__(256) edge_det_fixup_kernel(EdgeArgs a) {
     else a.tsum[(size_t)r * 3 + (j - kH)] = acc;
   }
 }
+template <bool kLive = false>
 inline cudaError_t launch_edge_det_fixup(const EdgeArgs& a, cudaStream_t st) {
   const int nb = (a.E + kTM - 1) / kTM - 1;      // tile boundaries
   if (nb <= 0) return cudaSuccess;
-  if (cudaError_t e_ = launch_pdl(edge_det_fixup_kernel, (nb + 7) / 8, 256, 0, st, a)) return e_;
+  if (cudaError_t e_ = launch_pdl(edge_det_fixup_kernel<kLive>, (nb + 7) / 8, 256, 0, st, a)) return e_;
   return cudaGetLastError();
 }
 
@@ -222,7 +240,8 @@ constexpr size_t kEdgeFwdSmem = (2 * kWFloats + 2 * kTileFloats) * sizeof(float)
 constexpr size_t kEdgeBwdSmem = (2 * kWFloats + 5 * kTileFloats) * sizeof(float) + sizeof(EdgeSmemVec);
 
 // kDet: msum / tsum through edge_det_msum / edge_det_tsum and the boundary slab (same terms, summed in row order)
-template <bool kDet>
+// kLive: the live edge count (live_edges) bounds the tiles instead of the capacity a.E
+template <bool kDet, bool kLive = false>
 __global__ void __launch_bounds__(kThreads, 2) edge_fwd_kernel(EdgeArgs a) {
   extern __shared__ __align__(16) float smem[];
   float* W2s = smem;
@@ -233,6 +252,10 @@ __global__ void __launch_bounds__(kThreads, 2) edge_fwd_kernel(EdgeArgs a) {
   const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15, lane = tid & 31;
   const bool att = a.flags & FEGNN_F_ATTENTION, use_tanh = a.flags & FEGNN_F_TANH;
   edge_stage_common(a, v, W2s, W3s);
+  if constexpr (kLive) {
+    pdl_wait();
+    a.E = live_edges(a);
+  }
   const int ntiles = (a.E + kTM - 1) / kTM;
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     __syncthreads();   // previous iteration's readers of v / tiles are done; weights staged
@@ -295,7 +318,8 @@ __global__ void __launch_bounds__(kThreads, 2) edge_fwd_kernel(EdgeArgs a) {
 }
 
 // kEa: also g_ea[perm[e]][f] += sum_k gz1[e][k] Wa[f][k] (edge_attr enters phi_e's first Linear only)
-template <bool kEa>
+// kLive: the live edge count (live_edges) bounds the tiles instead of the capacity a.E
+template <bool kEa, bool kLive = false>
 __global__ void __launch_bounds__(kThreads, 1) edge_bwd_kernel(EdgeArgs a) {
   extern __shared__ __align__(16) float smem[];
   float* W2s = smem;
@@ -323,6 +347,10 @@ __global__ void __launch_bounds__(kThreads, 1) edge_bwd_kernel(EdgeArgs a) {
     for (int j = 0; j < 4; ++j) cWa[f][j] = 0.f;
   float cba = 0.f;
 
+  if constexpr (kLive) {
+    pdl_wait();
+    a.E = live_edges(a);
+  }
   const int ntiles = (a.E + kTM - 1) / kTM;
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     __syncthreads();
@@ -512,33 +540,34 @@ __global__ void __launch_bounds__(kThreads, 1) edge_bwd_kernel(EdgeArgs a) {
 }
 
 // ---------------------------------------------------------------------------- host side
-template <bool kDet = false>
+// kLive: grid from the capacity a.E; the kernel reads the live count
+template <bool kDet = false, bool kLive = false>
 cudaError_t launch_edge_fwd(const EdgeArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(edge_fwd_kernel<kDet>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEdgeFwdSmem);
+    cudaError_t e = cudaFuncSetAttribute(edge_fwd_kernel<kDet, kLive>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEdgeFwdSmem);
     if (e != cudaSuccess) return e;
     attr.set();
   }
   int ntiles = (a.E + kTM - 1) / kTM;
   if (ntiles == 0) return cudaSuccess;
   int grid = ntiles < 2 * sms ? ntiles : 2 * sms;
-  edge_fwd_kernel<kDet><<<grid, kThreads, kEdgeFwdSmem, st>>>(a); ++g_launches;
+  edge_fwd_kernel<kDet, kLive><<<grid, kThreads, kEdgeFwdSmem, st>>>(a); ++g_launches;
   if (cudaError_t e_ = cudaGetLastError()) return e_;
-  return kDet ? launch_edge_det_fixup(a, st) : cudaSuccess;
+  return kDet ? launch_edge_det_fixup<kLive>(a, st) : cudaSuccess;
 }
-template <bool kEa = false>
+template <bool kEa = false, bool kLive = false>
 cudaError_t launch_edge_bwd(const EdgeArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(edge_bwd_kernel<kEa>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEdgeBwdSmem);
+    cudaError_t e = cudaFuncSetAttribute(edge_bwd_kernel<kEa, kLive>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEdgeBwdSmem);
     if (e != cudaSuccess) return e;
     attr.set();
   }
   int ntiles = (a.E + kTM - 1) / kTM;
   if (ntiles == 0) return cudaSuccess;
   int grid = ntiles < sms ? ntiles : sms;
-  edge_bwd_kernel<kEa><<<grid, kThreads, kEdgeBwdSmem, st>>>(a); ++g_launches;
+  edge_bwd_kernel<kEa, kLive><<<grid, kThreads, kEdgeBwdSmem, st>>>(a); ++g_launches;
   return cudaGetLastError();
 }
 

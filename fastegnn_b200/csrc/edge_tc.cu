@@ -132,8 +132,8 @@ __device__ __forceinline__ float tc_silu_hb(float z, float b) {
 }
 
 // kDet: msum / tsum through edge_det_msum / edge_det_tsum and the boundary slab (edge_kernels.cu; same terms, summed in row
-// order)
-template <int SPLIT, bool kDet>
+// order).  kLive: the live edge count (live_edges, after the wait) bounds the tiles instead of the capacity a.E
+template <int SPLIT, bool kDet, bool kLive = false>
 __global__ void __launch_bounds__(kTcThreads, EdgeTcSmem<SPLIT>::ctas_per_sm) edge_fwd_tc_kernel(EdgeArgs a) {
   using SM = EdgeTcSmem<SPLIT>;
   extern __shared__ uint8_t smem_raw[];
@@ -167,6 +167,7 @@ __global__ void __launch_bounds__(kTcThreads, EdgeTcSmem<SPLIT>::ctas_per_sm) ed
   __syncthreads();
   umma::fence_after();
   pdl_wait();
+  if constexpr (kLive) a.E = live_edges(a);
   const uint32_t tmem = v->tmem_slot;
   const uint32_t tlane = tmem + ((uint32_t)((warp & 3) * 32) << 16) + half * 32;
   const uint32_t idesc = umma::make_idesc_tf32(128, 64);
@@ -369,12 +370,12 @@ __global__ void __launch_bounds__(kTcThreads, EdgeTcSmem<SPLIT>::ctas_per_sm) ed
   if (warp == 0) umma::tmem_dealloc<128>(tmem);
 }
 
-template <int SPLIT, bool kDet = false>
+template <int SPLIT, bool kDet = false, bool kLive = false>
 cudaError_t launch_edge_fwd_tc(const EdgeArgs& a, int sms, cudaStream_t st) {
   static DevOnce attr;
   const size_t bytes = EdgeTcSmem<SPLIT>::bytes;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(edge_fwd_tc_kernel<SPLIT, kDet>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    cudaError_t e = cudaFuncSetAttribute(edge_fwd_tc_kernel<SPLIT, kDet, kLive>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
     attr.set();
   }
@@ -382,9 +383,9 @@ cudaError_t launch_edge_fwd_tc(const EdgeArgs& a, int sms, cudaStream_t st) {
   if (ntiles == 0) return cudaSuccess;
   const int per_sm = EdgeTcSmem<SPLIT>::ctas_per_sm;
   const int grid = ntiles < per_sm * sms ? ntiles : per_sm * sms;
-  if (cudaError_t e_ = launch_pdl(edge_fwd_tc_kernel<SPLIT, kDet>, grid, kTcThreads, bytes, st, a)) return e_;
+  if (cudaError_t e_ = launch_pdl(edge_fwd_tc_kernel<SPLIT, kDet, kLive>, grid, kTcThreads, bytes, st, a)) return e_;
   if (cudaError_t e_ = cudaGetLastError()) return e_;
-  return kDet ? launch_edge_det_fixup(a, st) : cudaSuccess;
+  return kDet ? launch_edge_det_fixup<kLive>(a, st) : cudaSuccess;
 }
 
 }  // namespace fegnn

@@ -169,7 +169,10 @@ __device__ __forceinline__ float pow2_to(float bound, int e_target) {   // large
 // claim: NULL = static split (group G of CTA b takes tiles 2 b + G + n 2 gridDim.x); else a zeroed counter from which
 // each group takes its tiles one at a time, two ahead of the one it works on, so that a CTA that starts late (its SM held
 // by a kernel of another stream) takes what is left instead of a fixed share.
-template <int CG, bool kEa>
+//
+// kLive: the live edge count (live_edges, read after the wait) bounds the tiles, the static split and the dynamic claim,
+// instead of the capacity a.E that sized the grid
+template <int CG, bool kEa, bool kLive = false>
 __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, const unsigned* stats, unsigned* claim) {
   VTR_DECL();
   constexpr int NTG = 128 * CG, NT = 2 * NTG, CPT = kH / CG, NP = CPT / 2, NWG = NTG / 32, RPW = kTM / NWG;
@@ -240,6 +243,7 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
   __syncthreads();
     VTR();
   pdl_wait();                                    // everything above read weights only; `stats` comes from the pre-pass
+  if constexpr (kLive) a.E = live_edges(a);
   // ---- per-launch power-of-two scales (every thread, identical arithmetic).  Bounds from the pre-pass `stats`:
   //      |gs| <= dmax * sqrt3 * max|gt|  ->  sa ;  |w4| -> sb ;  g3 is stored times s3 = sa sb (<= 2^14)
   //      |g2| <= (max|gm| + 64 |g3| max|W3|) -> s2 ;  |gz1| <= 64 |g2| max|W2| -> s1   (stored values <= 2^15)
@@ -791,13 +795,13 @@ __global__ void __launch_bounds__(256 * CG, 1) edge_bwd_tc4_kernel(EdgeArgs a, c
 
 // stats: 4 unsigned of caller scratch (device); claim: NULL (static tile split) or a zeroed word (tiles claimed dynamically);
 // sms: the grid's cap
-template <int CG, bool kEa = false>
+template <int CG, bool kEa = false, bool kLive = false>
 inline cudaError_t launch_edge_bwd_tc4(const EdgeArgs& a, unsigned* stats, int sms, cudaStream_t st, bool zero_stats = true,
                                        bool run_stats = true, unsigned* claim = nullptr) {
   static DevOnce attr;
   const size_t bytes = bwd4::Smem4<CG>::bytes;
   if (!attr.get()) {
-    cudaError_t e = cudaFuncSetAttribute(bwd4::edge_bwd_tc4_kernel<CG, kEa>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    cudaError_t e = cudaFuncSetAttribute(bwd4::edge_bwd_tc4_kernel<CG, kEa, kLive>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
     attr.set();
   }
@@ -816,7 +820,7 @@ inline cudaError_t launch_edge_bwd_tc4(const EdgeArgs& a, unsigned* stats, int s
     e = launch_pdl(bwd3::edge_bwd_stats_kernel, sblocks, 256, 0, st, a.N, a.Nl, a.x, a.gt, a.gm, stats);
     if (e != cudaSuccess) return e;
   }
-  e = launch_pdl(bwd4::edge_bwd_tc4_kernel<CG, kEa>, grid, 256 * CG, bytes, st, a, (const unsigned*)stats, claim);
+  e = launch_pdl(bwd4::edge_bwd_tc4_kernel<CG, kEa, kLive>, grid, 256 * CG, bytes, st, a, (const unsigned*)stats, claim);
   if (e != cudaSuccess) return e;
   return cudaGetLastError();
 }

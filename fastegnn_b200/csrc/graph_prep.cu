@@ -532,6 +532,35 @@ __global__ void iota_copy_kernel(int E, const int64_t* __restrict__ row64, int* 
   }
 }
 
+// ---------------------------------------------------------------- live edge count (fegnn_graph_prep_live)
+// The edge list is padded to the capacity E; *n_in is the caller's live count, clamped to [0, E].  Edges past it are never
+// read as indices: the live path counts only live rows and sorts from the keys below instead of from the int64 rows.
+__device__ __forceinline__ int live_count(int E, const int* n_in) {
+  const int n = *n_in;
+  return n < 0 ? 0 : (n > E ? E : n);
+}
+__global__ void count_live_rows_kernel(int E, const int* __restrict__ n_in, const int64_t* __restrict__ row64,
+                                       int* __restrict__ deg) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < live_count(E, n_in)) atomicAdd(deg + (int)row64[e], 1);
+}
+// the first pass's (key, value) pairs: a live edge its row, a padding edge the key N (it sorts after every row); thread 0
+// also writes the clamped count (the graph's own word) and flags a count outside [0, E] in the sticky status word
+__global__ void live_keys_kernel(int N, int E, const int* __restrict__ n_in, const int64_t* __restrict__ row64,
+                                 int* __restrict__ keys, int* __restrict__ vals, int* __restrict__ n_out,
+                                 unsigned* __restrict__ status) {
+  const int live = live_count(E, n_in);
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < E) {
+    keys[e] = e < live ? (int)row64[e] : N;
+    vals[e] = e;
+  }
+  if (e == 0) {
+    *n_out = live;
+    if (*n_in != live) atomicOr(status, FEGNN_LIVE_BAD_COUNT);
+  }
+}
+
 __global__ void finalize_kernel(int E, int Fe, const int* __restrict__ keys, const int* __restrict__ vals,
                                 const int64_t* __restrict__ col64, const float* __restrict__ ea,
                                 int* __restrict__ perm, int* __restrict__ row, int* __restrict__ col,
@@ -555,9 +584,12 @@ size_t graph_prep_workspace_bytes(int N, int E) {
   return ((size_t)4 * E + 256 * G + 2 * sums + 64) * sizeof(int);      // two scan scratch areas: the two chains overlap
 }
 
+// n_live_in != nullptr: the live path of fegnn_graph_prep_live (E is the capacity; n_live_out / status as documented there)
 cudaError_t graph_prep(int N, int E, int B, int Fe, const int64_t* edge_index, const int64_t* data_batch,
                        const float* edge_attr, int* perm, int* rowptr, int* row, int* col, int* batch, int* gptr,
-                       float* ea_sorted, float* dinv, float* inv_nb, void* ws, cudaStream_t st, cudaStream_t st_counts) {
+                       float* ea_sorted, float* dinv, float* inv_nb, void* ws, cudaStream_t st, cudaStream_t st_counts,
+                       const int* n_live_in = nullptr, int* n_live_out = nullptr, unsigned* status = nullptr) {
+  const bool live = n_live_in != nullptr;
   const int G = (E + kSortTile - 1) / kSortTile;
   const int Gf = (E + kFusedTile - 1) / kFusedTile;
   static const bool fused_ok = getenv("FEGNN_SORT_FUSED") == nullptr || atoi(getenv("FEGNN_SORT_FUSED")) != 0;   // experiment switch
@@ -577,11 +609,17 @@ cudaError_t graph_prep(int N, int E, int B, int Fe, const int64_t* edge_index, c
     if ((e = cudaMemsetAsync(rowptr, 0, sizeof(int) * ((size_t)N + 1), sc)) != cudaSuccess) return e;
     if ((e = cudaMemsetAsync(gptr, 0, sizeof(int) * ((size_t)B + 1), sc)) != cudaSuccess) return e;
     if (fused_ok && N > 0 && B > 0 && N + 1 <= kSmemScan && B + 1 <= kSmemScan) {
-      const int n = E > N ? E : N;
-      count_rows_batch_kernel<<<(n + 255) / 256, 256, 0, sc>>>(E, N, edge_index, data_batch, rowptr, batch, gptr); ++g_launches;
+      if (live) {       // rows up to the live count; the fused kernel does the batch part alone (E = 0)
+        if (E > 0) { count_live_rows_kernel<<<(E + 255) / 256, 256, 0, sc>>>(E, n_live_in, edge_index, rowptr); ++g_launches; }
+        count_rows_batch_kernel<<<(N + 255) / 256, 256, 0, sc>>>(0, N, edge_index, data_batch, rowptr, batch, gptr); ++g_launches;
+      } else {
+        const int n = E > N ? E : N;
+        count_rows_batch_kernel<<<(n + 255) / 256, 256, 0, sc>>>(E, N, edge_index, data_batch, rowptr, batch, gptr); ++g_launches;
+      }
       scan2_recip_kernel<<<2, 1024, 0, sc>>>(rowptr, N + 1, dinv, gptr, B + 1, inv_nb); ++g_launches;
     } else {
-      if (E > 0) { count_rows_kernel<<<(E + 255) / 256, 256, 0, sc>>>(E, edge_index, rowptr); ++g_launches; }
+      if (E > 0 && live) { count_live_rows_kernel<<<(E + 255) / 256, 256, 0, sc>>>(E, n_live_in, edge_index, rowptr); ++g_launches; }
+      else if (E > 0) { count_rows_kernel<<<(E + 255) / 256, 256, 0, sc>>>(E, edge_index, rowptr); ++g_launches; }
       if (N > 0) { batch_kernel<<<(N + 255) / 256, 256, 0, sc>>>(N, data_batch, batch, gptr); ++g_launches; }
       if ((e = exclusive_scan(rowptr, N + 1, rowptr, nullptr, sums2, sc)) != cudaSuccess) return e;
       if ((e = exclusive_scan(gptr, B + 1, gptr, nullptr, sums2, sc)) != cudaSuccess) return e;
@@ -589,21 +627,27 @@ cudaError_t graph_prep(int N, int E, int B, int Fe, const int64_t* edge_index, c
       if (B > 0) { recip_kernel<<<(B + 255) / 256, 256, 0, sc>>>(B, gptr, inv_nb); ++g_launches; }
     }
   }
+  // live: the first pass's keys (padding -> N) into keysA / valsA, the clamped count and the status bit; the passes then
+  // all read keys from the workspace, on enough bits for the key N
+  if (live) {
+    live_keys_kernel<<<E > 0 ? (E + 255) / 256 : 1, 256, 0, st>>>(N, E, n_live_in, edge_index, keysA, valsA, n_live_out,
+                                                                  status); ++g_launches;
+  }
   if (E == 0) return cudaGetLastError();
   // radix sort (row, edge id)
   int bits = 1;
-  while (bits < 31 && (1ll << bits) < (long long)N) ++bits;
+  while (bits < 31 && (1ll << bits) < (long long)(live ? N + 1 : N)) ++bits;
   const int passes = (bits + 7) / 8;
-  const int* kin = nullptr;
-  const int* vin = nullptr;
-  int* kout = keysA;
-  int* vout = valsA;
+  const int* kin = live ? keysA : nullptr;
+  const int* vin = live ? valsA : nullptr;
+  int* kout = live ? keysB : keysA;
+  int* vout = live ? valsB : valsA;
   if (Gf <= kFusedMaxTiles && fused_ok) {
     // short chain: per pass one histogram launch and one scatter launch that scans for itself; the last one emits the CSR
     const CsrOut o{edge_index + E, edge_attr, perm, row, col, ea_sorted, Fe};
     for (int p = 0; p < passes; ++p) {
       const int shift = 8 * p;
-      const bool first = p == 0, lastp = p == passes - 1;
+      const bool first = p == 0 && !live, lastp = p == passes - 1;
       if (first) radix_hist_fused_kernel<true><<<Gf, kSortThreads, 0, st>>>(E, shift, edge_index, nullptr, hist);
       else radix_hist_fused_kernel<false><<<Gf, kSortThreads, 0, st>>>(E, shift, nullptr, kin, hist);
       ++g_launches;
@@ -625,11 +669,11 @@ cudaError_t graph_prep(int N, int E, int B, int Fe, const int64_t* edge_index, c
   }
   for (int p = 0; p < passes; ++p) {
     const int shift = 8 * p;
-    if (p == 0) radix_hist_kernel<true><<<G, kSortThreads, 0, st>>>(E, shift, edge_index, nullptr, G, hist);
+    if (p == 0 && !live) radix_hist_kernel<true><<<G, kSortThreads, 0, st>>>(E, shift, edge_index, nullptr, G, hist);
     else radix_hist_kernel<false><<<G, kSortThreads, 0, st>>>(E, shift, nullptr, kin, G, hist);
     ++g_launches;
     if ((e = exclusive_scan(hist, 256 * G, hist, nullptr, sums, st)) != cudaSuccess) return e;
-    if (p == 0)
+    if (p == 0 && !live)
       radix_scatter_kernel<true><<<G, kSortThreads, 0, st>>>(E, shift, edge_index, nullptr, nullptr, G, hist, kout, vout);
     else
       radix_scatter_kernel<false><<<G, kSortThreads, 0, st>>>(E, shift, nullptr, kin, vin, G, hist, kout, vout);

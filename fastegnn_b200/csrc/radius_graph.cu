@@ -441,6 +441,15 @@ static Workspace carve(void* base, int N, int B) {
   return w;
 }
 
+// fegnn_radius_graph_fill_live: the live count out of the uncapped totals, and the sticky overflow bits
+__global__ void live_status_kernel(const int* __restrict__ n_cand, int cand_cap, const int* __restrict__ n_edges, int out_cap,
+                                   int* __restrict__ n_live, unsigned* __restrict__ status) {
+  const int nc = *n_cand, ne = *n_edges;
+  *n_live = ne < 0 ? 0 : (ne > out_cap ? out_cap : ne);
+  const unsigned bits = (nc > cand_cap ? FEGNN_LIVE_CAND_OVERFLOW : 0u) | (ne > out_cap ? FEGNN_LIVE_EDGE_OVERFLOW : 0u);
+  if (bits != 0u) atomicOr(status, bits);
+}
+
 }  // namespace rg
 
 size_t radius_graph_workspace_bytes(int N, int B) { return rg::carve(nullptr, N, B).bytes; }

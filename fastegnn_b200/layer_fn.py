@@ -13,7 +13,7 @@ from typing import Optional
 import torch
 
 from . import _lib as L
-from .ops import CsrGraph, SavedBlock, _on, _require_cuda, _stream, layer_ptrs, make_dims
+from .ops import CsrGraph, SavedBlock, _on, _require_cuda, _stream, layer_ptrs, live_flag, make_dims
 
 lib = L.lib
 
@@ -136,7 +136,9 @@ class _LayerFn(torch.autograd.Function):
         named = dict(zip(names, params))
         ptrs = layer_ptrs(named, "")
         Fa = 0 if node_attr is None else node_attr.size(1)
-        dims = make_dims(graph.N, graph.N, graph.E, graph.B, Cc, graph.Fe, flags, grav, Fa=Fa, node_attr=node_attr)
+        # a live graph (CsrGraph.live): E is its capacity and the phases read the live count (FEGNN_F_LIVE_EDGES)
+        dims = make_dims(graph.N, graph.N, graph.E, graph.B, Cc, graph.Fe, flags | live_flag(graph), grav, Fa=Fa,
+                         node_attr=node_attr)
         ph = LayerPhases(dims, graph, ptrs, dev)
         xsum = torch.empty(graph.B, 3, device=dev, dtype=torch.float32)
         with _on(dev):

@@ -43,16 +43,44 @@ def _prep_stream(dev) -> "torch.cuda.Stream":
     return _PREP_STREAMS[key]
 
 
+def _live_count_arg(n_edges: torch.Tensor) -> None:
+    """The live edge count of CsrGraph(..., n_edges=): checked before any device work."""
+    if not isinstance(n_edges, torch.Tensor) or n_edges.numel() != 1 or n_edges.dim() > 1:
+        raise L.FegnnError("n_edges must be a one-element tensor holding the live edge count")
+    if n_edges.dtype not in (torch.int32, torch.int64):
+        raise L.FegnnError(f"n_edges must be int32 or int64 (got {n_edges.dtype})")
+
+
 class CsrGraph:
     """CSR-by-row view of one batch (output of fegnn_graph_prep), shared by all layers
     and by backward.  Replaces the per-layer int64 gathers / scatter_add of
-    models/FastEGNN.py:182,210,279-294."""
+    models/FastEGNN.py:182,210,279-294.
+
+    A LIVE graph (`live` is True; CsrGraph(..., n_edges=t) or from_radius(..., capacity=c)) keeps its edge count on the
+    device: E is a capacity, the arrays have E rows, and the edge kernels read the live count `n_edges` (an int32 [1]
+    tensor) themselves (FEGNN_F_LIVE_EDGES).  Nothing is read back to the host, so a training step or a rollout that builds
+    such a graph can be captured once and replayed over batches whose edge count changes.  Overflow (more edges than the
+    capacity, a count outside [0, E]) runs without any out-of-bounds access but gives undefined results: check() is the
+    guard."""
+
+    live = False
 
     def __init__(self, edge_index: torch.Tensor, data_batch: torch.Tensor, edge_attr: Optional[torch.Tensor],
-                 n_graphs: int, n_local: Optional[int] = None, overlap: bool = False):
+                 n_graphs: int, n_local: Optional[int] = None, overlap: bool = False,
+                 n_edges: Optional[torch.Tensor] = None):
         """overlap=True runs the sort on a per-device side stream and leaves `ready_event` in the pointer table:
         fegnn_model_forward joins it right before its first use of the CSR arrays (the embedding and the first layer's
-        node phase run under the sort).  Any other consumer must call wait() first."""
+        node phase run under the sort).  Any other consumer must call wait() first.
+
+        n_edges: a one-element int32 / int64 CUDA tensor with the live edge count of an edge_index (and edge_attr) padded
+        to a fixed capacity E = edge_index.size(1), e.g. at collate time: the graph is live (fegnn_graph_prep_live).
+        Entries at and past the count are never read as indices.  With every host input of a fixed shape, such batches go
+        through PipelinedStep unchanged."""
+        if n_edges is not None:
+            _live_count_arg(n_edges)
+            if n_local is not None and n_local != int(data_batch.numel()):
+                raise L.FegnnError("a live graph has no halo rows (n_local is for the partitioned runner)")
+            _require_cuda(n_edges, "n_edges")
         _require_cuda(edge_index, "edge_index")
         dev = edge_index.device
         N = int(data_batch.numel())
@@ -79,6 +107,12 @@ class CsrGraph:
         nbytes = int(lib.fegnn_graph_prep_workspace_bytes(N, E))
         ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
         self._ready = None
+        n_in = None
+        if n_edges is not None:
+            self.live = True
+            n_in = n_edges.reshape(1).to(device=dev, dtype=torch.int32)
+            self.n_edges = torch.empty(1, **i32)                  # the graph's own word: the clamped live count
+            self.status = torch.zeros(1, **i32)                   # sticky FEGNN_LIVE_* bits
         with _on(dev):
             # every buffer above was allocated under the caller's stream; with overlap the side stream first joins that
             # stream (inputs and recycled memory are ordered), then runs the sort while the caller's stream goes on
@@ -87,22 +121,30 @@ class CsrGraph:
             if overlap:
                 st = _prep_stream(dev)
                 st.wait_stream(main)
-            L.check(lib.fegnn_graph_prep(N, E, n_graphs, Fe, L.ptr(ei), L.ptr(db), L.ptr(ea), L.ptr(self.perm),
-                                         L.ptr(self.rowptr), L.ptr(self.row), L.ptr(self.col), L.ptr(self.batch),
-                                         L.ptr(self.gptr), L.ptr(self.edge_attr), L.ptr(self.dinv), L.ptr(self.inv_nb),
-                                         L.ptr(ws), nbytes, st.cuda_stream), "fegnn_graph_prep")
+            if n_in is not None:
+                L.check(lib.fegnn_graph_prep_live(N, E, n_graphs, Fe, L.ptr(ei), L.ptr(db), L.ptr(ea), L.ptr(self.perm),
+                                                  L.ptr(self.rowptr), L.ptr(self.row), L.ptr(self.col), L.ptr(self.batch),
+                                                  L.ptr(self.gptr), L.ptr(self.edge_attr), L.ptr(self.dinv),
+                                                  L.ptr(self.inv_nb), L.ptr(ws), nbytes, L.ptr(n_in), L.ptr(self.n_edges),
+                                                  L.ptr(self.status), st.cuda_stream), "fegnn_graph_prep_live")
+            else:
+                L.check(lib.fegnn_graph_prep(N, E, n_graphs, Fe, L.ptr(ei), L.ptr(db), L.ptr(ea), L.ptr(self.perm),
+                                             L.ptr(self.rowptr), L.ptr(self.row), L.ptr(self.col), L.ptr(self.batch),
+                                             L.ptr(self.gptr), L.ptr(self.edge_attr), L.ptr(self.dinv), L.ptr(self.inv_nb),
+                                             L.ptr(ws), nbytes, st.cuda_stream), "fegnn_graph_prep")
             if overlap:
                 self._ready = torch.cuda.Event()
                 self._ready.record(st)
         self._ws = ws   # stream-ordered: keep alive until the kernels that use it have been enqueued
-        self._keep = (ei, db, ea)   # inputs of a sort that may still be running on the side stream
+        self._keep = (ei, db, ea, n_in)   # inputs of a sort that may still be running on the side stream
         self.rebind()
 
     def rebind(self) -> None:
         """(Re)build the fegnn_graph pointer table from the current tensors (after slicing / renumbering them)."""
         ready = getattr(self, "_ready", None)
         self.c = L.Graph(L.ptr(self.row), L.ptr(self.col), L.ptr(self.batch), L.ptr(self.edge_attr),
-                         L.ptr(self.dinv), L.ptr(self.inv_nb), None if ready is None else ready.cuda_event)
+                         L.ptr(self.dinv), L.ptr(self.inv_nb), None if ready is None else ready.cuda_event,
+                         L.ptr(self.n_edges) if self.live else None)
 
     def wait(self) -> None:
         """Order the current stream behind a sort that runs on the side stream (no-op otherwise)."""
@@ -114,13 +156,26 @@ class CsrGraph:
 
     @classmethod
     def from_radius(cls, node_loc: torch.Tensor, data_batch: torch.Tensor, n_graphs: int, r: float,
-                    cutoff_rate: float = 0.0, edge_attr_nf: int = 2) -> "CsrGraph":
+                    cutoff_rate: float = 0.0, edge_attr_nf: int = 2, capacity: Optional[int] = None,
+                    candidate_capacity: Optional[int] = None) -> "CsrGraph":
         """Build the graph ON THE DEVICE (fegnn_radius_graph_count / _fill): every ordered pair of distinct nodes of
         the same graph closer than r, the shortest int(E_b (1 - cutoff_rate)) of them per graph, in CSR order with
         edge_attr = length in each of the edge_attr_nf columns.  Replaces radius_graph + cutoff_edge + norm of
         datasets/simulation/dataset.py:80-82,96-101 (r = math.inf: the complete-graph / topk selection of
-        datasets/nbody/dataset.py:102-113) and the per-forward CSR sort.  One host read of the candidate count
-        sizes the buffers (this is dataset-time work, not part of the captured training step)."""
+        datasets/nbody/dataset.py:102-113) and the per-forward CSR sort.
+
+        capacity=None: one host read of the candidate count sizes the buffers exactly, and E is the edge count.
+        capacity=c: a LIVE graph of c edge rows (candidate_capacity rows of candidates, default c; with cutoff_rate > 0
+        there are more candidates than kept edges, so size it for them).  Nothing is read back: the call can sit inside a
+        captured step or rollout, and rebuild_() refills the same buffers from new positions.  check() raises, naming the
+        capacity needed, if either was too small."""
+        if capacity is not None:
+            capacity = int(capacity)
+            candidate_capacity = capacity if candidate_capacity is None else int(candidate_capacity)
+            if capacity < 0 or candidate_capacity < 0:
+                raise L.FegnnError(f"capacity ({capacity}) and candidate_capacity ({candidate_capacity}) must be >= 0")
+        elif candidate_capacity is not None:
+            raise L.FegnnError("candidate_capacity needs a capacity (the exact path sizes its candidates itself)")
         _require_cuda(node_loc, "node_loc")
         dev = node_loc.device
         x = node_loc.detach().contiguous().float()
@@ -146,6 +201,20 @@ class CsrGraph:
         counts = torch.zeros(2, **i32)                        # [n_cand, n_edges]
         nbytes = int(lib.fegnn_radius_graph_workspace_bytes(N, B))
         ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
+        if capacity is not None:
+            self.live = True
+            self.E, self.candidate_capacity = capacity, candidate_capacity
+            self._radius = (db, float(r), 1.0 - float(cutoff_rate), cand_rowptr, counts, ws, nbytes)
+            self._cand = tuple(torch.empty(max(candidate_capacity, 1), **dt) for dt in (i32, f32, i32))   # col, dist, row
+            self.row = torch.empty(max(capacity, 1), **i32)
+            self.col = torch.empty(max(capacity, 1), **i32)
+            self.edge_attr = torch.empty(max(capacity, 1), max(Fe, 1), **f32) if Fe else torch.empty(0, **f32)
+            self.n_edges = torch.empty(1, **i32)
+            self.status = torch.zeros(1, **i32)
+            self._peak = torch.zeros(2, **i32)                # largest uncapped [n_cand, n_edges] of any build (check())
+            self.rebuild_(x)
+            self.rebind()
+            return self
         st = _stream(dev)
         with _on(dev):
             L.check(lib.fegnn_radius_graph_count(N, B, L.ptr(x), L.ptr(db), float(r), L.ptr(self.batch), L.ptr(self.gptr),
@@ -175,9 +244,80 @@ class CsrGraph:
         self.rebind()
         return self
 
+    def rebuild_(self, node_loc: torch.Tensor) -> "CsrGraph":
+        """Refill a live from_radius graph IN PLACE from new positions (same data_batch, r, cutoff_rate and buffers, so
+        the pointer table stays valid): what a captured rollout calls every step.  No host read, no allocation."""
+        if getattr(self, "_radius", None) is None:
+            raise L.FegnnError("rebuild_ needs a graph made by CsrGraph.from_radius(..., capacity=...)")
+        if node_loc.dim() != 2 or node_loc.size(0) != self.N or node_loc.size(1) != 3:
+            raise L.FegnnError(f"node_loc has shape {tuple(node_loc.shape)}, the graph has {self.N} nodes")
+        _require_cuda(node_loc, "node_loc")
+        x = node_loc.detach().contiguous().float()
+        db, r, keep_frac, cand_rowptr, counts, ws, nbytes = self._radius
+        ccol, cdist, crow = self._cand
+        st = _stream(x.device)
+        with _on(x.device):
+            L.check(lib.fegnn_radius_graph_count(self.N, self.B, L.ptr(x), L.ptr(db), r, L.ptr(self.batch),
+                                                 L.ptr(self.gptr), L.ptr(self.inv_nb), L.ptr(cand_rowptr),
+                                                 L.ptr(counts[0:1]), L.ptr(ws), nbytes, st), "fegnn_radius_graph_count")
+            L.check(lib.fegnn_radius_graph_fill_live(self.N, self.B, self.Fe, r, keep_frac, L.ptr(self.batch),
+                                                     L.ptr(self.gptr), L.ptr(cand_rowptr), L.ptr(counts[0:1]),
+                                                     self.candidate_capacity, L.ptr(ccol), L.ptr(cdist), L.ptr(crow),
+                                                     self.E, L.ptr(self.rowptr), L.ptr(self.row), L.ptr(self.col),
+                                                     L.ptr(self.edge_attr), L.ptr(self.dinv), L.ptr(counts[1:2]),
+                                                     L.ptr(self.n_edges), L.ptr(self.status), L.ptr(ws), nbytes, st),
+                    "fegnn_radius_graph_fill_live")
+            # the status bits are sticky over rebuilds, so are the totals check() names: a running maximum on the device
+            torch.maximum(self._peak, counts, out=self._peak)
+        return self
+
+    def check(self) -> None:
+        """Live graphs: one host read; raises FegnnError if the graph overflowed its capacities or was given a count
+        outside [0, E] (at any build since it was made: the status bits are sticky), naming the capacity needed.  A graph
+        with a host-known edge count has nothing to check."""
+        if not self.live:
+            return
+        self.wait()
+        parts = [self.status, self.n_edges]
+        radius = getattr(self, "_radius", None)
+        if radius is not None:
+            parts.append(self._peak)                               # largest uncapped [n_cand, n_edges] of every build
+        else:
+            parts.append(self._keep[3])                            # the caller's count
+        vals = [int(v) for v in torch.cat(parts).cpu()]
+        status = vals[0]
+        if status == 0:
+            return
+        msgs = []
+        if status & L.LIVE_BAD_COUNT:
+            n_in = vals[2]
+            msgs.append(f"the edge count {n_in} is outside [0, {self.E}]" +
+                        (f": a capacity of at least {n_in} edges is needed" if n_in > self.E else ""))
+        if status & L.LIVE_CAND_OVERFLOW:
+            msgs.append(f"{vals[2]} radius-graph candidates exceed candidate_capacity={self.candidate_capacity}: "
+                        f"candidate_capacity >= {vals[2]} is needed")
+        if status & L.LIVE_EDGE_OVERFLOW:
+            msgs.append(f"{vals[3]} edges exceed capacity={self.E}: capacity >= {vals[3]} is needed"
+                        + (" (at least; candidates were truncated too)" if status & L.LIVE_CAND_OVERFLOW else ""))
+        raise L.FegnnError("live graph overflow (its results are undefined): " + "; ".join(msgs))
+
+    def num_edges(self) -> int:
+        """The live edge count (one host read on a live graph)."""
+        if not self.live:
+            return self.E
+        self.wait()
+        return int(self.n_edges.item())
+
     def edge_index(self) -> torch.Tensor:
-        """int64 [2,E] view of the CSR edge list for callers that want the reference's tensor (a cast, no arithmetic)."""
-        return torch.stack([self.row.long(), self.col.long()])
+        """int64 [2,E] view of the CSR edge list for callers that want the reference's tensor (a cast, no arithmetic).
+        A live graph returns its live edges (one host read of the count)."""
+        n = self.num_edges()
+        return torch.stack([self.row[:n].long(), self.col[:n].long()])
+
+
+def live_flag(graph) -> int:
+    """FEGNN_F_LIVE_EDGES for a graph whose edge count lives on the device (CsrGraph.live), else 0."""
+    return L.F_LIVE_EDGES if getattr(graph, "live", False) else 0
 
 
 def make_dims(N: int, Nl: int, E: int, B: int, C_: int, Fe: int, flags: int,

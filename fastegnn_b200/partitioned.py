@@ -613,6 +613,9 @@ class PartitionedFastEGNN:
             graph = edge_index
             if edge_attr is not None:
                 raise TypeError("edge_attr must be None when edge_index is a prebuilt CsrGraph (it carries its own)")
+            if graph.live:
+                raise L.FegnnError("the partitioned runner takes graphs with a host-known edge count: a live graph "
+                                   "(CsrGraph.from_radius(capacity=...) or CsrGraph(..., n_edges=...)) is not supported here")
             if graph.N != N or graph.Nl != self.comm.Nl:
                 raise L.FegnnError(f"prebuilt slab graph (N={graph.N}, Nl={graph.Nl}) does not match the plan "
                                    f"(N={N}, Nl={self.comm.Nl})")

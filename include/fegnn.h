@@ -83,6 +83,20 @@ extern "C" {
                                     too (it then also rebuilds the top two layers).  Without FEGNN_F_RECOMPUTE the backward
                                     refuses it with FEGNN_EINVAL; the forward entries ignore it; every other per-layer entry
                                     refuses it like FEGNN_F_RECOMPUTE. */
+#define FEGNN_F_LIVE_EDGES 8192u /* the edge count lives on the device: fegnn_dims.E is a CAPACITY (rows of the graph's row / col /
+                                   edge_attr arrays) and the live count is the int32 word *fegnn_graph.n_edges, read as
+                                   min(max(*n_edges, 0), E) by the edge kernels themselves, after their griddepcontrol.wait (an
+                                   earlier kernel of the stream may have written it: fegnn_graph_prep_live, fegnn_radius_graph_fill_live).
+                                   Entries >= the live count are never read.  The host sizes grids and workspaces from the capacity,
+                                   so a CTA may find no live tile and exit: one captured step serves batches whose edge count
+                                   changes.  Honoured by every entry that takes a fegnn_graph; with n_edges == NULL they return
+                                   FEGNN_EINVAL before any launch, as do "edge_backward" modes 1, 2, 4 and 5 (which have no live
+                                   form); auto (6) takes mode 7 or the fp32 kernel.  The partitioned runner does not take it. */
+
+/* bits of the sticky status word of fegnn_graph_prep_live / fegnn_radius_graph_fill_live (never cleared by the library) */
+#define FEGNN_LIVE_BAD_COUNT 1u     /* the caller's edge count was below 0 or above the capacity: clamped         */
+#define FEGNN_LIVE_CAND_OVERFLOW 2u /* more radius-graph candidates than cand_capacity: the graph is truncated    */
+#define FEGNN_LIVE_EDGE_OVERFLOW 4u /* more kept edges than out_capacity: the graph is truncated                   */
 
 typedef struct fegnn_dims {
   int32_t N;        /* owned real nodes                                             */
@@ -111,6 +125,7 @@ typedef struct fegnn_graph {
                              waits for it right before its first use of the arrays above (the embedding and the first layer's
                              node phase run under the sort), fegnn_model_forward_inference at its start; NULL = same stream.
                              Every other entry point ignores it: the caller orders them (ops.CsrGraph.wait)                    */
+  const int32_t* n_edges; /* [1] live edge count (device), read only with FEGNN_F_LIVE_EDGES in fegnn_dims.flags            */
 } fegnn_graph;
 
 /* One layer's parameters in reference layout (models/FastEGNN.py:28-99).
@@ -213,6 +228,19 @@ int fegnn_graph_prep(int32_t N, int32_t E, int32_t B, int32_t Fe,
                      int32_t* batch /*[N]*/, int32_t* gptr /*[B+1]*/, float* edge_attr_sorted /*[E,Fe]*/,
                      float* dinv /*[N]*/, float* inv_nb /*[B]*/,
                      void* workspace, size_t workspace_bytes, void* stream);
+/* The same for an edge list padded to the capacity E whose live count is the device word *n_edges_in (FEGNN_F_LIVE_EDGES):
+ * nothing is read back, so one captured step serves batches of any edge count up to E.  Edges >= the live count are never
+ * read as indices (their edge_index / edge_attr may hold anything); they take the sort key N, so they land after every
+ * live edge, and rowptr / dinv / gptr / inv_nb count live edges only.  *n_edges_out receives min(max(*n_edges_in, 0), E)
+ * (the graph's own word for fegnn_graph.n_edges); a count outside [0, E] also ORs FEGNN_LIVE_BAD_COUNT into *status.  The
+ * CSR arrays are written over the whole capacity; entries >= the live count hold no edge.  Workspace as fegnn_graph_prep. */
+int fegnn_graph_prep_live(int32_t N, int32_t E, int32_t B, int32_t Fe,
+                          const int64_t* edge_index /*[2,E]*/, const int64_t* data_batch /*[N]*/,
+                          const float* edge_attr /*[E,Fe] or NULL*/,
+                          int32_t* perm, int32_t* rowptr, int32_t* row, int32_t* col, int32_t* batch, int32_t* gptr,
+                          float* edge_attr_sorted, float* dinv, float* inv_nb, void* workspace, size_t workspace_bytes,
+                          const int32_t* n_edges_in /*[1]*/, int32_t* n_edges_out /*[1]*/, uint32_t* status /*[1]*/,
+                          void* stream);
 
 /* ------------------------------------------------------------------ graph construction on the device
  * Replaces the step right before the path: torch_cluster.radius_graph + cutoff_edge (torch.sort of the lengths, keep
@@ -241,6 +269,18 @@ int fegnn_radius_graph_fill(int32_t N, int32_t B, int32_t Fe, float r, double ke
                             int32_t out_capacity, int32_t* rowptr /*[N+1]*/, int32_t* row, int32_t* col,
                             float* edge_attr /*[out_capacity,Fe]*/, float* dinv /*[N]*/, int32_t* n_edges /*[1]*/,
                             void* workspace, size_t workspace_bytes, void* stream);
+/* fegnn_radius_graph_fill for fixed capacities chosen up front (no host read of *n_cand between the calls): the graph of a
+ * rollout or of a captured step, rebuilt from new positions every time.  *n_cand and *n_edges keep the uncapped totals
+ * (so an error can name the capacity that would have been enough; with candidates truncated *n_edges counts the kept
+ * edges among those that were written); *n_live receives min(*n_edges, out_capacity), the word for fegnn_graph.n_edges.
+ * Candidates over cand_capacity OR FEGNN_LIVE_CAND_OVERFLOW, kept edges over out_capacity FEGNN_LIVE_EDGE_OVERFLOW into
+ * *status (sticky).  Every write stays inside the capacities; a truncated graph's results are undefined. */
+int fegnn_radius_graph_fill_live(int32_t N, int32_t B, int32_t Fe, float r, double keep_frac, const int32_t* batch,
+                                 const int32_t* gptr, const int32_t* cand_rowptr, const int32_t* n_cand,
+                                 int32_t cand_capacity, int32_t* cand_col, float* cand_dist, int32_t* cand_row,
+                                 int32_t out_capacity, int32_t* rowptr, int32_t* row, int32_t* col, float* edge_attr,
+                                 float* dinv, int32_t* n_edges /*[1]*/, int32_t* n_live /*[1]*/, uint32_t* status /*[1]*/,
+                                 void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------ phases of one layer (forward)
  * Names follow oracle/staged.py, which spells the same pipeline out on the CPU.  */

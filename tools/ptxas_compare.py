@@ -11,7 +11,8 @@ Kernels are matched by mangled name, a name the parent lacks after renamings tha
 namespace of api.cu (its hash depends on the source path), the `kEa = false` instantiations of edge_bwd_kernel /
 edge_bwd_tc4_kernel and the `kDet = false` instantiations of the forward kernels (edge_fwd_kernel, edge_fwd_tc_kernel,
 virtual_fwd_kernel, virtual_fwd_tc_kernel, node_h_z_kernel), the `kSaved = false` instantiations of virtual_fwd_kernel,
-virtual_fwd_tc_kernel and node_h_fwd_tc_kernel, which are a parent's untemplated (resp. one-parameter fewer) kernels.  Every kernel of both builds is listed with its resource
+virtual_fwd_tc_kernel and node_h_fwd_tc_kernel, and the `kLive = false` instantiations of the kernels that walk edges
+(LIVE_ADDED), which are a parent's untemplated (resp. one-parameter fewer) kernels.  Every kernel of both builds is listed with its resource
 lines (stack frame, spills, registers, barriers, shared memory; constant-bank sizes are left out)."""
 import re
 import sys
@@ -38,11 +39,19 @@ BOOL_ADDED = ("edge_bwd_kernel", "edge_bwd_tc4_kernel", "edge_fwd_kernel", "edge
               "virtual_fwd_tc_kernel", "node_h_z_kernel", "node_h_fwd_tc_kernel")
 # a second trailing bool (the kSaved = false forms of the recompute, FEGNN_F_RECOMPUTE) after the kDet one
 BOOL2_ADDED = ("virtual_fwd_kernel", "virtual_fwd_tc_kernel")
+# the kLive = false forms of the kernels that walk edges (FEGNN_F_LIVE_EDGES): a trailing bool after the parent's parameters
+LIVE_ADDED = ("edge_fwd_kernel", "edge_fwd_tc_kernel", "edge_bwd_kernel", "edge_bwd_tc4_kernel", "edge_det_fixup_kernel")
 
 
 def to_parent(name, parent):
     if name in parent:
         return name
+    for k in LIVE_ADDED:
+        if f"{len(k)}{k}I" in name:
+            trimmed = name.replace(f"{k}ILb0EEEvNS_", f"{k}ENS_")
+            trimmed = re.sub(rf"({k}I(?:L[ib]\d+E)+)Lb0EEEv", r"\1EEv", trimmed)
+            if trimmed != name:
+                return to_parent(trimmed, parent)
     for k in BOOL2_ADDED:
         if f"{len(k)}{k}I" in name:
             trimmed = re.sub(rf"({k}I(?:L[ib]\d+E)+)Lb0EEEv", r"\1EEv", name)
