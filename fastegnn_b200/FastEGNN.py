@@ -15,7 +15,10 @@ Differences a caller can observe
     of the unmodified reference covers node_attr_nf > 0.
   * node_vel, node_attr and edge_attr receive gradients as in the reference, computed only when they require grad
     (fegnn_model_backward_inputs).  Exceptions: FastRF's node_vel (none), and the edge_attr a prebuilt CsrGraph carries
-    (data of the graph: pass graph.edge_index() and a tensor to differentiate it).
+    unless the graph was made with differentiable=True (else data of the graph).  A differentiable
+    CsrGraph(edge_index, data_batch, edge_attr, B) gives the caller's edge_attr its gradient; a differentiable
+    CsrGraph.from_radius(node_loc, ...) gives node_loc the gradient through its edge lengths (the topology is piecewise
+    constant), and raises in the backward if it was rebuilt (rebuild_) after the forward.
   * the number of graphs is taken from loc_mean.size(0) instead of data_batch[-1].item()
     (:267), which removes a device synchronisation; the two agree for valid batches.
 """
@@ -144,6 +147,7 @@ class _StackFn(torch.autograd.Function):
                                             L.ptr(x0), L.ptr(v), L.ptr(loc_mean), L.ptr(x_out), L.ptr(Z_out), L.ptr(ws),
                                             ws_floats, _stream(dev)), "fegnn_model_forward")
         ctx.mod, ctx.graph, ctx.dims, ctx.ws, ctx.Fin = mod, graph, dims, ws, Fin
+        ctx.build = graph.builds                                # a differentiable graph's backward checks it (rebuild_)
         ctx.recompute = recompute                               # the backward follows this step's forward
         ctx.blocks_consumed = False                             # recompute: set by the first backward (see above)
         ctx.save_for_backward(node_feat, v, node_attr)          # node_attr: dims points at it until the backward
@@ -157,6 +161,8 @@ class _StackFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gx, gZ):
         mod, graph, dims = ctx.mod, ctx.graph, ctx.dims
+        if getattr(graph, "differentiable", False):
+            graph.check_build(ctx.build)
         L.deterministic(type(mod).__name__ + " backward", L.NO_DET_LAYERS)
         node_feat, v, _ = ctx.saved_tensors
         dev = v.device
@@ -332,8 +338,10 @@ class FastEGNN(nn.Module):
             if graph.Fe != self._edge_attr_nf or graph.N != node_loc.size(0) or graph.B != loc_mean.size(0):
                 raise RuntimeError(f"prebuilt graph (N={graph.N}, B={graph.B}, Fe={graph.Fe}) does not match the inputs "
                                    f"(N={node_loc.size(0)}, B={loc_mean.size(0)}, edge_attr_nf={self._edge_attr_nf})")
-            # node_attr still gets its gradient; the graph's edge_attr is data of the graph (no autograd input here)
-            return self._run_stack(graph, node_attr, attr_in, None, node_feat, node_loc, node_vel, loc_mean)
+            # node_attr still gets its gradient; the graph's edge_attr is data of the graph unless the graph is
+            # differentiable, which hands the training forward the tensor (or the function of node_loc) to differentiate
+            ea_in = graph.edge_attr_input() if graph.differentiable and not self._inference_route() else None
+            return self._run_stack(graph, node_attr, attr_in, ea_in, node_feat, node_loc, node_vel, loc_mean)
         if edge_attr is None:
             if self._edge_attr_nf != 0:
                 raise TypeError("edge_attr is required when edge_attr_nf > 0 (the reference's torch.cat fails on None, "

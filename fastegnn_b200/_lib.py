@@ -149,6 +149,7 @@ SIGNATURES = {
     "fegnn_virtual_backward_inputs": (C.c_int, [_PD, _PG, _PP, _PP, vp, vp, vp, _PS] + [vp] * 12 + [_PI, vp]),
     "fegnn_edge_backward_inputs": (C.c_int, [_PD, _PG, _PP, _PP, vp, _PS, vp, vp, vp, vp, vp, _PI, vp]),
     "fegnn_node_pre_backward_inputs": (C.c_int, [_PD, _PP, _PP, vp, vp, vp, vp, vp, vp, vp, vp, _PI, vp]),
+    "fegnn_edge_length_backward": (C.c_int, [_PD, _PG, vp, vp, vp, vp, vp]),
     "fegnn_halo_push": (C.c_int, [i32, vp, vp, vp, vp, vp, vp]),
     "fegnn_halo_reduce_push": (C.c_int, [i32, i32, vp, vp, vp, vp, vp]),
     "fegnn_halo_push_signal": (C.c_int, [C.POINTER(P2P), i32, i32, vp, i32, vp, vp, vp, vp, vp]),

@@ -1017,6 +1017,19 @@ int fegnn_node_pre_backward_inputs(const fegnn_dims* d, const fegnn_layer_params
   return 0;
 }
 
+int fegnn_edge_length_backward(const fegnn_dims* d, const fegnn_graph* g, const int32_t* rowptr, const float* x,
+                               const float* g_ea, float* g_x, void* stream) {
+  NO_DET("the col side of the position gradient is a scatter with float atomics");
+  TRY(check_dims(d));
+  if (d->Fe == 0) return fail(FEGNN_EINVAL, "fegnn_edge_length_backward: the graph has no edge_attr (Fe = 0)");
+  RQ(g != nullptr);
+  TRY(check_live(d, g, false));
+  RQ(d->N == 0 || d->E == 0 || (rowptr && g->col && g->edge_attr && x && g_ea && g_x));
+  CK(launch_edge_length_bwd(d->N, d->E, d->Fe, rowptr, g->col, g->edge_attr, x, g_ea,
+                            (d->flags & FEGNN_F_LIVE_EDGES) ? g->n_edges : nullptr, g_x, sm_count(), S(stream)));
+  return 0;
+}
+
 // ------------------------------------------------------------------ halo exchange over peer memory (partitioned path)
 int fegnn_halo_push(int32_t n, const int32_t* src_row, const uint64_t* dst_q, const uint64_t* dst_x, const float* Q,
                     const float* x, void* stream) {

@@ -50,6 +50,66 @@ __global__ void __launch_bounds__(kGaThreads) input_grad_attr_kernel(int N, int 
   ga[idx] += s;
 }
 
+// Edge lengths of a graph built from positions x (fegnn_edge_length_backward): edge_attr[e, k] = len_e for every k, with
+// len_e = |x_row - x_col| the graph's own edge_attr[e, 0] (radius_graph.cu: __fsqrt_rn of the no-FMA d2), so
+//   g_x[row_e] += u_e,  g_x[col_e] -= u_e,  u_e = (sum_k g_ea[e, k]) (x_row - x_col) / len_e,  u_e = 0 where len_e == 0
+// (coincident distinct nodes: torch's norm subgradient).  One warp per CSR row over rowptr, lanes over its edges: the row
+// side is summed in registers and added once per row, the col side with red.global.add per edge.  Persistent grid; kLive
+// bounds every row by the live edge count (read after the wait, as live_edges() does), so no edge at or past it is read.
+constexpr int kElThreads = 256;
+template <bool kLive>
+__global__ void __launch_bounds__(kElThreads) edge_length_bwd_kernel(int N, int E, int Fe, const int* __restrict__ rowptr,
+                                                                     const int* __restrict__ col, const float* __restrict__ ea,
+                                                                     const float* __restrict__ x, const float* __restrict__ g_ea,
+                                                                     const int* __restrict__ n_edges, float* __restrict__ g_x) {
+  pdl_trigger();
+  pdl_wait();
+  if constexpr (kLive) {
+    const int n = __ldcg(n_edges);
+    E = n < 0 ? 0 : (n > E ? E : n);
+  }
+  const int lane = threadIdx.x & 31;
+  const int warps = gridDim.x * (kElThreads / 32);
+  for (int i = blockIdx.x * (kElThreads / 32) + (threadIdx.x >> 5); i < N; i += warps) {
+    const int e0 = min(rowptr[i], E), e1 = min(rowptr[i + 1], E);
+    if (e0 >= e1) continue;
+    const float xi0 = x[3 * i], xi1 = x[3 * i + 1], xi2 = x[3 * i + 2];
+    float r0 = 0.f, r1 = 0.f, r2 = 0.f;
+    for (int e = e0 + lane; e < e1; e += 32) {
+      const float len = ea[(size_t)e * Fe];
+      if (len == 0.f) continue;
+      float s = 0.f;
+      for (int k = 0; k < Fe; ++k) s += g_ea[(size_t)e * Fe + k];
+      const int j = col[e];
+      const float f = s / len;
+      const float u0 = f * (xi0 - x[3 * j]), u1 = f * (xi1 - x[3 * j + 1]), u2 = f * (xi2 - x[3 * j + 2]);
+      r0 += u0; r1 += u1; r2 += u2;
+      atomicAdd(g_x + 3 * j, -u0);
+      atomicAdd(g_x + 3 * j + 1, -u1);
+      atomicAdd(g_x + 3 * j + 2, -u2);
+    }
+    r0 = warpsum(r0); r1 = warpsum(r1); r2 = warpsum(r2);
+    if (lane == 0) {
+      atomicAdd(g_x + 3 * i, r0);          // other rows' col terms land on this row too
+      atomicAdd(g_x + 3 * i + 1, r1);
+      atomicAdd(g_x + 3 * i + 2, r2);
+    }
+  }
+}
+
+inline cudaError_t launch_edge_length_bwd(int N, int E, int Fe, const int* rowptr, const int* col, const float* ea,
+                                          const float* x, const float* g_ea, const int* n_edges, float* g_x, int sms,
+                                          cudaStream_t st) {
+  if (N == 0 || E == 0) return cudaSuccess;
+  const int rows_per_cta = kElThreads / 32;
+  const int grid = min(4 * sms, (N + rows_per_cta - 1) / rows_per_cta);
+  cudaError_t e = n_edges != nullptr
+      ? launch_pdl(edge_length_bwd_kernel<true>, grid, kElThreads, 0, st, N, E, Fe, rowptr, col, ea, x, g_ea, n_edges, g_x)
+      : launch_pdl(edge_length_bwd_kernel<false>, grid, kElThreads, 0, st, N, E, Fe, rowptr, col, ea, x, g_ea, n_edges, g_x);
+  if (e != cudaSuccess) return e;
+  return cudaGetLastError();
+}
+
 inline cudaError_t launch_input_grad_vel(int N, const float* sv, const float* gx_new, const float* gxsum_next,
                                          const int* batch, float* gv, cudaStream_t st) {
   if (N == 0) return cudaSuccess;

@@ -61,13 +61,20 @@ class CsrGraph:
     tensor) themselves (FEGNN_F_LIVE_EDGES).  Nothing is read back to the host, so a training step or a rollout that builds
     such a graph can be captured once and replayed over batches whose edge count changes.  Overflow (more edges than the
     capacity, a count outside [0, E]) runs without any out-of-bounds access but gives undefined results: check() is the
-    guard."""
+    guard.
+
+    A DIFFERENTIABLE graph (`differentiable` is True; CsrGraph(..., differentiable=True) or from_radius(...,
+    differentiable=True)) lets the training forward of FastEGNN / FastRF differentiate its edge_attr: the caller's edge_attr
+    tensor, or the edge lengths as a function of the node_loc the graph was built from (DESIGN 3.10).  Every other graph's
+    edge_attr is data."""
 
     live = False
+    differentiable = False
+    builds = 0          # from_radius: builds of the arrays (rebuild_ counts up); a backward checks its forward's build
 
     def __init__(self, edge_index: torch.Tensor, data_batch: torch.Tensor, edge_attr: Optional[torch.Tensor],
                  n_graphs: int, n_local: Optional[int] = None, overlap: bool = False,
-                 n_edges: Optional[torch.Tensor] = None):
+                 n_edges: Optional[torch.Tensor] = None, differentiable: bool = False):
         """overlap=True runs the sort on a per-device side stream and leaves `ready_event` in the pointer table:
         fegnn_model_forward joins it right before its first use of the CSR arrays (the embedding and the first layer's
         node phase run under the sort).  Any other consumer must call wait() first.
@@ -75,7 +82,13 @@ class CsrGraph:
         n_edges: a one-element int32 / int64 CUDA tensor with the live edge count of an edge_index (and edge_attr) padded
         to a fixed capacity E = edge_index.size(1), e.g. at collate time: the graph is live (fegnn_graph_prep_live).
         Entries at and past the count are never read as indices.  With every host input of a fixed shape, such batches go
-        through PipelinedStep unchanged."""
+        through PipelinedStep unchanged.
+
+        differentiable=True: the graph keeps the caller's edge_attr tensor, and a training forward on it gives that tensor
+        its gradient in the caller's edge order, as a per-call edge_index + edge_attr does (padding rows of a live graph
+        get zero)."""
+        if differentiable and edge_attr is None:
+            raise L.FegnnError("differentiable=True needs an edge_attr (there is nothing to differentiate)")
         if n_edges is not None:
             _live_count_arg(n_edges)
             if n_local is not None and n_local != int(data_batch.numel()):
@@ -137,6 +150,9 @@ class CsrGraph:
                 self._ready.record(st)
         self._ws = ws   # stream-ordered: keep alive until the kernels that use it have been enqueued
         self._keep = (ei, db, ea, n_in)   # inputs of a sort that may still be running on the side stream
+        if differentiable:
+            self.differentiable = True
+            self._ea_src = edge_attr
         self.rebind()
 
     def rebind(self) -> None:
@@ -157,7 +173,7 @@ class CsrGraph:
     @classmethod
     def from_radius(cls, node_loc: torch.Tensor, data_batch: torch.Tensor, n_graphs: int, r: float,
                     cutoff_rate: float = 0.0, edge_attr_nf: int = 2, capacity: Optional[int] = None,
-                    candidate_capacity: Optional[int] = None) -> "CsrGraph":
+                    candidate_capacity: Optional[int] = None, differentiable: bool = False) -> "CsrGraph":
         """Build the graph ON THE DEVICE (fegnn_radius_graph_count / _fill): every ordered pair of distinct nodes of
         the same graph closer than r, the shortest int(E_b (1 - cutoff_rate)) of them per graph, in CSR order with
         edge_attr = length in each of the edge_attr_nf columns.  Replaces radius_graph + cutoff_edge + norm of
@@ -168,7 +184,15 @@ class CsrGraph:
         capacity=c: a LIVE graph of c edge rows (candidate_capacity rows of candidates, default c; with cutoff_rate > 0
         there are more candidates than kept edges, so size it for them).  Nothing is read back: the call can sit inside a
         captured step or rollout, and rebuild_() refills the same buffers from new positions.  check() raises, naming the
-        capacity needed, if either was too small."""
+        capacity needed, if either was too small.
+
+        differentiable=True: the graph keeps node_loc, with its autograd history (rebuild_ rebinds it to the new
+        positions), and a training forward of FastEGNN / FastRF on the graph takes its edge lengths as a function of
+        node_loc: node_loc receives the gradient that flows through them (fegnn_edge_length_backward), as it would
+        through a torch norm of node_loc[row] - node_loc[col].  The topology stays piecewise constant.  A rebuild_ between
+        a forward and that forward's backward makes the backward raise."""
+        if differentiable and int(edge_attr_nf) == 0:
+            raise L.FegnnError("differentiable=True needs edge_attr_nf > 0 (the edge lengths are what it differentiates)")
         if capacity is not None:
             capacity = int(capacity)
             candidate_capacity = capacity if candidate_capacity is None else int(candidate_capacity)
@@ -191,6 +215,7 @@ class CsrGraph:
         f32 = dict(device=dev, dtype=torch.float32)
         self = cls.__new__(cls)
         self.N, self.B, self.Fe, self.Nl = N, B, Fe, N
+        self.differentiable = bool(differentiable)
         self.perm = None                                      # there is no caller-side edge list to permute
         self.batch = torch.empty(N, **i32)
         self.gptr = torch.empty(B + 1, **i32)
@@ -212,7 +237,7 @@ class CsrGraph:
             self.n_edges = torch.empty(1, **i32)
             self.status = torch.zeros(1, **i32)
             self._peak = torch.zeros(2, **i32)                # largest uncapped [n_cand, n_edges] of any build (check())
-            self.rebuild_(x)
+            self.rebuild_(node_loc)
             self.rebind()
             return self
         st = _stream(dev)
@@ -241,12 +266,35 @@ class CsrGraph:
         self.row, self.col = row[:E], col[:E]
         self.edge_attr = ea[:E] if Fe else torch.empty(0, **f32)
         self._ws = ws
+        self._built_from(node_loc, x)
         self.rebind()
         return self
 
+    def _built_from(self, node_loc: torch.Tensor, x: torch.Tensor) -> None:
+        """Counts a build; a differentiable graph keeps the positions (node_loc with its history, x the fp32 copy the
+        kernels read) for the backward of its edge lengths."""
+        self.builds += 1
+        if self.differentiable:
+            self.node_loc, self._x = node_loc, x
+
+    def check_build(self, build: int) -> None:
+        """Raises FegnnError unless the arrays are still those of build `build` (a backward's guard against rebuild_)."""
+        if self.builds != build:
+            raise L.FegnnError(f"the graph was rebuilt (rebuild_) after the forward this backward belongs to (build {build}, "
+                               f"now {self.builds}): the backward would read the new topology.  Use one graph per step "
+                               "of an unrolled rollout.")
+
+    def edge_attr_input(self) -> torch.Tensor:
+        """What a training forward on a differentiable graph passes as its edge_attr input: the caller's tensor, or (from_radius)
+        graph.edge_attr itself (no copy) as a function of node_loc."""
+        if getattr(self, "_ea_src", None) is not None:
+            return self._ea_src
+        return _EdgeLengthFn.apply(self.node_loc, self)
+
     def rebuild_(self, node_loc: torch.Tensor) -> "CsrGraph":
         """Refill a live from_radius graph IN PLACE from new positions (same data_batch, r, cutoff_rate and buffers, so
-        the pointer table stays valid): what a captured rollout calls every step.  No host read, no allocation."""
+        the pointer table stays valid): what a captured rollout calls every step.  No host read, no allocation.  A
+        differentiable graph now takes its edge lengths as a function of this node_loc."""
         if getattr(self, "_radius", None) is None:
             raise L.FegnnError("rebuild_ needs a graph made by CsrGraph.from_radius(..., capacity=...)")
         if node_loc.dim() != 2 or node_loc.size(0) != self.N or node_loc.size(1) != 3:
@@ -269,6 +317,7 @@ class CsrGraph:
                     "fegnn_radius_graph_fill_live")
             # the status bits are sticky over rebuilds, so are the totals check() names: a running maximum on the device
             torch.maximum(self._peak, counts, out=self._peak)
+        self._built_from(node_loc, x)
         return self
 
     def check(self) -> None:
@@ -331,6 +380,32 @@ def make_dims(N: int, Nl: int, E: int, B: int, C_: int, Fe: int, flags: int,
     d.eps = eps
     d.Fa, d.node_attr = Fa, L.ptr(node_attr)
     return d
+
+
+class _EdgeLengthFn(torch.autograd.Function):
+    """graph.edge_attr of a differentiable from_radius graph (its rows, no copy) as a function of the node_loc it was built
+    from: the backward is fegnn_edge_length_backward on the gradient the stack gives edge_attr (CSR order: perm is NULL)."""
+
+    @staticmethod
+    def forward(ctx, node_loc, graph):
+        ctx.graph, ctx.build, ctx.dtype = graph, graph.builds, node_loc.dtype
+        ctx.save_for_backward(graph._x)
+        return graph.edge_attr[:graph.E]
+
+    @staticmethod
+    def backward(ctx, g_ea):
+        graph = ctx.graph
+        graph.check_build(ctx.build)
+        L.deterministic("CsrGraph edge-length backward", "the col side of the position gradient adds with float atomics")
+        x, = ctx.saved_tensors
+        dev = x.device
+        g_x = torch.zeros(graph.N, 3, device=dev, dtype=torch.float32)
+        g_ea = g_ea.contiguous().float()
+        dims = make_dims(graph.N, graph.N, graph.E, graph.B, 1, graph.Fe, live_flag(graph))
+        with _on(dev):
+            L.check(lib.fegnn_edge_length_backward(C.byref(dims), C.byref(graph.c), L.ptr(graph.rowptr), L.ptr(x),
+                                                   L.ptr(g_ea), L.ptr(g_x), _stream(dev)), "fegnn_edge_length_backward")
+        return g_x.to(ctx.dtype), None
 
 
 def node_attr_arg(node_attr, node_attr_nf: int, n_nodes: int) -> Optional[torch.Tensor]:

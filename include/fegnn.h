@@ -387,6 +387,17 @@ int fegnn_node_pre_backward_inputs(const fegnn_dims* d, const fegnn_layer_params
                                    const float* h, const float* gP, const float* gQ, const float* gAv,
                                    const float* gUh, const float* gsv, const float* gsg, float* gh,
                                    const fegnn_input_grads* ig /*node_attr +=*/, void* stream);
+/* Gradient through the edge lengths of a graph built from positions x (fegnn_radius_graph_fill / _fill_live: edge_attr[e, k]
+ * = len_e = |x_row - x_col| in every column): for every edge e of the CSR arrays (g->col, g->edge_attr, rowptr),
+ *   g_x[row_e] += u_e,  g_x[col_e] -= u_e,  u_e = (sum_k g_ea[e, k]) (x_row - x_col) / len_e,
+ * with len_e the graph's own edge_attr[e, 0] and u_e = 0 where len_e == 0 (coincident distinct nodes: the subgradient
+ * torch's norm takes).  g_ea [E,Fe] is in CSR order (what fegnn_model_backward_inputs writes when perm is NULL).  ADDS into
+ * g_x [N,3].  Honours FEGNN_F_LIVE_EDGES (no edge at or past the live count is read).  Refused with FEGNN_EINVAL before
+ * any launch: Fe == 0, the live flag with a NULL n_edges, and the "deterministic" mode (the col side adds with float
+ * atomics).  Never allocates or synchronises. */
+int fegnn_edge_length_backward(const fegnn_dims* d, const fegnn_graph* g, const int32_t* rowptr,
+                               const float* x /*[N,3] positions the graph was built from*/,
+                               const float* g_ea /*[E,Fe] CSR order*/, float* g_x /*[N,3] +=*/, void* stream);
 
 /* ------------------------------------------------------------------ halo exchange over peer memory
  * Multi-GPU form of the layer (one big graph in spatial slabs, fastegnn_b200/partitioned.py): a node is owned by one
